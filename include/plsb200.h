@@ -145,6 +145,20 @@ int plsb200_boot_moments_f64(const double* X, int N, int64_t p, int64_t ldx, con
                              int R, const double* pivot, double* sum, double* sumsq,
                              void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- K4 collapsed (task methods, exact FP64): the bootstrap variance as a quadratic form ------------------
+ * Each salience is linear in the draw, so R . Var_r(VS_r[v,k]) = x_v^T S_k x_v with S_k = R . Cov_r(c_rk) (N x N).
+ *   q[v,k] = x_v^T S_k x_v   (p x K, overwritten)
+ * Step 1 packs S ([K][N][N], row-major, k slowest) into the B-fragment order of the bootstrap GEMM
+ * (`coef`, plsb200_boot_quad_coef_bytes bytes); step 2 evaluates the p x K quadratic forms on the FP64 tensor cores.
+ * Feeding (sum = 0, sumsq = q) to plsb200_boot_finalize_f64 gives the bootstrap standard errors.
+ * Supported shapes: N <= 320 and K <= 24 per call (split wider problems by column), else PLSB200_EUNSUPPORTED
+ * (the size queries return 0).                                                                                  */
+size_t plsb200_boot_quad_coef_bytes(int N, int K);
+int plsb200_boot_quad_coef_pack_f64(const double* S, int N, int K, double* coef, void* stream);
+size_t plsb200_boot_quad_f64_workspace(int N, int64_t p, int K);
+int plsb200_boot_quad_f64(const double* X, int N, int64_t p, int64_t ldx, const double* coef, int K, double* q,
+                          void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- K4 fast mode: the same moments on the tcgen05 tensor cores with the 3xTF32 split ---------------------
  * (x = xh + xl, c = ch + cl, each TF32-exact; xh.cl + xl.ch + xh.ch accumulated in FP32 in tensor memory, the
  * moments in FP64).  Relative error of a salience ~1e-6; std_errs / boot_ratios agree with the FP64 path to

@@ -11,7 +11,9 @@ boot_ratios, [LVcorr], boot_debug_dict, CI`; "NA" placeholders when a test is sk
 Extra keyword-only arguments (not in the reference): `perm_indices`, `boot_indices` (index matrices
 generated elsewhere -- each an int array, or a (task, behaviour) tuple for mb/cmb), `engine`
 (an `Engine` that already holds X on the device), `device` (CUDA device of the engine built here), `precision` ("fp64" exact mode, or "tf32x3": the
-bootstrap moment GEMM of the task methods on the tcgen05 tensor cores; p-values stay FP64-exact).
+bootstrap moment GEMM of the task methods on the tcgen05 tensor cores; p-values stay FP64-exact), `boot_algo`
+("direct", default: the bootstrap moments from the B x p x K salience GEMM; "collapsed": mct / cst in the exact mode
+only, the same standard errors from the closed form x_v^T Cov_r(c_rk) x_v -- see `check_boot_algo`).
 """
 import abc
 
@@ -353,6 +355,54 @@ def _task_operators(pls_alg, cond_order, mctype, U, contrast):
     return Lop, Ucoef, Lop.T @ Ucoef
 
 
+BOOT_ALGOS = ("direct", "collapsed")
+
+
+def check_boot_algo(boot_algo, pls_alg, precision, N):
+    """Validates the bootstrap formulation before any GPU work.
+
+    "direct" (default) accumulates the moments of the B x p x K bootstrap saliences VS_r = X^T C_r.  "collapsed" uses
+    that every task-method salience is linear in the draw: Var_r(x_v^T c_rk) = x_v^T Cov_r(c_rk) x_v, so the
+    standard errors come from K covariance matrices of N x N and one p x K quadratic form (2 p N^2 K flops instead of
+    2 p N K B: fewer when B > N, more when B < N).  Exact FP64 like the direct form; results agree to rounding."""
+    if boot_algo not in BOOT_ALGOS:
+        raise ValueError(f'boot_algo must be one of {BOOT_ALGOS}, got {boot_algo!r}')
+    if boot_algo == "direct":
+        return
+    if precision != "fp64":
+        raise ValueError(f'boot_algo="collapsed" is an exact (precision="fp64") formulation, got precision={precision!r}')
+    if pls_alg not in ("mct", "cst"):
+        raise exceptions.NotImplementedError(
+            'boot_algo="collapsed" applies to the task methods (mct, cst): the block standardisation of the behaviour '
+            'and multiblock methods makes their saliences non-linear in the bootstrap draw')
+    if N is not None and N > Engine.QUAD_MAX_ROWS:
+        raise exceptions.NotImplementedError(
+            f'boot_algo="collapsed" supports designs of at most {Engine.QUAD_MAX_ROWS} rows (this one has {N}); '
+            'use boot_algo="direct"')
+
+
+def _collapsed_sumsq(eng, E, idx_dev, niter, lo, hi):
+    """Collapsed bootstrap: q[v,k] = x_v^T S_k x_v with S_k = sum_r (c_rk - e_k)(c_rk - e_k)^T - s1_k s1_k^T / niter
+    (= niter . Cov_r(c_rk)): the sum of squares of (VS_r - mean) over all `niter` resamples, p x K, the same on every
+    rank.  Multi-process: one all-reduce of the N-space partial sums, each rank evaluates the quadratic form on its
+    share of the voxels and the shares are gathered."""
+    E = eng.to_device(E, torch.float64)
+    eng._x_ranges()          # (starts a deferred upload of X: the covariance build below overlaps it)
+    if hi > lo:
+        S1, S2 = eng.boot_cov(E, idx_dev)
+    else:
+        K = E.shape[1]
+        S1 = torch.zeros(eng.N, K, dtype=torch.float64, device=eng.device)
+        S2 = torch.zeros(K, eng.N, eng.N, dtype=torch.float64, device=eng.device)
+    dist.allreduce_packed_([S1, S2])
+    s1t = S1.T
+    Sig = S2 - s1t[:, :, None] * s1t[:, None, :] / niter
+    if dist.world()[1] == 1:
+        return eng.boot_quad(Sig)
+    v0, v1 = dist.shard(eng.p)
+    return dist.gather_rows(eng.boot_quad(Sig, v0, v1), eng.p, v0)
+
+
 @ResampleTest._register_subclass("mct")
 @ResampleTest._register_subclass("rb")
 @ResampleTest._register_subclass("cst")
@@ -365,8 +415,11 @@ class _ResampleTestPLS(ResampleTest):
     def __init__(self, X, Y, U, s, V, cond_order, mctype, contrast=None, preprocess=None, nperm=1000,
                  nboot=1000, bscan=None, Xbscan=None, Ybscan=None, lvcorrs_orig=None, Tvsc_orig=None,
                  CI=0.95, *, perm_indices=None, boot_indices=None, engine=None, precision="fp64", rotate_method=2,
-                 device=None):
+                 device=None, boot_algo="direct"):
         self.CI = CI
+        check_boot_algo(boot_algo, self.pls_alg, engine.precision if engine is not None else precision,
+                        engine.N if engine is not None else (int(X.shape[0]) if X is not None else None))
+        self.boot_algo = boot_algo
         if rotate_method not in (0, 1, 2):
             raise ValueError("rotate_method must be 0 (SVD), 1 (Procrustes) or 2 (derived)")
         if rotate_method == 0 and self.pls_alg not in ("mct", "rb", "mb"):
@@ -396,7 +449,7 @@ class _ResampleTestPLS(ResampleTest):
                 boot_indices = resample.bootstrap_indices(self.pls_alg, nboot, cond_order, Y=Y, bscan=bscan,
                                                           Ybscan=Ybscan)
             early = self._bootstrap_moments_early(eng, U, s, V, cond_order, mctype, nboot, self.pls_alg, contrast,
-                                                  boot_indices)
+                                                  boot_indices, boot_algo=boot_algo)
         if nperm > 0:
             # the permutation kernels and their device->host copies are enqueued here; the host only waits for
             # them after the bootstrap work has been enqueued too, so the GPU never idles between the two tests
@@ -411,7 +464,7 @@ class _ResampleTestPLS(ResampleTest):
             out = self._bootstrap_test(
                 X, Y, U, s, V, cond_order, mctype, nboot, self.pls_alg, preprocess=preprocess, contrast=contrast,
                 bscan=bscan, Xbscan=Xbscan, Ybscan=Ybscan, lvcorrs_orig=lvcorrs_orig, Tvsc_orig=Tvsc_orig, CI=CI,
-                indices=boot_indices, engine=eng, _early=early)
+                indices=boot_indices, engine=eng, _early=early, boot_algo=boot_algo)
             if self.pls_alg in ("rb", "csb"):
                 self.conf_ints, self.std_errs, self.boot_ratios, self.LVcorr, self.boot_debug_dict = out
             elif self.pls_alg in ("mb", "cmb"):
@@ -555,9 +608,9 @@ class _ResampleTestPLS(ResampleTest):
     @staticmethod
     def _bootstrap_test(X, Y, U, s, V, cond_order, mctype, niter, pls_alg, preprocess=None, dist_=(0.05, 0.95),
                         contrast=None, bscan=None, Xbscan=None, Ybscan=None, lvcorrs_orig=None, Tvsc_orig=None,
-                        CI=0.95, indices=None, engine=None, _early=None):
+                        CI=0.95, indices=None, engine=None, _early=None, boot_algo="direct"):
         """bootstrap_permutation.py:466-766 for the task methods (mct, cst).  `_early`: moments already enqueued by
-        `_bootstrap_moments_early` (pipelined upload of X)."""
+        `_bootstrap_moments_early` (pipelined upload of X).  `boot_algo`: see `check_boot_algo`."""
         eng = engine if engine is not None else Engine(X)
         if indices is None:
             indices = resample.bootstrap_indices(pls_alg, niter, cond_order, Y=Y, bscan=bscan, Ybscan=Ybscan)
@@ -597,13 +650,18 @@ class _ResampleTestPLS(ResampleTest):
         defer = dist.world()[1] > 1
         fetch_small = (eng.to_host_async(eng.colstd(Tdist), side=True) if defer
                        else eng.to_host_async(eng.colstd(Tdist), Tdist, left, side=True))
-        if _early is not None:
-            s1, s2 = _early
-        elif hi > lo:
-            s1, s2 = eng.boot_moments(E, idx_dev, pivot=numer, packed=packed)   # K4
+        if boot_algo == "collapsed":
+            # sum of squares about the bootstrap mean, already complete on every rank: no p x K all-reduce
+            s2 = _early if _early is not None else _collapsed_sumsq(eng, E, idx_dev, niter, lo, hi)
+            s1 = torch.zeros_like(s2)
         else:
-            s1 = torch.zeros_like(numer); s2 = torch.zeros_like(numer)
-        dist.allreduce_packed_([s1, s2])
+            if _early is not None:
+                s1, s2 = _early
+            elif hi > lo:
+                s1, s2 = eng.boot_moments(E, idx_dev, pivot=numer, packed=packed)   # K4
+            else:
+                s1 = torch.zeros_like(numer); s2 = torch.zeros_like(numer)
+            dist.allreduce_packed_([s1, s2])
         std_errs, boot_ratios = eng.boot_finalize(s1, s2, niter, numer=numer)   # (:695-703)
         z = norm.ppf(1 - (1 - CI) / 2)                                      # (:709)
         std_errs_h, boot_ratios_h = _p_sized_to_host(eng, std_errs, boot_ratios)
@@ -638,11 +696,16 @@ class _ResampleTestPLS(ResampleTest):
 
     # ------------------------------------------------------------------------------------------
     @staticmethod
-    def _bootstrap_moments_early(eng, U, s, V, cond_order, mctype, niter, pls_alg, contrast, indices):
-        """The moment GEMM of `_bootstrap_test` for the task methods, on its own (single process)."""
+    def _bootstrap_moments_early(eng, U, s, V, cond_order, mctype, niter, pls_alg, contrast, indices,
+                                 boot_algo="direct"):
+        """The moment GEMM of `_bootstrap_test` for the task methods, on its own (single process).  Collapsed: the
+        N-space covariance build needs no X, so it runs while X is still crossing PCIe; the quadratic form follows
+        range by range as X arrives."""
         if isinstance(indices, tuple):
             indices = indices[0]
         _, _, E = _task_operators(pls_alg, cond_order, mctype, U, contrast)
+        if boot_algo == "collapsed":
+            return _collapsed_sumsq(eng, E, _index_shard(eng, indices, niter, 0, niter), niter, 0, niter)
         Vd = eng.to_device(V, torch.float64)
         numer = Vd * eng.to_device(np.asarray(s, dtype=float), torch.float64) if contrast is None else Vd
         idx_dev = _index_shard(eng, indices, niter, 0, niter)

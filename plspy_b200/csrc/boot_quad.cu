@@ -1,0 +1,261 @@
+// Collapsed bootstrap (task methods): the quadratic forms q[v,k] = x_v^T S_k x_v on the FP64 tensor cores.
+//
+// Every bootstrap salience is linear in the draw, VS_r[v,k] = x_v^T c_rk (c_rk = column k of C_r = scatter(E, idx_r)),
+// so its spread over the resamples is a quadratic form in the covariance of the coefficients:
+//       R . Var_r(VS_r[v,k]) = x_v^T S_k x_v,        S_k = sum_r d_rk d_rk^T - s1_k s1_k^T / R   (N x N)
+// with d_r = C_r - E and s1_k = sum_r d_rk (DESIGN.md section 3).  Engine.boot_cov forms the S_k in N-space; this
+// file evaluates the p x K quadratic forms, 2 p N^2 K flops instead of the 2 p N K B of the direct moment GEMM.
+//
+// The kernel is boot_moments_kernel (boot.cu) with N "pseudo-resamples" in place of the B resamples: pseudo-resample m
+// has the N x K coefficient matrix P_m[n,k] = S_k[n,m], packed in exactly the B-fragment / period order of
+// boot_coef_pack_kernel, so the plan, the ring of bulk copies and the mbarriers are the same.  A D element is then
+// (S_k x_v)[m]; the epilogue folds it as acc[v,k] += X[m,v] . d.  X[m,v] comes from an __ldg issued before the
+// period's MMA stream (the A registers cannot serve it: m is a runtime index).  Pseudo-resamples m >= N and columns
+// k >= K are zero in the pack; the loads of rows m >= N are masked.
+#include "common.cuh"
+#include "boot_plan.cuh"
+
+namespace plsb {
+
+// S ([K][N][N], row-major) -> B-fragment order: offset ((per*nks + s)*nblk + jb)*32 + lane, lane = 4*n + qq,
+// column c = 8*jb + n = slot*Kp + k of pseudo-resample m = per*nb + slot, row i = 4*s + qq.
+__global__ void quad_coef_pack_kernel(const double* __restrict__ S, int N, int K, int Kp, int nblk, int nb, int nks,
+                                      long long total, double* __restrict__ coef) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= total) return;
+    const int lane = (int)(i & 31);
+    long long t = i >> 5;
+    const int jb = (int)(t % nblk); t /= nblk;
+    const int s = (int)(t % nks);
+    const int per = (int)(t / nks);
+    const int c = 8 * jb + (lane >> 2), row = 4 * s + (lane & 3);
+    const int k = c % Kp, m = per * nb + c / Kp;
+    coef[i] = (row < N && m < N && k < K) ? S[((size_t)k * N + row) * N + m] : 0.0;
+}
+
+template <int NKS, int NBLK>
+__global__ void __launch_bounds__(BM_THREADS, 1)
+boot_quad_kernel(const double* __restrict__ X, long long ldx, int N, long long p, const double* __restrict__ coef,
+                 int nper, int per_per_split, int nstage, int Kp, int K, double* __restrict__ out) {
+    extern __shared__ __align__(128) unsigned char smraw[];
+    constexpr int stage_doubles = NKS * NBLK * 32;
+    constexpr uint32_t stage_bytes = (uint32_t)stage_doubles * 8u;
+    double* ring = reinterpret_cast<double*>(smraw);
+    double* red = ring + (size_t)nstage * stage_doubles;              // [8 warps][8][Kp] (the plan reserves twice that)
+    uint64_t* full = reinterpret_cast<uint64_t*>(red + BM_WARPS * 16 * Kp);
+    uint64_t* empty = full + nstage;
+
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int q = lane & 3, vr = lane >> 2;
+    const long long v = (long long)blockIdx.x * BM_VOX + warp * 8 + vr;
+    const int per0 = blockIdx.y * per_per_split;
+    const int per1 = min(nper, per0 + per_per_split);
+    const int nit = per1 - per0;
+
+    if (tid == 0) {
+        for (int s = 0; s < nstage; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, BM_WARPS); }
+        mbar_fence_init();
+    }
+    __syncthreads();
+
+    auto issue = [&](int it, int slot) {   // thread 0 only: stream period per0+it into `slot`
+        mbar_expect_tx(full + slot, stage_bytes);
+        const char* src = reinterpret_cast<const char*>(coef + (size_t)(per0 + it) * stage_doubles);
+        char* dst = reinterpret_cast<char*>(ring + (size_t)slot * stage_doubles);
+#pragma unroll 1
+        for (uint32_t off = 0; off < stage_bytes; off += 16384u)
+            bulk_g2s(dst + off, src + off, min(16384u, stage_bytes - off), full + slot);
+    };
+    if (tid == 0)
+        for (int it = 0; it < min(nstage, nit); ++it) issue(it, it);
+
+    // ---- A fragments: this warp's 8 voxels x all rows, resident in registers
+    double a[NKS];
+#pragma unroll
+    for (int s = 0; s < NKS; ++s) {
+        const int row = 4 * s + q;
+        a[s] = (row < N && v < p) ? __ldg(X + (long long)row * ldx + v) : 0.0;
+    }
+    const long long vc = v < p ? v : 0;                                // (address of the masked lanes' X loads)
+
+    // ---- per-thread column bookkeeping (fixed for the whole kernel): pseudo-resample slot of each column
+    int slot_of[NBLK][2];
+    double acc[NBLK][2];
+#pragma unroll
+    for (int j = 0; j < NBLK; ++j)
+#pragma unroll
+        for (int e = 0; e < 2; ++e) { slot_of[j][e] = (8 * j + 2 * q + e) / Kp; acc[j][e] = 0.0; }
+    const int nb = 8 * NBLK / Kp;
+
+    if (warp >= 4) __nanosleep((unsigned)(NKS * NBLK * 8));
+
+    int slot = 0, prev_slot = 0;
+    uint32_t phase = 0, prev_phase = 0;
+    for (int it = 0; it < nit; ++it) {
+        if (tid == 0 && it > 0) {
+            const int nx = it - 1 + nstage;
+            if (nx < nit) {
+                mbar_wait(empty + prev_slot, prev_phase);
+                issue(nx, prev_slot);
+            }
+        }
+        // X[m, v] of this thread's columns, loaded before the MMA stream so that its latency is hidden
+        const int mbase = (per0 + it) * nb;
+        double xm[NBLK][2];
+#pragma unroll
+        for (int j = 0; j < NBLK; ++j)
+#pragma unroll
+            for (int e = 0; e < 2; ++e) {
+                const int m = mbase + slot_of[j][e];
+                xm[j][e] = m < N ? __ldg(X + (long long)m * ldx + vc) : 0.0;
+            }
+        __syncwarp();
+        mbar_wait(full + slot, phase);
+
+        double d[NBLK][2];
+#pragma unroll
+        for (int j = 0; j < NBLK; ++j) { d[j][0] = 0.0; d[j][1] = 0.0; }
+        // volatile: keeps the loads in program order, so the NBLK accumulator chains stay interleaved (see boot.cu)
+        const volatile double* bs = ring + (size_t)slot * stage_doubles + lane;
+#pragma unroll
+        for (int s = 0; s < NKS; ++s) {
+#pragma unroll
+            for (int j = 0; j < NBLK; ++j) {
+                const double b = bs[(s * NBLK + j) * 32];
+                dmma884(d[j][0], d[j][1], a[s], b);
+            }
+        }
+        __syncwarp();
+        if (lane == 0) mbar_arrive(empty + slot);
+#pragma unroll
+        for (int j = 0; j < NBLK; ++j)
+#pragma unroll
+            for (int e = 0; e < 2; ++e) acc[j][e] = fma(xm[j][e], d[j][e], acc[j][e]);
+        prev_slot = slot; prev_phase = phase;
+        if (++slot == nstage) { slot = 0; phase ^= 1u; }
+    }
+
+    // ---- fold the nb pseudo-resample slots of a period onto k, in slot order (deterministic)
+    double* r1 = red + warp * (8 * Kp);
+    for (int i = lane; i < 8 * Kp; i += 32) r1[i] = 0.0;
+    __syncwarp();
+    for (int round = 0; round < nb; ++round) {
+#pragma unroll
+        for (int j = 0; j < NBLK; ++j)
+#pragma unroll
+            for (int e = 0; e < 2; ++e) {
+                const int c = 8 * j + 2 * q + e;
+                if (slot_of[j][e] == round) r1[vr * Kp + c % Kp] += acc[j][e];
+            }
+        __syncwarp();
+    }
+    const long long vbase = (long long)blockIdx.x * BM_VOX + warp * 8;
+    double* o = out + (size_t)blockIdx.y * p * K;
+    for (int i = lane; i < 8 * K; i += 32) {
+        const int rr = i / K, k = i % K;
+        if (vbase + rr < p) o[(vbase + rr) * K + k] = r1[rr * Kp + k];
+    }
+}
+
+// q = sum of the split partials, in split order (deterministic)
+__global__ void quad_reduce_kernel(const double* __restrict__ part, int nsplit, long long n, double* __restrict__ q) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    double a = 0.0;
+    for (int s = 0; s < nsplit; ++s) a += part[(size_t)s * n + i];
+    q[i] = a;
+}
+
+template <int NKS, int NBLK>
+static int launch_quad(const BootPlan& b, const double* X, int N, int64_t p, int64_t ldx, const double* coef, int K,
+                       double* o, cudaStream_t st) {
+    PLSB_CUDA(cudaFuncSetAttribute(boot_quad_kernel<NKS, NBLK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   (int)b.smem_bytes));
+    dim3 grid((unsigned)cdiv(p, BM_VOX), (unsigned)b.nsplit);
+    boot_quad_kernel<NKS, NBLK><<<grid, BM_THREADS, b.smem_bytes, st>>>(X, ldx, N, p, coef, b.nper, b.per_per_split,
+                                                                       b.nstage, b.Kp, K, o);
+    PLSB_LAUNCH_CHECK("boot_quad_kernel");
+    return PLSB200_OK;
+}
+
+template <int NBLK>
+static int quad_dispatch_nks(const BootPlan& b, const double* X, int N, int64_t p, int64_t ldx, const double* coef,
+                             int K, double* o, cudaStream_t st) {
+    switch (b.nks) {
+#define PLSB_CASE(n) case n: return launch_quad<n, NBLK>(b, X, N, p, ldx, coef, K, o, st);
+        PLSB_CASE(4) PLSB_CASE(8) PLSB_CASE(12) PLSB_CASE(16) PLSB_CASE(20) PLSB_CASE(24) PLSB_CASE(28)
+        PLSB_CASE(32) PLSB_CASE(36) PLSB_CASE(40) PLSB_CASE(44) PLSB_CASE(48) PLSB_CASE(52) PLSB_CASE(56)
+        PLSB_CASE(60) PLSB_CASE(64) PLSB_CASE(68) PLSB_CASE(72) PLSB_CASE(76) PLSB_CASE(80)
+#undef PLSB_CASE
+        default:
+            set_err("boot_quad_f64: no kernel for nks=%d", b.nks);
+            return PLSB200_EUNSUPPORTED;
+    }
+}
+
+}  // namespace plsb
+
+using namespace plsb;
+
+// the plan of the quadratic form: N pseudo-resamples of N x K coefficients
+static bool quad_plan(int N, int K, int64_t p, BootPlan& b) { return N <= 320 && boot_plan(N, K, N, p, b); }
+
+extern "C" size_t plsb200_boot_quad_coef_bytes(int N, int K) {
+    BootPlan b;
+    if (!quad_plan(N, K, 1, b)) return 0;
+    return (size_t)b.nper * b.stage_doubles * sizeof(double);
+}
+
+extern "C" int plsb200_boot_quad_coef_pack_f64(const double* S, int N, int K, double* coef, void* stream) {
+    PLSB_CHECK_ARG(S && coef, "boot_quad_coef_pack_f64: null pointer");
+    BootPlan b;
+    if (!quad_plan(N, K, 1, b)) {
+        set_err("boot_quad_coef_pack_f64: unsupported shape N=%d K=%d (need N<=320, K<=24)", N, K);
+        return PLSB200_EUNSUPPORTED;
+    }
+    const long long total = (long long)b.nper * b.stage_doubles;
+    quad_coef_pack_kernel<<<(unsigned)cdiv(total, 256), 256, 0, (cudaStream_t)stream>>>(S, N, K, b.Kp, b.nblk, b.nb,
+                                                                                       b.nks, total, coef);
+    PLSB_LAUNCH_CHECK("quad_coef_pack_kernel");
+    return PLSB200_OK;
+}
+
+extern "C" size_t plsb200_boot_quad_f64_workspace(int N, int64_t p, int K) {
+    BootPlan b;
+    if (p <= 0 || !quad_plan(N, K, p, b)) return 0;
+    return b.nsplit > 1 ? (size_t)b.nsplit * p * K * sizeof(double) : 16;
+}
+
+extern "C" int plsb200_boot_quad_f64(const double* X, int N, int64_t p, int64_t ldx, const double* coef, int K,
+                                     double* q, void* workspace, size_t workspace_bytes, void* stream) {
+    PLSB_CHECK_ARG(X && coef && q, "boot_quad_f64: null pointer");
+    PLSB_CHECK_ARG(p > 0 && ldx >= p, "boot_quad_f64: bad shape p=%lld ldx=%lld", (long long)p, (long long)ldx);
+    BootPlan b;
+    if (!quad_plan(N, K, p, b)) {
+        set_err("boot_quad_f64: unsupported shape N=%d K=%d (need N<=320, K<=24)", N, K);
+        return PLSB200_EUNSUPPORTED;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    double* o = q;
+    if (b.nsplit > 1) {
+        const size_t need = (size_t)b.nsplit * p * K * sizeof(double);
+        if (!workspace || workspace_bytes < need) {
+            set_err("boot_quad_f64: workspace %zu < %zu bytes", workspace_bytes, need);
+            return PLSB200_EWORKSPACE;
+        }
+        o = (double*)workspace;
+    }
+    int rc;
+    switch (b.nblk) {
+        case 1: rc = quad_dispatch_nks<1>(b, X, N, p, ldx, coef, K, o, st); break;
+        case 2: rc = quad_dispatch_nks<2>(b, X, N, p, ldx, coef, K, o, st); break;
+        default: rc = quad_dispatch_nks<3>(b, X, N, p, ldx, coef, K, o, st); break;
+    }
+    if (rc != PLSB200_OK) return rc;
+    if (b.nsplit > 1) {
+        const long long n = (long long)p * K;
+        quad_reduce_kernel<<<(unsigned)cdiv(n, 256), 256, 0, st>>>(o, b.nsplit, n, q);
+        PLSB_LAUNCH_CHECK("quad_reduce_kernel");
+    }
+    return PLSB200_OK;
+}

@@ -607,6 +607,68 @@ class Engine:
                 self._mark("boot_moments")
         return s1, s2
 
+    QUAD_MAX_ROWS = 320     # designs the collapsed bootstrap's register-resident quadratic-form kernel holds
+
+    def boot_cov(self, E, idx, max_bytes=1 << 30):
+        """Partial sums of the collapsed bootstrap over the resamples in `idx`, pivoted at the original coefficients
+        (d_r = scatter(E, idx_r) - E): S1 = sum_r d_r (N x K) and S2[k] = sum_r d_rk d_rk^T (K x N x N).  They add up
+        over any split of the resamples (a multi-process run all-reduces them).  N-space only -- X is not read.
+        Per chunk of resamples (at most `max_bytes` of workspace) the K matrices [d_1k ... d_Rk; 1 ... 1] ((N + 1) x R)
+        go through the FP64 Gram kernel: their Gram matrix holds S2[k] and, in its last column, S1[:, k].  Chunks
+        are summed in a fixed order."""
+        E = self.to_device(E, F64); idx = self.to_device(idx, I32)
+        R, N, K = int(idx.shape[0]), int(E.shape[0]), int(E.shape[1])
+        S = torch.zeros(K, N + 1, N + 1, dtype=F64, device=self.device)
+        rc = max(1, min(R, int(max_bytes // (8 * (N * K + K * (N + 1))))))
+        Et = E.T.contiguous()
+        for r0 in range(0, R, rc):
+            n = min(rc, R - r0)
+            C = self.scatter_coef(E, idx[r0:r0 + n])                      # n x N x K
+            M = torch.ones(K, N + 1, n, dtype=F64, device=self.device)
+            M[:, :N, :].copy_(C.permute(2, 1, 0)).sub_(Et[:, :, None])
+            del C
+            for k in range(K):
+                S[k] += self.gram_of(M[k])
+            del M
+        return S[:, :N, N].T.contiguous(), S[:, :N, :N].contiguous()
+
+    def boot_quad(self, Sig, v0=0, v1=None):
+        """Collapsed bootstrap: q[v,k] = x_v^T Sig[k] x_v for the voxels v0 <= v < v1 ((v1 - v0) x K).  With
+        Sig[k] = R . Cov_r(c_rk), (sum = 0, sumsq = q) are the moments `boot_finalize` turns into standard errors.
+        One launch per voxel range of a pipelined upload, each after its range has arrived.  Designs of at most
+        320 rows."""
+        Sig = self.to_device(Sig, F64)
+        K, N = int(Sig.shape[0]), int(Sig.shape[1])
+        v1 = self.p if v1 is None else int(v1)
+        if N != self.N or tuple(Sig.shape) != (K, N, N):
+            raise ValueError(f"boot_quad: Sig must be K x {self.N} x {self.N}")
+        if K > self.KMAX:   # columns are independent: split wide problems
+            return torch.cat([self.boot_quad(Sig[k0:k0 + self.KMAX], v0, v1) for k0 in range(0, K, self.KMAX)], dim=1)
+        q = self._empty(max(v1 - v0, 0), K)
+        if v1 <= v0:
+            return q
+        with torch.cuda.device(self.device):
+            nbytes = lib.plsb200_boot_quad_coef_bytes(N, K)
+            if nbytes == 0:
+                raise _lib.PlsB200Error(f"boot_quad: unsupported shape N={N} K={K} (N <= {self.QUAD_MAX_ROWS})")
+            coef = self._ws(nbytes)
+            check(lib.plsb200_boot_quad_coef_pack_f64(self._p(Sig), N, K, self._p(coef), self._stream()),
+                  "boot_quad_coef_pack_f64")
+            cur = torch.cuda.current_stream(self.device)
+            for a, b, ev in self._x_ranges():
+                lo, hi = max(a, v0), min(b, v1)
+                if lo >= hi:
+                    continue
+                if ev is not None:
+                    cur.wait_event(ev)
+                ws = self._ws(lib.plsb200_boot_quad_f64_workspace(N, hi - lo, K))
+                self._mark("boot_quad")
+                check(lib.plsb200_boot_quad_f64(self._X.data_ptr() + 8 * lo, N, hi - lo, self.ldx, self._p(coef), K,
+                                                q.data_ptr() + 8 * (lo - v0) * K, self._p(ws), ws.numel(),
+                                                self._stream()), "boot_quad_f64")
+                self._mark("boot_quad")
+        return q
+
     def boot_finalize(self, s1, s2, R_total, numer=None):
         K = int(s1.shape[1])
         se = self._empty(self.p, K)

@@ -1,5 +1,5 @@
 """`PLS(...)` driver with the reference's signature and argument validation (plspy/core/pls.py:21-93)."""
-from . import pls_classes
+from . import bootstrap_permutation, pls_classes
 
 methods = {
     "mct": pls_classes._MeanCentreTaskPLS,
@@ -22,7 +22,10 @@ def PLS(*args, **kwargs):
     `rotate_method` (2 = derived, the reference's behaviour and the default; 1 = Procrustes; 0 = per-permutation SVD,
     mct only -- see `_ResampleTestPLS._permutation_test`), `analysis` ("host" = LAPACK on the cross-block matrix as
     in the reference, default; "device" = through the Gram matrix on the GPU, sign of each latent
-    variable fixed by convention -- see device_analysis.py).
+    variable fixed by convention -- see device_analysis.py), `boot_algo` ("direct" = the bootstrap moments of the
+    B x p x K salience GEMM, default; "collapsed" = mct / cst with precision="fp64" and at most 320 rows: the same exact
+    standard errors from K covariance matrices of N x N and one p x K quadratic form, about N / B of the direct
+    form's flops, so faster when num_boot > N -- see bootstrap_permutation.check_boot_algo).
     """
     pls_method = kwargs.pop("pls_method", "mct")
     kwargs["pls_alg"] = pls_method
@@ -41,4 +44,10 @@ def PLS(*args, **kwargs):
     if "num_perm" in kwargs:
         if kwargs["num_perm"] < 0 or not isinstance(kwargs["num_perm"], int):
             raise ValueError("Invalid number of permutations provided. Value must be a positive integer.")
+    if "boot_algo" in kwargs:        # before any GPU work (the engine's upload of X starts with the analysis)
+        X = args[0] if args else kwargs.get("X")
+        engine = kwargs.get("engine")
+        bootstrap_permutation.check_boot_algo(
+            kwargs["boot_algo"], pls_method, engine.precision if engine is not None else kwargs.get("precision", "fp64"),
+            engine.N if engine is not None else (int(X.shape[0]) if X is not None and hasattr(X, "shape") else None))
     return pls_classes.PLSBase._create(pls_method, *args, **kwargs)

@@ -45,7 +45,8 @@ class PLSBase(abc.ABC):
         return cls._subclasses[pls_method](*args, **kwargs)
 
     # ---- shared helpers -------------------------------------------------------------------
-    _ENGINE_KWARGS = ("perm_indices", "boot_indices", "engine", "device", "precision", "rotate_method", "analysis")
+    _ENGINE_KWARGS = ("perm_indices", "boot_indices", "engine", "device", "precision", "rotate_method", "analysis",
+                      "boot_algo")
 
     def _take_kwargs(self, kwargs):
         self.pls_alg = kwargs["pls_alg"]
@@ -212,7 +213,8 @@ class PLSBase(abc.ABC):
             perm_indices=self._engine_kwargs.get("perm_indices"),
             boot_indices=self._engine_kwargs.get("boot_indices"),
             engine=self._engine_kwargs.get("engine"), precision=self._engine_kwargs.get("precision", "fp64"),
-            rotate_method=self._engine_kwargs.get("rotate_method", 2), device=self._engine_kwargs.get("device"), **kw)
+            rotate_method=self._engine_kwargs.get("rotate_method", 2), device=self._engine_kwargs.get("device"),
+            boot_algo=self._engine_kwargs.get("boot_algo", "direct"), **kw)
 
     def _split_half(self, Y, mctype, contrasts, **kw):
         """pls_classes.py:285-318 (identical block in every class)."""

@@ -29,7 +29,7 @@ from .engine import Engine
 METHODS = ("mct", "rb", "cst", "csb", "mb", "cmb")
 
 _state = None          # what install() replaced, for uninstall()
-_options = {"precision": "fp64"}
+_options = {"precision": "fp64", "boot_algo": "direct"}
 _shared = {"ref": None, "engine": None}
 
 
@@ -63,6 +63,7 @@ class _InstalledResampleTest(_bp._ResampleTestPLS):
         if "engine" not in kwargs and (nperm > 0 or nboot > 0):
             kwargs["engine"] = shared_engine(X)
         kwargs.setdefault("precision", _options["precision"])
+        kwargs.setdefault("boot_algo", _options["boot_algo"])
         super().__init__(X, Y, U, s, V, cond_order, mctype, *args, **kwargs)
 
 
@@ -87,12 +88,18 @@ def _split_half(pls_alg, matrix, Y, cond_order, num_split, mctype=None, contrast
                           Xbscan=Xbscan, Ybscan=Ybscan, lv=lv, CI=CI, engine=shared_engine(matrix))
 
 
-def install(plspy_module=None, precision="fp64"):
+def install(plspy_module=None, precision="fp64", boot_algo="direct"):
     """Route the permutation / bootstrap / split-half loops of `plspy_module` (default: `import plspy`) through the
-    GPU engine.  Idempotent; returns the module.  `precision`: "fp64" (exact) or "tf32x3" (fast bootstrap GEMM)."""
+    GPU engine.  Idempotent; returns the module.  `precision`: "fp64" (exact) or "tf32x3" (fast bootstrap GEMM).
+    `boot_algo`: "direct" or "collapsed" (mct / cst in the exact mode: see `bootstrap_permutation.check_boot_algo`);
+    a per-call option, applied to every resampling test while installed."""
     global _state
     if precision not in ("fp64", "tf32x3", "tf32x3+gram"):
         raise ValueError('precision must be "fp64", "tf32x3" or "tf32x3+gram"')
+    if boot_algo not in _bp.BOOT_ALGOS:
+        raise ValueError(f"boot_algo must be one of {_bp.BOOT_ALGOS}")
+    if boot_algo == "collapsed" and precision != "fp64":
+        raise ValueError('boot_algo="collapsed" is an exact (precision="fp64") formulation')
     if plspy_module is None:
         import plspy as plspy_module
     ref_bp = plspy_module.core.bootstrap_permutation
@@ -100,6 +107,7 @@ def install(plspy_module=None, precision="fp64"):
     if _state is not None and _state["module"] is not plspy_module:
         uninstall()
     _options["precision"] = precision
+    _options["boot_algo"] = boot_algo
     if _state is None:
         _state = {
             "module": plspy_module,
