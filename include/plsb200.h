@@ -58,6 +58,13 @@ int plsb200_copy2d_h2d(void* dst, size_t dst_pitch, const void* src_host, size_t
  * file holds are float32 / int16; plspy/io/io.py:10-700 assembles them into a float64 matrix on the host)         */
 int plsb200_widen_f32_f64(const float* src, double* dst, int64_t n, void* stream);
 
+/* ---- float32-resident X.  Every entry point named *_x32* is its FP64 twin with X given as float32 (N x p, leading
+ * dimension ldx in elements, any 4-byte aligned address and any ldx): each element is widened to float64 where the
+ * kernel loads it, so the results are bit-identical to the twin's on the widened matrix.  Sizes and workspaces are
+ * the twin's (plsb200_gram_f64_workspace, plsb200_xv_f64_workspace, plsb200_boot_moments_f64_workspace,
+ * plsb200_boot_quad_f64_workspace, plsb200_tf32_ximage_bytes, plsb200_gram_tf32_image_bytes).  The row-split tall
+ * kernel (PLSB200_TALL=rs) has no float32 variant: boot_moments_x32_f64 returns PLSB200_EUNSUPPORTED there. */
+
 /* ---- K1: Gram matrix G = X . X^T (N x N), FP64 DMMA, split over voxel chunks, deterministic --------
  * Replaces the N x p work that every resample redoes in the reference (row gather + means + projection,
  * resample.py:79,153 + class_functions.py:7-95 + bootstrap_permutation.py:404): once G is known every
@@ -66,6 +73,8 @@ int plsb200_widen_f32_f64(const float* src, double* dst, int64_t n, void* stream
 size_t plsb200_gram_f64_workspace(int N, int64_t p);
 int plsb200_gram_f64(const double* X, int N, int64_t p, int64_t ldx, double* G,
                      void* workspace, size_t workspace_bytes, void* stream);
+int plsb200_gram_x32_f64(const float* X, int N, int64_t p, int64_t ldx, double* G,
+                         void* workspace, size_t workspace_bytes, void* stream);
 /* The same for the row stack [X1; X2] ((N1 + N2) x p) without materialising it: the multiblock methods need the Gram
  * matrix of [X; Zb] (class_functions.py:454-516 through N-space quadratic forms).  Workspace:
  * plsb200_gram_f64_workspace(N1 + N2, p).                                                                      */
@@ -78,6 +87,8 @@ int plsb200_gram_stacked_f64(const double* X1, int N1, int64_t ld1, const double
 size_t plsb200_xv_f64_workspace(int N, int64_t p, int K);
 int plsb200_xv_f64(const double* X, int N, int64_t p, int64_t ldx, const double* V, int K,
                    double* XL, void* workspace, size_t workspace_bytes, void* stream);
+int plsb200_xv_x32_f64(const float* X, int N, int64_t p, int64_t ldx, const double* V, int K,
+                       double* XL, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- K2/K6: N-space pass over a batch of resamples ------------------------------------------------
  * For each resample r (index vector idx[r, 0..N)):
@@ -124,6 +135,7 @@ int plsb200_uhat_f64(const double* XL, int64_t xl_stride, int N, int K, const do
  * every permutation (plspy/core/bootstrap_permutation.py:323-452) like plsb200_gram_f64.                        */
 size_t plsb200_gram_tf32_image_bytes(int N, int64_t p);
 int plsb200_gram_tf32_split(const double* X, int N, int64_t p, int64_t ldx, void* image, void* stream);
+int plsb200_gram_tf32_split_x32(const float* X, int N, int64_t p, int64_t ldx, void* image, void* stream);
 size_t plsb200_gram_tf32_workspace(int N, int64_t p);
 int plsb200_gram_tf32(const void* image, int N, int64_t p, double* G, int accumulate, void* workspace,
                       size_t workspace_bytes, void* stream);
@@ -144,6 +156,9 @@ size_t plsb200_boot_moments_f64_workspace(int N, int64_t p, int K, int R);
 int plsb200_boot_moments_f64(const double* X, int N, int64_t p, int64_t ldx, const double* coef, int K,
                              int R, const double* pivot, double* sum, double* sumsq,
                              void* workspace, size_t workspace_bytes, void* stream);
+int plsb200_boot_moments_x32_f64(const float* X, int N, int64_t p, int64_t ldx, const double* coef, int K,
+                                 int R, const double* pivot, double* sum, double* sumsq,
+                                 void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- K4 collapsed (task methods, exact FP64): the bootstrap variance as a quadratic form ------------------
  * Each salience is linear in the draw, so R . Var_r(VS_r[v,k]) = x_v^T S_k x_v with S_k = R . Cov_r(c_rk) (N x N).
@@ -158,6 +173,8 @@ int plsb200_boot_quad_coef_pack_f64(const double* S, int N, int K, double* coef,
 size_t plsb200_boot_quad_f64_workspace(int N, int64_t p, int K);
 int plsb200_boot_quad_f64(const double* X, int N, int64_t p, int64_t ldx, const double* coef, int K, double* q,
                           void* workspace, size_t workspace_bytes, void* stream);
+int plsb200_boot_quad_x32_f64(const float* X, int N, int64_t p, int64_t ldx, const double* coef, int K, double* q,
+                              void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- K4 fast mode: the same moments on the tcgen05 tensor cores with the 3xTF32 split ---------------------
  * (x = xh + xl, c = ch + cl, each TF32-exact; xh.cl + xl.ch + xh.ch accumulated in FP32 in tensor memory, the
@@ -169,6 +186,7 @@ int plsb200_boot_quad_f64(const double* X, int N, int64_t p, int64_t ldx, const 
  * boot_moments_tf32: sum_r (VS_r - pivot), sum_r (VS_r - pivot)^2 (p x K each, overwritten).              */
 size_t plsb200_tf32_ximage_bytes(int N, int64_t p);
 int plsb200_tf32_split_x(const double* X, int N, int64_t p, int64_t ldx, void* ximage, void* stream);
+int plsb200_tf32_split_x32(const float* X, int N, int64_t p, int64_t ldx, void* ximage, void* stream);
 size_t plsb200_boot_coef_bytes_tf32(int N, int K, int R);
 int plsb200_boot_coef_pack_tf32(const double* E, int N, int K, const int32_t* idx, int R, void* coef, void* stream);
 size_t plsb200_boot_moments_tf32_workspace(int N, int64_t p, int K, int R);
@@ -201,10 +219,14 @@ int plsb200_percentile_f64(const double* samples, int B, int64_t nseries, int64_
  * boot_debug_dict["right_sv_sampled"] on problems small enough to hold it.                          */
 int plsb200_salience_f64(const double* X, int N, int64_t p, int64_t ldx, const double* E, int K,
                          const int32_t* idx, int R, double* VS, void* stream);
+int plsb200_salience_x32_f64(const float* X, int N, int64_t p, int64_t ldx, const double* E, int K,
+                             const int32_t* idx, int R, double* VS, void* stream);
 /* the same saliences series-major, VS[v][k][r] (p x K x R): the R samples of an element are contiguous, which is the
  * layout plsb200_percentile_f64 sorts fastest (stride_sample = 1, stride_series = R); p <= 65535 * 128 per call.   */
 int plsb200_salience_series_f64(const double* X, int N, int64_t p, int64_t ldx, const double* E, int K,
                                 const int32_t* idx, int R, double* VS, void* stream);
+int plsb200_salience_series_x32_f64(const float* X, int N, int64_t p, int64_t ldx, const double* E, int K,
+                                    const int32_t* idx, int R, double* VS, void* stream);
 
 /* ---- K5: behaviour PLS (rb / csb) -----------------------------------------------------------------
  * Cells = (group, condition) blocks of consecutive rows, given as ncell+1 int32 offsets `cell_start`.

@@ -40,15 +40,19 @@ SIGNATURES = {
     "plsb200_widen_f32_f64": (c_int, [c_void_p, c_double_p, c_int64, c_void_p]),
     "plsb200_gram_f64_workspace": (c_size_t, [c_int, c_int64]),
     "plsb200_gram_f64": (c_int, [c_double_p, c_int, c_int64, c_int64, c_double_p, c_void_p, c_size_t, c_void_p]),
+    "plsb200_gram_x32_f64": (c_int, [c_void_p, c_int, c_int64, c_int64, c_double_p, c_void_p, c_size_t, c_void_p]),
     "plsb200_gram_stacked_f64": (c_int, [c_double_p, c_int, c_int64, c_double_p, c_int, c_int64, c_int64, c_double_p,
                                          c_void_p, c_size_t, c_void_p]),
     "plsb200_gram_tf32_image_bytes": (c_size_t, [c_int, c_int64]),
     "plsb200_gram_tf32_split": (c_int, [c_double_p, c_int, c_int64, c_int64, c_void_p, c_void_p]),
+    "plsb200_gram_tf32_split_x32": (c_int, [c_void_p, c_int, c_int64, c_int64, c_void_p, c_void_p]),
     "plsb200_gram_tf32_workspace": (c_size_t, [c_int, c_int64]),
     "plsb200_gram_tf32": (c_int, [c_void_p, c_int, c_int64, c_double_p, c_int, c_void_p, c_size_t, c_void_p]),
     "plsb200_xv_f64_workspace": (c_size_t, [c_int, c_int64, c_int]),
     "plsb200_xv_f64": (c_int, [c_double_p, c_int, c_int64, c_int64, c_double_p, c_int, c_double_p, c_void_p,
                                c_size_t, c_void_p]),
+    "plsb200_xv_x32_f64": (c_int, [c_void_p, c_int, c_int64, c_int64, c_double_p, c_int, c_double_p, c_void_p,
+                                   c_size_t, c_void_p]),
     "plsb200_nspace_f64": (c_int, [c_double_p, c_int, c_double_p, c_int, c_int32_p, c_int, c_double_p, c_int,
                                    c_double_p, c_double_p, c_void_p]),
     "plsb200_nspace_dmma_f64_workspace": (c_size_t, [c_int, c_int, c_int, c_int]),
@@ -68,13 +72,18 @@ SIGNATURES = {
     "plsb200_boot_moments_f64_workspace": (c_size_t, [c_int, c_int64, c_int, c_int]),
     "plsb200_boot_moments_f64": (c_int, [c_double_p, c_int, c_int64, c_int64, c_double_p, c_int, c_int,
                                          c_double_p, c_double_p, c_double_p, c_void_p, c_size_t, c_void_p]),
+    "plsb200_boot_moments_x32_f64": (c_int, [c_void_p, c_int, c_int64, c_int64, c_double_p, c_int, c_int,
+                                             c_double_p, c_double_p, c_double_p, c_void_p, c_size_t, c_void_p]),
     "plsb200_boot_quad_coef_bytes": (c_size_t, [c_int, c_int]),
     "plsb200_boot_quad_coef_pack_f64": (c_int, [c_double_p, c_int, c_int, c_double_p, c_void_p]),
     "plsb200_boot_quad_f64_workspace": (c_size_t, [c_int, c_int64, c_int]),
     "plsb200_boot_quad_f64": (c_int, [c_double_p, c_int, c_int64, c_int64, c_double_p, c_int, c_double_p, c_void_p,
                                       c_size_t, c_void_p]),
+    "plsb200_boot_quad_x32_f64": (c_int, [c_void_p, c_int, c_int64, c_int64, c_double_p, c_int, c_double_p, c_void_p,
+                                          c_size_t, c_void_p]),
     "plsb200_tf32_ximage_bytes":(c_size_t, [c_int, c_int64]),
     "plsb200_tf32_split_x": (c_int, [c_double_p, c_int, c_int64, c_int64, c_void_p, c_void_p]),
+    "plsb200_tf32_split_x32": (c_int, [c_void_p, c_int, c_int64, c_int64, c_void_p, c_void_p]),
     "plsb200_boot_coef_bytes_tf32": (c_size_t, [c_int, c_int, c_int]),
     "plsb200_boot_coef_pack_tf32": (c_int, [c_double_p, c_int, c_int, c_int32_p, c_int, c_void_p, c_void_p]),
     "plsb200_boot_moments_tf32_workspace": (c_size_t, [c_int, c_int64, c_int, c_int]),
@@ -128,6 +137,10 @@ SIGNATURES = {
                                      c_double_p, c_void_p]),
     "plsb200_salience_series_f64": (c_int, [c_double_p, c_int, c_int64, c_int64, c_double_p, c_int, c_int32_p, c_int,
                                      c_double_p, c_void_p]),
+    "plsb200_salience_x32_f64": (c_int, [c_void_p, c_int, c_int64, c_int64, c_double_p, c_int, c_int32_p, c_int,
+                                         c_double_p, c_void_p]),
+    "plsb200_salience_series_x32_f64": (c_int, [c_void_p, c_int, c_int64, c_int64, c_double_p, c_int, c_int32_p,
+                                                c_int, c_double_p, c_void_p]),
 }
 
 for _name, (_res, _args) in SIGNATURES.items():

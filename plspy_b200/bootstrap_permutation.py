@@ -381,6 +381,24 @@ def check_boot_algo(boot_algo, pls_alg, precision, N):
             'use boot_algo="direct"')
 
 
+X_STORAGES = ("fp64", "fp32")
+
+
+def check_x_storage(x_storage, pls_alg):
+    """Validates the device storage of X before any GPU work.
+
+    "fp64" (default) holds X as float64.  "fp32" analyses X.astype(float32): the device holds that float32 matrix
+    (half the memory and half the bytes of every pass over X) and every kernel widens an element where it loads it,
+    so all results equal, bit for bit, those of the "fp64" run on the widened matrix.  Task methods (mct, cst) only:
+    the block standardisation kernels of the behaviour and multiblock methods read float64."""
+    if x_storage not in X_STORAGES:
+        raise ValueError(f'x_storage must be one of {X_STORAGES}, got {x_storage!r}')
+    if x_storage == "fp32" and pls_alg not in ("mct", "cst"):
+        raise exceptions.NotImplementedError(
+            'x_storage="fp32" applies to the task methods (mct, cst); the behaviour and multiblock methods keep X '
+            'in float64')
+
+
 def _collapsed_sumsq(eng, E, idx_dev, niter, lo, hi):
     """Collapsed bootstrap: q[v,k] = x_v^T S_k x_v with S_k = sum_r (c_rk - e_k)(c_rk - e_k)^T - s1_k s1_k^T / niter
     (= niter . Cov_r(c_rk)): the sum of squares of (VS_r - mean) over all `niter` resamples, p x K, the same on every
@@ -415,10 +433,13 @@ class _ResampleTestPLS(ResampleTest):
     def __init__(self, X, Y, U, s, V, cond_order, mctype, contrast=None, preprocess=None, nperm=1000,
                  nboot=1000, bscan=None, Xbscan=None, Ybscan=None, lvcorrs_orig=None, Tvsc_orig=None,
                  CI=0.95, *, perm_indices=None, boot_indices=None, engine=None, precision="fp64", rotate_method=2,
-                 device=None, boot_algo="direct"):
+                 device=None, boot_algo="direct", x_storage="fp64"):
         self.CI = CI
         check_boot_algo(boot_algo, self.pls_alg, engine.precision if engine is not None else precision,
                         engine.N if engine is not None else (int(X.shape[0]) if X is not None else None))
+        check_x_storage(x_storage, self.pls_alg)
+        if engine is not None:
+            check_x_storage(engine.x_storage, self.pls_alg)
         self.boot_algo = boot_algo
         if rotate_method not in (0, 1, 2):
             raise ValueError("rotate_method must be 0 (SVD), 1 (Procrustes) or 2 (derived)")
@@ -429,7 +450,7 @@ class _ResampleTestPLS(ResampleTest):
         self.rotate_method = rotate_method
         _log(f"PLS ALG: {self.pls_alg}")
         eng = engine if engine is not None else (
-            Engine(X, device=device, precision=precision) if (nperm > 0 or nboot > 0) else None)
+            Engine(X, device=device, precision=precision, x_storage=x_storage) if (nperm > 0 or nboot > 0) else None)
         self._engine = eng
         if eng is not None and self.pls_alg in ("mct", "cst") and dist.world()[1] > 1:
             eng.gram_collective()          # all ranks are here: Gram from per-rank voxel ranges + one all-reduce

@@ -79,10 +79,11 @@ __global__ void __launch_bounds__(256) boot_coef_pack_kernel(const double* __res
 // ------------------------------------------------------------------------------------------------
 // NKS (k-steps of 4 rows) is a compile-time constant so that the whole period is one straight-line
 // stream of NKS*NBLK {LDS.64, DMMA} pairs that ptxas can software-pipeline; kernels are instantiated
-// for every multiple of 4 up to 80 (N <= 320).
-template <int NKS, int NBLK>
+// for every multiple of 4 up to 80 (N <= 320).  T: element type of X (float: X stored as float32, widened as the A
+// fragments are loaded -- the same DMMA operands as from the widened matrix).
+template <typename T, int NKS, int NBLK>
 __global__ void __launch_bounds__(BM_THREADS, 1)
-boot_moments_kernel(const double* __restrict__ X, long long ldx, int N, long long p,
+boot_moments_kernel(const T* __restrict__ X, long long ldx, int N, long long p,
                     const double* __restrict__ coef, int nper, int per_per_split, int nstage,
                     int R, int Kp, int K, const double* __restrict__ pivot,
                     double* __restrict__ osum, double* __restrict__ osumsq) {
@@ -125,7 +126,7 @@ boot_moments_kernel(const double* __restrict__ X, long long ldx, int N, long lon
 #pragma unroll
     for (int s = 0; s < NKS; ++s) {
         const int row = 4 * s + q;
-        a[s] = (row < N && v < p) ? __ldg(X + (long long)row * ldx + v) : 0.0;
+        a[s] = (row < N && v < p) ? (double)__ldg(X + (long long)row * ldx + v) : 0.0;
     }
 
     // ---- per-thread column bookkeeping (fixed for the whole kernel)
@@ -412,8 +413,8 @@ __global__ void boot_finalize_kernel(const double* __restrict__ sum, const doubl
 // SERIES: output [v][k][r] (the R samples of an element contiguous: the layout percentile_kernel sorts fastest) with the
 // resample as the FAST grid index, so that the CTAs running at one time share their rows of X in L2 and write
 // neighbouring 8-byte slots of the same sectors.
-template <int KT, bool SERIES>
-__global__ void __launch_bounds__(128) salience_kernel(const double* __restrict__ X, int N, long long p, long long ldx,
+template <typename T, int KT, bool SERIES>
+__global__ void __launch_bounds__(128) salience_kernel(const T* __restrict__ X, int N, long long p, long long ldx,
                                                       const double* __restrict__ E, int K,
                                                       const int32_t* __restrict__ idx, int R, double* __restrict__ VS) {
     extern __shared__ __align__(16) double sms[];
@@ -430,7 +431,7 @@ __global__ void __launch_bounds__(128) salience_kernel(const double* __restrict_
 #pragma unroll
         for (int t = 0; t < KT; ++t) acc[t] = 0.0;
         for (int i = 0; i < N; ++i) {
-            const double x = __ldg(X + (long long)ids[i] * ldx + v);
+            const double x = (double)__ldg(X + (long long)ids[i] * ldx + v);
 #pragma unroll
             for (int t = 0; t < KT; ++t)
                 if (k0 + t < K) acc[t] = fma(x, Es[i * K + k0 + t], acc[t]);
@@ -450,8 +451,8 @@ __global__ void __launch_bounds__(128) salience_kernel(const double* __restrict_
 // partial sums are combined by shuffles in a fixed order (deterministic).  HBM-bound: X is read once.
 constexpr int XV_CHUNK = 512;
 constexpr int XV_RG = 2;
-template <int KT>
-__global__ void __launch_bounds__(256, 3) xv_partial_kernel(const double* __restrict__ X, int N, long long p, long long ldx,
+template <typename T, int KT>
+__global__ void __launch_bounds__(256, 3) xv_partial_kernel(const T* __restrict__ X, int N, long long p, long long ldx,
                                                         const double* __restrict__ V, int K,
                                                         double* __restrict__ part) {
     extern __shared__ __align__(16) double smv[];   // [KT][XV_CHUNK]
@@ -472,12 +473,12 @@ __global__ void __launch_bounds__(256, 3) xv_partial_kernel(const double* __rest
             for (int r = 0; r < XV_RG; ++r)
 #pragma unroll
                 for (int t = 0; t < KT; ++t) acc[r][t] = 0.0;
-            const double* x = X + (long long)r0 * ldx + v0;
+            const T* x = X + (long long)r0 * ldx + v0;
 #pragma unroll 2
             for (int c = lane; c < nv; c += 32) {
                 double xr[XV_RG];
 #pragma unroll
-                for (int r = 0; r < XV_RG; ++r) xr[r] = (r0 + r < N) ? __ldg(x + (long long)r * ldx + c) : 0.0;
+                for (int r = 0; r < XV_RG; ++r) xr[r] = (r0 + r < N) ? (double)__ldg(x + (long long)r * ldx + c) : 0.0;
 #pragma unroll
                 for (int t = 0; t < KT; ++t) {
                     const double vv = smv[t * XV_CHUNK + c];
@@ -507,23 +508,23 @@ __global__ void xv_reduce_kernel(const double* __restrict__ part, int nchunk, in
     out[i] = s;
 }
 
-template <int NKS, int NBLK>
-static int launch_moments(const BootPlan& b, const double* X, int N, int64_t p, int64_t ldx, const double* coef, int K,
+template <typename T, int NKS, int NBLK>
+static int launch_moments(const BootPlan& b, const T* X, int N, int64_t p, int64_t ldx, const double* coef, int K,
                           int R, const double* pivot, double* o1, double* o2, cudaStream_t st) {
-    PLSB_CUDA(cudaFuncSetAttribute(boot_moments_kernel<NKS, NBLK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    PLSB_CUDA(cudaFuncSetAttribute(boot_moments_kernel<T, NKS, NBLK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                    (int)b.smem_bytes));
     dim3 grid((unsigned)cdiv(p, BM_VOX), (unsigned)b.nsplit);
-    boot_moments_kernel<NKS, NBLK><<<grid, BM_THREADS, b.smem_bytes, st>>>(
+    boot_moments_kernel<T, NKS, NBLK><<<grid, BM_THREADS, b.smem_bytes, st>>>(
         X, ldx, N, p, coef, b.nper, b.per_per_split, b.nstage, R, b.Kp, K, pivot, o1, o2);
     PLSB_LAUNCH_CHECK("boot_moments_kernel");
     return PLSB200_OK;
 }
 
-template <int NBLK>
-static int dispatch_nks(const BootPlan& b, const double* X, int N, int64_t p, int64_t ldx, const double* coef, int K,
+template <typename T, int NBLK>
+static int dispatch_nks(const BootPlan& b, const T* X, int N, int64_t p, int64_t ldx, const double* coef, int K,
                         int R, const double* pivot, double* o1, double* o2, cudaStream_t st) {
     switch (b.nks) {
-#define PLSB_CASE(n) case n: return launch_moments<n, NBLK>(b, X, N, p, ldx, coef, K, R, pivot, o1, o2, st);
+#define PLSB_CASE(n) case n: return launch_moments<T, n, NBLK>(b, X, N, p, ldx, coef, K, R, pivot, o1, o2, st);
         PLSB_CASE(4) PLSB_CASE(8) PLSB_CASE(12) PLSB_CASE(16) PLSB_CASE(20) PLSB_CASE(24) PLSB_CASE(28)
         PLSB_CASE(32) PLSB_CASE(36) PLSB_CASE(40) PLSB_CASE(44) PLSB_CASE(48) PLSB_CASE(52) PLSB_CASE(56)
         PLSB_CASE(60) PLSB_CASE(64) PLSB_CASE(68) PLSB_CASE(72) PLSB_CASE(76) PLSB_CASE(80)
@@ -585,19 +586,37 @@ extern "C" size_t plsb200_boot_moments_f64_workspace(int N, int64_t p, int K, in
     return b.nsplit > 1 ? (size_t)2 * b.nsplit * p * K * sizeof(double) : 16;
 }
 
-extern "C" int plsb200_boot_moments_f64(const double* X, int N, int64_t p, int64_t ldx, const double* coef, int K, int R,
-                                        const double* pivot, double* sum, double* sumsq, void* workspace,
-                                        size_t workspace_bytes, void* stream) {
-    PLSB_CHECK_ARG(X && coef && sum && sumsq, "boot_moments_f64: null pointer");
-    PLSB_CHECK_ARG(p > 0 && ldx >= p, "boot_moments_f64: bad shape p=%lld ldx=%lld", (long long)p, (long long)ldx);
+// tall designs: the output-stationary or (PLSB200_TALL=rs) the row-split kernel; the row-split kernel reads FP64 X only
+static int tall_moments(const double* X, int N, int64_t p, int64_t ldx, const double* coef, int K, int R,
+                        const double* pivot, double* sum, double* sumsq, void* workspace, size_t workspace_bytes,
+                        cudaStream_t st) {
+    return use_os(N) ? boot_os_moments(X, N, p, ldx, coef, K, R, pivot, sum, sumsq, workspace, workspace_bytes, st,
+                                       "boot_moments_f64")
+                     : boot_rs_moments(X, N, p, ldx, coef, K, R, pivot, sum, sumsq, workspace, workspace_bytes, st);
+}
+static int tall_moments(const float* X, int N, int64_t p, int64_t ldx, const double* coef, int K, int R,
+                        const double* pivot, double* sum, double* sumsq, void* workspace, size_t workspace_bytes,
+                        cudaStream_t st) {
+    if (!use_os(N)) {
+        set_err("boot_moments_x32_f64: the row-split kernel (PLSB200_TALL=rs) has no float32 variant; "
+                "unset PLSB200_TALL or store X as float64");
+        return PLSB200_EUNSUPPORTED;
+    }
+    return boot_os_moments(X, N, p, ldx, coef, K, R, pivot, sum, sumsq, workspace, workspace_bytes, st,
+                           "boot_moments_x32_f64");
+}
+
+template <typename T>
+static int boot_moments(const T* X, int N, int64_t p, int64_t ldx, const double* coef, int K, int R,
+                        const double* pivot, double* sum, double* sumsq, void* workspace, size_t workspace_bytes,
+                        void* stream, const char* what) {
+    PLSB_CHECK_ARG(X && coef && sum && sumsq, "%s: null pointer", what);
+    PLSB_CHECK_ARG(p > 0 && ldx >= p, "%s: bad shape p=%lld ldx=%lld", what, (long long)p, (long long)ldx);
     if (use_other(N))
-        return use_os(N) ? boot_os_moments(X, N, p, ldx, coef, K, R, pivot, sum, sumsq, workspace, workspace_bytes,
-                                           (cudaStream_t)stream)
-                         : boot_rs_moments(X, N, p, ldx, coef, K, R, pivot, sum, sumsq, workspace, workspace_bytes,
-                                           (cudaStream_t)stream);
+        return tall_moments(X, N, p, ldx, coef, K, R, pivot, sum, sumsq, workspace, workspace_bytes, (cudaStream_t)stream);
     BootPlan b;
     if (!boot_plan(N, K, R, p, b)) {
-        set_err("boot_moments_f64: unsupported shape N=%d K=%d R=%d (need K<=24, N<=320)", N, K, R);
+        set_err("%s: unsupported shape N=%d K=%d R=%d (need K<=24, N<=320)", what, N, K, R);
         return PLSB200_EUNSUPPORTED;
     }
     cudaStream_t st = (cudaStream_t)stream;
@@ -605,7 +624,7 @@ extern "C" int plsb200_boot_moments_f64(const double* X, int N, int64_t p, int64
     if (b.nsplit > 1) {
         size_t need = (size_t)2 * b.nsplit * p * K * sizeof(double);
         if (!workspace || workspace_bytes < need) {
-            set_err("boot_moments_f64: workspace %zu < %zu bytes", workspace_bytes, need);
+            set_err("%s: workspace %zu < %zu bytes", what, workspace_bytes, need);
             return PLSB200_EWORKSPACE;
         }
         o1 = (double*)workspace;
@@ -613,9 +632,9 @@ extern "C" int plsb200_boot_moments_f64(const double* X, int N, int64_t p, int64
     }
     int rc;
     switch (b.nblk) {
-        case 1: rc = dispatch_nks<1>(b, X, N, p, ldx, coef, K, R, pivot, o1, o2, st); break;
-        case 2: rc = dispatch_nks<2>(b, X, N, p, ldx, coef, K, R, pivot, o1, o2, st); break;
-        default: rc = dispatch_nks<3>(b, X, N, p, ldx, coef, K, R, pivot, o1, o2, st); break;
+        case 1: rc = dispatch_nks<T, 1>(b, X, N, p, ldx, coef, K, R, pivot, o1, o2, st); break;
+        case 2: rc = dispatch_nks<T, 2>(b, X, N, p, ldx, coef, K, R, pivot, o1, o2, st); break;
+        default: rc = dispatch_nks<T, 3>(b, X, N, p, ldx, coef, K, R, pivot, o1, o2, st); break;
     }
     if (rc != PLSB200_OK) return rc;
     if (b.nsplit > 1) {
@@ -624,6 +643,20 @@ extern "C" int plsb200_boot_moments_f64(const double* X, int N, int64_t p, int64
         PLSB_LAUNCH_CHECK("moments_reduce_kernel");
     }
     return PLSB200_OK;
+}
+
+extern "C" int plsb200_boot_moments_f64(const double* X, int N, int64_t p, int64_t ldx, const double* coef, int K, int R,
+                                        const double* pivot, double* sum, double* sumsq, void* workspace,
+                                        size_t workspace_bytes, void* stream) {
+    return boot_moments(X, N, p, ldx, coef, K, R, pivot, sum, sumsq, workspace, workspace_bytes, stream,
+                        "boot_moments_f64");
+}
+
+extern "C" int plsb200_boot_moments_x32_f64(const float* X, int N, int64_t p, int64_t ldx, const double* coef, int K,
+                                            int R, const double* pivot, double* sum, double* sumsq, void* workspace,
+                                            size_t workspace_bytes, void* stream) {
+    return boot_moments(X, N, p, ldx, coef, K, R, pivot, sum, sumsq, workspace, workspace_bytes, stream,
+                        "boot_moments_x32_f64");
 }
 
 extern "C" int plsb200_boot_finalize_f64(const double* sum, const double* sumsq, int64_t p, int K, int64_t R_total,
@@ -638,42 +671,50 @@ extern "C" int plsb200_boot_finalize_f64(const double* sum, const double* sumsq,
     return PLSB200_OK;
 }
 
-static int salience_launch(const double* X, int N, int64_t p, int64_t ldx, const double* E, int K, const int32_t* idx, int R,
-                           double* VS, bool series, void* stream);
+template <typename T>
+static int salience_launch(const T* X, int N, int64_t p, int64_t ldx, const double* E, int K, const int32_t* idx, int R,
+                           double* VS, bool series, void* stream, const char* what) {
+    PLSB_CHECK_ARG(X && E && idx && VS, "%s: null pointer", what);
+    PLSB_CHECK_ARG(N > 0 && p > 0 && K > 0 && R >= 0 && ldx >= p, "%s: bad shape", what);
+    if (R == 0) return PLSB200_OK;
+    size_t smem = (size_t)N * K * sizeof(double) + (size_t)N * sizeof(int);
+    if (smem > 200 * 1024) {
+        set_err("%s: N*K too large", what);
+        return PLSB200_EUNSUPPORTED;
+    }
+    if (series) {
+        PLSB_CHECK_ARG(cdiv(p, 128) <= 65535, "%s: more than 65535 voxel blocks per call", what);
+        PLSB_CUDA(cudaFuncSetAttribute(salience_kernel<T, 12, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        dim3 grid((unsigned)R, (unsigned)cdiv(p, 128));
+        salience_kernel<T, 12, true><<<grid, 128, smem, (cudaStream_t)stream>>>(X, N, p, ldx, E, K, idx, R, VS);
+    } else {
+        PLSB_CHECK_ARG(R <= 65535, "%s: more than 65535 resamples per call", what);
+        PLSB_CUDA(cudaFuncSetAttribute(salience_kernel<T, 12, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        dim3 grid((unsigned)cdiv(p, 128), (unsigned)R);
+        salience_kernel<T, 12, false><<<grid, 128, smem, (cudaStream_t)stream>>>(X, N, p, ldx, E, K, idx, R, VS);
+    }
+    PLSB_LAUNCH_CHECK("salience_kernel");
+    return PLSB200_OK;
+}
 
 extern "C" int plsb200_salience_f64(const double* X, int N, int64_t p, int64_t ldx, const double* E, int K,
                                     const int32_t* idx, int R, double* VS, void* stream) {
-    return salience_launch(X, N, p, ldx, E, K, idx, R, VS, false, stream);
+    return salience_launch(X, N, p, ldx, E, K, idx, R, VS, false, stream, "salience_f64");
 }
 
 extern "C" int plsb200_salience_series_f64(const double* X, int N, int64_t p, int64_t ldx, const double* E, int K,
                                            const int32_t* idx, int R, double* VS, void* stream) {
-    return salience_launch(X, N, p, ldx, E, K, idx, R, VS, true, stream);
+    return salience_launch(X, N, p, ldx, E, K, idx, R, VS, true, stream, "salience_series_f64");
 }
 
-static int salience_launch(const double* X, int N, int64_t p, int64_t ldx, const double* E, int K, const int32_t* idx, int R,
-                           double* VS, bool series, void* stream) {
-    PLSB_CHECK_ARG(X && E && idx && VS, "salience_f64: null pointer");
-    PLSB_CHECK_ARG(N > 0 && p > 0 && K > 0 && R >= 0 && ldx >= p, "salience_f64: bad shape");
-    if (R == 0) return PLSB200_OK;
-    size_t smem = (size_t)N * K * sizeof(double) + (size_t)N * sizeof(int);
-    if (smem > 200 * 1024) {
-        set_err("salience_f64: N*K too large");
-        return PLSB200_EUNSUPPORTED;
-    }
-    if (series) {
-        PLSB_CHECK_ARG(cdiv(p, 128) <= 65535, "salience_series_f64: more than 65535 voxel blocks per call");
-        PLSB_CUDA(cudaFuncSetAttribute(salience_kernel<12, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        dim3 grid((unsigned)R, (unsigned)cdiv(p, 128));
-        salience_kernel<12, true><<<grid, 128, smem, (cudaStream_t)stream>>>(X, N, p, ldx, E, K, idx, R, VS);
-    } else {
-        PLSB_CHECK_ARG(R <= 65535, "salience_f64: more than 65535 resamples per call");
-        PLSB_CUDA(cudaFuncSetAttribute(salience_kernel<12, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        dim3 grid((unsigned)cdiv(p, 128), (unsigned)R);
-        salience_kernel<12, false><<<grid, 128, smem, (cudaStream_t)stream>>>(X, N, p, ldx, E, K, idx, R, VS);
-    }
-    PLSB_LAUNCH_CHECK("salience_kernel");
-    return PLSB200_OK;
+extern "C" int plsb200_salience_x32_f64(const float* X, int N, int64_t p, int64_t ldx, const double* E, int K,
+                                        const int32_t* idx, int R, double* VS, void* stream) {
+    return salience_launch(X, N, p, ldx, E, K, idx, R, VS, false, stream, "salience_x32_f64");
+}
+
+extern "C" int plsb200_salience_series_x32_f64(const float* X, int N, int64_t p, int64_t ldx, const double* E, int K,
+                                               const int32_t* idx, int R, double* VS, void* stream) {
+    return salience_launch(X, N, p, ldx, E, K, idx, R, VS, true, stream, "salience_series_x32_f64");
 }
 
 extern "C" size_t plsb200_xv_f64_workspace(int N, int64_t p, int K) {
@@ -681,24 +722,35 @@ extern "C" size_t plsb200_xv_f64_workspace(int N, int64_t p, int K) {
     return (size_t)cdiv(p, XV_CHUNK) * N * K * sizeof(double);
 }
 
-extern "C" int plsb200_xv_f64(const double* X, int N, int64_t p, int64_t ldx, const double* V, int K, double* XL,
-                              void* workspace, size_t workspace_bytes, void* stream) {
-    PLSB_CHECK_ARG(X && V && XL && workspace, "xv_f64: null pointer");
-    PLSB_CHECK_ARG(N > 0 && p > 0 && K > 0 && ldx >= p, "xv_f64: bad shape");
+template <typename T>
+static int xv_launch(const T* X, int N, int64_t p, int64_t ldx, const double* V, int K, double* XL, void* workspace,
+                     size_t workspace_bytes, void* stream, const char* what) {
+    PLSB_CHECK_ARG(X && V && XL && workspace, "%s: null pointer", what);
+    PLSB_CHECK_ARG(N > 0 && p > 0 && K > 0 && ldx >= p, "%s: bad shape", what);
     const int nchunk = (int)cdiv(p, XV_CHUNK);
     size_t need = (size_t)nchunk * N * K * sizeof(double);
     if (workspace_bytes < need) {
-        set_err("xv_f64: workspace %zu < %zu bytes", workspace_bytes, need);
+        set_err("%s: workspace %zu < %zu bytes", what, workspace_bytes, need);
         return PLSB200_EWORKSPACE;
     }
     size_t smem = (size_t)XV_CHUNK * 12 * sizeof(double);
     cudaStream_t st = (cudaStream_t)stream;
-    PLSB_CUDA(cudaFuncSetAttribute(xv_partial_kernel<12>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    xv_partial_kernel<12><<<nchunk, 256, smem, st>>>(X, N, p, ldx, V, K, (double*)workspace);
+    PLSB_CUDA(cudaFuncSetAttribute(xv_partial_kernel<T, 12>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    xv_partial_kernel<T, 12><<<nchunk, 256, smem, st>>>(X, N, p, ldx, V, K, (double*)workspace);
     PLSB_LAUNCH_CHECK("xv_partial_kernel");
     xv_reduce_kernel<<<(unsigned)cdiv((int64_t)N * K, 256), 256, 0, st>>>((const double*)workspace, nchunk, N * K, XL);
     PLSB_LAUNCH_CHECK("xv_reduce_kernel");
     return PLSB200_OK;
+}
+
+extern "C" int plsb200_xv_f64(const double* X, int N, int64_t p, int64_t ldx, const double* V, int K, double* XL,
+                              void* workspace, size_t workspace_bytes, void* stream) {
+    return xv_launch(X, N, p, ldx, V, K, XL, workspace, workspace_bytes, stream, "xv_f64");
+}
+
+extern "C" int plsb200_xv_x32_f64(const float* X, int N, int64_t p, int64_t ldx, const double* V, int K, double* XL,
+                                  void* workspace, size_t workspace_bytes, void* stream) {
+    return xv_launch(X, N, p, ldx, V, K, XL, workspace, workspace_bytes, stream, "xv_x32_f64");
 }
 
 // ---- N-space pass on DMMA (see nspace_dmma_kernel) -----------------------------------------------------------

@@ -117,8 +117,10 @@ __global__ void __launch_bounds__(256) boot_os_pack_kernel(const double* __restr
 
 // Tile-major image of X: block (t, sb) = rows [4 ks sb, 4 ks (sb + 1)) x voxels [128 t, 128 t + 128) at a pitch of 132
 // doubles, zero-filled beyond N rows / p voxels (and in the 4 padding columns).  One pass over X per call
-// (3.5 ms for the 9.6 GB of BASELINE config 5, against 2.4 s of GEMM).
-__global__ void __launch_bounds__(256) os_ximage_kernel(const double* __restrict__ X, long long ldx, int N, long long p,
+// (3.5 ms for the 9.6 GB of BASELINE config 5, against 2.4 s of GEMM).  T = float: X stored as float32, widened here,
+// so the image -- and everything after it -- is that of the widened matrix.
+template <typename T>
+__global__ void __launch_bounds__(256) os_ximage_kernel(const T* __restrict__ X, long long ldx, int N, long long p,
                                                        int nsb, int ks, double* __restrict__ img) {
     const long long t = blockIdx.x;
     const int sb = blockIdx.y;
@@ -128,7 +130,7 @@ __global__ void __launch_bounds__(256) os_ximage_kernel(const double* __restrict
         const int r = i / OS_PITCH, c = i % OS_PITCH;
         const int row = sb * 4 * ks + r;
         const long long v = t * OS_TM + c;
-        out[i] = (c < OS_TM && row < N && v < p) ? __ldg(X + (long long)row * ldx + v) : 0.0;
+        out[i] = (c < OS_TM && row < N && v < p) ? (double)__ldg(X + (long long)row * ldx + v) : 0.0;
     }
 }
 
@@ -359,21 +361,23 @@ int boot_os_pack(const double* E, int N, int K, const int32_t* idx, int R, doubl
     return PLSB200_OK;
 }
 
-int boot_os_moments(const double* X, int N, int64_t p, int64_t ldx, const double* coef, int K, int R, const double* pivot,
-                    double* sum, double* sumsq, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+template <typename T>
+static int os_moments(const T* X, int N, int64_t p, int64_t ldx, const double* coef, int K, int R, const double* pivot,
+                      double* sum, double* sumsq, void* workspace, size_t workspace_bytes, cudaStream_t st,
+                      const char* what) {
     OsPlan b;
     if (!os_plan(N, K, R, p, b)) {
-        set_err("boot_moments_f64: unsupported shape N=%d K=%d R=%d (need K<=24)", N, K, R);
+        set_err("%s: unsupported shape N=%d K=%d R=%d (need K<=24)", what, N, K, R);
         return PLSB200_EUNSUPPORTED;
     }
     const size_t pbytes = os_partial_bytes(b, p, K), need = pbytes + os_image_bytes(b, p);
     if (!workspace || workspace_bytes < need) {
-        set_err("boot_moments_f64: workspace %zu < %zu bytes", workspace_bytes, need);
+        set_err("%s: workspace %zu < %zu bytes", what, workspace_bytes, need);
         return PLSB200_EWORKSPACE;
     }
     char* base = reinterpret_cast<char*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255);
     if ((size_t)(base - (char*)workspace) + need > workspace_bytes) {
-        set_err("boot_moments_f64: workspace too small after alignment");
+        set_err("%s: workspace too small after alignment", what);
         return PLSB200_EWORKSPACE;
     }
     double *o1 = sum, *o2 = sumsq;
@@ -381,7 +385,7 @@ int boot_os_moments(const double* X, int N, int64_t p, int64_t ldx, const double
     double* img = (double*)(base + pbytes);
     {
         dim3 grid((unsigned)cdiv(p, OS_TM), (unsigned)(b.nks / b.ks));
-        os_ximage_kernel<<<grid, 256, 0, st>>>(X, ldx, N, p, b.nks / b.ks, b.ks, img);
+        os_ximage_kernel<T><<<grid, 256, 0, st>>>(X, ldx, N, p, b.nks / b.ks, b.ks, img);
         PLSB_LAUNCH_CHECK("os_ximage_kernel");
     }
     int rc;
@@ -397,6 +401,18 @@ int boot_os_moments(const double* X, int N, int64_t p, int64_t ldx, const double
         PLSB_LAUNCH_CHECK("os_moments_reduce_kernel");
     }
     return PLSB200_OK;
+}
+
+int boot_os_moments(const double* X, int N, int64_t p, int64_t ldx, const double* coef, int K, int R, const double* pivot,
+                    double* sum, double* sumsq, void* workspace, size_t workspace_bytes, cudaStream_t st,
+                    const char* what) {
+    return os_moments(X, N, p, ldx, coef, K, R, pivot, sum, sumsq, workspace, workspace_bytes, st, what);
+}
+
+int boot_os_moments(const float* X, int N, int64_t p, int64_t ldx, const double* coef, int K, int R, const double* pivot,
+                    double* sum, double* sumsq, void* workspace, size_t workspace_bytes, cudaStream_t st,
+                    const char* what) {
+    return os_moments(X, N, p, ldx, coef, K, R, pivot, sum, sumsq, workspace, workspace_bytes, st, what);
 }
 
 }  // namespace plsb

@@ -33,9 +33,11 @@ __global__ void quad_coef_pack_kernel(const double* __restrict__ S, int N, int K
     coef[i] = (row < N && m < N && k < K) ? S[((size_t)k * N + row) * N + m] : 0.0;
 }
 
-template <int NKS, int NBLK>
+// T: element type of X (float: X stored as float32, widened at every load -- the same FP64 operations as on the
+// widened matrix).
+template <typename T, int NKS, int NBLK>
 __global__ void __launch_bounds__(BM_THREADS, 1)
-boot_quad_kernel(const double* __restrict__ X, long long ldx, int N, long long p, const double* __restrict__ coef,
+boot_quad_kernel(const T* __restrict__ X, long long ldx, int N, long long p, const double* __restrict__ coef,
                  int nper, int per_per_split, int nstage, int Kp, int K, double* __restrict__ out) {
     extern __shared__ __align__(128) unsigned char smraw[];
     constexpr int stage_doubles = NKS * NBLK * 32;
@@ -74,7 +76,7 @@ boot_quad_kernel(const double* __restrict__ X, long long ldx, int N, long long p
 #pragma unroll
     for (int s = 0; s < NKS; ++s) {
         const int row = 4 * s + q;
-        a[s] = (row < N && v < p) ? __ldg(X + (long long)row * ldx + v) : 0.0;
+        a[s] = (row < N && v < p) ? (double)__ldg(X + (long long)row * ldx + v) : 0.0;
     }
     const long long vc = v < p ? v : 0;                                // (address of the masked lanes' X loads)
 
@@ -107,7 +109,7 @@ boot_quad_kernel(const double* __restrict__ X, long long ldx, int N, long long p
 #pragma unroll
             for (int e = 0; e < 2; ++e) {
                 const int m = mbase + slot_of[j][e];
-                xm[j][e] = m < N ? __ldg(X + (long long)m * ldx + vc) : 0.0;
+                xm[j][e] = m < N ? (double)__ldg(X + (long long)m * ldx + vc) : 0.0;
             }
         __syncwarp();
         mbar_wait(full + slot, phase);
@@ -166,23 +168,23 @@ __global__ void quad_reduce_kernel(const double* __restrict__ part, int nsplit, 
     q[i] = a;
 }
 
-template <int NKS, int NBLK>
-static int launch_quad(const BootPlan& b, const double* X, int N, int64_t p, int64_t ldx, const double* coef, int K,
+template <typename T, int NKS, int NBLK>
+static int launch_quad(const BootPlan& b, const T* X, int N, int64_t p, int64_t ldx, const double* coef, int K,
                        double* o, cudaStream_t st) {
-    PLSB_CUDA(cudaFuncSetAttribute(boot_quad_kernel<NKS, NBLK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    PLSB_CUDA(cudaFuncSetAttribute(boot_quad_kernel<T, NKS, NBLK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                    (int)b.smem_bytes));
     dim3 grid((unsigned)cdiv(p, BM_VOX), (unsigned)b.nsplit);
-    boot_quad_kernel<NKS, NBLK><<<grid, BM_THREADS, b.smem_bytes, st>>>(X, ldx, N, p, coef, b.nper, b.per_per_split,
+    boot_quad_kernel<T, NKS, NBLK><<<grid, BM_THREADS, b.smem_bytes, st>>>(X, ldx, N, p, coef, b.nper, b.per_per_split,
                                                                        b.nstage, b.Kp, K, o);
     PLSB_LAUNCH_CHECK("boot_quad_kernel");
     return PLSB200_OK;
 }
 
-template <int NBLK>
-static int quad_dispatch_nks(const BootPlan& b, const double* X, int N, int64_t p, int64_t ldx, const double* coef,
+template <typename T, int NBLK>
+static int quad_dispatch_nks(const BootPlan& b, const T* X, int N, int64_t p, int64_t ldx, const double* coef,
                              int K, double* o, cudaStream_t st) {
     switch (b.nks) {
-#define PLSB_CASE(n) case n: return launch_quad<n, NBLK>(b, X, N, p, ldx, coef, K, o, st);
+#define PLSB_CASE(n) case n: return launch_quad<T, n, NBLK>(b, X, N, p, ldx, coef, K, o, st);
         PLSB_CASE(4) PLSB_CASE(8) PLSB_CASE(12) PLSB_CASE(16) PLSB_CASE(20) PLSB_CASE(24) PLSB_CASE(28)
         PLSB_CASE(32) PLSB_CASE(36) PLSB_CASE(40) PLSB_CASE(44) PLSB_CASE(48) PLSB_CASE(52) PLSB_CASE(56)
         PLSB_CASE(60) PLSB_CASE(64) PLSB_CASE(68) PLSB_CASE(72) PLSB_CASE(76) PLSB_CASE(80)
@@ -226,13 +228,14 @@ extern "C" size_t plsb200_boot_quad_f64_workspace(int N, int64_t p, int K) {
     return b.nsplit > 1 ? (size_t)b.nsplit * p * K * sizeof(double) : 16;
 }
 
-extern "C" int plsb200_boot_quad_f64(const double* X, int N, int64_t p, int64_t ldx, const double* coef, int K,
-                                     double* q, void* workspace, size_t workspace_bytes, void* stream) {
-    PLSB_CHECK_ARG(X && coef && q, "boot_quad_f64: null pointer");
-    PLSB_CHECK_ARG(p > 0 && ldx >= p, "boot_quad_f64: bad shape p=%lld ldx=%lld", (long long)p, (long long)ldx);
+template <typename T>
+static int boot_quad(const T* X, int N, int64_t p, int64_t ldx, const double* coef, int K, double* q, void* workspace,
+                     size_t workspace_bytes, void* stream, const char* what) {
+    PLSB_CHECK_ARG(X && coef && q, "%s: null pointer", what);
+    PLSB_CHECK_ARG(p > 0 && ldx >= p, "%s: bad shape p=%lld ldx=%lld", what, (long long)p, (long long)ldx);
     BootPlan b;
     if (!quad_plan(N, K, p, b)) {
-        set_err("boot_quad_f64: unsupported shape N=%d K=%d (need N<=320, K<=24)", N, K);
+        set_err("%s: unsupported shape N=%d K=%d (need N<=320, K<=24)", what, N, K);
         return PLSB200_EUNSUPPORTED;
     }
     cudaStream_t st = (cudaStream_t)stream;
@@ -240,16 +243,16 @@ extern "C" int plsb200_boot_quad_f64(const double* X, int N, int64_t p, int64_t 
     if (b.nsplit > 1) {
         const size_t need = (size_t)b.nsplit * p * K * sizeof(double);
         if (!workspace || workspace_bytes < need) {
-            set_err("boot_quad_f64: workspace %zu < %zu bytes", workspace_bytes, need);
+            set_err("%s: workspace %zu < %zu bytes", what, workspace_bytes, need);
             return PLSB200_EWORKSPACE;
         }
         o = (double*)workspace;
     }
     int rc;
     switch (b.nblk) {
-        case 1: rc = quad_dispatch_nks<1>(b, X, N, p, ldx, coef, K, o, st); break;
-        case 2: rc = quad_dispatch_nks<2>(b, X, N, p, ldx, coef, K, o, st); break;
-        default: rc = quad_dispatch_nks<3>(b, X, N, p, ldx, coef, K, o, st); break;
+        case 1: rc = quad_dispatch_nks<T, 1>(b, X, N, p, ldx, coef, K, o, st); break;
+        case 2: rc = quad_dispatch_nks<T, 2>(b, X, N, p, ldx, coef, K, o, st); break;
+        default: rc = quad_dispatch_nks<T, 3>(b, X, N, p, ldx, coef, K, o, st); break;
     }
     if (rc != PLSB200_OK) return rc;
     if (b.nsplit > 1) {
@@ -258,4 +261,14 @@ extern "C" int plsb200_boot_quad_f64(const double* X, int N, int64_t p, int64_t 
         PLSB_LAUNCH_CHECK("quad_reduce_kernel");
     }
     return PLSB200_OK;
+}
+
+extern "C" int plsb200_boot_quad_f64(const double* X, int N, int64_t p, int64_t ldx, const double* coef, int K,
+                                     double* q, void* workspace, size_t workspace_bytes, void* stream) {
+    return boot_quad(X, N, p, ldx, coef, K, q, workspace, workspace_bytes, stream, "boot_quad_f64");
+}
+
+extern "C" int plsb200_boot_quad_x32_f64(const float* X, int N, int64_t p, int64_t ldx, const double* coef, int K,
+                                         double* q, void* workspace, size_t workspace_bytes, void* stream) {
+    return boot_quad(X, N, p, ldx, coef, K, q, workspace, workspace_bytes, stream, "boot_quad_x32_f64");
 }

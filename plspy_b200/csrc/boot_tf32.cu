@@ -102,8 +102,10 @@ __device__ __forceinline__ void split_tf32(double x, float& hi, float& lo) {
 }
 
 // X (N x p, FP64, row-major) -> image [voxel tile][k-block][hi|lo][128 voxels x 16 rows], each plane in the
-// K-major SWIZZLE_64B order: voxel r, row j -> r*64 + ((j/4) ^ ((r/2)&3))*16 + (j%4)*4 bytes.
-__global__ void __launch_bounds__(TF_MV) split_x_tf32_kernel(const double* __restrict__ X, int N, long long p,
+// K-major SWIZZLE_64B order: voxel r, row j -> r*64 + ((j/4) ^ ((r/2)&3))*16 + (j%4)*4 bytes.  T = float: X stored
+// as float32; its widened value is split, so the planes are those of the widened matrix.
+template <typename T>
+__global__ void __launch_bounds__(TF_MV) split_x_tf32_kernel(const T* __restrict__ X, int N, long long p,
                                                             long long ldx, int nkb, float* __restrict__ img) {
     const int r = threadIdx.x;
     const long long vt = blockIdx.x;
@@ -113,7 +115,7 @@ __global__ void __launch_bounds__(TF_MV) split_x_tf32_kernel(const double* __res
 #pragma unroll
     for (int j = 0; j < TF_KB; ++j) {
         const int row = kb * TF_KB + j;
-        const double x = (row < N && v < p) ? __ldg(X + (long long)row * ldx + v) : 0.0;
+        const double x = (row < N && v < p) ? (double)__ldg(X + (long long)row * ldx + v) : 0.0;
         split_tf32(x, hi[j], lo[j]);
     }
     float* base = img + ((size_t)vt * nkb + kb) * (TF_A_STAGE / 4);
@@ -568,15 +570,24 @@ extern "C" size_t plsb200_tf32_ximage_bytes(int N, int64_t p) {
     return (size_t)(2 * cdiv(cdiv(p, TF_MV), 2)) * (size_t)cdiv(N, TF_KB) * TF_A_STAGE;   // tile count padded to even
 }
 
-extern "C" int plsb200_tf32_split_x(const double* X, int N, int64_t p, int64_t ldx, void* ximage, void* stream) {
+template <typename T>
+static int tf32_split_x(const T* X, int N, int64_t p, int64_t ldx, void* ximage, void* stream) {
     PLSB_CHECK_ARG(X && ximage, "tf32_split_x: null pointer");
     PLSB_CHECK_ARG(N > 0 && p > 0 && ldx >= p, "tf32_split_x: bad shape");
     const int nkb = (int)cdiv(N, TF_KB);
     PLSB_CHECK_ARG(nkb <= 65535, "tf32_split_x: N too large");
     dim3 grid((unsigned)(2 * cdiv(cdiv(p, TF_MV), 2)), (unsigned)nkb);      // padding tile is written as zeros
-    split_x_tf32_kernel<<<grid, TF_MV, 0, (cudaStream_t)stream>>>(X, N, p, ldx, nkb, (float*)ximage);
+    split_x_tf32_kernel<T><<<grid, TF_MV, 0, (cudaStream_t)stream>>>(X, N, p, ldx, nkb, (float*)ximage);
     PLSB_LAUNCH_CHECK("split_x_tf32_kernel");
     return PLSB200_OK;
+}
+
+extern "C" int plsb200_tf32_split_x(const double* X, int N, int64_t p, int64_t ldx, void* ximage, void* stream) {
+    return tf32_split_x(X, N, p, ldx, ximage, stream);
+}
+
+extern "C" int plsb200_tf32_split_x32(const float* X, int N, int64_t p, int64_t ldx, void* ximage, void* stream) {
+    return tf32_split_x(X, N, p, ldx, ximage, stream);
 }
 
 extern "C" size_t plsb200_boot_coef_bytes_tf32(int N, int K, int R) {

@@ -70,7 +70,12 @@ size_t boot_os_workspace(int N, int64_t p, int K, int R);
 int boot_os_pack(const double* E, int N, int K, const int32_t* idx, int R, double* coef, cudaStream_t st);
 int boot_os_moments(const double* X, int N, int64_t p, int64_t ldx, const double* coef, int K, int R,
                     const double* pivot, double* sum, double* sumsq, void* workspace, size_t workspace_bytes,
-                    cudaStream_t st);
+                    cudaStream_t st, const char* what);
+// the same with X stored as float32 (widened as the tile-major FP64 image is built); `what` names the entry point in
+// error messages
+int boot_os_moments(const float* X, int N, int64_t p, int64_t ldx, const double* coef, int K, int R,
+                    const double* pivot, double* sum, double* sumsq, void* workspace, size_t workspace_bytes,
+                    cudaStream_t st, const char* what);
 
 // ---------------------------------------------------------------- device side
 #ifdef __CUDACC__
@@ -229,8 +234,13 @@ __device__ __forceinline__ void cp_async_zfill(void* dst_smem, const void* src_g
         asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;\n" ::"r"(smem_u32(dst_smem)), "l"(src_gmem),
                      "r"(src_bytes)
                      : "memory");
-    } else {
+    } else if constexpr (BYTES == 8) {
         asm volatile("cp.async.ca.shared.global [%0], [%1], 8, %2;\n" ::"r"(smem_u32(dst_smem)), "l"(src_gmem),
+                     "r"(src_bytes)
+                     : "memory");
+    } else {
+        static_assert(BYTES == 4, "cp.async copies 4, 8 or 16 bytes");
+        asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;\n" ::"r"(smem_u32(dst_smem)), "l"(src_gmem),
                      "r"(src_bytes)
                      : "memory");
     }

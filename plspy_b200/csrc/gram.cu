@@ -51,9 +51,12 @@ static GramPlan gram_plan(int N, int64_t p) {
     return g;
 }
 
-template <int VEC>  // doubles per cp.async (2 when rows are 16-B aligned, else 1)
-__global__ void __launch_bounds__(GTHREADS) gram_partial_kernel(const double* __restrict__ X, int N, long long p,
-                                                               long long ldx, const double* __restrict__ X2, int n1,
+// T: element type of X (double, or float widened when the fragments are formed: the same FP64 products in the same
+// order, so the same G as from the widened matrix).  VEC: elements per cp.async (16 bytes when rows are 16-B aligned,
+// else one element).
+template <typename T, int VEC>
+__global__ void __launch_bounds__(GTHREADS) gram_partial_kernel(const T* __restrict__ X, int N, long long p,
+                                                               long long ldx, const T* __restrict__ X2, int n1,
                                                                long long ld2, long long chunk, int ntile,
                                                                double* __restrict__ part) {
     extern __shared__ __align__(16) double sm[];
@@ -72,8 +75,8 @@ __global__ void __launch_bounds__(GTHREADS) gram_partial_kernel(const double* __
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int wi = (warp >> 1) * 32, wj = (warp & 1) * 32;
-    double* As = sm;                            // [GSTAGES][GT][GSTR]
-    double* Bs = sm + GSTAGES * GT * GSTR;      // same shape (unused on diagonal tiles)
+    T* As = reinterpret_cast<T*>(sm);           // [GSTAGES][GT][GSTR]
+    T* Bs = As + GSTAGES * GT * GSTR;           // same shape (unused on diagonal tiles)
 
     // rows [0, n1) live in X, rows [n1, N) in X2 (the Gram matrix of the stack [X; X2] without materialising it;
     // n1 == N: a single matrix)
@@ -87,15 +90,15 @@ __global__ void __launch_bounds__(GTHREADS) gram_partial_kernel(const double* __
             long long left = v1 - v; if (left < 0) left = 0; if (left > VEC) left = VEC;
             {
                 const int row = ti * GT + r;
-                const int nb = row < N ? (int)left * 8 : 0;
-                const double* src = nb ? rowp(row) + v : X;
-                cp_async_zfill<VEC * 8>(As + (st * GT + r) * GSTR + cc, src, nb);
+                const int nb = row < N ? (int)left * (int)sizeof(T) : 0;
+                const T* src = nb ? rowp(row) + v : X;
+                cp_async_zfill<VEC * sizeof(T)>(As + (st * GT + r) * GSTR + cc, src, nb);
             }
             if (!diag) {
                 const int row = tj * GT + r;
-                const int nb = row < N ? (int)left * 8 : 0;
-                const double* src = nb ? rowp(row) + v : X;
-                cp_async_zfill<VEC * 8>(Bs + (st * GT + r) * GSTR + cc, src, nb);
+                const int nb = row < N ? (int)left * (int)sizeof(T) : 0;
+                const T* src = nb ? rowp(row) + v : X;
+                cp_async_zfill<VEC * sizeof(T)>(Bs + (st * GT + r) * GSTR + cc, src, nb);
             }
         }
     };
@@ -121,15 +124,15 @@ __global__ void __launch_bounds__(GTHREADS) gram_partial_kernel(const double* __
             cp_async_commit();
         }
         const int st = kt % GSTAGES;
-        const double* a_base = As + (st * GT + wi + fr) * GSTR + fk;
-        const double* b_base = (diag ? As : Bs) + (st * GT + wj + fr) * GSTR + fk;
+        const T* a_base = As + (st * GT + wi + fr) * GSTR + fk;
+        const T* b_base = (diag ? As : Bs) + (st * GT + wj + fr) * GSTR + fk;
 #pragma unroll
         for (int ks = 0; ks < GKC / 4; ++ks) {
             double af[4], bf[4];
 #pragma unroll
             for (int t = 0; t < 4; ++t) {
-                af[t] = a_base[t * 8 * GSTR + ks * 4];
-                bf[t] = b_base[t * 8 * GSTR + ks * 4];
+                af[t] = (double)a_base[t * 8 * GSTR + ks * 4];
+                bf[t] = (double)b_base[t * 8 * GSTR + ks * 4];
             }
 #pragma unroll
             for (int a = 0; a < 4; ++a)
@@ -177,7 +180,8 @@ extern "C" size_t plsb200_gram_f64_workspace(int N, int64_t p) {
     return (size_t)g.nsplit * g.npair * GT * GT * sizeof(double);
 }
 
-static int gram_launch(const double* X, int n1, int64_t ldx, const double* X2, int n2, int64_t ld2, int64_t p, double* G,
+template <typename T>
+static int gram_launch(const T* X, int n1, int64_t ldx, const T* X2, int n2, int64_t ld2, int64_t p, double* G,
                        void* workspace, size_t workspace_bytes, void* stream, const char* what) {
     const int N = n1 + n2;
     GramPlan g = gram_plan(N, p);
@@ -187,16 +191,17 @@ static int gram_launch(const double* X, int n1, int64_t ldx, const double* X2, i
         return PLSB200_EWORKSPACE;
     }
     cudaStream_t st = (cudaStream_t)stream;
-    const size_t smem = (size_t)2 * GSTAGES * GT * GSTR * sizeof(double);
-    const bool vec2 = ((reinterpret_cast<uintptr_t>(X) & 15) == 0) && (ldx % 2 == 0) &&
-                      (n2 == 0 || (((reinterpret_cast<uintptr_t>(X2) & 15) == 0) && (ld2 % 2 == 0)));
+    const size_t smem = (size_t)2 * GSTAGES * GT * GSTR * sizeof(T);
+    constexpr int V = 16 / (int)sizeof(T);      // elements of a 16-byte copy
+    const bool vec = ((reinterpret_cast<uintptr_t>(X) & 15) == 0) && (ldx % V == 0) &&
+                     (n2 == 0 || (((reinterpret_cast<uintptr_t>(X2) & 15) == 0) && (ld2 % V == 0)));
     dim3 grid(g.npair, g.nsplit);
-    if (vec2) {
-        PLSB_CUDA(cudaFuncSetAttribute(gram_partial_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        gram_partial_kernel<2><<<grid, GTHREADS, smem, st>>>(X, N, p, ldx, X2, n1, ld2, g.chunk, g.ntile, (double*)workspace);
+    if (vec) {
+        PLSB_CUDA(cudaFuncSetAttribute(gram_partial_kernel<T, V>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        gram_partial_kernel<T, V><<<grid, GTHREADS, smem, st>>>(X, N, p, ldx, X2, n1, ld2, g.chunk, g.ntile, (double*)workspace);
     } else {
-        PLSB_CUDA(cudaFuncSetAttribute(gram_partial_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        gram_partial_kernel<1><<<grid, GTHREADS, smem, st>>>(X, N, p, ldx, X2, n1, ld2, g.chunk, g.ntile, (double*)workspace);
+        PLSB_CUDA(cudaFuncSetAttribute(gram_partial_kernel<T, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        gram_partial_kernel<T, 1><<<grid, GTHREADS, smem, st>>>(X, N, p, ldx, X2, n1, ld2, g.chunk, g.ntile, (double*)workspace);
     }
     PLSB_LAUNCH_CHECK("gram_partial_kernel");
     gram_reduce_kernel<<<g.npair, 256, 0, st>>>((const double*)workspace, g.npair, g.nsplit, g.ntile, N, G);
@@ -209,12 +214,21 @@ extern "C" int plsb200_gram_f64(const double* X, int N, int64_t p, int64_t ldx, 
     PLSB_CHECK_ARG(X && G && workspace, "gram_f64: null pointer");
     PLSB_CHECK_ARG(N > 0 && p > 0 && ldx >= p, "gram_f64: bad shape N=%d p=%lld ldx=%lld", N, (long long)p,
                    (long long)ldx);
-    return gram_launch(X, N, ldx, nullptr, 0, 0, p, G, workspace, workspace_bytes, stream, "gram_f64");
+    return gram_launch<double>(X, N, ldx, nullptr, 0, 0, p, G, workspace, workspace_bytes, stream, "gram_f64");
+}
+
+// X stored as float32: the same partial sums as plsb200_gram_f64 on the widened matrix (workspace: gram_f64_workspace)
+extern "C" int plsb200_gram_x32_f64(const float* X, int N, int64_t p, int64_t ldx, double* G, void* workspace,
+                                    size_t workspace_bytes, void* stream) {
+    PLSB_CHECK_ARG(X && G && workspace, "gram_x32_f64: null pointer");
+    PLSB_CHECK_ARG(N > 0 && p > 0 && ldx >= p, "gram_x32_f64: bad shape N=%d p=%lld ldx=%lld", N, (long long)p,
+                   (long long)ldx);
+    return gram_launch<float>(X, N, ldx, nullptr, 0, 0, p, G, workspace, workspace_bytes, stream, "gram_x32_f64");
 }
 
 extern "C" int plsb200_gram_stacked_f64(const double* X1, int N1, int64_t ld1, const double* X2, int N2, int64_t ld2,
                                         int64_t p, double* G, void* workspace, size_t workspace_bytes, void* stream) {
     PLSB_CHECK_ARG(X1 && X2 && G && workspace, "gram_stacked_f64: null pointer");
     PLSB_CHECK_ARG(N1 > 0 && N2 > 0 && p > 0 && ld1 >= p && ld2 >= p, "gram_stacked_f64: bad shape");
-    return gram_launch(X1, N1, ld1, X2, N2, ld2, p, G, workspace, workspace_bytes, stream, "gram_stacked_f64");
+    return gram_launch<double>(X1, N1, ld1, X2, N2, ld2, p, G, workspace, workspace_bytes, stream, "gram_stacked_f64");
 }

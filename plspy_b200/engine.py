@@ -14,6 +14,7 @@ from . import _lib
 from ._lib import lib, check
 
 F64 = torch.float64
+F32 = torch.float32
 I32 = torch.int32
 
 
@@ -26,26 +27,37 @@ def _require_cuda():
 
 
 class Engine:
-    """Holds X (N x p, float64) on one GPU together with its Gram matrix and runs the batched kernels.
+    """Holds X (N x p, float64, or float32 with x_storage="fp32") on one GPU together with its Gram matrix and runs the batched kernels.
 
     Replaces, for one analysis, the per-iteration bodies of `_permutation_test` / `_bootstrap_test`
     (plspy/core/bootstrap_permutation.py:323-452, 537-675).
     """
 
     PRECISIONS = ("fp64", "tf32x3", "tf32x3+gram")
+    X_STORAGES = ("fp64", "fp32")
     GRAM_TF32_MAX_ROWS = 320
 
-    def __init__(self, X, device=None, precision="fp64"):
+    def __init__(self, X, device=None, precision="fp64", x_storage="fp64"):
         """precision: "fp64" (exact mode, FP64 DMMA) or "tf32x3" (fast mode: the bootstrap moment GEMM runs on the
         tcgen05 tensor cores with the 3xTF32 split; every N-space quantity -- Gram matrix, permutation p-values,
         Tdistrib, U_hat -- stays FP64) or "tf32x3+gram" (fast mode whose Gram matrix G = X X^T is ALSO formed on the
         tcgen05 tensor cores with the 3xTF32 split: permuted singular values then carry
         a relative error of ~1e-6 instead of being exact, inside the fast mode's tolerance of 1e-5, and a permutation
         p-value can differ by one count where a permuted value ties with the observed one at that level; designs
-        beyond 320 rows keep the exact Gram kernel)."""
+        beyond 320 rows keep the exact Gram kernel).
+
+        x_storage: "fp64" (default) holds X as float64; "fp32" holds `X.astype(float32)` (a float32 input as it is, a
+        float64 one rounded once) and never allocates a float64 copy of X: the task-method kernels widen each element
+        where they load it, so every result equals, bit for bit, the "fp64" result for the widened float32 matrix.
+        Half the device memory and half the HBM traffic of every pass over X.  The behaviour / multiblock kernels
+        (cell_standardize, rb_boot, half_gram, gram_stacked) take float64 operands only."""
         _require_cuda()
         if precision not in self.PRECISIONS:
             raise ValueError(f"precision must be one of {self.PRECISIONS}")
+        if x_storage not in self.X_STORAGES:
+            raise ValueError(f"x_storage must be one of {self.X_STORAGES}, got {x_storage!r}")
+        self.x_storage = x_storage
+        self._xdt = F32 if x_storage == "fp32" else F64
         self.gram_tf32 = precision == "tf32x3+gram"
         self.precision = "tf32x3" if self.gram_tf32 else precision
         self._tf32_ranges = None
@@ -60,7 +72,22 @@ class Engine:
         self._G = None
         self.kernel_events = None     # set to {} to record CUDA events around named kernels (bench.py)
         self.on_mark = None           # optional callable(name) invoked at every _mark (bench.py: clock sampling)
-        self.h2d_bytes = 0 if (torch.is_tensor(X) and X.is_cuda) else self._X.numel() * 8
+        self.h2d_bytes = 0 if (torch.is_tensor(X) and X.is_cuda) else self._X.numel() * self._X.element_size()
+
+    def _xp(self, v0=0):
+        """Address of column v0 of the device copy of X (float32 or float64 elements)."""
+        return self._X.data_ptr() + self._X.element_size() * v0
+
+    @staticmethod
+    def _x32(M):
+        return M.dtype == F32
+
+    @staticmethod
+    def _need_f64(M, what):
+        """The behaviour / multiblock kernels read float64 operands only (x_storage="fp32" is for mct / cst)."""
+        if M is not None and M.dtype != F64:
+            raise _lib.PlsB200Error(f"{what}: needs a float64 data matrix, got {M.dtype} (x_storage='fp32' applies to "
+                                    "the task methods mct and cst)")
 
     # ------------------------------------------------------------------ plumbing
     PIPELINED_UPLOAD_MIN_BYTES = 64 << 20
@@ -97,7 +124,7 @@ class Engine:
         n, p = int(Xh.shape[0]), int(Xh.shape[1])
         self._x_host = Xh            # keep the pinned source alive until the copies have been consumed
         self._pending = []           # empty list = upload not started yet
-        return torch.empty((n, p), dtype=F64, device=self.device)
+        return torch.empty((n, p), dtype=Xh.dtype, device=self.device)
 
     def _start_upload(self):
         if self._pending is None or len(self._pending) > 0:
@@ -121,11 +148,12 @@ class Engine:
             step = -(-(-(-p // 4)) // 256) * 256          # whole pairs of 128-voxel tiles
             bounds = list(range(0, p, step)) + [p]
         pend = []
+        es = Xd.element_size()
         with torch.cuda.device(self.device):
             for v0, v1 in zip(bounds[:-1], bounds[1:]):
                 # (torch's copy_ of a column block goes through a contiguous temporary and synchronises)
-                check(lib.plsb200_copy2d_h2d(Xd.data_ptr() + 8 * v0, 8 * p, Xh.data_ptr() + 8 * v0, 8 * p,
-                                             8 * (v1 - v0), n, side.cuda_stream), "copy2d_h2d")
+                check(lib.plsb200_copy2d_h2d(Xd.data_ptr() + es * v0, es * p, Xh.data_ptr() + es * v0, es * p,
+                                             es * (v1 - v0), n, side.cuda_stream), "copy2d_h2d")
                 ev = torch.cuda.Event()
                 ev.record(side)
                 pend.append((v0, v1, ev))
@@ -139,7 +167,8 @@ class Engine:
         time took 17 ms each, a share plus the all-gather takes 2."""
         from . import dist
         size = dist.world()[1]
-        if torch.is_tensor(X) and X.dtype == torch.float32 and X.dim() == 2:
+        dt = self._xdt
+        if dt == F64 and torch.is_tensor(X) and X.dtype == torch.float32 and X.dim() == 2:
             # float32 storage (plspy_b200/io.py): half the bytes over PCIe, widened on the device
             x32 = X.to(self.device, non_blocking=True).contiguous()
             out = torch.empty(x32.shape, dtype=F64, device=self.device)
@@ -148,19 +177,20 @@ class Engine:
                       "widen_f32_f64")
             return out
         on_host = not (torch.is_tensor(X) and X.is_cuda)
-        if (size == 1 and on_host and torch.is_tensor(X) and X.dim() == 2 and X.dtype == F64 and X.is_pinned()
-                and X.is_contiguous() and X.numel() * 8 >= self.PIPELINED_UPLOAD_MIN_BYTES):
+        if (size == 1 and on_host and torch.is_tensor(X) and X.dim() == 2 and X.dtype == dt and X.is_pinned()
+                and X.is_contiguous() and X.numel() * X.element_size() >= self.PIPELINED_UPLOAD_MIN_BYTES):
             return self._upload_pipelined(X)
-        if (size == 1 and on_host and len(X.shape) == 2 and not torch.is_tensor(X) and X.dtype == np.float64
-                and X.flags.c_contiguous and X.nbytes >= self.PIPELINED_UPLOAD_MIN_BYTES and self.PAGEABLE_UPLOAD_THREADS > 1):
+        if (size == 1 and on_host and len(X.shape) == 2 and not torch.is_tensor(X)
+                and X.dtype == (np.float64 if dt == F64 else np.float32) and X.flags.c_contiguous
+                and X.nbytes >= self.PIPELINED_UPLOAD_MIN_BYTES and self.PAGEABLE_UPLOAD_THREADS > 1):
             return self._upload_pageable(X)
         if size == 1 or not on_host or len(X.shape) != 2:
-            return self.to_device(X, F64)
+            return self.to_device(X, dt)
         n = int(X.shape[0])
         lo, hi = dist.shard(n)
-        part = self.to_device(X[lo:hi], F64)
+        part = self.to_device(X[lo:hi], dt)
         if part.shape[0] == 0:
-            part = torch.zeros((0, int(X.shape[1])), dtype=F64, device=self.device)
+            part = torch.zeros((0, int(X.shape[1])), dtype=dt, device=self.device)
         return dist.gather_rows(part, n, lo).contiguous()
 
     PAGEABLE_UPLOAD_THREADS = int(os.environ.get("PLSB200_UPLOAD_THREADS", str(max(1, min(8, (os.cpu_count() or 2) // 2)))))
@@ -182,12 +212,13 @@ class Engine:
     def _upload_pageable_locked(self, X):
         import concurrent.futures
         n, p = int(X.shape[0]), int(X.shape[1])
-        out = torch.empty((n, p), dtype=F64, device=self.device)
+        dt = self._xdt
+        out = torch.empty((n, p), dtype=dt, device=self.device)
         nt = max(1, self.PAGEABLE_UPLOAD_THREADS)
-        rows = max(1, self.STAGING_BLOCK_BYTES // (8 * p))
-        bufs = Engine._staging.get("bufs")
-        if bufs is None or bufs[0].numel() < rows * p:            # one pair per process, grown when a row is longer
-            bufs = Engine._staging["bufs"] = [torch.empty(rows * p, dtype=F64).pin_memory() for _ in range(2)]
+        rows = max(1, self.STAGING_BLOCK_BYTES // (X.itemsize * p))
+        bufs = Engine._staging.get(dt)
+        if bufs is None or bufs[0].numel() < rows * p:            # one pair per process and dtype, grown when a row is longer
+            bufs = Engine._staging[dt] = [torch.empty(rows * p, dtype=dt).pin_memory() for _ in range(2)]
         side = getattr(self, "_copy_stream", None)
         if side is None:
             side = self._copy_stream = torch.cuda.Stream(device=self.device)
@@ -295,17 +326,18 @@ class Engine:
     def gram_of(self, M):
         """K1: M M^T for a device matrix M (rows x p)."""
         n, p, ld = int(M.shape[0]), int(M.shape[1]), int(M.stride(0))
+        fn, what = (lib.plsb200_gram_x32_f64, "gram_x32_f64") if self._x32(M) else (lib.plsb200_gram_f64, "gram_f64")
         with torch.cuda.device(self.device):
             ws = self._ws(lib.plsb200_gram_f64_workspace(n, p))
             G = self._empty(n, n)
-            check(lib.plsb200_gram_f64(self._p(M), n, p, ld, self._p(G), self._p(ws), ws.numel(), self._stream()),
-                  "gram_f64")
+            check(fn(self._p(M), n, p, ld, self._p(G), self._p(ws), ws.numel(), self._stream()), what)
         return G
 
     def gram_stacked(self, M1, M2):
         """Gram matrix of the row stack [M1; M2] ((n1 + n2) x p) without building it (multiblock: [X; Zb])."""
         n1, n2, p = int(M1.shape[0]), int(M2.shape[0]), int(M1.shape[1])
         assert int(M2.shape[1]) == p
+        self._need_f64(M1, "gram_stacked"); self._need_f64(M2, "gram_stacked")
         with torch.cuda.device(self.device):
             ws = self._ws(lib.plsb200_gram_f64_workspace(n1 + n2, p))
             G = self._empty(n1 + n2, n1 + n2)
@@ -336,6 +368,7 @@ class Engine:
         into the Gram kernel's operand image, then its partial Gram, accumulated in a fixed order)."""
         G = self._empty(self.N, self.N)
         cur = torch.cuda.current_stream(self.device)
+        split = lib.plsb200_gram_tf32_split_x32 if self._x32(self._X) else lib.plsb200_gram_tf32_split
         with torch.cuda.device(self.device):
             for i, (v0, v1, ev) in enumerate(self._x_ranges() if ranges is None else ranges):
                 if ev is not None:
@@ -345,8 +378,7 @@ class Engine:
                 nb = lib.plsb200_gram_tf32_workspace(self.N, pc)
                 ws = self._ws(nb)
                 self._mark("gram_tf32")
-                check(lib.plsb200_gram_tf32_split(self._X.data_ptr() + 8 * v0, self.N, pc, self.ldx, self._p(img),
-                                                  self._stream()), "gram_tf32_split")
+                check(split(self._xp(v0), self.N, pc, self.ldx, self._p(img), self._stream()), "gram_tf32_split")
                 check(lib.plsb200_gram_tf32(self._p(img), self.N, pc, self._p(G), 1 if i else 0, self._p(ws), nb,
                                             self._stream()), "gram_tf32")
                 self._mark("gram_tf32")
@@ -375,11 +407,13 @@ class Engine:
         """XL = X @ V (N x K)."""
         V = self.to_device(V, F64)
         K = int(V.shape[1])
+        X = self.X
+        fn, what = (lib.plsb200_xv_x32_f64, "xv_x32_f64") if self._x32(X) else (lib.plsb200_xv_f64, "xv_f64")
         with torch.cuda.device(self.device):
             ws = self._ws(lib.plsb200_xv_f64_workspace(self.N, self.p, K))
             out = self._empty(self.N, K)
-            check(lib.plsb200_xv_f64(self._p(self.X), self.N, self.p, self.ldx, self._p(V), K, self._p(out),
-                                     self._p(ws), ws.numel(), self._stream()), "xv_f64")
+            check(fn(self._p(X), self.N, self.p, self.ldx, self._p(V), K, self._p(out), self._p(ws), ws.numel(),
+                     self._stream()), what)
         return out
 
     def nspace_coef(self, G, C, Lmat=None):
@@ -538,8 +572,8 @@ class Engine:
                 torch.cuda.current_stream(self.device).wait_event(ev)
             with torch.cuda.device(self.device):
                 img = self._ws(lib.plsb200_tf32_ximage_bytes(self.N, v1 - v0))
-                check(lib.plsb200_tf32_split_x(self._X.data_ptr() + 8 * v0, self.N, v1 - v0, self.ldx,
-                                               self._p(img), self._stream()), "tf32_split_x")
+                split = lib.plsb200_tf32_split_x32 if self._x32(self._X) else lib.plsb200_tf32_split_x
+                check(split(self._xp(v0), self.N, v1 - v0, self.ldx, self._p(img), self._stream()), "tf32_split_x")
             self._ximage[i] = (v0, v1, img)
         return self._ximage[i][2]
 
@@ -594,16 +628,18 @@ class Engine:
             coef = packed["coef"]
             s1 = self._empty(self.p, K); s2 = self._empty(self.p, K)
             cur = torch.cuda.current_stream(self.device)
+            fn, what = ((lib.plsb200_boot_moments_x32_f64, "boot_moments_x32_f64") if self._x32(self._X)
+                        else (lib.plsb200_boot_moments_f64, "boot_moments_f64"))
             for v0, v1, ev in self._x_ranges():          # one launch per voxel range still arriving, else one in all
                 if ev is not None:
                     cur.wait_event(ev)
                 pc = v1 - v0
                 ws = self._ws(lib.plsb200_boot_moments_f64_workspace(self.N, pc, K, R))
                 self._mark("boot_moments")
-                check(lib.plsb200_boot_moments_f64(self._X.data_ptr() + 8 * v0, self.N, pc, self.ldx, self._p(coef),
-                                                   K, R, None if pivot is None else pivot.data_ptr() + 8 * v0 * K,
-                                                   s1.data_ptr() + 8 * v0 * K, s2.data_ptr() + 8 * v0 * K,
-                                                   self._p(ws), ws.numel(), self._stream()), "boot_moments_f64")
+                check(fn(self._xp(v0), self.N, pc, self.ldx, self._p(coef), K, R,
+                         None if pivot is None else pivot.data_ptr() + 8 * v0 * K,
+                         s1.data_ptr() + 8 * v0 * K, s2.data_ptr() + 8 * v0 * K,
+                         self._p(ws), ws.numel(), self._stream()), what)
                 self._mark("boot_moments")
         return s1, s2
 
@@ -655,6 +691,8 @@ class Engine:
             check(lib.plsb200_boot_quad_coef_pack_f64(self._p(Sig), N, K, self._p(coef), self._stream()),
                   "boot_quad_coef_pack_f64")
             cur = torch.cuda.current_stream(self.device)
+            fn, what = ((lib.plsb200_boot_quad_x32_f64, "boot_quad_x32_f64") if self._x32(self._X)
+                        else (lib.plsb200_boot_quad_f64, "boot_quad_f64"))
             for a, b, ev in self._x_ranges():
                 lo, hi = max(a, v0), min(b, v1)
                 if lo >= hi:
@@ -663,9 +701,8 @@ class Engine:
                     cur.wait_event(ev)
                 ws = self._ws(lib.plsb200_boot_quad_f64_workspace(N, hi - lo, K))
                 self._mark("boot_quad")
-                check(lib.plsb200_boot_quad_f64(self._X.data_ptr() + 8 * lo, N, hi - lo, self.ldx, self._p(coef), K,
-                                                q.data_ptr() + 8 * (lo - v0) * K, self._p(ws), ws.numel(),
-                                                self._stream()), "boot_quad_f64")
+                check(fn(self._xp(lo), N, hi - lo, self.ldx, self._p(coef), K, q.data_ptr() + 8 * (lo - v0) * K,
+                         self._p(ws), ws.numel(), self._stream()), what)
                 self._mark("boot_quad")
         return q
 
@@ -711,6 +748,7 @@ class Engine:
         lo = self._empty(self.p, K); hi = self._empty(self.p, K)
         vc = max(128, min(self.p, int(max_bytes // (R * K * 8)) // 128 * 128))
         X = self.X
+        series = lib.plsb200_salience_series_x32_f64 if self._x32(X) else lib.plsb200_salience_series_f64
         nb = lib.plsb200_percentile_f64_workspace(R)
         with torch.cuda.device(self.device):
             ws = self._ws(nb)
@@ -719,8 +757,8 @@ class Engine:
                 # series-major chunk [voxel][k][resample]: the sort reads every series as one contiguous run (the
                 # resample-major cube read in place with a stride of the chunk size cost 23-41 ms per chunk against 17)
                 cube = self._empty(v1 - v0, K, R)
-                check(lib.plsb200_salience_series_f64(X.data_ptr() + 8 * v0, self.N, v1 - v0, self.ldx, self._p(E), K,
-                                                      self._p(idx), R, self._p(cube), self._stream()), "salience_series_f64")
+                check(series(self._xp(v0), self.N, v1 - v0, self.ldx, self._p(E), K, self._p(idx), R, self._p(cube),
+                             self._stream()), "salience_series_f64")
                 check(lib.plsb200_percentile_f64(self._p(cube), R, (v1 - v0) * K, 1, R, float(conf[0]), float(conf[1]),
                                                  lo.data_ptr() + 8 * v0 * K, hi.data_ptr() + 8 * v0 * K, self._p(ws), nb,
                                                  self._stream()), "percentile_f64")
@@ -734,9 +772,9 @@ class Engine:
         n, p, ld = int(M.shape[0]), int(M.shape[1]), int(M.stride(0))
         R, K = int(idx.shape[0]), int(E.shape[1])
         out = self._empty(R, p, K)
+        fn = lib.plsb200_salience_x32_f64 if self._x32(M) else lib.plsb200_salience_f64
         with torch.cuda.device(self.device):
-            check(lib.plsb200_salience_f64(self._p(M), n, p, ld, self._p(E), K, self._p(idx), R,
-                                           self._p(out), self._stream()), "salience_f64")
+            check(fn(self._p(M), n, p, ld, self._p(E), K, self._p(idx), R, self._p(out), self._stream()), "salience_f64")
         return out
 
     # ------------------------------------------------------------------ split-half (K3)
@@ -794,6 +832,7 @@ class Engine:
         """Xc = M - block means, Z = block z-score(M) / sqrt(n) (both rows x p, dense); M defaults to X."""
         cs = self.to_device(np.asarray(cell_start, dtype=np.int32), I32)
         M = self.X if M is None else M
+        self._need_f64(M, "cell_standardize")
         n, p, ld = int(M.shape[0]), int(M.shape[1]), int(M.stride(0))
         Xc = self._empty(n, p)
         Z = self._empty(n, p) if want_z else None
@@ -830,6 +869,7 @@ class Engine:
         Runs on the FP64 tensor path (plsb200_rb_boot_dmma_f64) when the design fits its register-resident
         fragments, else on the general FMA kernel.  `X2`: the data matrix is the row stack [Xc; X2] (not built: the
         kernels take the two row segments; multiblock bootstraps pass [Xcb; X])."""
+        self._need_f64(Xc, "rb_boot"); self._need_f64(X2, "rb_boot")
         cs_host = np.ascontiguousarray(np.asarray(cell_start, dtype=np.int32))
         R, N, K = int(Q.shape[0]), int(Q.shape[1]), int(Q.shape[2])
         p = int(Xc.shape[1])
@@ -906,6 +946,7 @@ class Engine:
         The windowed kernel (half_gram.cu, DMMA Gram) is used: the non-zero column window of every block is read
         off Q (blocks wider than 8 columns become several segments); `dense=True` forces the older FMA kernel of
         rb.cu (K <= 24), kept as the in-library cross-check."""
+        self._need_f64(Xstd, "half_gram"); self._need_f64(Xlin, "half_gram")
         ids = self.to_device(ids, I32); Q = self.to_device(Q, F64)
         cells_h = np.asarray(cells.cpu() if torch.is_tensor(cells) else cells, dtype=np.int32)
         S, nmax, K = int(ids.shape[0]), int(ids.shape[2]), int(Q.shape[3])

@@ -25,7 +25,10 @@ def PLS(*args, **kwargs):
     variable fixed by convention -- see device_analysis.py), `boot_algo` ("direct" = the bootstrap moments of the
     B x p x K salience GEMM, default; "collapsed" = mct / cst with precision="fp64" and at most 320 rows: the same exact
     standard errors from K covariance matrices of N x N and one p x K quadratic form, about N / B of the direct
-    form's flops, so faster when num_boot > N -- see bootstrap_permutation.check_boot_algo).
+    form's flops, so faster when num_boot > N -- see bootstrap_permutation.check_boot_algo), `x_storage` ("fp64" =
+    X held as float64 on the device, default; "fp32" = mct / cst: X.astype(float32) held as float32 -- half the device
+    memory -- with every result bit-identical to the "fp64" run on the widened float32 matrix; the host-side steps see
+    the same widened values -- see bootstrap_permutation.check_x_storage).
     """
     pls_method = kwargs.pop("pls_method", "mct")
     kwargs["pls_alg"] = pls_method
@@ -50,4 +53,6 @@ def PLS(*args, **kwargs):
         bootstrap_permutation.check_boot_algo(
             kwargs["boot_algo"], pls_method, engine.precision if engine is not None else kwargs.get("precision", "fp64"),
             engine.N if engine is not None else (int(X.shape[0]) if X is not None and hasattr(X, "shape") else None))
+    if "x_storage" in kwargs:
+        bootstrap_permutation.check_x_storage(kwargs["x_storage"], pls_method)
     return pls_classes.PLSBase._create(pls_method, *args, **kwargs)

@@ -46,7 +46,7 @@ class PLSBase(abc.ABC):
 
     # ---- shared helpers -------------------------------------------------------------------
     _ENGINE_KWARGS = ("perm_indices", "boot_indices", "engine", "device", "precision", "rotate_method", "analysis",
-                      "boot_algo")
+                      "boot_algo", "x_storage")
 
     def _take_kwargs(self, kwargs):
         self.pls_alg = kwargs["pls_alg"]
@@ -58,6 +58,13 @@ class PLSBase(abc.ABC):
                 continue
             setattr(self, k, v)
             self._user_defined_attrs.add(k)
+        # storage of X on the device: the option, else that of a given engine (before any GPU work)
+        eng = self._engine_kwargs.get("engine")
+        xs = self._engine_kwargs.get("x_storage", eng.x_storage if eng is not None else "fp64")
+        if eng is not None and eng.x_storage != xs:
+            raise ValueError(f"x_storage={xs!r} but the engine holds X as {eng.x_storage!r}")
+        bootstrap_permutation.check_x_storage(xs, self.pls_alg)
+        self._engine_kwargs["x_storage"] = xs
 
     @staticmethod
     def _get_groups_info(groups_tuple):
@@ -84,9 +91,18 @@ class PLSBase(abc.ABC):
         if hasattr(X, "is_pinned") and hasattr(X, "numpy") and not X.is_cuda:
             # a host tensor from plspy_b200.io.assemble_pinned: the engine uploads the (pinned) tensor itself, the
             # host-side code works on its numpy view (float32 storage: a widened copy, meant for analysis="device")
+            if self._engine_kwargs["x_storage"] == "fp32" and X.element_size() != 4:
+                X = X.float()                                     # rounded once
             if self._engine_kwargs.get("engine") is None:
                 self._x_tensor = X
             X = X.numpy() if X.dtype.is_floating_point and X.element_size() == 8 else X.numpy().astype(np.float64)
+        elif self._engine_kwargs["x_storage"] == "fp32":
+            # x_storage="fp32": the analysis is that of X.astype(float32).  The engine uploads the float32 matrix (a
+            # float32 input as it is); the host-side steps work on its values widened to float64, as the kernels do
+            x32 = np.ascontiguousarray(X, dtype=np.float32)
+            if self._engine_kwargs.get("engine") is None:
+                self._x_tensor = x32
+            X = x32.astype(np.float64)
         self.X = X
         if need_y:
             self.Y = Y
@@ -162,7 +178,8 @@ class PLSBase(abc.ABC):
         def work():
             out = {}
             if want_eng:
-                out["engine"] = Engine(xsrc, device=device, precision=ek.get("precision", "fp64"))
+                out["engine"] = Engine(xsrc, device=device, precision=ek.get("precision", "fp64"),
+                                       x_storage=ek["x_storage"])
             if want_idx:
                 if self.num_perm > 0:
                     out["perm_indices"] = resample.permutation_indices(self.pls_alg, self.num_perm, self.cond_order, Y=Y,
@@ -196,7 +213,8 @@ class PLSBase(abc.ABC):
             from .engine import Engine
             self._engine_kwargs["engine"] = Engine(getattr(self, "_x_tensor", None) if getattr(self, "_x_tensor", None)
                                                    is not None else self.X, device=self._engine_kwargs.get("device"),
-                                                   precision=self._engine_kwargs.get("precision", "fp64"))
+                                                   precision=self._engine_kwargs.get("precision", "fp64"),
+                                                   x_storage=self._engine_kwargs["x_storage"])
         return True
 
     def _resample(self, Y, mctype, preprocess, **kw):
@@ -206,7 +224,8 @@ class PLSBase(abc.ABC):
         if xt is not None and self._engine_kwargs.get("engine") is None and (self.num_perm > 0 or self.num_boot > 0):
             from .engine import Engine
             self._engine_kwargs["engine"] = Engine(xt, device=self._engine_kwargs.get("device"),
-                                                   precision=self._engine_kwargs.get("precision", "fp64"))
+                                                   precision=self._engine_kwargs.get("precision", "fp64"),
+                                                   x_storage=self._engine_kwargs["x_storage"])
         self.resample_tests = bootstrap_permutation.ResampleTest._create(
             self.pls_alg, self.X, Y, self.U, self.s, self.V if V is None else V, self.cond_order, mctype, preprocess=preprocess,
             nperm=self.num_perm, nboot=self.num_boot, CI=self.CI,
@@ -214,7 +233,7 @@ class PLSBase(abc.ABC):
             boot_indices=self._engine_kwargs.get("boot_indices"),
             engine=self._engine_kwargs.get("engine"), precision=self._engine_kwargs.get("precision", "fp64"),
             rotate_method=self._engine_kwargs.get("rotate_method", 2), device=self._engine_kwargs.get("device"),
-            boot_algo=self._engine_kwargs.get("boot_algo", "direct"), **kw)
+            boot_algo=self._engine_kwargs.get("boot_algo", "direct"), x_storage=self._engine_kwargs["x_storage"], **kw)
 
     def _split_half(self, Y, mctype, contrasts, **kw):
         """pls_classes.py:285-318 (identical block in every class)."""
@@ -227,6 +246,11 @@ class PLSBase(abc.ABC):
                           f"Using lv={max_lv} instead.")
                     self.lv = max_lv
                 eng = getattr(self.resample_tests, "_engine", None) or self._engine_kwargs.get("engine")
+                if eng is None and self._engine_kwargs["x_storage"] == "fp32":
+                    # no resampling engine: the split-half functions would each upload the widened host copy as
+                    # float64; one engine holding the float32 matrix (exact mode, as theirs) serves both instead
+                    from .engine import Engine
+                    eng = Engine(self._x_tensor, device=self._engine_kwargs.get("device"), x_storage="fp32")
                 self.pls_repro_tt = split_half_resampling.split_half_test_train(
                     self.pls_alg, self.X, Y, self.cond_order, num_split=self.num_split, mctype=mctype,
                     contrasts=contrasts, engine=eng, **kw)

@@ -29,7 +29,7 @@ from .engine import Engine
 METHODS = ("mct", "rb", "cst", "csb", "mb", "cmb")
 
 _state = None          # what install() replaced, for uninstall()
-_options = {"precision": "fp64", "boot_algo": "direct"}
+_options = {"precision": "fp64", "boot_algo": "direct", "x_storage": "fp64"}
 _shared = {"ref": None, "engine": None}
 
 
@@ -44,7 +44,7 @@ def shared_engine(X):
     ref = _shared["ref"]
     if ref is not None and ref() is X and _shared["engine"] is not None:
         return _shared["engine"]
-    eng = Engine(X, precision=_options["precision"])
+    eng = Engine(X, precision=_options["precision"], x_storage=_options["x_storage"])
     try:
         _shared["ref"] = weakref.ref(X, _drop_engine)
     except TypeError:           # not weak-referenceable (a torch tensor is; a list is not): do not cache
@@ -60,6 +60,8 @@ class _InstalledResampleTest(_bp._ResampleTestPLS):
     def __init__(self, X, Y, U, s, V, cond_order, mctype, *args, **kwargs):
         nperm = kwargs.get("nperm", 1000)
         nboot = kwargs.get("nboot", 1000)
+        kwargs.setdefault("x_storage", _options["x_storage"])
+        _bp.check_x_storage(kwargs["x_storage"], self.pls_alg)        # before the engine uploads X
         if "engine" not in kwargs and (nperm > 0 or nboot > 0):
             kwargs["engine"] = shared_engine(X)
         kwargs.setdefault("precision", _options["precision"])
@@ -88,11 +90,14 @@ def _split_half(pls_alg, matrix, Y, cond_order, num_split, mctype=None, contrast
                           Xbscan=Xbscan, Ybscan=Ybscan, lv=lv, CI=CI, engine=shared_engine(matrix))
 
 
-def install(plspy_module=None, precision="fp64", boot_algo="direct"):
+def install(plspy_module=None, precision="fp64", boot_algo="direct", x_storage="fp64"):
     """Route the permutation / bootstrap / split-half loops of `plspy_module` (default: `import plspy`) through the
     GPU engine.  Idempotent; returns the module.  `precision`: "fp64" (exact) or "tf32x3" (fast bootstrap GEMM).
     `boot_algo`: "direct" or "collapsed" (mct / cst in the exact mode: see `bootstrap_permutation.check_boot_algo`);
-    a per-call option, applied to every resampling test while installed."""
+    a per-call option, applied to every resampling test while installed.  `x_storage`: "fp64" or "fp32" (mct / cst:
+    the engine holds X as float32, see `bootstrap_permutation.check_x_storage`; the reference's own host analysis
+    still sees X as passed, so the results are bit-identical to "fp64" when X holds float32 values).  Behaviour and
+    multiblock analyses raise NotImplementedError with "fp32"."""
     global _state
     if precision not in ("fp64", "tf32x3", "tf32x3+gram"):
         raise ValueError('precision must be "fp64", "tf32x3" or "tf32x3+gram"')
@@ -100,6 +105,8 @@ def install(plspy_module=None, precision="fp64", boot_algo="direct"):
         raise ValueError(f"boot_algo must be one of {_bp.BOOT_ALGOS}")
     if boot_algo == "collapsed" and precision != "fp64":
         raise ValueError('boot_algo="collapsed" is an exact (precision="fp64") formulation')
+    if x_storage not in _bp.X_STORAGES:
+        raise ValueError(f"x_storage must be one of {_bp.X_STORAGES}")
     if plspy_module is None:
         import plspy as plspy_module
     ref_bp = plspy_module.core.bootstrap_permutation
@@ -108,6 +115,9 @@ def install(plspy_module=None, precision="fp64", boot_algo="direct"):
         uninstall()
     _options["precision"] = precision
     _options["boot_algo"] = boot_algo
+    if _options["x_storage"] != x_storage:
+        _drop_engine()                                     # a cached engine holds X in the other storage
+    _options["x_storage"] = x_storage
     if _state is None:
         _state = {
             "module": plspy_module,
