@@ -13,7 +13,8 @@ generated elsewhere -- each an int array, or a (task, behaviour) tuple for mb/cm
 (an `Engine` that already holds X on the device), `device` (CUDA device of the engine built here), `precision` ("fp64" exact mode, or "tf32x3": the
 bootstrap moment GEMM of the task methods on the tcgen05 tensor cores; p-values stay FP64-exact), `boot_algo`
 ("direct", default: the bootstrap moments from the B x p x K salience GEMM; "collapsed": mct / cst in the exact mode
-only, the same standard errors from the closed form x_v^T Cov_r(c_rk) x_v -- see `check_boot_algo`).
+only, the same standard errors from the closed form x_v^T Cov_r(c_rk) x_v -- see `check_boot_algo`), `shard`
+("resamples", default, or "voxels": the layout of X in a multi-process run -- see `check_shard`).
 """
 import abc
 
@@ -399,11 +400,31 @@ def check_x_storage(x_storage, pls_alg):
             'in float64')
 
 
+SHARDS = Engine.SHARDS
+
+
+def check_shard(shard, pls_alg):
+    """Validates the multi-process layout of X before any GPU work.
+
+    "resamples" (default): every rank holds the whole of X and takes a share of the resamples.  "voxels": every rank
+    holds only its columns of X (dist.voxel_shard: 1/world of the device memory for X and for the tall-design image of
+    the bootstrap GEMM) and runs every bootstrap on them; the permutations and the per-bootstrap N-space outputs stay
+    resample-sharded through the all-reduced Gram matrix, and the p x K results are gathered.  Task methods (mct,
+    cst): the behaviour and multiblock bootstraps reduce over voxels per resample.  One process: the two are the
+    same."""
+    if shard not in SHARDS:
+        raise ValueError(f'shard must be one of {SHARDS}, got {shard!r}')
+    if shard == "voxels" and pls_alg not in ("mct", "cst"):
+        raise exceptions.NotImplementedError(
+            'shard="voxels" applies to the task methods (mct, cst); the behaviour and multiblock bootstraps need '
+            'per-resample norms over all voxels')
+
+
 def _collapsed_sumsq(eng, E, idx_dev, niter, lo, hi):
     """Collapsed bootstrap: q[v,k] = x_v^T S_k x_v with S_k = sum_r (c_rk - e_k)(c_rk - e_k)^T - s1_k s1_k^T / niter
     (= niter . Cov_r(c_rk)): the sum of squares of (VS_r - mean) over all `niter` resamples, p x K, the same on every
     rank.  Multi-process: one all-reduce of the N-space partial sums, each rank evaluates the quadratic form on its
-    share of the voxels and the shares are gathered."""
+    share of the voxels and the shares are gathered (a voxel-sharded engine: its own voxels, gathered later)."""
     E = eng.to_device(E, torch.float64)
     eng._x_ranges()          # (starts a deferred upload of X: the covariance build below overlaps it)
     if hi > lo:
@@ -415,7 +436,7 @@ def _collapsed_sumsq(eng, E, idx_dev, niter, lo, hi):
     dist.allreduce_packed_([S1, S2])
     s1t = S1.T
     Sig = S2 - s1t[:, :, None] * s1t[:, None, :] / niter
-    if dist.world()[1] == 1:
+    if dist.world()[1] == 1 or eng.voxel_sharded:
         return eng.boot_quad(Sig)
     v0, v1 = dist.shard(eng.p)
     return dist.gather_rows(eng.boot_quad(Sig, v0, v1), eng.p, v0)
@@ -433,13 +454,18 @@ class _ResampleTestPLS(ResampleTest):
     def __init__(self, X, Y, U, s, V, cond_order, mctype, contrast=None, preprocess=None, nperm=1000,
                  nboot=1000, bscan=None, Xbscan=None, Ybscan=None, lvcorrs_orig=None, Tvsc_orig=None,
                  CI=0.95, *, perm_indices=None, boot_indices=None, engine=None, precision="fp64", rotate_method=2,
-                 device=None, boot_algo="direct", x_storage="fp64"):
+                 device=None, boot_algo="direct", x_storage="fp64", shard=None):
         self.CI = CI
         check_boot_algo(boot_algo, self.pls_alg, engine.precision if engine is not None else precision,
                         engine.N if engine is not None else (int(X.shape[0]) if X is not None else None))
         check_x_storage(x_storage, self.pls_alg)
         if engine is not None:
             check_x_storage(engine.x_storage, self.pls_alg)
+        if shard is None:                   # the layout of a given engine, else the default
+            shard = engine.shard if engine is not None else "resamples"
+        check_shard(shard, self.pls_alg)
+        if engine is not None and engine.shard != shard:
+            raise ValueError(f"shard={shard!r} but the engine holds X laid out for shard={engine.shard!r}")
         self.boot_algo = boot_algo
         if rotate_method not in (0, 1, 2):
             raise ValueError("rotate_method must be 0 (SVD), 1 (Procrustes) or 2 (derived)")
@@ -450,7 +476,8 @@ class _ResampleTestPLS(ResampleTest):
         self.rotate_method = rotate_method
         _log(f"PLS ALG: {self.pls_alg}")
         eng = engine if engine is not None else (
-            Engine(X, device=device, precision=precision, x_storage=x_storage) if (nperm > 0 or nboot > 0) else None)
+            Engine(X, device=device, precision=precision, x_storage=x_storage, shard=shard)
+            if (nperm > 0 or nboot > 0) else None)
         self._engine = eng
         if eng is not None and self.pls_alg in ("mct", "cst") and dist.world()[1] > 1:
             eng.gram_collective()          # all ranks are here: Gram from per-rank voxel ranges + one all-reduce
@@ -524,7 +551,8 @@ class _ResampleTestPLS(ResampleTest):
     def salience_percentile_intervals(self, conf=None, max_bytes=4 << 30):
         """Percentile interval of every brain salience over the bootstrap samples (element-wise
         `confidence_interval(right_sv_sampled)`), streamed in voxel chunks so the B x p x K cube the reference stores
-        (bootstrap_permutation.py:497, 626) never exists.  Task methods (mct, cst).  Returns (lower, upper), p x K."""
+        (bootstrap_permutation.py:497, 626) never exists.  Task methods (mct, cst).  Returns (lower, upper), p x K.
+        With shard="voxels" every rank works on its voxels and the intervals are gathered: every rank must call it."""
         fn = getattr(getattr(self, "boot_debug_dict", None), "salience_percentiles", None)
         if fn is None:
             raise exceptions.NotImplementedError(
@@ -631,7 +659,9 @@ class _ResampleTestPLS(ResampleTest):
                         contrast=None, bscan=None, Xbscan=None, Ybscan=None, lvcorrs_orig=None, Tvsc_orig=None,
                         CI=0.95, indices=None, engine=None, _early=None, boot_algo="direct"):
         """bootstrap_permutation.py:466-766 for the task methods (mct, cst).  `_early`: moments already enqueued by
-        `_bootstrap_moments_early` (pipelined upload of X).  `boot_algo`: see `check_boot_algo`."""
+        `_bootstrap_moments_early` (pipelined upload of X).  `boot_algo`: see `check_boot_algo`.  A voxel-sharded engine
+        runs the moment GEMM of ALL bootstraps on its voxels (no moment all-reduce) and gathers the p x K results; the
+        lazy `right_sv_sampled` and the salience percentiles are then gathered too, so every rank must ask for them."""
         eng = engine if engine is not None else Engine(X)
         if indices is None:
             indices = resample.bootstrap_indices(pls_alg, niter, cond_order, Y=Y, bscan=bscan, Ybscan=Ybscan)
@@ -652,9 +682,16 @@ class _ResampleTestPLS(ResampleTest):
 
         lo, hi = dist.shard(niter)
         idx_dev = _index_shard(eng, indices, niter, lo, hi)
+        vox = eng.voxel_sharded
+        if vox:         # this rank's voxels: rows [v0, v1) of the p x K operands, every bootstrap
+            v0, v1 = eng.voxel_range
+            numer_v = numer[v0:v1].contiguous()
+            idx_all = _index_shard(eng, indices, niter, 0, niter)
+        else:
+            numer_v = numer
         # exact mode, single launch: the packed coefficients serve the N-space pass and the moment GEMM
         packed = (eng.pack_coef(E, idx_dev) if (hi > lo and eng.precision == "fp64" and _early is None
-                                                and E.shape[1] <= eng.KMAX) else None)
+                                                and E.shape[1] <= eng.KMAX and not vox) else None)
         d2, Tdist = eng.nspace(E, idx_dev, Lmat=Abar, packed=packed)        # Tdistrib (:633-634, :665-666)
         if pls_alg == "mct":
             XL = eng.xv(Vd)                                                 # X @ V once
@@ -678,12 +715,19 @@ class _ResampleTestPLS(ResampleTest):
         else:
             if _early is not None:
                 s1, s2 = _early
+            elif vox:
+                s1, s2 = eng.boot_moments(E, idx_all, pivot=numer_v)
             elif hi > lo:
                 s1, s2 = eng.boot_moments(E, idx_dev, pivot=numer, packed=packed)   # K4
             else:
                 s1 = torch.zeros_like(numer); s2 = torch.zeros_like(numer)
-            dist.allreduce_packed_([s1, s2])
-        std_errs, boot_ratios = eng.boot_finalize(s1, s2, niter, numer=numer)   # (:695-703)
+            if not vox:
+                dist.allreduce_packed_([s1, s2])
+        std_errs, boot_ratios = eng.boot_finalize(s1, s2, niter, numer=numer_v)   # (:695-703)
+        if vox:                                                             # ONE gather of [std_errs | boot_ratios]
+            K = int(std_errs.shape[1])
+            both = eng.gather_voxels(torch.cat([std_errs, boot_ratios], dim=1))
+            std_errs, boot_ratios = both[:, :K], both[:, K:]
         z = norm.ppf(1 - (1 - CI) / 2)                                      # (:709)
         std_errs_h, boot_ratios_h = _p_sized_to_host(eng, std_errs, boot_ratios)
         std_T, Tdist_h, left_h = (fetch_small(), None, None) if defer else fetch_small()
@@ -702,15 +746,22 @@ class _ResampleTestPLS(ResampleTest):
         debug.set_lazy("indices", lambda: _indices_to_host(indices, niter))
 
         def _right():   # the reference's B x p x K cube, only on request
-            nbytes = niter * eng.p * E.shape[1] * 8
+            nbytes = niter * eng.p_total * E.shape[1] * 8
             if nbytes > (2 << 30):
                 raise MemoryError(f"right_sv_sampled would need {nbytes / 2**30:.1f} GiB; the B200 path "
                                   "accumulates its moments on the fly instead of storing it")
-            return eng.salience(E, _index_shard(eng, indices, niter, 0, niter)).cpu().numpy()
+            VS = eng.salience(E, _index_shard(eng, indices, niter, 0, niter))
+            if vox:     # voxel-major for the gather
+                VS = eng.gather_voxels(VS.transpose(0, 1).contiguous()).transpose(0, 1).contiguous()
+            return VS.cpu().numpy()
         debug.set_lazy("right_sv_sampled", _right)
 
         def _salience_percentiles(conf, max_bytes=4 << 30):
             lo_, hi_ = eng.salience_percentiles(E, _index_shard(eng, indices, niter, 0, niter), conf, max_bytes)
+            if vox:
+                K = int(lo_.shape[1])
+                both = eng.gather_voxels(torch.cat([lo_, hi_], dim=1))
+                lo_, hi_ = both[:, :K], both[:, K:]
             return tuple(eng.to_host(lo_, hi_))
         debug.salience_percentiles = _salience_percentiles
         return conf_int, std_errs_h, boot_ratios_h, debug

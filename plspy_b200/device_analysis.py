@@ -19,6 +19,9 @@ Differences from the host path, all inherent to going through the Gram matrix:
     which the permutation test's own 1e-12 threshold zeroes as well);
   * relative accuracy of s_k is ~1e-16 (s_1 / s_k)^2 rather than 1e-16 (s_1 / s_k).
 The contrast methods have no SVD at all (U = contrasts), so their device path agrees with the host path to rounding.
+
+A voxel-sharded engine (shard="voxels", mct / cst) holds only its columns of X: G is all-reduced (Engine.G), every
+projection runs on the rank's slice and is gathered to p rows (`_project_x`), X V is all-reduced (Engine.xv).
 """
 import numpy as np
 import torch
@@ -56,6 +59,13 @@ def _project(eng, W, coef):
                      dim=1)
 
 
+def _project_x(eng, coef):
+    """X^T coef (p x K) on every rank: the projection of this rank's columns, gathered when X is voxel-sharded (an
+    engine without the `voxel_sharded` flag holds the whole of X)."""
+    P = _project(eng, eng.X, coef)
+    return eng.gather_voxels(P) if getattr(eng, "voxel_sharded", False) else P
+
+
 def _svd_through_gram(eng, W, Gw, coef, project=None):
     """U (K x K), s (K,), V (p x K, device) of M = coef^T W given Gw = W W^T; `project(c)` = W^T c when W is not
     held as one matrix."""
@@ -80,8 +90,8 @@ def task(eng, cond_order, mctype):
     """mct (pls_classes.py:258-266): X_means, X_mc, U, s, V (device), X_latent, Tvsc_orig."""
     A = cf._centring_operator(cond_order, mctype)
     Abar = cf._cell_mean_operator(cond_order)
-    U, s, V = _svd_through_gram(eng, eng.X, eng.G, A.T)
-    both = _project(eng, eng.X, np.concatenate([Abar.T, A.T], axis=1))         # one pass: cell means and M
+    U, s, V = _svd_through_gram(eng, None, eng.G, A.T, project=lambda c: _project_x(eng, c))
+    both = _project_x(eng, np.concatenate([Abar.T, A.T], axis=1))               # one pass: cell means and M
     K = A.shape[0]
     X_means, X_mc = both[:, :K].T.contiguous(), both[:, K:].T.contiguous()
     XL = eng.xv(V)
@@ -93,7 +103,7 @@ def contrast_task(eng, cond_order, contrasts):
     """cst (pls_classes.py:854-866): R = cell means, U = contrasts, V = (C^T R)^T un-normalised, s = its column norms."""
     Abar = cf._cell_mean_operator(cond_order)
     E = Abar.T @ contrasts                                                     # N x L
-    both = _project(eng, eng.X, np.concatenate([Abar.T, E], axis=1))
+    both = _project_x(eng, np.concatenate([Abar.T, E], axis=1))
     K = Abar.shape[0]
     R, V = both[:, :K].T.contiguous(), both[:, K:].contiguous()
     Ed = eng.to_device(E, torch.float64)

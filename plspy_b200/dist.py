@@ -1,7 +1,10 @@
-"""Resample-level data parallelism (SURVEY.md section 8e): X replicated, the resample index range is
-cut into one contiguous shard per rank, and only the tiny permutation counters, the two p x K moment
-matrices and the per-resample K x K outputs cross NVLink, through torch.distributed (NCCL on GPUs;
-the same code runs under gloo on CPU tensors for the host-logic tests).
+"""Multi-process layouts (SURVEY.md section 8e), through torch.distributed (NCCL on GPUs; the same code runs under gloo
+on CPU tensors for the host-logic tests).
+
+Resample sharding (the default): X replicated, the resample index range cut into one contiguous shard per rank
+(`shard`); only the tiny permutation counters, the two p x K moment matrices and the per-resample K x K outputs cross
+NVLink.  Voxel sharding (`shard="voxels"`, task methods): each rank holds the columns `voxel_shard` gives it; the
+N x N Gram matrix and the N x K product X V are all-reduced and the p x K results are gathered (`gather_spans`).
 """
 import torch
 
@@ -102,14 +105,36 @@ def allreduce_packed_(tensors):
     return tensors
 
 
+VOXEL_ALIGN = 256          # voxel_shard cut points: whole pairs of 128-voxel tiles, 16-byte aligned float32 rows
+
+
+def voxel_shard(p, rank=None, size=None):
+    """Contiguous [v0, v1) voxel range owned by `rank` in a voxel-sharded run: every cut point is a multiple of
+    VOXEL_ALIGN (the last range ends at p) and range sizes differ by at most VOXEL_ALIGN.  With p < VOXEL_ALIGN x size
+    the last ranks get empty ranges."""
+    if rank is None:
+        rank, size = world()
+    p = int(p)
+    lo, hi = shard(-(-p // VOXEL_ALIGN), rank, size)
+    return min(p, lo * VOXEL_ALIGN), min(p, hi * VOXEL_ALIGN)
+
+
 def gather_rows(local, n_total, lo):
     """Assemble per-resample rows computed on each rank's shard into the full [n_total, ...] tensor on
     every rank with ONE all_gather (shards padded to the largest shard, then trimmed)."""
-    import torch.distributed as dist
     rank, size = world()
     if size == 1:
         return local
-    spans = [shard(n_total, r, size) for r in range(size)]
+    return gather_spans(local, [shard(n_total, r, size) for r in range(size)])
+
+
+def gather_spans(local, spans):
+    """Concatenate along the first axis the blocks of rows [lo, hi) that rank r holds (`spans[r]`; any sizes, empty
+    ones included), on every rank, with ONE all_gather (blocks padded to the largest, then trimmed).  COLLECTIVE."""
+    import torch.distributed as dist
+    size = len(spans)
+    if size == 1:
+        return local
     mx = max(hi - l for l, hi in spans)
     tail = tuple(local.shape[1:])
     buf = local

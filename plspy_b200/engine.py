@@ -35,9 +35,10 @@ class Engine:
 
     PRECISIONS = ("fp64", "tf32x3", "tf32x3+gram")
     X_STORAGES = ("fp64", "fp32")
+    SHARDS = ("resamples", "voxels")
     GRAM_TF32_MAX_ROWS = 320
 
-    def __init__(self, X, device=None, precision="fp64", x_storage="fp64"):
+    def __init__(self, X, device=None, precision="fp64", x_storage="fp64", shard="resamples"):
         """precision: "fp64" (exact mode, FP64 DMMA) or "tf32x3" (fast mode: the bootstrap moment GEMM runs on the
         tcgen05 tensor cores with the 3xTF32 split; every N-space quantity -- Gram matrix, permutation p-values,
         Tdistrib, U_hat -- stays FP64) or "tf32x3+gram" (fast mode whose Gram matrix G = X X^T is ALSO formed on the
@@ -50,12 +51,28 @@ class Engine:
         float64 one rounded once) and never allocates a float64 copy of X: the task-method kernels widen each element
         where they load it, so every result equals, bit for bit, the "fp64" result for the widened float32 matrix.
         Half the device memory and half the HBM traffic of every pass over X.  The behaviour / multiblock kernels
-        (cell_standardize, rb_boot, half_gram, gram_stacked) take float64 operands only."""
+        (cell_standardize, rb_boot, half_gram, gram_stacked) take float64 operands only.
+
+        shard: the layout of X in a multi-process run.  "resamples" (default): every rank holds the whole of X.
+        "voxels" (task methods): every rank is handed the whole host matrix and holds only its columns
+        `voxel_range` = dist.voxel_shard(p); `p` is then the width of that slice and `p_total` the width of X.  The
+        Gram matrix (`G`) and `xv` become collectives: the partial product of the slice plus one all-reduce, so every
+        rank must call them at the same point.  With one process (or inside dist.local_only) the two layouts are the
+        same."""
         _require_cuda()
         if precision not in self.PRECISIONS:
             raise ValueError(f"precision must be one of {self.PRECISIONS}")
         if x_storage not in self.X_STORAGES:
             raise ValueError(f"x_storage must be one of {self.X_STORAGES}, got {x_storage!r}")
+        if shard not in self.SHARDS:
+            raise ValueError(f"shard must be one of {self.SHARDS}, got {shard!r}")
+        from . import dist
+        self.shard = shard
+        self._world = dist.world()
+        self.voxel_sharded = shard == "voxels" and self._world[1] > 1
+        p_total = int(X.shape[1]) if len(X.shape) == 2 else 0
+        self.voxel_range = dist.voxel_shard(p_total, *self._world) if self.voxel_sharded else (0, p_total)
+        self.p_total = p_total
         self.x_storage = x_storage
         self._xdt = F32 if x_storage == "fp32" else F64
         self.gram_tf32 = precision == "tf32x3+gram"
@@ -67,7 +84,7 @@ class Engine:
         self._X = self._upload_x(X)
         if self._X.dim() != 2:
             raise ValueError("X must be 2-dimensional")
-        self.N, self.p = int(self._X.shape[0]), int(self._X.shape[1])
+        self.N, self.p = int(self._X.shape[0]), int(self._X.shape[1])     # p: the width held here
         self.ldx = int(self._X.stride(0))
         self._G = None
         self.kernel_events = None     # set to {} to record CUDA events around named kernels (bench.py)
@@ -81,6 +98,29 @@ class Engine:
     @staticmethod
     def _x32(M):
         return M.dtype == F32
+
+    def _collective(self):
+        """The world this voxel-sharded engine was cut for must be the current one: a voxel-sharded engine used inside
+        dist.local_only (or in another process group) would silently compute on its slice alone."""
+        from . import dist
+        if self.voxel_sharded and dist.world() != self._world:
+            raise RuntimeError(f"this engine holds the voxels {self.voxel_range} of {self.p_total} for rank "
+                               f"{self._world[0]} of {self._world[1]}; it cannot be used outside that process group")
+        return dist
+
+    def gather_voxels(self, T):
+        """The p_total x ... tensor whose rows [v0, v1) are the voxel rows `T` of every rank (voxel-sharded: ONE
+        all-gather, COLLECTIVE); T itself otherwise."""
+        if not self.voxel_sharded:
+            return T
+        dist = self._collective()
+        return dist.gather_spans(T, [dist.voxel_shard(self.p_total, r, self._world[1]) for r in range(self._world[1])])
+
+    def _need_whole_x(self, what):
+        """The behaviour / multiblock kernels need every voxel of X (shard="voxels" is for mct / cst)."""
+        if self.voxel_sharded:
+            raise _lib.PlsB200Error(f"{what}: needs the whole of X, this engine holds the voxels {self.voxel_range} "
+                                    "(shard='voxels' applies to the task methods mct and cst)")
 
     @staticmethod
     def _need_f64(M, what):
@@ -121,16 +161,17 @@ class Engine:
         the rest is still crossing PCIe.  The copies are only enqueued at the first use of X (`_start_upload`):
         host->device copies execute in issue order, so the small uploads of an analysis (index matrices, V, weights)
         must be issued before the 480 MB of X or they would wait behind it -- and with them the first kernels."""
-        n, p = int(Xh.shape[0]), int(Xh.shape[1])
+        v0, v1 = self.voxel_range   # (the columns this rank holds: all of them unless voxel-sharded)
         self._x_host = Xh            # keep the pinned source alive until the copies have been consumed
         self._pending = []           # empty list = upload not started yet
-        return torch.empty((n, p), dtype=Xh.dtype, device=self.device)
+        return torch.empty((int(Xh.shape[0]), v1 - v0), dtype=Xh.dtype, device=self.device)
 
     def _start_upload(self):
         if self._pending is None or len(self._pending) > 0:
             return
         Xh, Xd = self._x_host, self._X
-        n, p = int(Xh.shape[0]), int(Xh.shape[1])
+        n, p = int(Xd.shape[0]), int(Xd.shape[1])
+        c0, ph = self.voxel_range[0], int(Xh.shape[1])       # first column held here, host row length
         if getattr(self, "_copy_stream", None) is None:
             self._copy_stream = torch.cuda.Stream(device=self.device)
         side = self._copy_stream
@@ -152,7 +193,7 @@ class Engine:
         with torch.cuda.device(self.device):
             for v0, v1 in zip(bounds[:-1], bounds[1:]):
                 # (torch's copy_ of a column block goes through a contiguous temporary and synchronises)
-                check(lib.plsb200_copy2d_h2d(Xd.data_ptr() + es * v0, es * p, Xh.data_ptr() + es * v0, es * p,
+                check(lib.plsb200_copy2d_h2d(Xd.data_ptr() + es * v0, es * p, Xh.data_ptr() + es * (c0 + v0), es * ph,
                                              es * (v1 - v0), n, side.cuda_stream), "copy2d_h2d")
                 ev = torch.cuda.Event()
                 ev.record(side)
@@ -164,26 +205,33 @@ class Engine:
         """X -> device.  In a multi-process run X is replicated (every rank is handed the same host matrix), so
         each rank uploads only its 1/world share of the rows over PCIe and the ranks exchange the shares with one
         all-gather over NVLink: eight ranks pulling the same 480 MB through the host's memory system at the same
-        time took 17 ms each, a share plus the all-gather takes 2."""
+        time took 17 ms each, a share plus the all-gather takes 2.  Voxel-sharded, each rank uploads only its columns
+        (`voxel_range`) by the same paths and nothing is gathered."""
         from . import dist
         size = dist.world()[1]
         dt = self._xdt
+        cols = self.voxel_sharded and len(X.shape) == 2
+        v0, v1 = self.voxel_range
         if dt == F64 and torch.is_tensor(X) and X.dtype == torch.float32 and X.dim() == 2:
             # float32 storage (plspy_b200/io.py): half the bytes over PCIe, widened on the device
-            x32 = X.to(self.device, non_blocking=True).contiguous()
+            x32 = (X[:, v0:v1] if cols else X).to(self.device, non_blocking=True).contiguous()
             out = torch.empty(x32.shape, dtype=F64, device=self.device)
             with torch.cuda.device(self.device):
                 check(lib.plsb200_widen_f32_f64(x32.data_ptr(), out.data_ptr(), x32.numel(), self._stream()),
                       "widen_f32_f64")
             return out
         on_host = not (torch.is_tensor(X) and X.is_cuda)
-        if (size == 1 and on_host and torch.is_tensor(X) and X.dim() == 2 and X.dtype == dt and X.is_pinned()
-                and X.is_contiguous() and X.numel() * X.element_size() >= self.PIPELINED_UPLOAD_MIN_BYTES):
+        whole = size == 1 or cols                     # this rank uploads everything it holds over PCIe itself
+        if (whole and on_host and torch.is_tensor(X) and X.dim() == 2 and X.dtype == dt and X.is_pinned()
+                and X.is_contiguous() and X.shape[0] * (v1 - v0) * X.element_size() >= self.PIPELINED_UPLOAD_MIN_BYTES):
             return self._upload_pipelined(X)
-        if (size == 1 and on_host and len(X.shape) == 2 and not torch.is_tensor(X)
+        if (whole and on_host and len(X.shape) == 2 and not torch.is_tensor(X)
                 and X.dtype == (np.float64 if dt == F64 else np.float32) and X.flags.c_contiguous
-                and X.nbytes >= self.PIPELINED_UPLOAD_MIN_BYTES and self.PAGEABLE_UPLOAD_THREADS > 1):
+                and X.shape[0] * (v1 - v0) * X.itemsize >= self.PIPELINED_UPLOAD_MIN_BYTES
+                and self.PAGEABLE_UPLOAD_THREADS > 1):
             return self._upload_pageable(X)
+        if cols:
+            return self.to_device(X[:, v0:v1], dt)
         if size == 1 or not on_host or len(X.shape) != 2:
             return self.to_device(X, dt)
         n = int(X.shape[0])
@@ -211,7 +259,8 @@ class Engine:
 
     def _upload_pageable_locked(self, X):
         import concurrent.futures
-        n, p = int(X.shape[0]), int(X.shape[1])
+        v0, v1 = self.voxel_range
+        n, p = int(X.shape[0]), v1 - v0
         dt = self._xdt
         out = torch.empty((n, p), dtype=dt, device=self.device)
         nt = max(1, self.PAGEABLE_UPLOAD_THREADS)
@@ -233,7 +282,8 @@ class Engine:
                     free[b % 2].synchronize()
                 dst = buf.numpy()
                 cuts = [r0 + (r1 - r0) * i // nt for i in range(nt + 1)]
-                list(pool.map(lambda i: np.copyto(dst[cuts[i] - r0:cuts[i + 1] - r0], X[cuts[i]:cuts[i + 1]]), range(nt)))
+                list(pool.map(lambda i: np.copyto(dst[cuts[i] - r0:cuts[i + 1] - r0], X[cuts[i]:cuts[i + 1], v0:v1]),
+                              range(nt)))
                 with torch.cuda.stream(side):
                     out[r0:r1].copy_(buf, non_blocking=True)
                     free[b % 2] = torch.cuda.Event()
@@ -337,7 +387,7 @@ class Engine:
         """Gram matrix of the row stack [M1; M2] ((n1 + n2) x p) without building it (multiblock: [X; Zb])."""
         n1, n2, p = int(M1.shape[0]), int(M2.shape[0]), int(M1.shape[1])
         assert int(M2.shape[1]) == p
-        self._need_f64(M1, "gram_stacked"); self._need_f64(M2, "gram_stacked")
+        self._need_f64(M1, "gram_stacked"); self._need_f64(M2, "gram_stacked"); self._need_whole_x("gram_stacked")
         with torch.cuda.device(self.device):
             ws = self._ws(lib.plsb200_gram_f64_workspace(n1 + n2, p))
             G = self._empty(n1 + n2, n1 + n2)
@@ -347,9 +397,12 @@ class Engine:
 
     @property
     def G(self):
-        """G = X X^T (N x N), computed once per engine."""
+        """G = X X^T (N x N), computed once per engine.  Voxel-sharded: the Gram matrix of this rank's columns plus one
+        all-reduce of N x N doubles (COLLECTIVE at its first use)."""
         if self._G is None:
-            if self.gram_tf32 and self.N <= self.GRAM_TF32_MAX_ROWS:
+            if self.p == 0:
+                self._G = torch.zeros(self.N, self.N, dtype=F64, device=self.device)
+            elif self.gram_tf32 and self.N <= self.GRAM_TF32_MAX_ROWS:
                 self._G = self._gram_tf32()
             elif self._pending is None:
                 self._G = self.gram_of(self.X)
@@ -361,6 +414,8 @@ class Engine:
                     Gc = self.gram_of(self._X[:, v0:v1])
                     G = Gc if G is None else G.add_(Gc)
                 self._G = G
+            if self.voxel_sharded:
+                self._collective().allreduce_sum_(self._G)
         return self._G
 
     def _gram_tf32(self, ranges=None):
@@ -388,10 +443,11 @@ class Engine:
         """COLLECTIVE in a multi-process run (every rank must call it at the same point): G from the partial Gram
         matrix of this rank's voxel range plus one all-reduce of N x N doubles, instead of every rank forming the whole
         G redundantly -- the Gram is the largest piece of per-rank work that does not shrink with the shard of
-        resamples.  Single process, G already there, or PLSB200_SHARD_GRAM=0: the plain property."""
+        resamples.  Single process, G already there, a voxel-sharded engine (whose G is collective anyway) or
+        PLSB200_SHARD_GRAM=0: the plain property."""
         from . import dist
         rank, size = dist.world()
-        if (self._G is None and size > 1 and self.p >= 4096 * size
+        if (self._G is None and size > 1 and not self.voxel_sharded and self.p >= 4096 * size
                 and os.environ.get("PLSB200_SHARD_GRAM", "1") != "0"):
             cut = [(self.p * r // size) // 64 * 64 for r in range(size)] + [self.p]
             if self.gram_tf32 and self.N <= self.GRAM_TF32_MAX_ROWS:
@@ -404,16 +460,26 @@ class Engine:
         return self.G
 
     def xv(self, V):
-        """XL = X @ V (N x K)."""
+        """XL = X @ V (N x K) for V of p_total x K.  Voxel-sharded: the product of this rank's columns with its rows of V
+        plus one all-reduce of N x K doubles (COLLECTIVE)."""
         V = self.to_device(V, F64)
         K = int(V.shape[1])
+        if self.voxel_sharded:
+            if int(V.shape[0]) != self.p_total:
+                raise ValueError(f"xv: V must have {self.p_total} rows, got {int(V.shape[0])}")
+            V = V[self.voxel_range[0]:self.voxel_range[1]].contiguous()
         X = self.X
-        fn, what = (lib.plsb200_xv_x32_f64, "xv_x32_f64") if self._x32(X) else (lib.plsb200_xv_f64, "xv_f64")
-        with torch.cuda.device(self.device):
-            ws = self._ws(lib.plsb200_xv_f64_workspace(self.N, self.p, K))
-            out = self._empty(self.N, K)
-            check(fn(self._p(X), self.N, self.p, self.ldx, self._p(V), K, self._p(out), self._p(ws), ws.numel(),
-                     self._stream()), what)
+        if self.p == 0:
+            out = torch.zeros(self.N, K, dtype=F64, device=self.device)
+        else:
+            fn, what = (lib.plsb200_xv_x32_f64, "xv_x32_f64") if self._x32(X) else (lib.plsb200_xv_f64, "xv_f64")
+            with torch.cuda.device(self.device):
+                ws = self._ws(lib.plsb200_xv_f64_workspace(self.N, self.p, K))
+                out = self._empty(self.N, K)
+                check(fn(self._p(X), self.N, self.p, self.ldx, self._p(V), K, self._p(out), self._p(ws), ws.numel(),
+                         self._stream()), what)
+        if self.voxel_sharded:
+            self._collective().allreduce_sum_(out)
         return out
 
     def nspace_coef(self, G, C, Lmat=None):
@@ -618,6 +684,8 @@ class Engine:
                                                None if pivot is None else pivot[:, sl].contiguous()))
             return torch.cat([a for a, _ in parts], dim=1), torch.cat([b for _, b in parts], dim=1)
         self._x_ranges()          # (starts a deferred upload of X now: every small input is already on its way)
+        if self.p == 0:           # the empty voxel slice of a voxel-sharded rank
+            return self._empty(0, K), self._empty(0, K)
         if self.precision == "tf32x3":
             return self._boot_moments_tf32(E, idx, pivot, R, K)
         with torch.cuda.device(self.device):
@@ -712,6 +780,8 @@ class Engine:
         br = self._empty(self.p, K) if numer is not None else None
         if numer is not None:
             numer = self.to_device(numer, F64)
+        if self.p == 0:
+            return se, br
         with torch.cuda.device(self.device):
             check(lib.plsb200_boot_finalize_f64(self._p(s1), self._p(s2), self.p, K, int(R_total), self._p(numer),
                                                 self._p(se), self._p(br), self._stream()), "boot_finalize_f64")
@@ -772,6 +842,8 @@ class Engine:
         n, p, ld = int(M.shape[0]), int(M.shape[1]), int(M.stride(0))
         R, K = int(idx.shape[0]), int(E.shape[1])
         out = self._empty(R, p, K)
+        if p == 0:
+            return out
         fn = lib.plsb200_salience_x32_f64 if self._x32(M) else lib.plsb200_salience_f64
         with torch.cuda.device(self.device):
             check(fn(self._p(M), n, p, ld, self._p(E), K, self._p(idx), R, self._p(out), self._stream()), "salience_f64")
@@ -832,7 +904,7 @@ class Engine:
         """Xc = M - block means, Z = block z-score(M) / sqrt(n) (both rows x p, dense); M defaults to X."""
         cs = self.to_device(np.asarray(cell_start, dtype=np.int32), I32)
         M = self.X if M is None else M
-        self._need_f64(M, "cell_standardize")
+        self._need_f64(M, "cell_standardize"); self._need_whole_x("cell_standardize")
         n, p, ld = int(M.shape[0]), int(M.shape[1]), int(M.stride(0))
         Xc = self._empty(n, p)
         Z = self._empty(n, p) if want_z else None
@@ -869,7 +941,7 @@ class Engine:
         Runs on the FP64 tensor path (plsb200_rb_boot_dmma_f64) when the design fits its register-resident
         fragments, else on the general FMA kernel.  `X2`: the data matrix is the row stack [Xc; X2] (not built: the
         kernels take the two row segments; multiblock bootstraps pass [Xcb; X])."""
-        self._need_f64(Xc, "rb_boot"); self._need_f64(X2, "rb_boot")
+        self._need_f64(Xc, "rb_boot"); self._need_f64(X2, "rb_boot"); self._need_whole_x("rb_boot")
         cs_host = np.ascontiguousarray(np.asarray(cell_start, dtype=np.int32))
         R, N, K = int(Q.shape[0]), int(Q.shape[1]), int(Q.shape[2])
         p = int(Xc.shape[1])
@@ -946,7 +1018,7 @@ class Engine:
         The windowed kernel (half_gram.cu, DMMA Gram) is used: the non-zero column window of every block is read
         off Q (blocks wider than 8 columns become several segments); `dense=True` forces the older FMA kernel of
         rb.cu (K <= 24), kept as the in-library cross-check."""
-        self._need_f64(Xstd, "half_gram"); self._need_f64(Xlin, "half_gram")
+        self._need_f64(Xstd, "half_gram"); self._need_f64(Xlin, "half_gram"); self._need_whole_x("half_gram")
         ids = self.to_device(ids, I32); Q = self.to_device(Q, F64)
         cells_h = np.asarray(cells.cpu() if torch.is_tensor(cells) else cells, dtype=np.int32)
         S, nmax, K = int(ids.shape[0]), int(ids.shape[2]), int(Q.shape[3])

@@ -28,7 +28,10 @@ def PLS(*args, **kwargs):
     form's flops, so faster when num_boot > N -- see bootstrap_permutation.check_boot_algo), `x_storage` ("fp64" =
     X held as float64 on the device, default; "fp32" = mct / cst: X.astype(float32) held as float32 -- half the device
     memory -- with every result bit-identical to the "fp64" run on the widened float32 matrix; the host-side steps see
-    the same widened values -- see bootstrap_permutation.check_x_storage).
+    the same widened values -- see bootstrap_permutation.check_x_storage), `shard` ("resamples" = in a multi-process
+    run every GPU holds the whole of X and takes a share of the resamples, default; "voxels" = mct / cst: every GPU
+    holds only its share of the columns of X and runs every bootstrap on them, so an X larger than one GPU's memory
+    can be analysed -- see bootstrap_permutation.check_shard).
     """
     pls_method = kwargs.pop("pls_method", "mct")
     kwargs["pls_alg"] = pls_method
@@ -55,4 +58,6 @@ def PLS(*args, **kwargs):
             engine.N if engine is not None else (int(X.shape[0]) if X is not None and hasattr(X, "shape") else None))
     if "x_storage" in kwargs:
         bootstrap_permutation.check_x_storage(kwargs["x_storage"], pls_method)
+    if "shard" in kwargs:
+        bootstrap_permutation.check_shard(kwargs["shard"], pls_method)
     return pls_classes.PLSBase._create(pls_method, *args, **kwargs)

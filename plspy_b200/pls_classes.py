@@ -46,7 +46,7 @@ class PLSBase(abc.ABC):
 
     # ---- shared helpers -------------------------------------------------------------------
     _ENGINE_KWARGS = ("perm_indices", "boot_indices", "engine", "device", "precision", "rotate_method", "analysis",
-                      "boot_algo", "x_storage")
+                      "boot_algo", "x_storage", "shard")
 
     def _take_kwargs(self, kwargs):
         self.pls_alg = kwargs["pls_alg"]
@@ -65,6 +65,17 @@ class PLSBase(abc.ABC):
             raise ValueError(f"x_storage={xs!r} but the engine holds X as {eng.x_storage!r}")
         bootstrap_permutation.check_x_storage(xs, self.pls_alg)
         self._engine_kwargs["x_storage"] = xs
+        # multi-process layout of X: the option, else that of a given engine
+        sh = self._engine_kwargs.get("shard", eng.shard if eng is not None else "resamples")
+        if eng is not None and eng.shard != sh:
+            raise ValueError(f"shard={sh!r} but the engine holds X laid out for shard={eng.shard!r}")
+        bootstrap_permutation.check_shard(sh, self.pls_alg)
+        self._engine_kwargs["shard"] = sh
+
+    def _shard_kw(self):
+        """Engine keyword for the layout of X: none for the default (the same construction as without the option)."""
+        sh = self._engine_kwargs["shard"]
+        return {} if sh == "resamples" else {"shard": sh}
 
     @staticmethod
     def _get_groups_info(groups_tuple):
@@ -179,7 +190,7 @@ class PLSBase(abc.ABC):
             out = {}
             if want_eng:
                 out["engine"] = Engine(xsrc, device=device, precision=ek.get("precision", "fp64"),
-                                       x_storage=ek["x_storage"])
+                                       x_storage=ek["x_storage"], **self._shard_kw())
             if want_idx:
                 if self.num_perm > 0:
                     out["perm_indices"] = resample.permutation_indices(self.pls_alg, self.num_perm, self.cond_order, Y=Y,
@@ -214,7 +225,7 @@ class PLSBase(abc.ABC):
             self._engine_kwargs["engine"] = Engine(getattr(self, "_x_tensor", None) if getattr(self, "_x_tensor", None)
                                                    is not None else self.X, device=self._engine_kwargs.get("device"),
                                                    precision=self._engine_kwargs.get("precision", "fp64"),
-                                                   x_storage=self._engine_kwargs["x_storage"])
+                                                   x_storage=self._engine_kwargs["x_storage"], **self._shard_kw())
         return True
 
     def _resample(self, Y, mctype, preprocess, **kw):
@@ -225,7 +236,7 @@ class PLSBase(abc.ABC):
             from .engine import Engine
             self._engine_kwargs["engine"] = Engine(xt, device=self._engine_kwargs.get("device"),
                                                    precision=self._engine_kwargs.get("precision", "fp64"),
-                                                   x_storage=self._engine_kwargs["x_storage"])
+                                                   x_storage=self._engine_kwargs["x_storage"], **self._shard_kw())
         self.resample_tests = bootstrap_permutation.ResampleTest._create(
             self.pls_alg, self.X, Y, self.U, self.s, self.V if V is None else V, self.cond_order, mctype, preprocess=preprocess,
             nperm=self.num_perm, nboot=self.num_boot, CI=self.CI,
@@ -233,7 +244,8 @@ class PLSBase(abc.ABC):
             boot_indices=self._engine_kwargs.get("boot_indices"),
             engine=self._engine_kwargs.get("engine"), precision=self._engine_kwargs.get("precision", "fp64"),
             rotate_method=self._engine_kwargs.get("rotate_method", 2), device=self._engine_kwargs.get("device"),
-            boot_algo=self._engine_kwargs.get("boot_algo", "direct"), x_storage=self._engine_kwargs["x_storage"], **kw)
+            boot_algo=self._engine_kwargs.get("boot_algo", "direct"), x_storage=self._engine_kwargs["x_storage"],
+            shard=self._engine_kwargs["shard"], **kw)
 
     def _split_half(self, Y, mctype, contrasts, **kw):
         """pls_classes.py:285-318 (identical block in every class)."""
@@ -246,11 +258,14 @@ class PLSBase(abc.ABC):
                           f"Using lv={max_lv} instead.")
                     self.lv = max_lv
                 eng = getattr(self.resample_tests, "_engine", None) or self._engine_kwargs.get("engine")
-                if eng is None and self._engine_kwargs["x_storage"] == "fp32":
-                    # no resampling engine: the split-half functions would each upload the widened host copy as
-                    # float64; one engine holding the float32 matrix (exact mode, as theirs) serves both instead
+                if eng is None and (self._engine_kwargs["x_storage"] == "fp32"
+                                    or self._engine_kwargs["shard"] == "voxels"):
+                    # no resampling engine: the split-half functions would each upload the (widened) host copy as
+                    # float64 and whole; one engine holding X as asked (exact mode, as theirs) serves both instead
                     from .engine import Engine
-                    eng = Engine(self._x_tensor, device=self._engine_kwargs.get("device"), x_storage="fp32")
+                    src = getattr(self, "_x_tensor", None)
+                    eng = Engine(self.X if src is None else src, device=self._engine_kwargs.get("device"),
+                                 x_storage=self._engine_kwargs["x_storage"], **self._shard_kw())
                 self.pls_repro_tt = split_half_resampling.split_half_test_train(
                     self.pls_alg, self.X, Y, self.cond_order, num_split=self.num_split, mctype=mctype,
                     contrasts=contrasts, engine=eng, **kw)

@@ -29,7 +29,7 @@ from .engine import Engine
 METHODS = ("mct", "rb", "cst", "csb", "mb", "cmb")
 
 _state = None          # what install() replaced, for uninstall()
-_options = {"precision": "fp64", "boot_algo": "direct", "x_storage": "fp64"}
+_options = {"precision": "fp64", "boot_algo": "direct", "x_storage": "fp64", "shard": "resamples"}
 _shared = {"ref": None, "engine": None}
 
 
@@ -44,7 +44,7 @@ def shared_engine(X):
     ref = _shared["ref"]
     if ref is not None and ref() is X and _shared["engine"] is not None:
         return _shared["engine"]
-    eng = Engine(X, precision=_options["precision"], x_storage=_options["x_storage"])
+    eng = Engine(X, precision=_options["precision"], x_storage=_options["x_storage"], shard=_options["shard"])
     try:
         _shared["ref"] = weakref.ref(X, _drop_engine)
     except TypeError:           # not weak-referenceable (a torch tensor is; a list is not): do not cache
@@ -61,7 +61,9 @@ class _InstalledResampleTest(_bp._ResampleTestPLS):
         nperm = kwargs.get("nperm", 1000)
         nboot = kwargs.get("nboot", 1000)
         kwargs.setdefault("x_storage", _options["x_storage"])
+        kwargs.setdefault("shard", _options["shard"])
         _bp.check_x_storage(kwargs["x_storage"], self.pls_alg)        # before the engine uploads X
+        _bp.check_shard(kwargs["shard"], self.pls_alg)
         if "engine" not in kwargs and (nperm > 0 or nboot > 0):
             kwargs["engine"] = shared_engine(X)
         kwargs.setdefault("precision", _options["precision"])
@@ -79,6 +81,7 @@ PINNED = {key: _pinned(key) for key in METHODS}
 def _split_half_test_train(pls_alg, matrix, Y, cond_order, num_split, mctype=None, contrasts=None, bscan=None,
                            Xbscan=None, Ybscan=None):
     """split_half_resampling.py:23 -- the reference's signature; X is reused from the resampling step."""
+    _bp.check_shard(_options["shard"], pls_alg)
     return _sh.split_half_test_train(pls_alg, matrix, Y, cond_order, num_split, mctype=mctype, contrasts=contrasts,
                                      bscan=bscan, Xbscan=Xbscan, Ybscan=Ybscan, engine=shared_engine(matrix))
 
@@ -86,18 +89,21 @@ def _split_half_test_train(pls_alg, matrix, Y, cond_order, num_split, mctype=Non
 def _split_half(pls_alg, matrix, Y, cond_order, num_split, mctype=None, contrasts=None, bscan=None, Xbscan=None,
                 Ybscan=None, lv=1, CI=0.95):
     """split_half_resampling.py:404."""
+    _bp.check_shard(_options["shard"], pls_alg)
     return _sh.split_half(pls_alg, matrix, Y, cond_order, num_split, mctype=mctype, contrasts=contrasts, bscan=bscan,
                           Xbscan=Xbscan, Ybscan=Ybscan, lv=lv, CI=CI, engine=shared_engine(matrix))
 
 
-def install(plspy_module=None, precision="fp64", boot_algo="direct", x_storage="fp64"):
+def install(plspy_module=None, precision="fp64", boot_algo="direct", x_storage="fp64", shard="resamples"):
     """Route the permutation / bootstrap / split-half loops of `plspy_module` (default: `import plspy`) through the
     GPU engine.  Idempotent; returns the module.  `precision`: "fp64" (exact) or "tf32x3" (fast bootstrap GEMM).
     `boot_algo`: "direct" or "collapsed" (mct / cst in the exact mode: see `bootstrap_permutation.check_boot_algo`);
     a per-call option, applied to every resampling test while installed.  `x_storage`: "fp64" or "fp32" (mct / cst:
     the engine holds X as float32, see `bootstrap_permutation.check_x_storage`; the reference's own host analysis
     still sees X as passed, so the results are bit-identical to "fp64" when X holds float32 values).  Behaviour and
-    multiblock analyses raise NotImplementedError with "fp32"."""
+    multiblock analyses raise NotImplementedError with "fp32".  `shard`: "resamples" or "voxels" (mct / cst in a
+    multi-process run: every rank holds only its columns of X, see `bootstrap_permutation.check_shard`); behaviour and
+    multiblock analyses raise NotImplementedError with "voxels"."""
     global _state
     if precision not in ("fp64", "tf32x3", "tf32x3+gram"):
         raise ValueError('precision must be "fp64", "tf32x3" or "tf32x3+gram"')
@@ -107,6 +113,8 @@ def install(plspy_module=None, precision="fp64", boot_algo="direct", x_storage="
         raise ValueError('boot_algo="collapsed" is an exact (precision="fp64") formulation')
     if x_storage not in _bp.X_STORAGES:
         raise ValueError(f"x_storage must be one of {_bp.X_STORAGES}")
+    if shard not in _bp.SHARDS:
+        raise ValueError(f"shard must be one of {_bp.SHARDS}")
     if plspy_module is None:
         import plspy as plspy_module
     ref_bp = plspy_module.core.bootstrap_permutation
@@ -115,9 +123,10 @@ def install(plspy_module=None, precision="fp64", boot_algo="direct", x_storage="
         uninstall()
     _options["precision"] = precision
     _options["boot_algo"] = boot_algo
-    if _options["x_storage"] != x_storage:
-        _drop_engine()                                     # a cached engine holds X in the other storage
+    if _options["x_storage"] != x_storage or _options["shard"] != shard:
+        _drop_engine()                                     # a cached engine holds X in the other storage or layout
     _options["x_storage"] = x_storage
+    _options["shard"] = shard
     if _state is None:
         _state = {
             "module": plspy_module,
