@@ -159,6 +159,14 @@ int plsb200_boot_moments_f64(const double* X, int N, int64_t p, int64_t ldx, con
 int plsb200_boot_moments_x32_f64(const float* X, int N, int64_t p, int64_t ldx, const double* coef, int K,
                                  int R, const double* pivot, double* sum, double* sumsq,
                                  void* workspace, size_t workspace_bytes, void* stream);
+/* Factored collapsed bootstrap (task methods; DESIGN.md section 3): J pseudo-resamples with the coefficients
+ * c_j[n,k] = E[n,k] . L[sid[n], j] (L: ns x J row-major, sid: N subjects) packed for plsb200_boot_moments_f64 /
+ * _x32_f64, which then run with R = J and pivot = NULL: their `sumsq` is q[v,k] = sum_j (x_v^T c_jk)^2.  The size
+ * query returns 0 (and the pack PLSB200_EUNSUPPORTED) where boot_moments reads another layout (N > 320 or
+ * PLSB200_EXACT=os) or K > 24.                                                                                  */
+size_t plsb200_boot_factor_coef_bytes(int N, int K, int J);
+int plsb200_boot_factor_pack_f64(const double* E, int N, int K, const double* L, int J, const int32_t* sid,
+                                 double* coef, void* stream);
 
 /* ---- K4 collapsed (task methods, exact FP64): the bootstrap variance as a quadratic form ------------------
  * Each salience is linear in the draw, so R . Var_r(VS_r[v,k]) = x_v^T S_k x_v with S_k = R . Cov_r(c_rk) (N x N).
@@ -175,6 +183,21 @@ int plsb200_boot_quad_f64(const double* X, int N, int64_t p, int64_t ldx, const 
                           void* workspace, size_t workspace_bytes, void* stream);
 int plsb200_boot_quad_x32_f64(const float* X, int N, int64_t p, int64_t ldx, const double* coef, int K, double* q,
                               void* workspace, size_t workspace_bytes, void* stream);
+/* The factor of the draw-count covariance.  layout (int32, 2N + ns): base[n] = first row of n's cell, sid[n] = subject of
+ * row n, row0[s] = row of subject s in the first condition of its group.
+ * boot_counts_f64: for every draw r of idx (R x N) sets *bad |= 1 unless each row keeps its cell and follows the
+ * first condition's subject map (bad may be NULL); with counts != NULL writes counts[s * ldc + r] = m_r[s] - 1 (draws of
+ * subject s) and counts[ns * ldc + r] = 1 -- their Gram matrix (plsb200_gram_f64) holds sum_r (m_r - 1)(m_r - 1)^T and,
+ * in its last column, s1 = sum_r (m_r - 1).
+ * boot_factor_f64: one CTA.  From that (ns + 1)-square Gram matrix Mg, M = Mg[:ns,:ns] - s1 s1^T / R_total, and L
+ * (ns x J, J = ns - G, row-major) with L L^T = M: Cholesky of M without the last subject of each group (gstart: G + 1
+ * subject offsets), a dropped subject's row = minus the sum of its group's other rows; non-positive pivots give zero
+ * columns.  workspace: plsb200_boot_factor_f64_workspace bytes.                                                 */
+int plsb200_boot_counts_f64(const int32_t* idx, int N, int R, const int32_t* layout, int ns, double* counts,
+                            int64_t ldc, int32_t* bad, void* stream);
+size_t plsb200_boot_factor_f64_workspace(int ns, int G);
+int plsb200_boot_factor_f64(const double* Mg, int ns, int64_t R_total, const int32_t* gstart, int G, double* L,
+                            void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- K4 fast mode: the same moments on the tcgen05 tensor cores with the 3xTF32 split ---------------------
  * (x = xh + xl, c = ch + cl, each TF32-exact; xh.cl + xl.ch + xh.ch accumulated in FP32 in tensor memory, the

@@ -74,6 +74,9 @@ SIGNATURES = {
                                          c_double_p, c_double_p, c_double_p, c_void_p, c_size_t, c_void_p]),
     "plsb200_boot_moments_x32_f64": (c_int, [c_void_p, c_int, c_int64, c_int64, c_double_p, c_int, c_int,
                                              c_double_p, c_double_p, c_double_p, c_void_p, c_size_t, c_void_p]),
+    "plsb200_boot_factor_coef_bytes": (c_size_t, [c_int, c_int, c_int]),
+    "plsb200_boot_factor_pack_f64": (c_int, [c_double_p, c_int, c_int, c_double_p, c_int, c_int32_p, c_double_p,
+                                             c_void_p]),
     "plsb200_boot_quad_coef_bytes": (c_size_t, [c_int, c_int]),
     "plsb200_boot_quad_coef_pack_f64": (c_int, [c_double_p, c_int, c_int, c_double_p, c_void_p]),
     "plsb200_boot_quad_f64_workspace": (c_size_t, [c_int, c_int64, c_int]),
@@ -81,6 +84,11 @@ SIGNATURES = {
                                       c_size_t, c_void_p]),
     "plsb200_boot_quad_x32_f64": (c_int, [c_void_p, c_int, c_int64, c_int64, c_double_p, c_int, c_double_p, c_void_p,
                                           c_size_t, c_void_p]),
+    "plsb200_boot_counts_f64": (c_int, [c_int32_p, c_int, c_int, c_int32_p, c_int, c_double_p, c_int64, c_int32_p,
+                                        c_void_p]),
+    "plsb200_boot_factor_f64_workspace": (c_size_t, [c_int, c_int]),
+    "plsb200_boot_factor_f64": (c_int, [c_double_p, c_int, c_int64, c_int32_p, c_int, c_double_p, c_void_p, c_size_t,
+                                        c_void_p]),
     "plsb200_tf32_ximage_bytes":(c_size_t, [c_int, c_int64]),
     "plsb200_tf32_split_x": (c_int, [c_double_p, c_int, c_int64, c_int64, c_void_p, c_void_p]),
     "plsb200_tf32_split_x32": (c_int, [c_void_p, c_int, c_int64, c_int64, c_void_p, c_void_p]),

@@ -12,8 +12,9 @@ Extra keyword-only arguments (not in the reference): `perm_indices`, `boot_indic
 generated elsewhere -- each an int array, or a (task, behaviour) tuple for mb/cmb), `engine`
 (an `Engine` that already holds X on the device), `device` (CUDA device of the engine built here), `precision` ("fp64" exact mode, or "tf32x3": the
 bootstrap moment GEMM of the task methods on the tcgen05 tensor cores; p-values stay FP64-exact), `boot_algo`
-("direct", default: the bootstrap moments from the B x p x K salience GEMM; "collapsed": mct / cst in the exact mode
-only, the same standard errors from the closed form x_v^T Cov_r(c_rk) x_v -- see `check_boot_algo`), `shard`
+("auto", default: "collapsed" where it does fewer flops, else "direct"; "direct": the bootstrap moments from the
+B x p x K salience GEMM; "collapsed": mct / cst in the exact mode only, the same standard errors from the closed form
+x_v^T Cov_r(c_rk) x_v -- see `check_boot_algo`; `boot_algo` of the result is the one that ran), `shard`
 ("resamples", default, or "voxels": the layout of X in a multi-process run -- see `check_shard`).
 """
 import abc
@@ -356,20 +357,27 @@ def _task_operators(pls_alg, cond_order, mctype, U, contrast):
     return Lop, Ucoef, Lop.T @ Ucoef
 
 
-BOOT_ALGOS = ("direct", "collapsed")
+BOOT_ALGOS = ("auto", "direct", "collapsed")
 
 
-def check_boot_algo(boot_algo, pls_alg, precision, N):
-    """Validates the bootstrap formulation before any GPU work.
+def check_boot_algo(boot_algo, pls_alg, precision, N, nboot=None):
+    """Validates the bootstrap formulation before any GPU work and returns the one that runs.
 
-    "direct" (default) accumulates the moments of the B x p x K bootstrap saliences VS_r = X^T C_r.  "collapsed" uses
-    that every task-method salience is linear in the draw: Var_r(x_v^T c_rk) = x_v^T Cov_r(c_rk) x_v, so the
-    standard errors come from K covariance matrices of N x N and one p x K quadratic form (2 p N^2 K flops instead of
-    2 p N K B: fewer when B > N, more when B < N).  Exact FP64 like the direct form; results agree to rounding."""
+    "direct" accumulates the moments of the B x p x K bootstrap saliences VS_r = X^T C_r.  "collapsed" uses that every
+    task-method salience is linear in the draw: Var_r(x_v^T c_rk) = x_v^T Cov_r(c_rk) x_v.  When the draws have the
+    subject structure of resample.bootstrap_indices, the covariance factors through the draw counts of the ns subjects
+    (DESIGN.md section 3) and the standard errors come from the bootstrap GEMM over ns - G pseudo-resamples
+    (2 p N K (ns - G) flops instead of 2 p N K B); otherwise from K covariance matrices of N x N and one p x K
+    quadratic form (2 p N^2 K flops).  Exact FP64 like the direct form; results agree to rounding.
+    "auto" (default) is "collapsed" for mct / cst with precision="fp64", N <= 320 and more bootstraps (`nboot`, the
+    whole run's) than rows, else "direct"."""
     if boot_algo not in BOOT_ALGOS:
         raise ValueError(f'boot_algo must be one of {BOOT_ALGOS}, got {boot_algo!r}')
+    if boot_algo == "auto":
+        fits = N is not None and N <= Engine.QUAD_MAX_ROWS and nboot is not None and nboot > N
+        return "collapsed" if (pls_alg in ("mct", "cst") and precision == "fp64" and fits) else "direct"
     if boot_algo == "direct":
-        return
+        return boot_algo
     if precision != "fp64":
         raise ValueError(f'boot_algo="collapsed" is an exact (precision="fp64") formulation, got precision={precision!r}')
     if pls_alg not in ("mct", "cst"):
@@ -380,6 +388,7 @@ def check_boot_algo(boot_algo, pls_alg, precision, N):
         raise exceptions.NotImplementedError(
             f'boot_algo="collapsed" supports designs of at most {Engine.QUAD_MAX_ROWS} rows (this one has {N}); '
             'use boot_algo="direct"')
+    return boot_algo
 
 
 X_STORAGES = ("fp64", "fp32")
@@ -420,13 +429,61 @@ def check_shard(shard, pls_alg):
             'per-resample norms over all voxels')
 
 
-def _collapsed_sumsq(eng, E, idx_dev, niter, lo, hi):
+def _factor_plan(eng, pls_alg, U, contrast, cond_order, mctype, niter, indices):
+    """The subject layout for the factored collapsed bootstrap (DESIGN.md section 3), or None when its preconditions
+    do not hold and the N x N covariance route runs instead: every group has the same number of subjects in each
+    condition, E = Lop^T Ucoef is bit-identical within each cell, there are more bootstraps than the factor's ns - G
+    columns (fewer make the count covariance singular), and every draw keeps each row in its cell with one subject map
+    for all conditions.  Indices drawn here (`indices` None) have that structure by construction; given ones are
+    checked on the device, each rank its shard, with the flag all-reduced."""
+    co = np.asarray(cond_order)
+    if co.ndim != 2 or (co != co[:, :1]).any():
+        return None
+    sizes = co[:, 0].astype(np.int64)
+    G, C, ns = co.shape[0], co.shape[1], int(sizes.sum())
+    if niter <= ns - G or ns <= G:
+        return None
+    _, _, E = _task_operators(pls_alg, cond_order, mctype, U, contrast)
+    cells = _cell_offsets(co)
+    if any((E[a:b] != E[a]).any() for a, b in zip(cells[:-1], cells[1:])):
+        return None
+    gstart = np.concatenate(([0], np.cumsum(sizes))).astype(np.int32)
+    base = np.repeat(cells[:-1], co.reshape(-1))                         # first row of each row's cell
+    sid = np.concatenate([gstart[g] + np.arange(sizes[g]) for g in range(G) for _ in range(C)])
+    row0 = np.concatenate([cells[g * C] + np.arange(sizes[g]) for g in range(G)])
+    plan = {"layout": eng.to_device(np.concatenate([base, sid, row0]).astype(np.int32), torch.int32),
+            "sid": eng.to_device(sid.astype(np.int32), torch.int32), "gstart": gstart}
+    if indices is not None:
+        if isinstance(indices, tuple):
+            indices = indices[0]
+        lo, hi = dist.shard(niter)
+        bad = (eng.boot_draw_check(_index_shard(eng, indices, niter, lo, hi), plan["layout"]) if hi > lo
+               else torch.zeros(1, dtype=torch.int32, device=eng.device)).to(torch.int64)
+        dist.allreduce_sum_(bad)
+        if int(bad.item()) != 0:
+            return None
+    return plan
+
+
+def _collapsed_sumsq(eng, E, idx_dev, niter, lo, hi, factor=None):
     """Collapsed bootstrap: q[v,k] = x_v^T S_k x_v with S_k = sum_r (c_rk - e_k)(c_rk - e_k)^T - s1_k s1_k^T / niter
     (= niter . Cov_r(c_rk)): the sum of squares of (VS_r - mean) over all `niter` resamples, p x K, the same on every
-    rank.  Multi-process: one all-reduce of the N-space partial sums, each rank evaluates the quadratic form on its
+    rank.  `factor` (a `_factor_plan`): S_k = D_k P M P^T D_k through the ns x ns covariance M of the subjects' draw
+    counts, M = L L^T, and q is the bootstrap GEMM over the ns - G columns of L; else the K N x N matrices S_k.
+    Multi-process: one all-reduce of the N-space partial sums ([s1 | M] or [S1 | S2]), each rank evaluates q on its
     share of the voxels and the shares are gathered (a voxel-sharded engine: its own voxels, gathered later)."""
     E = eng.to_device(E, torch.float64)
     eng._x_ranges()          # (starts a deferred upload of X: the covariance build below overlaps it)
+    if factor is not None:
+        ns = int(factor["gstart"][-1])
+        Mg = (eng.boot_count_gram(idx_dev, factor["layout"]) if hi > lo
+              else torch.zeros(ns + 1, ns + 1, dtype=torch.float64, device=eng.device))
+        dist.allreduce_sum_(Mg)
+        L = eng.boot_factor(Mg, niter, factor["gstart"])
+        if dist.world()[1] == 1 or eng.voxel_sharded:
+            return eng.boot_factor_quad(E, L, factor["sid"])
+        v0, v1 = dist.shard(eng.p)
+        return dist.gather_rows(eng.boot_factor_quad(E, L, factor["sid"], v0, v1), eng.p, v0)
     if hi > lo:
         S1, S2 = eng.boot_cov(E, idx_dev)
     else:
@@ -454,10 +511,11 @@ class _ResampleTestPLS(ResampleTest):
     def __init__(self, X, Y, U, s, V, cond_order, mctype, contrast=None, preprocess=None, nperm=1000,
                  nboot=1000, bscan=None, Xbscan=None, Ybscan=None, lvcorrs_orig=None, Tvsc_orig=None,
                  CI=0.95, *, perm_indices=None, boot_indices=None, engine=None, precision="fp64", rotate_method=2,
-                 device=None, boot_algo="direct", x_storage="fp64", shard=None):
+                 device=None, boot_algo="auto", x_storage="fp64", shard=None):
         self.CI = CI
-        check_boot_algo(boot_algo, self.pls_alg, engine.precision if engine is not None else precision,
-                        engine.N if engine is not None else (int(X.shape[0]) if X is not None else None))
+        boot_algo = check_boot_algo(boot_algo, self.pls_alg, engine.precision if engine is not None else precision,
+                                    engine.N if engine is not None else (int(X.shape[0]) if X is not None else None),
+                                    nboot)
         check_x_storage(x_storage, self.pls_alg)
         if engine is not None:
             check_x_storage(engine.x_storage, self.pls_alg)
@@ -483,6 +541,10 @@ class _ResampleTestPLS(ResampleTest):
             eng.gram_collective()          # all ranks are here: Gram from per-rank voxel ranges + one all-reduce
         perm_pending = None
         early = None
+        factor = None
+        if eng is not None and nboot > 0 and boot_algo == "collapsed":
+            # (given indices are checked here, before the permutation work is enqueued: one small kernel and one wait)
+            factor = _factor_plan(eng, self.pls_alg, U, contrast, cond_order, mctype, nboot, boot_indices)
         if (eng is not None and eng.upload_in_flight and nboot > 0 and self.pls_alg in ("mct", "cst")
                 and dist.world()[1] == 1):
             # X is still crossing PCIe in voxel ranges (Engine._upload_pipelined): the bootstrap moment GEMM is the
@@ -497,7 +559,7 @@ class _ResampleTestPLS(ResampleTest):
                 boot_indices = resample.bootstrap_indices(self.pls_alg, nboot, cond_order, Y=Y, bscan=bscan,
                                                           Ybscan=Ybscan)
             early = self._bootstrap_moments_early(eng, U, s, V, cond_order, mctype, nboot, self.pls_alg, contrast,
-                                                  boot_indices, boot_algo=boot_algo)
+                                                  boot_indices, boot_algo=boot_algo, _factor=factor)
         if nperm > 0:
             # the permutation kernels and their device->host copies are enqueued here; the host only waits for
             # them after the bootstrap work has been enqueued too, so the GPU never idles between the two tests
@@ -512,7 +574,7 @@ class _ResampleTestPLS(ResampleTest):
             out = self._bootstrap_test(
                 X, Y, U, s, V, cond_order, mctype, nboot, self.pls_alg, preprocess=preprocess, contrast=contrast,
                 bscan=bscan, Xbscan=Xbscan, Ybscan=Ybscan, lvcorrs_orig=lvcorrs_orig, Tvsc_orig=Tvsc_orig, CI=CI,
-                indices=boot_indices, engine=eng, _early=early, boot_algo=boot_algo)
+                indices=boot_indices, engine=eng, _early=early, boot_algo=boot_algo, _factor=factor)
             if self.pls_alg in ("rb", "csb"):
                 self.conf_ints, self.std_errs, self.boot_ratios, self.LVcorr, self.boot_debug_dict = out
             elif self.pls_alg in ("mb", "cmb"):
@@ -657,12 +719,14 @@ class _ResampleTestPLS(ResampleTest):
     @staticmethod
     def _bootstrap_test(X, Y, U, s, V, cond_order, mctype, niter, pls_alg, preprocess=None, dist_=(0.05, 0.95),
                         contrast=None, bscan=None, Xbscan=None, Ybscan=None, lvcorrs_orig=None, Tvsc_orig=None,
-                        CI=0.95, indices=None, engine=None, _early=None, boot_algo="direct"):
+                        CI=0.95, indices=None, engine=None, _early=None, boot_algo="direct", _factor=None):
         """bootstrap_permutation.py:466-766 for the task methods (mct, cst).  `_early`: moments already enqueued by
-        `_bootstrap_moments_early` (pipelined upload of X).  `boot_algo`: see `check_boot_algo`.  A voxel-sharded engine
+        `_bootstrap_moments_early` (pipelined upload of X).  `boot_algo`: see `check_boot_algo` ("auto" resolves here;
+        `_factor`: a `_factor_plan` for "collapsed").  A voxel-sharded engine
         runs the moment GEMM of ALL bootstraps on its voxels (no moment all-reduce) and gathers the p x K results; the
         lazy `right_sv_sampled` and the salience percentiles are then gathered too, so every rank must ask for them."""
         eng = engine if engine is not None else Engine(X)
+        boot_algo = check_boot_algo(boot_algo, pls_alg, eng.precision, eng.N, niter)
         if indices is None:
             indices = resample.bootstrap_indices(pls_alg, niter, cond_order, Y=Y, bscan=bscan, Ybscan=Ybscan)
         if pls_alg in ("mb", "cmb"):
@@ -710,7 +774,7 @@ class _ResampleTestPLS(ResampleTest):
                        else eng.to_host_async(eng.colstd(Tdist), Tdist, left, side=True))
         if boot_algo == "collapsed":
             # sum of squares about the bootstrap mean, already complete on every rank: no p x K all-reduce
-            s2 = _early if _early is not None else _collapsed_sumsq(eng, E, idx_dev, niter, lo, hi)
+            s2 = _early if _early is not None else _collapsed_sumsq(eng, E, idx_dev, niter, lo, hi, factor=_factor)
             s1 = torch.zeros_like(s2)
         else:
             if _early is not None:
@@ -769,7 +833,7 @@ class _ResampleTestPLS(ResampleTest):
     # ------------------------------------------------------------------------------------------
     @staticmethod
     def _bootstrap_moments_early(eng, U, s, V, cond_order, mctype, niter, pls_alg, contrast, indices,
-                                 boot_algo="direct"):
+                                 boot_algo="direct", _factor=None):
         """The moment GEMM of `_bootstrap_test` for the task methods, on its own (single process).  Collapsed: the
         N-space covariance build needs no X, so it runs while X is still crossing PCIe; the quadratic form follows
         range by range as X arrives."""
@@ -777,7 +841,8 @@ class _ResampleTestPLS(ResampleTest):
             indices = indices[0]
         _, _, E = _task_operators(pls_alg, cond_order, mctype, U, contrast)
         if boot_algo == "collapsed":
-            return _collapsed_sumsq(eng, E, _index_shard(eng, indices, niter, 0, niter), niter, 0, niter)
+            return _collapsed_sumsq(eng, E, _index_shard(eng, indices, niter, 0, niter), niter, 0, niter,
+                                    factor=_factor)
         Vd = eng.to_device(V, torch.float64)
         numer = Vd * eng.to_device(np.asarray(s, dtype=float), torch.float64) if contrast is None else Vd
         idx_dev = _index_shard(eng, indices, niter, 0, niter)

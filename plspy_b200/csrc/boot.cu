@@ -76,6 +76,34 @@ __global__ void __launch_bounds__(256) boot_coef_pack_kernel(const double* __res
     for (int i = threadIdx.x; i < stage_doubles / 2; i += blockDim.x) out[i] = in[i];
 }
 
+// The factored collapsed bootstrap (boot_quad.cu, boot_factor_kernel): pseudo-resample j has the coefficients
+// c_j[n,k] = E[n,k] . L[sid[n], j] (L: ns x J, row-major), written in the layout of boot_coef_pack_kernel so that
+// boot_moments_kernel runs on them unchanged.  One CTA per period; slots j >= J stay zero.
+__global__ void __launch_bounds__(256) boot_factor_pack_kernel(const double* __restrict__ E, int N, int K,
+                                                              const double* __restrict__ L, int J,
+                                                              const int32_t* __restrict__ sid, int Kp, int nblk,
+                                                              int nb, int nks, double* __restrict__ coef) {
+    extern __shared__ __align__(16) double smf[];
+    const int stage_doubles = nks * nblk * 32;
+    const int per = blockIdx.x;
+    for (int i = threadIdx.x; i < stage_doubles; i += blockDim.x) smf[i] = 0.0;
+    __syncthreads();
+    for (int e = threadIdx.x; e < nb * N; e += blockDim.x) {
+        const int slot = e / N, i = e % N, j = per * nb + slot;
+        if (j >= J) continue;
+        const double w = L[(size_t)sid[i] * J + j];
+        const int s = i >> 2, q = i & 3;
+        for (int k = 0; k < K; ++k) {
+            const int c = slot * Kp + k;
+            smf[(s * nblk + (c >> 3)) * 32 + 4 * (c & 7) + q] = E[(size_t)i * K + k] * w;
+        }
+    }
+    __syncthreads();
+    double2* out = reinterpret_cast<double2*>(coef + (size_t)per * stage_doubles);
+    const double2* in = reinterpret_cast<const double2*>(smf);
+    for (int i = threadIdx.x; i < stage_doubles / 2; i += blockDim.x) out[i] = in[i];
+}
+
 // ------------------------------------------------------------------------------------------------
 // NKS (k-steps of 4 rows) is a compile-time constant so that the whole period is one straight-line
 // stream of NKS*NBLK {LDS.64, DMMA} pairs that ptxas can software-pipeline; kernels are instantiated
@@ -576,6 +604,31 @@ extern "C" int plsb200_boot_coef_pack_f64(const double* E, int N, int K, const i
     PLSB_CUDA(cudaFuncSetAttribute(boot_coef_pack_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     boot_coef_pack_kernel<<<b.nper, 256, smem, st>>>(E, N, K, idx, R, b.Kp, b.nblk, b.nb, b.nks, coef);
     PLSB_LAUNCH_CHECK("boot_coef_pack_kernel");
+    return PLSB200_OK;
+}
+
+// the register-resident layout only: with PLSB200_EXACT=os (or N > 320) boot_moments_f64 reads another one
+extern "C" size_t plsb200_boot_factor_coef_bytes(int N, int K, int J) {
+    if (use_other(N)) return 0;
+    BootPlan b;
+    if (!boot_plan(N, K, J, 1, b)) return 0;
+    return (size_t)b.nper * b.stage_doubles * sizeof(double);
+}
+
+extern "C" int plsb200_boot_factor_pack_f64(const double* E, int N, int K, const double* L, int J, const int32_t* sid,
+                                            double* coef, void* stream) {
+    PLSB_CHECK_ARG(E && L && sid && coef, "boot_factor_pack_f64: null pointer");
+    BootPlan b;
+    if (use_other(N) || !boot_plan(N, K, J, 1, b)) {
+        set_err("boot_factor_pack_f64: unsupported shape N=%d K=%d J=%d (need K<=24, N<=320, PLSB200_EXACT unset)",
+                N, K, J);
+        return PLSB200_EUNSUPPORTED;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t smem = b.stage_doubles * sizeof(double);
+    PLSB_CUDA(cudaFuncSetAttribute(boot_factor_pack_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    boot_factor_pack_kernel<<<b.nper, 256, smem, st>>>(E, N, K, L, J, sid, b.Kp, b.nblk, b.nb, b.nks, coef);
+    PLSB_LAUNCH_CHECK("boot_factor_pack_kernel");
     return PLSB200_OK;
 }
 

@@ -12,6 +12,8 @@
 // (S_k x_v)[m]; the epilogue folds it as acc[v,k] += X[m,v] . d.  X[m,v] comes from an __ldg issued before the
 // period's MMA stream (the A registers cannot serve it: m is a runtime index).  Pseudo-resamples m >= N and columns
 // k >= K are zero in the pack; the loads of rows m >= N are masked.
+#include <float.h>
+
 #include "common.cuh"
 #include "boot_plan.cuh"
 
@@ -195,9 +197,138 @@ static int quad_dispatch_nks(const BootPlan& b, const T* X, int N, int64_t p, in
     }
 }
 
+// ------------------------------------------------------------------------------------------------
+// Factored form (DESIGN.md section 3).  A draw of resample.bootstrap_indices keeps every row in its cell and uses one
+// subject map for all conditions, and E is constant within a cell, so c_rk[n] = E[n,k] . m_r[subj(n)] with m_r the
+// draw counts of the subjects and S_k = D_k P M P^T D_k, M = sum_r (m_r - 1)(m_r - 1)^T - s1 s1^T / R (ns x ns, the
+// same for every k).  With M = L L^T the quadratic form is a sum of squares over ns - G "pseudo-resamples" c_jk[n] =
+// E[n,k] . L[subj(n), j]: the bootstrap GEMM of boot.cu, run on those.
+//
+// Row layout (int32, 2N + ns): base[n] = first row of n's cell, sid[n] = subject of row n, row0[s] = row of subject s
+// in the first condition of its group.  One CTA per draw: checks the structure (`bad` |= 1 when a row leaves its cell
+// or its subject map differs from the first condition's) and counts the draws of each subject from the first-condition
+// rows (shared-memory integer atomics: the result does not depend on their order).  counts[s][r] = m_r[s] - 1 and
+// counts[ns][r] = 1, so the Gram matrix of `counts` holds sum_r (m_r - 1)(m_r - 1)^T and, in its last column, s1.
+__global__ void boot_counts_kernel(const int32_t* __restrict__ idx, int N, const int32_t* __restrict__ layout, int ns,
+                                   double* __restrict__ counts, long long ldc, int32_t* __restrict__ bad) {
+    extern __shared__ int cnt[];
+    const int32_t* base = layout;
+    const int32_t* sid = layout + N;
+    const int32_t* row0 = layout + 2 * N;
+    const int r = blockIdx.x;
+    const int32_t* id = idx + (size_t)r * N;
+    for (int s = threadIdx.x; s < ns; s += blockDim.x) cnt[s] = 0;
+    __syncthreads();
+    bool ok = true;
+    for (int n = threadIdx.x; n < N; n += blockDim.x) {
+        const int src = id[n], n0 = row0[sid[n]];
+        const int src0 = id[n0];
+        const bool in = src >= 0 && src < N && src0 >= 0 && src0 < N && base[src] == base[n]
+                        && src - base[n] == src0 - base[n0];
+        ok = ok && in;
+        if (in && n == n0) atomicAdd(&cnt[sid[src]], 1);
+    }
+    if (!ok && bad != nullptr) atomicOr(bad, 1);
+    __syncthreads();
+    if (counts == nullptr) return;
+    for (int s = threadIdx.x; s <= ns; s += blockDim.x) counts[(size_t)s * ldc + r] = s < ns ? cnt[s] - 1.0 : 1.0;
+}
+
+// One CTA.  Every m_r - 1 sums to zero within each group, so M has rank <= ns - G: drop the last subject of each
+// group, factor the remaining J x J block A (J = ns - G) by Cholesky, and rebuild a dropped subject's row of L as minus
+// the sum of its group's other rows (L L^T = M).  A pivot <= J eps max(diag A) (a singular A: draws that do not span the
+// subject space) gives a zero column -- the factor of a semidefinite matrix.  A: J x J workspace (global, L2-resident);
+// every element is written by one thread in a fixed order (deterministic).
+__global__ void __launch_bounds__(256) boot_factor_kernel(const double* __restrict__ Mg, int ns, double R,
+                                                          const int32_t* __restrict__ gstart, int G,
+                                                          double* __restrict__ A, double* __restrict__ L) {
+    extern __shared__ int keep[];                       // kept index -> subject
+    __shared__ double piv, tol;
+    const int J = ns - G, ld = ns + 1, tid = threadIdx.x, nt = blockDim.x;
+    for (int a = tid; a < J; a += nt) {
+        int g = 0;
+        while (a >= gstart[g + 1] - (g + 1)) ++g;        // group g keeps gstart[g+1] - gstart[g] - 1 subjects
+        keep[a] = a + g;
+    }
+    __syncthreads();
+    for (int i = tid; i < J * J; i += nt) {
+        const int sa = keep[i / J], sb = keep[i % J];
+        A[i] = Mg[(size_t)sa * ld + sb] - Mg[(size_t)sa * ld + ns] * Mg[(size_t)sb * ld + ns] / R;
+    }
+    __syncthreads();
+    if (tid == 0) {
+        double m = 0.0;
+        for (int a = 0; a < J; ++a) m = fmax(m, A[(size_t)a * J + a]);
+        tol = J * DBL_EPSILON * m;
+    }
+    __syncthreads();
+    for (int j = 0; j < J; ++j) {
+        if (tid == 0) {
+            const double d = A[(size_t)j * J + j];
+            piv = d > tol ? sqrt(d) : 0.0;
+            A[(size_t)j * J + j] = piv;
+        }
+        __syncthreads();
+        const double pj = piv;
+        for (int i = j + 1 + tid; i < J; i += nt) A[(size_t)i * J + j] = pj > 0.0 ? A[(size_t)i * J + j] / pj : 0.0;
+        __syncthreads();
+        const int w = J - j - 1;
+        for (int t = tid; t < w * w; t += nt) {
+            const int i = j + 1 + t / w, k = j + 1 + t % w;
+            if (k <= i) A[(size_t)i * J + k] -= A[(size_t)i * J + j] * A[(size_t)k * J + j];
+        }
+        __syncthreads();
+    }
+    for (int i = tid; i < ns * J; i += nt) {
+        const int s = i / J, j = i % J;
+        int g = 0;
+        while (s >= gstart[g + 1]) ++g;
+        double v = 0.0;
+        if (s == gstart[g + 1] - 1) {                   // dropped subject: minus the sum of the group's kept rows
+            for (int a = gstart[g] - g; a < gstart[g + 1] - g - 1; ++a) v -= j <= a ? A[(size_t)a * J + j] : 0.0;
+        } else {
+            const int a = s - g;
+            v = j <= a ? A[(size_t)a * J + j] : 0.0;
+        }
+        L[i] = v;
+    }
+}
+
 }  // namespace plsb
 
 using namespace plsb;
+
+extern "C" int plsb200_boot_counts_f64(const int32_t* idx, int N, int R, const int32_t* layout, int ns, double* counts,
+                                       int64_t ldc, int32_t* bad, void* stream) {
+    PLSB_CHECK_ARG(idx && layout && (counts || bad), "boot_counts_f64: null pointer");
+    PLSB_CHECK_ARG(N > 0 && R >= 0 && ns > 0 && ns <= N && (counts == nullptr || ldc >= R),
+                   "boot_counts_f64: bad shape N=%d R=%d ns=%d", N, R, ns);
+    if (R == 0) return PLSB200_OK;
+    boot_counts_kernel<<<(unsigned)R, 128, (size_t)ns * sizeof(int), (cudaStream_t)stream>>>(idx, N, layout, ns, counts,
+                                                                                           (long long)ldc, bad);
+    PLSB_LAUNCH_CHECK("boot_counts_kernel");
+    return PLSB200_OK;
+}
+
+extern "C" size_t plsb200_boot_factor_f64_workspace(int ns, int G) {
+    const int J = ns - G;
+    return (G >= 1 && J >= 1) ? (size_t)J * J * sizeof(double) : 0;
+}
+
+extern "C" int plsb200_boot_factor_f64(const double* Mg, int ns, int64_t R_total, const int32_t* gstart, int G,
+                                       double* L, void* workspace, size_t workspace_bytes, void* stream) {
+    PLSB_CHECK_ARG(Mg && gstart && L && workspace, "boot_factor_f64: null pointer");
+    PLSB_CHECK_ARG(G >= 1 && ns > G && R_total > 0, "boot_factor_f64: bad shape ns=%d G=%d", ns, G);
+    const size_t need = plsb200_boot_factor_f64_workspace(ns, G);
+    if (workspace_bytes < need) {
+        set_err("boot_factor_f64: workspace %zu < %zu bytes", workspace_bytes, need);
+        return PLSB200_EWORKSPACE;
+    }
+    boot_factor_kernel<<<1, 256, (size_t)(ns - G) * sizeof(int), (cudaStream_t)stream>>>(
+        Mg, ns, (double)R_total, gstart, G, (double*)workspace, L);
+    PLSB_LAUNCH_CHECK("boot_factor_kernel");
+    return PLSB200_OK;
+}
 
 // the plan of the quadratic form: N pseudo-resamples of N x K coefficients
 static bool quad_plan(int N, int K, int64_t p, BootPlan& b) { return N <= 320 && boot_plan(N, K, N, p, b); }

@@ -774,6 +774,82 @@ class Engine:
                 self._mark("boot_quad")
         return q
 
+    def boot_draw_check(self, idx, layout):
+        """A one-element int32 device tensor, nonzero unless every draw in `idx` keeps each row in its cell and uses one
+        subject map for all conditions (the structure of resample.bootstrap_indices).  `layout`: the int32 row layout of
+        plsb200_boot_counts_f64."""
+        idx = self.to_device(idx, I32); layout = self.to_device(layout, I32)
+        R = int(idx.shape[0])
+        ns = int(layout.numel()) - 2 * self.N
+        bad = torch.zeros(1, dtype=I32, device=self.device)
+        with torch.cuda.device(self.device):
+            check(lib.plsb200_boot_counts_f64(self._p(idx), self.N, R, self._p(layout), ns, None, 0, self._p(bad),
+                                              self._stream()), "boot_counts_f64")
+        return bad
+
+    def boot_count_gram(self, idx, layout):
+        """Factored collapsed bootstrap, N-space part of the resamples in `idx`: the (ns + 1)-square Gram matrix of
+        [m_r - 1; 1] over the draws (m_r: draws of each subject).  Integer entries, so exact in any summation order; a
+        multi-process run all-reduces it."""
+        idx = self.to_device(idx, I32); layout = self.to_device(layout, I32)
+        R = int(idx.shape[0])
+        ns = int(layout.numel()) - 2 * self.N
+        counts = self._empty(ns + 1, R)
+        with torch.cuda.device(self.device):
+            check(lib.plsb200_boot_counts_f64(self._p(idx), self.N, R, self._p(layout), ns, self._p(counts), R, None,
+                                              self._stream()), "boot_counts_f64")
+        return self.gram_of(counts)
+
+    def boot_factor(self, Mg, R_total, gstart):
+        """L (ns x (ns - G)) with L L^T = sum_r (m_r - 1)(m_r - 1)^T - s1 s1^T / R_total from `boot_count_gram`'s
+        matrix (summed over every resample); one CTA, no host synchronisation."""
+        gstart = self.to_device(gstart, I32)
+        ns, G = int(Mg.shape[0]) - 1, int(gstart.numel()) - 1
+        L = self._empty(ns, ns - G)
+        with torch.cuda.device(self.device):
+            ws = self._ws(lib.plsb200_boot_factor_f64_workspace(ns, G))
+            check(lib.plsb200_boot_factor_f64(self._p(Mg), ns, int(R_total), self._p(gstart), G, self._p(L), self._p(ws),
+                                              ws.numel(), self._stream()), "boot_factor_f64")
+        return L
+
+    def boot_factor_quad(self, E, L, sid, v0=0, v1=None):
+        """q[v,k] = sum_j (x_v^T c_jk)^2 with c_jk[n] = E[n,k] L[sid[n], j], for the voxels v0 <= v < v1: the bootstrap
+        moment GEMM on the J columns of L as pseudo-resamples (no pivot).  With L L^T the draw-count covariance this is
+        the q of `boot_quad`.  One launch per voxel range of a pipelined upload, each after its range has arrived."""
+        E = self.to_device(E, F64); sid = self.to_device(sid, I32)
+        K, J = int(E.shape[1]), int(L.shape[1])
+        v1 = self.p if v1 is None else int(v1)
+        if K > self.KMAX:   # columns are independent: split wide problems
+            return torch.cat([self.boot_factor_quad(E[:, k0:k0 + self.KMAX].contiguous(), L, sid, v0, v1)
+                              for k0 in range(0, K, self.KMAX)], dim=1)
+        q = self._empty(max(v1 - v0, 0), K)
+        if v1 <= v0:
+            return q
+        s1 = self._empty(v1 - v0, K)                 # sum_j x_v^T c_jk: not needed, the kernel writes it
+        with torch.cuda.device(self.device):
+            nbytes = lib.plsb200_boot_factor_coef_bytes(self.N, K, J)
+            if nbytes == 0:
+                raise _lib.PlsB200Error(f"boot_factor_quad: unsupported shape N={self.N} K={K} J={J}")
+            coef = self._ws(nbytes)
+            check(lib.plsb200_boot_factor_pack_f64(self._p(E), self.N, K, self._p(L), J, self._p(sid), self._p(coef),
+                                                   self._stream()), "boot_factor_pack_f64")
+            cur = torch.cuda.current_stream(self.device)
+            fn, what = ((lib.plsb200_boot_moments_x32_f64, "boot_moments_x32_f64") if self._x32(self._X)
+                        else (lib.plsb200_boot_moments_f64, "boot_moments_f64"))
+            for a, b, ev in self._x_ranges():
+                lo, hi = max(a, v0), min(b, v1)
+                if lo >= hi:
+                    continue
+                if ev is not None:
+                    cur.wait_event(ev)
+                ws = self._ws(lib.plsb200_boot_moments_f64_workspace(self.N, hi - lo, K, J))
+                off = 8 * (lo - v0) * K
+                self._mark("boot_moments")
+                check(fn(self._xp(lo), self.N, hi - lo, self.ldx, self._p(coef), K, J, None, s1.data_ptr() + off,
+                         q.data_ptr() + off, self._p(ws), ws.numel(), self._stream()), what)
+                self._mark("boot_moments")
+        return q
+
     def boot_finalize(self, s1, s2, R_total, numer=None):
         K = int(s1.shape[1])
         se = self._empty(self.p, K)

@@ -22,10 +22,12 @@ def PLS(*args, **kwargs):
     `rotate_method` (2 = derived, the reference's behaviour and the default; 1 = Procrustes; 0 = per-permutation SVD,
     mct only -- see `_ResampleTestPLS._permutation_test`), `analysis` ("host" = LAPACK on the cross-block matrix as
     in the reference, default; "device" = through the Gram matrix on the GPU, sign of each latent
-    variable fixed by convention -- see device_analysis.py), `boot_algo` ("direct" = the bootstrap moments of the
-    B x p x K salience GEMM, default; "collapsed" = mct / cst with precision="fp64" and at most 320 rows: the same exact
-    standard errors from K covariance matrices of N x N and one p x K quadratic form, about N / B of the direct
-    form's flops, so faster when num_boot > N -- see bootstrap_permutation.check_boot_algo), `x_storage` ("fp64" =
+    variable fixed by convention -- see device_analysis.py), `boot_algo` ("auto" = "collapsed" for mct / cst
+    with precision="fp64", at most 320 rows and num_boot > N, else "direct", default; "direct" = the bootstrap moments of
+    the B x p x K salience GEMM; "collapsed" = mct / cst with precision="fp64" and at most 320 rows: the same exact
+    standard errors from the covariance of the subjects' draw counts (a GEMM over ns - G pseudo-resamples, ns subjects
+    in G groups) or, for draws without that structure, from K covariance matrices of N x N -- see
+    bootstrap_permutation.check_boot_algo; `resample_tests.boot_algo` reports the one that ran), `x_storage` ("fp64" =
     X held as float64 on the device, default; "fp32" = mct / cst: X.astype(float32) held as float32 -- half the device
     memory -- with every result bit-identical to the "fp64" run on the widened float32 matrix; the host-side steps see
     the same widened values -- see bootstrap_permutation.check_x_storage), `shard` ("resamples" = in a multi-process

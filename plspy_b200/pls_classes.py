@@ -244,7 +244,7 @@ class PLSBase(abc.ABC):
             boot_indices=self._engine_kwargs.get("boot_indices"),
             engine=self._engine_kwargs.get("engine"), precision=self._engine_kwargs.get("precision", "fp64"),
             rotate_method=self._engine_kwargs.get("rotate_method", 2), device=self._engine_kwargs.get("device"),
-            boot_algo=self._engine_kwargs.get("boot_algo", "direct"), x_storage=self._engine_kwargs["x_storage"],
+            boot_algo=self._engine_kwargs.get("boot_algo", "auto"), x_storage=self._engine_kwargs["x_storage"],
             shard=self._engine_kwargs["shard"], **kw)
 
     def _split_half(self, Y, mctype, contrasts, **kw):

@@ -29,7 +29,7 @@ from .engine import Engine
 METHODS = ("mct", "rb", "cst", "csb", "mb", "cmb")
 
 _state = None          # what install() replaced, for uninstall()
-_options = {"precision": "fp64", "boot_algo": "direct", "x_storage": "fp64", "shard": "resamples"}
+_options = {"precision": "fp64", "boot_algo": "auto", "x_storage": "fp64", "shard": "resamples"}
 _shared = {"ref": None, "engine": None}
 
 
@@ -94,10 +94,11 @@ def _split_half(pls_alg, matrix, Y, cond_order, num_split, mctype=None, contrast
                           Xbscan=Xbscan, Ybscan=Ybscan, lv=lv, CI=CI, engine=shared_engine(matrix))
 
 
-def install(plspy_module=None, precision="fp64", boot_algo="direct", x_storage="fp64", shard="resamples"):
+def install(plspy_module=None, precision="fp64", boot_algo="auto", x_storage="fp64", shard="resamples"):
     """Route the permutation / bootstrap / split-half loops of `plspy_module` (default: `import plspy`) through the
     GPU engine.  Idempotent; returns the module.  `precision`: "fp64" (exact) or "tf32x3" (fast bootstrap GEMM).
-    `boot_algo`: "direct" or "collapsed" (mct / cst in the exact mode: see `bootstrap_permutation.check_boot_algo`);
+    `boot_algo`: "auto" (default), "direct" or "collapsed" (mct / cst in the exact mode: see
+    `bootstrap_permutation.check_boot_algo`);
     a per-call option, applied to every resampling test while installed.  `x_storage`: "fp64" or "fp32" (mct / cst:
     the engine holds X as float32, see `bootstrap_permutation.check_x_storage`; the reference's own host analysis
     still sees X as passed, so the results are bit-identical to "fp64" when X holds float32 values).  Behaviour and
