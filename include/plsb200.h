@@ -161,9 +161,10 @@ int plsb200_boot_moments_x32_f64(const float* X, int N, int64_t p, int64_t ldx, 
                                  void* workspace, size_t workspace_bytes, void* stream);
 /* Factored collapsed bootstrap (task methods; DESIGN.md section 3): J pseudo-resamples with the coefficients
  * c_j[n,k] = E[n,k] . L[sid[n], j] (L: ns x J row-major, sid: N subjects) packed for plsb200_boot_moments_f64 /
- * _x32_f64, which then run with R = J and pivot = NULL: their `sumsq` is q[v,k] = sum_j (x_v^T c_jk)^2.  The size
- * query returns 0 (and the pack PLSB200_EUNSUPPORTED) where boot_moments reads another layout (N > 320 or
- * PLSB200_EXACT=os) or K > 24.                                                                                  */
+ * _x32_f64, which then run with R = J and pivot = NULL: their `sumsq` is q[v,k] = sum_j (x_v^T c_jk)^2.  Any N:
+ * the pack writes the layout boot_moments reads (the register-resident kernel's for N <= 320, the output-stationary
+ * kernel's for N > 320 or with PLSB200_EXACT=os).  The size query returns 0 (and the pack PLSB200_EUNSUPPORTED) for
+ * K > 24 and where boot_moments runs the row-split kernel (N > 320 with PLSB200_TALL=rs).                        */
 size_t plsb200_boot_factor_coef_bytes(int N, int K, int J);
 int plsb200_boot_factor_pack_f64(const double* E, int N, int K, const double* L, int J, const int32_t* sid,
                                  double* coef, void* stream);

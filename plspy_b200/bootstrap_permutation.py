@@ -360,17 +360,20 @@ def _task_operators(pls_alg, cond_order, mctype, U, contrast):
 BOOT_ALGOS = ("auto", "direct", "collapsed")
 
 
-def check_boot_algo(boot_algo, pls_alg, precision, N, nboot=None):
+def check_boot_algo(boot_algo, pls_alg, precision, N, nboot=None, cond_order=None):
     """Validates the bootstrap formulation before any GPU work and returns the one that runs.
 
     "direct" accumulates the moments of the B x p x K bootstrap saliences VS_r = X^T C_r.  "collapsed" uses that every
     task-method salience is linear in the draw: Var_r(x_v^T c_rk) = x_v^T Cov_r(c_rk) x_v.  When the draws have the
     subject structure of resample.bootstrap_indices, the covariance factors through the draw counts of the ns subjects
     (DESIGN.md section 3) and the standard errors come from the bootstrap GEMM over ns - G pseudo-resamples
-    (2 p N K (ns - G) flops instead of 2 p N K B); otherwise from K covariance matrices of N x N and one p x K
-    quadratic form (2 p N^2 K flops).  Exact FP64 like the direct form; results agree to rounding.
-    "auto" (default) is "collapsed" for mct / cst with precision="fp64", N <= 320 and more bootstraps (`nboot`, the
-    whole run's) than rows, else "direct"."""
+    (2 p N K (ns - G) flops instead of 2 p N K B); otherwise, for N <= 320, from K covariance matrices of N x N and one
+    p x K quadratic form (2 p N^2 K flops).  Exact FP64 like the direct form; results agree to rounding.
+    Beyond 320 rows only the factored route exists, so "collapsed" there needs `cond_order` (G x C subject counts)
+    with every group the same size in each of its conditions (groups may differ) and more bootstraps (`nboot`, the
+    whole run's) than ns - G; draws passed in must also have the subject structure (checked on the device).
+    "auto" (default) is "collapsed" for mct / cst with precision="fp64", N <= 320 and more bootstraps than rows, else
+    "direct"."""
     if boot_algo not in BOOT_ALGOS:
         raise ValueError(f'boot_algo must be one of {BOOT_ALGOS}, got {boot_algo!r}')
     if boot_algo == "auto":
@@ -385,9 +388,17 @@ def check_boot_algo(boot_algo, pls_alg, precision, N, nboot=None):
             'boot_algo="collapsed" applies to the task methods (mct, cst): the block standardisation of the behaviour '
             'and multiblock methods makes their saliences non-linear in the bootstrap draw')
     if N is not None and N > Engine.QUAD_MAX_ROWS:
-        raise exceptions.NotImplementedError(
-            f'boot_algo="collapsed" supports designs of at most {Engine.QUAD_MAX_ROWS} rows (this one has {N}); '
-            'use boot_algo="direct"')
+        co = None if cond_order is None else np.asarray(cond_order)
+        balanced = co is not None and co.ndim == 2 and co.size > 0 and bool((co == co[:, :1]).all())
+        ns_g = int(co[:, 0].sum()) - co.shape[0] if balanced else None
+        if not (balanced and nboot is not None and nboot > ns_g >= 1):
+            have = ("no cond_order" if co is None else "unequal subject counts across conditions" if not balanced
+                    else f"num_boot={nboot}, ns - G = {ns_g}")
+            raise exceptions.NotImplementedError(
+                f'boot_algo="collapsed" for a design of {N} rows: the N x N covariance route is limited to '
+                f'{Engine.QUAD_MAX_ROWS} rows, and the factored route needs a cond_order in which every group has the '
+                f'same number of subjects in each condition and more bootstraps than ns - G (subjects minus groups) '
+                f'({have}); use boot_algo="direct"')
     return boot_algo
 
 
@@ -435,7 +446,20 @@ def _factor_plan(eng, pls_alg, U, contrast, cond_order, mctype, niter, indices):
     condition, E = Lop^T Ucoef is bit-identical within each cell, there are more bootstraps than the factor's ns - G
     columns (fewer make the count covariance singular), and every draw keeps each row in its cell with one subject map
     for all conditions.  Indices drawn here (`indices` None) have that structure by construction; given ones are
-    checked on the device, each rank its shard, with the flag all-reduced."""
+    checked on the device, each rank its shard, with the flag all-reduced.  Designs of more than 320 rows have no
+    N x N route: there exceptions.NotImplementedError replaces None (on every rank)."""
+    plan = _factor_plan_or_none(eng, pls_alg, U, contrast, cond_order, mctype, niter, indices)
+    if plan is None and eng.N > Engine.QUAD_MAX_ROWS:
+        raise exceptions.NotImplementedError(
+            f'boot_algo="collapsed" for a design of {eng.N} rows: the N x N covariance route is limited to '
+            f'{Engine.QUAD_MAX_ROWS} rows, and the factored route needs every group to have the same number of '
+            'subjects in each condition, more bootstraps than ns - G, design weights constant within each cell and '
+            'bootstrap draws with the subject structure of resample.bootstrap_indices (each row drawn from its own '
+            'cell, one subject map for all conditions); use boot_algo="direct"')
+    return plan
+
+
+def _factor_plan_or_none(eng, pls_alg, U, contrast, cond_order, mctype, niter, indices):
     co = np.asarray(cond_order)
     if co.ndim != 2 or (co != co[:, :1]).any():
         return None
@@ -515,7 +539,7 @@ class _ResampleTestPLS(ResampleTest):
         self.CI = CI
         boot_algo = check_boot_algo(boot_algo, self.pls_alg, engine.precision if engine is not None else precision,
                                     engine.N if engine is not None else (int(X.shape[0]) if X is not None else None),
-                                    nboot)
+                                    nboot, cond_order)
         check_x_storage(x_storage, self.pls_alg)
         if engine is not None:
             check_x_storage(engine.x_storage, self.pls_alg)
@@ -726,9 +750,11 @@ class _ResampleTestPLS(ResampleTest):
         runs the moment GEMM of ALL bootstraps on its voxels (no moment all-reduce) and gathers the p x K results; the
         lazy `right_sv_sampled` and the salience percentiles are then gathered too, so every rank must ask for them."""
         eng = engine if engine is not None else Engine(X)
-        boot_algo = check_boot_algo(boot_algo, pls_alg, eng.precision, eng.N, niter)
+        boot_algo = check_boot_algo(boot_algo, pls_alg, eng.precision, eng.N, niter, cond_order)
         if indices is None:
             indices = resample.bootstrap_indices(pls_alg, niter, cond_order, Y=Y, bscan=bscan, Ybscan=Ybscan)
+        if boot_algo == "collapsed" and _factor is None and _early is None and eng.N > Engine.QUAD_MAX_ROWS:
+            _factor = _factor_plan(eng, pls_alg, U, contrast, cond_order, mctype, niter, indices)   # the only route
         if pls_alg in ("mb", "cmb"):
             return _boot_multiblock(eng, U, s, V, cond_order, mctype, niter, pls_alg, contrast, bscan, Ybscan,
                                     lvcorrs_orig, Tvsc_orig, CI, indices)

@@ -607,9 +607,10 @@ extern "C" int plsb200_boot_coef_pack_f64(const double* E, int N, int K, const i
     return PLSB200_OK;
 }
 
-// the register-resident layout only: with PLSB200_EXACT=os (or N > 320) boot_moments_f64 reads another one
+// the layout boot_moments_f64 reads: the register-resident one, else (N > 320 or PLSB200_EXACT=os) that of the
+// output-stationary kernel; the row-split kernel (PLSB200_TALL=rs) has no factored pack
 extern "C" size_t plsb200_boot_factor_coef_bytes(int N, int K, int J) {
-    if (use_other(N)) return 0;
+    if (use_other(N)) return use_os(N) ? boot_os_coef_bytes(N, K, J) : 0;
     BootPlan b;
     if (!boot_plan(N, K, J, 1, b)) return 0;
     return (size_t)b.nper * b.stage_doubles * sizeof(double);
@@ -618,13 +619,21 @@ extern "C" size_t plsb200_boot_factor_coef_bytes(int N, int K, int J) {
 extern "C" int plsb200_boot_factor_pack_f64(const double* E, int N, int K, const double* L, int J, const int32_t* sid,
                                             double* coef, void* stream) {
     PLSB_CHECK_ARG(E && L && sid && coef, "boot_factor_pack_f64: null pointer");
+    PLSB_CHECK_ARG(N > 0 && J > 0, "boot_factor_pack_f64: bad shape N=%d J=%d", N, J);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (use_other(N)) {
+        if (!use_os(N)) {
+            set_err("boot_factor_pack_f64: the row-split kernel (PLSB200_TALL=rs) has no factored layout; "
+                    "unset PLSB200_TALL");
+            return PLSB200_EUNSUPPORTED;
+        }
+        return boot_os_factor_pack(E, N, K, L, J, sid, coef, st);
+    }
     BootPlan b;
-    if (use_other(N) || !boot_plan(N, K, J, 1, b)) {
-        set_err("boot_factor_pack_f64: unsupported shape N=%d K=%d J=%d (need K<=24, N<=320, PLSB200_EXACT unset)",
-                N, K, J);
+    if (!boot_plan(N, K, J, 1, b)) {
+        set_err("boot_factor_pack_f64: unsupported shape N=%d K=%d J=%d (need K<=24)", N, K, J);
         return PLSB200_EUNSUPPORTED;
     }
-    cudaStream_t st = (cudaStream_t)stream;
     const size_t smem = b.stage_doubles * sizeof(double);
     PLSB_CUDA(cudaFuncSetAttribute(boot_factor_pack_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     boot_factor_pack_kernel<<<b.nper, 256, smem, st>>>(E, N, K, L, J, sid, b.Kp, b.nblk, b.nb, b.nks, coef);

@@ -115,6 +115,27 @@ __global__ void __launch_bounds__(256) boot_os_pack_kernel(const double* __restr
     }
 }
 
+// The factored collapsed bootstrap (boot_quad.cu, boot_factor_kernel) for this kernel: pseudo-resample j has the
+// coefficients c_j[n,k] = E[n,k] . L[sid[n], j] (L: ns x J, row-major), written at the offsets of boot_os_pack_kernel
+// (r = j).  No scatter, so no source lists: one CTA per pseudo-resample, a thread per row.  The padding (rows up to
+// 4 nks, k >= K inside Kp, the tail of the last column tile) is the memset of boot_os_factor_pack.
+__global__ void __launch_bounds__(256) boot_os_factor_pack_kernel(const double* __restrict__ E, int N, int K,
+                                                                 const double* __restrict__ L, int J,
+                                                                 const int32_t* __restrict__ sid, int Kp, int nks,
+                                                                 double* __restrict__ coef) {
+    const int j = blockIdx.x;
+    for (int i = threadIdx.x; i < N; i += blockDim.x) {
+        const double w = __ldg(L + (size_t)__ldg(sid + i) * J + j);
+        const int s = i >> 2, q = i & 3;
+        for (int k = 0; k < K; ++k) {
+            const long long c = (long long)j * Kp + k;
+            const long long ct = c / OS_TN;
+            const int cin = (int)(c % OS_TN);
+            coef[(((size_t)ct * nks + s) * OS_NB + (cin >> 3)) * 32 + 4 * (cin & 7) + q] = __ldg(E + (size_t)i * K + k) * w;
+        }
+    }
+}
+
 // Tile-major image of X: block (t, sb) = rows [4 ks sb, 4 ks (sb + 1)) x voxels [128 t, 128 t + 128) at a pitch of 132
 // doubles, zero-filled beyond N rows / p voxels (and in the 4 padding columns).  One pass over X per call
 // (3.5 ms for the 9.6 GB of BASELINE config 5, against 2.4 s of GEMM).  T = float: X stored as float32, widened here,
@@ -358,6 +379,20 @@ int boot_os_pack(const double* E, int N, int K, const int32_t* idx, int R, doubl
     PLSB_CUDA(cudaMemsetAsync(coef, 0, (size_t)b.nct * b.nks * OS_NB * 32 * sizeof(double), st));
     boot_os_pack_kernel<<<R, 256, (size_t)(4 * N + 1) * sizeof(int), st>>>(E, N, K, idx, b.Kp, b.nks, coef);
     PLSB_LAUNCH_CHECK("boot_os_pack_kernel");
+    return PLSB200_OK;
+}
+
+// the layout is that of boot_os_pack with R = J, so boot_os_coef_bytes(N, K, J) sizes it
+int boot_os_factor_pack(const double* E, int N, int K, const double* L, int J, const int32_t* sid, double* coef,
+                        cudaStream_t st) {
+    OsPlan b;
+    if (!os_plan(N, K, J, 1, b)) {
+        set_err("boot_factor_pack_f64: unsupported shape N=%d K=%d J=%d (need K<=24)", N, K, J);
+        return PLSB200_EUNSUPPORTED;
+    }
+    PLSB_CUDA(cudaMemsetAsync(coef, 0, (size_t)b.nct * b.nks * OS_NB * 32 * sizeof(double), st));
+    boot_os_factor_pack_kernel<<<J, 256, 0, st>>>(E, N, K, L, J, sid, b.Kp, b.nks, coef);
+    PLSB_LAUNCH_CHECK("boot_os_factor_pack_kernel");
     return PLSB200_OK;
 }
 

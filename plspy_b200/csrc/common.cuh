@@ -68,6 +68,9 @@ bool boot_os_usable(const double* X, int64_t p, int64_t ldx);
 size_t boot_os_coef_bytes(int N, int K, int R);
 size_t boot_os_workspace(int N, int64_t p, int K, int R);
 int boot_os_pack(const double* E, int N, int K, const int32_t* idx, int R, double* coef, cudaStream_t st);
+// the factored collapsed bootstrap's J pseudo-resamples in the same layout (boot_os_coef_bytes(N, K, J) bytes)
+int boot_os_factor_pack(const double* E, int N, int K, const double* L, int J, const int32_t* sid, double* coef,
+                        cudaStream_t st);
 int boot_os_moments(const double* X, int N, int64_t p, int64_t ldx, const double* coef, int K, int R,
                     const double* pivot, double* sum, double* sumsq, void* workspace, size_t workspace_bytes,
                     cudaStream_t st, const char* what);

@@ -829,7 +829,8 @@ class Engine:
         with torch.cuda.device(self.device):
             nbytes = lib.plsb200_boot_factor_coef_bytes(self.N, K, J)
             if nbytes == 0:
-                raise _lib.PlsB200Error(f"boot_factor_quad: unsupported shape N={self.N} K={K} J={J}")
+                raise _lib.PlsB200Error(f"boot_factor_quad: unsupported shape N={self.N} K={K} J={J} (the row-split "
+                                        "kernel of PLSB200_TALL=rs has no factored layout)")
             coef = self._ws(nbytes)
             check(lib.plsb200_boot_factor_pack_f64(self._p(E), self.N, K, self._p(L), J, self._p(sid), self._p(coef),
                                                    self._stream()), "boot_factor_pack_f64")

@@ -1,4 +1,8 @@
 """`PLS(...)` driver with the reference's signature and argument validation (plspy/core/pls.py:21-93)."""
+import inspect
+
+import numpy as np
+
 from . import bootstrap_permutation, pls_classes
 
 methods = {
@@ -9,6 +13,25 @@ methods = {
     "mb": pls_classes._MultiblockPLS,
     "cmb": pls_classes._ContrastMultiblockPLS,
 }
+
+
+def _boot_layout(pls_method, args, kwargs):
+    """(num_boot, cond_order) of a PLS(...) call as the method class will see them -- its defaults included, the
+    cond_order derived from groups_sizes and num_conditions when not given -- or None where they cannot be read (the
+    class reports malformed arguments itself)."""
+    try:
+        bound = inspect.signature(methods[pls_method]).bind(*args, **kwargs)
+    except (KeyError, TypeError):
+        return None, None
+    bound.apply_defaults()
+    a = bound.arguments
+    cond_order = a.get("cond_order")
+    if cond_order is None:
+        try:
+            cond_order = np.array([[int(n)] * int(a["num_conditions"]) for n in a["groups_sizes"]])
+        except (KeyError, TypeError, ValueError):
+            cond_order = None
+    return a.get("num_boot"), cond_order
 
 
 def PLS(*args, **kwargs):
@@ -24,9 +47,10 @@ def PLS(*args, **kwargs):
     in the reference, default; "device" = through the Gram matrix on the GPU, sign of each latent
     variable fixed by convention -- see device_analysis.py), `boot_algo` ("auto" = "collapsed" for mct / cst
     with precision="fp64", at most 320 rows and num_boot > N, else "direct", default; "direct" = the bootstrap moments of
-    the B x p x K salience GEMM; "collapsed" = mct / cst with precision="fp64" and at most 320 rows: the same exact
-    standard errors from the covariance of the subjects' draw counts (a GEMM over ns - G pseudo-resamples, ns subjects
-    in G groups) or, for draws without that structure, from K covariance matrices of N x N -- see
+    the B x p x K salience GEMM; "collapsed" = mct / cst with precision="fp64": the same exact standard errors from
+    the covariance of the subjects' draw counts (a GEMM over ns - G pseudo-resamples, ns subjects in G groups) or, for
+    draws without that structure and at most 320 rows, from K covariance matrices of N x N; beyond 320 rows it needs
+    every group to have the same number of subjects in each condition and num_boot > ns - G -- see
     bootstrap_permutation.check_boot_algo; `resample_tests.boot_algo` reports the one that ran), `x_storage` ("fp64" =
     X held as float64 on the device, default; "fp32" = mct / cst: X.astype(float32) held as float32 -- half the device
     memory -- with every result bit-identical to the "fp64" run on the widened float32 matrix; the host-side steps see
@@ -55,9 +79,11 @@ def PLS(*args, **kwargs):
     if "boot_algo" in kwargs:        # before any GPU work (the engine's upload of X starts with the analysis)
         X = args[0] if args else kwargs.get("X")
         engine = kwargs.get("engine")
+        nboot, cond_order = _boot_layout(pls_method, args, kwargs)
         bootstrap_permutation.check_boot_algo(
             kwargs["boot_algo"], pls_method, engine.precision if engine is not None else kwargs.get("precision", "fp64"),
-            engine.N if engine is not None else (int(X.shape[0]) if X is not None and hasattr(X, "shape") else None))
+            engine.N if engine is not None else (int(X.shape[0]) if X is not None and hasattr(X, "shape") else None),
+            nboot, cond_order)
     if "x_storage" in kwargs:
         bootstrap_permutation.check_x_storage(kwargs["x_storage"], pls_method)
     if "shard" in kwargs:

@@ -62,12 +62,16 @@ class _InstalledResampleTest(_bp._ResampleTestPLS):
         nboot = kwargs.get("nboot", 1000)
         kwargs.setdefault("x_storage", _options["x_storage"])
         kwargs.setdefault("shard", _options["shard"])
-        _bp.check_x_storage(kwargs["x_storage"], self.pls_alg)        # before the engine uploads X
-        _bp.check_shard(kwargs["shard"], self.pls_alg)
-        if "engine" not in kwargs and (nperm > 0 or nboot > 0):
-            kwargs["engine"] = shared_engine(X)
         kwargs.setdefault("precision", _options["precision"])
         kwargs.setdefault("boot_algo", _options["boot_algo"])
+        _bp.check_x_storage(kwargs["x_storage"], self.pls_alg)        # before the engine uploads X
+        _bp.check_shard(kwargs["shard"], self.pls_alg)
+        eng = kwargs.get("engine")
+        _bp.check_boot_algo(kwargs["boot_algo"], self.pls_alg, eng.precision if eng is not None else kwargs["precision"],
+                            eng.N if eng is not None else (int(X.shape[0]) if hasattr(X, "shape") else None), nboot,
+                            cond_order)
+        if "engine" not in kwargs and (nperm > 0 or nboot > 0):
+            kwargs["engine"] = shared_engine(X)
         super().__init__(X, Y, U, s, V, cond_order, mctype, *args, **kwargs)
 
 
@@ -97,8 +101,9 @@ def _split_half(pls_alg, matrix, Y, cond_order, num_split, mctype=None, contrast
 def install(plspy_module=None, precision="fp64", boot_algo="auto", x_storage="fp64", shard="resamples"):
     """Route the permutation / bootstrap / split-half loops of `plspy_module` (default: `import plspy`) through the
     GPU engine.  Idempotent; returns the module.  `precision`: "fp64" (exact) or "tf32x3" (fast bootstrap GEMM).
-    `boot_algo`: "auto" (default), "direct" or "collapsed" (mct / cst in the exact mode: see
-    `bootstrap_permutation.check_boot_algo`);
+    `boot_algo`: "auto" (default), "direct" or "collapsed" (mct / cst in the exact mode; beyond 320 rows every group
+    needs the same number of subjects in each condition and more bootstraps than subjects minus groups, checked per
+    resampling test before X is uploaded: see `bootstrap_permutation.check_boot_algo`);
     a per-call option, applied to every resampling test while installed.  `x_storage`: "fp64" or "fp32" (mct / cst:
     the engine holds X as float32, see `bootstrap_permutation.check_x_storage`; the reference's own host analysis
     still sees X as passed, so the results are bit-identical to "fp64" when X holds float32 values).  Behaviour and
