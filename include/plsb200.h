@@ -62,8 +62,7 @@ int plsb200_widen_f32_f64(const float* src, double* dst, int64_t n, void* stream
  * dimension ldx in elements, any 4-byte aligned address and any ldx): each element is widened to float64 where the
  * kernel loads it, so the results are bit-identical to the twin's on the widened matrix.  Sizes and workspaces are
  * the twin's (plsb200_gram_f64_workspace, plsb200_xv_f64_workspace, plsb200_boot_moments_f64_workspace,
- * plsb200_boot_quad_f64_workspace, plsb200_tf32_ximage_bytes, plsb200_gram_tf32_image_bytes).  The row-split tall
- * kernel (PLSB200_TALL=rs) has no float32 variant: boot_moments_x32_f64 returns PLSB200_EUNSUPPORTED there. */
+ * plsb200_boot_quad_f64_workspace, plsb200_tf32_ximage_bytes, plsb200_gram_tf32_image_bytes).                */
 
 /* ---- K1: Gram matrix G = X . X^T (N x N), FP64 DMMA, split over voxel chunks, deterministic --------
  * Replaces the N x p work that every resample redoes in the reference (row gather + means + projection,
@@ -148,7 +147,7 @@ int plsb200_gram_tf32(const void* image, int N, int64_t p, double* G, int accumu
  * Step 1 packs the coefficients C_r = scatter(E, idx_r) into the DMMA B-fragment order the kernel
  * streams through shared memory (`coef`, size from plsb200_boot_coef_bytes).
  * Step 2 runs the GEMM+moment kernel.  pivot (p x K) may be NULL (= 0).  sum, sumsq: p x K, overwritten.
- * Supported shapes: K <= 24 per call (split wider problems by column), N <= 320 * 4.               */
+ * Supported shapes: K <= 24 per call (split wider problems by column), any N.                     */
 size_t plsb200_boot_coef_bytes(int N, int K, int R);
 int plsb200_boot_coef_pack_f64(const double* E, int N, int K, const int32_t* idx, int R, double* coef,
                                void* stream);
@@ -164,7 +163,7 @@ int plsb200_boot_moments_x32_f64(const float* X, int N, int64_t p, int64_t ldx, 
  * _x32_f64, which then run with R = J and pivot = NULL: their `sumsq` is q[v,k] = sum_j (x_v^T c_jk)^2.  Any N:
  * the pack writes the layout boot_moments reads (the register-resident kernel's for N <= 320, the output-stationary
  * kernel's for N > 320 or with PLSB200_EXACT=os).  The size query returns 0 (and the pack PLSB200_EUNSUPPORTED) for
- * K > 24 and where boot_moments runs the row-split kernel (N > 320 with PLSB200_TALL=rs).                        */
+ * K > 24.                                                                                                       */
 size_t plsb200_boot_factor_coef_bytes(int N, int K, int J);
 int plsb200_boot_factor_pack_f64(const double* E, int N, int K, const double* L, int J, const int32_t* sid,
                                  double* coef, void* stream);

@@ -12,7 +12,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libplsb200.so")
-SOURCES = ["abi.cu", "gram.cu", "nspace.cu", "boot.cu", "boot_quad.cu", "boot_rs.cu", "boot_os.cu", "boot_tf32.cu", "gram_tf32.cu", "split.cu", "rb.cu", "rb_dmma.cu", "half_gram.cu", "percentile.cu", "host_rng.cpp"]
+SOURCES = ["abi.cu", "gram.cu", "nspace.cu", "boot.cu", "boot_quad.cu", "boot_os.cu", "boot_tf32.cu", "gram_tf32.cu", "split.cu", "rb.cu", "rb_dmma.cu", "half_gram.cu", "percentile.cu", "host_rng.cpp"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-O3", "--expt-relaxed-constexpr",

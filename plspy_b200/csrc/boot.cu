@@ -567,22 +567,17 @@ static int dispatch_nks(const BootPlan& b, const T* X, int N, int64_t p, int64_t
 
 using namespace plsb;
 
-// Tall designs (N > 320): the output-stationary kernel (boot_os.cu) unless PLSB200_TALL=rs selects the row-split one
-// (boot_rs.cu, N <= 1280).  Read once per process: the pack and the GEMM must agree on the coefficient layout.
-static bool tall_os() {
-    static const char* const env = getenv("PLSB200_TALL");
-    return !(env && env[0] == 'r');
-}
-// N <= 320: the register-resident kernel of this file unless PLSB200_EXACT=os routes every design through boot_os.cu
+// N <= 320: the register-resident kernel of this file unless PLSB200_EXACT=os routes every design through boot_os.cu.
+// Read once per process: the pack and the GEMM must agree on the coefficient layout.
 static bool short_os() {
     static const char* const env = getenv("PLSB200_EXACT");
     return env && env[0] == 'o';
 }
-static bool use_other(int N) { return N > 320 || short_os(); }
-static bool use_os(int N) { return N > 320 ? tall_os() : true; }
+// tall designs (N > 320) always take the output-stationary kernel (boot_os.cu)
+static bool use_os(int N) { return N > 320 || short_os(); }
 
 extern "C" size_t plsb200_boot_coef_bytes(int N, int K, int R) {
-    if (use_other(N)) return use_os(N) ? boot_os_coef_bytes(N, K, R) : boot_rs_coef_bytes(N, K, R);
+    if (use_os(N)) return boot_os_coef_bytes(N, K, R);
     BootPlan b;
     if (!boot_plan(N, K, R, 1, b)) return 0;
     return (size_t)b.nper * b.stage_doubles * sizeof(double);
@@ -591,9 +586,7 @@ extern "C" size_t plsb200_boot_coef_bytes(int N, int K, int R) {
 extern "C" int plsb200_boot_coef_pack_f64(const double* E, int N, int K, const int32_t* idx, int R, double* coef,
                                           void* stream) {
     PLSB_CHECK_ARG(E && idx && coef, "boot_coef_pack_f64: null pointer");
-    if (use_other(N))
-        return use_os(N) ? boot_os_pack(E, N, K, idx, R, coef, (cudaStream_t)stream)
-                         : boot_rs_pack(E, N, K, idx, R, coef, (cudaStream_t)stream);
+    if (use_os(N)) return boot_os_pack(E, N, K, idx, R, coef, (cudaStream_t)stream);
     BootPlan b;
     if (!boot_plan(N, K, R, 1, b)) {
         set_err("boot_coef_pack_f64: unsupported shape N=%d K=%d R=%d (need K<=24, N<=320)", N, K, R);
@@ -608,9 +601,9 @@ extern "C" int plsb200_boot_coef_pack_f64(const double* E, int N, int K, const i
 }
 
 // the layout boot_moments_f64 reads: the register-resident one, else (N > 320 or PLSB200_EXACT=os) that of the
-// output-stationary kernel; the row-split kernel (PLSB200_TALL=rs) has no factored pack
+// output-stationary kernel
 extern "C" size_t plsb200_boot_factor_coef_bytes(int N, int K, int J) {
-    if (use_other(N)) return use_os(N) ? boot_os_coef_bytes(N, K, J) : 0;
+    if (use_os(N)) return boot_os_coef_bytes(N, K, J);
     BootPlan b;
     if (!boot_plan(N, K, J, 1, b)) return 0;
     return (size_t)b.nper * b.stage_doubles * sizeof(double);
@@ -621,14 +614,7 @@ extern "C" int plsb200_boot_factor_pack_f64(const double* E, int N, int K, const
     PLSB_CHECK_ARG(E && L && sid && coef, "boot_factor_pack_f64: null pointer");
     PLSB_CHECK_ARG(N > 0 && J > 0, "boot_factor_pack_f64: bad shape N=%d J=%d", N, J);
     cudaStream_t st = (cudaStream_t)stream;
-    if (use_other(N)) {
-        if (!use_os(N)) {
-            set_err("boot_factor_pack_f64: the row-split kernel (PLSB200_TALL=rs) has no factored layout; "
-                    "unset PLSB200_TALL");
-            return PLSB200_EUNSUPPORTED;
-        }
-        return boot_os_factor_pack(E, N, K, L, J, sid, coef, st);
-    }
+    if (use_os(N)) return boot_os_factor_pack(E, N, K, L, J, sid, coef, st);
     BootPlan b;
     if (!boot_plan(N, K, J, 1, b)) {
         set_err("boot_factor_pack_f64: unsupported shape N=%d K=%d J=%d (need K<=24)", N, K, J);
@@ -642,30 +628,10 @@ extern "C" int plsb200_boot_factor_pack_f64(const double* E, int N, int K, const
 }
 
 extern "C" size_t plsb200_boot_moments_f64_workspace(int N, int64_t p, int K, int R) {
-    if (use_other(N)) return use_os(N) ? boot_os_workspace(N, p, K, R) : boot_rs_workspace(N, p, K, R);
+    if (use_os(N)) return boot_os_workspace(N, p, K, R);
     BootPlan b;
     if (!boot_plan(N, K, R, p, b)) return 0;
     return b.nsplit > 1 ? (size_t)2 * b.nsplit * p * K * sizeof(double) : 16;
-}
-
-// tall designs: the output-stationary or (PLSB200_TALL=rs) the row-split kernel; the row-split kernel reads FP64 X only
-static int tall_moments(const double* X, int N, int64_t p, int64_t ldx, const double* coef, int K, int R,
-                        const double* pivot, double* sum, double* sumsq, void* workspace, size_t workspace_bytes,
-                        cudaStream_t st) {
-    return use_os(N) ? boot_os_moments(X, N, p, ldx, coef, K, R, pivot, sum, sumsq, workspace, workspace_bytes, st,
-                                       "boot_moments_f64")
-                     : boot_rs_moments(X, N, p, ldx, coef, K, R, pivot, sum, sumsq, workspace, workspace_bytes, st);
-}
-static int tall_moments(const float* X, int N, int64_t p, int64_t ldx, const double* coef, int K, int R,
-                        const double* pivot, double* sum, double* sumsq, void* workspace, size_t workspace_bytes,
-                        cudaStream_t st) {
-    if (!use_os(N)) {
-        set_err("boot_moments_x32_f64: the row-split kernel (PLSB200_TALL=rs) has no float32 variant; "
-                "unset PLSB200_TALL or store X as float64");
-        return PLSB200_EUNSUPPORTED;
-    }
-    return boot_os_moments(X, N, p, ldx, coef, K, R, pivot, sum, sumsq, workspace, workspace_bytes, st,
-                           "boot_moments_x32_f64");
 }
 
 template <typename T>
@@ -674,8 +640,9 @@ static int boot_moments(const T* X, int N, int64_t p, int64_t ldx, const double*
                         void* stream, const char* what) {
     PLSB_CHECK_ARG(X && coef && sum && sumsq, "%s: null pointer", what);
     PLSB_CHECK_ARG(p > 0 && ldx >= p, "%s: bad shape p=%lld ldx=%lld", what, (long long)p, (long long)ldx);
-    if (use_other(N))
-        return tall_moments(X, N, p, ldx, coef, K, R, pivot, sum, sumsq, workspace, workspace_bytes, (cudaStream_t)stream);
+    if (use_os(N))
+        return boot_os_moments(X, N, p, ldx, coef, K, R, pivot, sum, sumsq, workspace, workspace_bytes,
+                               (cudaStream_t)stream, what);
     BootPlan b;
     if (!boot_plan(N, K, R, p, b)) {
         set_err("%s: unsupported shape N=%d K=%d R=%d (need K<=24, N<=320)", what, N, K, R);

@@ -4,11 +4,12 @@
 //   VS[v, (r,k)] = sum_i X[i, v] C_r[i, k]          M = voxels, N = R*Kp columns, K-dim = rows of X
 //
 // boot_moments_kernel (boot.cu) keeps a warp's A fragments -- 8 voxels x all rows -- in registers, which is ideal
-// while they fit (N <= 320) and makes every coefficient byte serve only the 64 voxels of a CTA.  For taller designs
-// the row-split kernel (boot_rs.cu) gets down to 16 voxels per SM: 63 GB/s of coefficient ingest per SM at N = 1200,
-// 0.76 of the DGEMM peak with a fifth of the warp samples waiting for stages (profiles/ncu_boot_rs_r02.md).
-// Here NOTHING is register-resident except the accumulators: a CTA owns a tile of 128 voxels x 96 columns
-// (4 whole resamples at K = 24), both operands stream through shared memory in stages of 32 rows --
+// while they fit (N <= 320) and makes every coefficient byte serve only the 64 voxels of a CTA.  Taller designs would
+// have to split those fragments over several warps, and a coefficient byte would serve fewer voxels still: 16 per SM,
+// 63 GB/s of coefficient ingest per SM at N = 1200, which held such a kernel to 0.76 of the DGEMM peak with a fifth of
+// the warp samples waiting for stages (DESIGN.md §5.1b).  Here NOTHING is register-resident except the accumulators:
+// a CTA owns a tile of 128 voxels x 96 columns (4 whole resamples at K = 24), both operands stream through shared
+// memory in stages of 32 rows --
 //   A: 32 rows x 128 voxels of X at a pitch of 132 doubles (so that the transposed fragment loads are bank-conflict-
 //      free), read from a TILE-MAJOR IMAGE of X built once per call (os_ximage_kernel: [voxel tile][32-row block]
 //      [32 x 132]), so that the block is three bulk copies of contiguous memory.  Fetching the 32 row segments of the
@@ -19,7 +20,7 @@
 // A coefficient byte now serves 128 voxels and an X byte 96 columns: 37 GB/s per SM at any N.  After the last row
 // the 48 accumulators of a thread hold (VS) for 4 voxel rows x 12 columns; they are folded into per-thread running
 // moments of (VS - pivot) -- the column -> k map is tile-invariant because 96 is a multiple of every padded K -- and
-// the CTA moves to the next column tile.  There is no limit on N any more (boot_rs: 1280).
+// the CTA moves to the next column tile.  There is no limit on N.
 #include "common.cuh"
 
 namespace plsb {
@@ -346,9 +347,6 @@ static int os_launch(const OsPlan& b, const double* Ximg, int N, int64_t p, cons
         default: return os_launch_ks<NACC, 8>(b, Ximg, N, p, coef, K, R, pivot, o1, o2, st);
     }
 }
-
-// (the image builder reads X with plain loads: no alignment requirement on X any more)
-bool boot_os_usable(const double*, int64_t, int64_t) { return true; }
 
 static size_t os_image_bytes(const OsPlan& b, int64_t p) {
     return (size_t)cdiv(p, OS_TM) * (b.nks / b.ks) * os_a_doubles(b.ks) * sizeof(double);

@@ -55,16 +55,7 @@ inline int num_sms() {
 
 inline int64_t cdiv(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
-// row-split bootstrap-moments path for N > 320 (boot_rs.cu), reached through the plsb200_boot_* entry points
-size_t boot_rs_coef_bytes(int N, int K, int R);
-size_t boot_rs_workspace(int N, int64_t p, int K, int R);
-int boot_rs_pack(const double* E, int N, int K, const int32_t* idx, int R, double* coef, cudaStream_t st);
-int boot_rs_moments(const double* X, int N, int64_t p, int64_t ldx, const double* coef, int K, int R,
-                    const double* pivot, double* sum, double* sumsq, void* workspace, size_t workspace_bytes,
-                    cudaStream_t st);
-
-// output-stationary bootstrap-moments path for N > 320 (boot_os.cu); same contract as the row-split path
-bool boot_os_usable(const double* X, int64_t p, int64_t ldx);
+// output-stationary bootstrap-moments path for N > 320 (boot_os.cu), reached through the plsb200_boot_* entry points
 size_t boot_os_coef_bytes(int N, int K, int R);
 size_t boot_os_workspace(int N, int64_t p, int K, int R);
 int boot_os_pack(const double* E, int N, int K, const int32_t* idx, int R, double* coef, cudaStream_t st);
@@ -151,7 +142,7 @@ __device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_gmem, u
         : "memory");
 }
 
-// ---- thread-block clusters: rank, cluster barrier, remote mbarrier arrive, multicast bulk copy ----
+// ---- thread-block clusters: rank, cluster barrier, remote mbarrier arrive ----
 __device__ __forceinline__ uint32_t cluster_ctarank() {
     uint32_t r;
     asm volatile("mov.u32 %0, %%cluster_ctarank;\n" : "=r"(r));
@@ -173,16 +164,6 @@ __device__ __forceinline__ uint32_t mapa_u32(uint32_t local_addr, uint32_t rank)
 // .release.cluster / .acquire.cluster compile to MEMBAR.ALL.GPU + CCTL.IVALL per pipeline stage.
 __device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
     asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];\n" ::"r"(cluster_addr) : "memory");
-}
-// global -> the SAME shared-memory offset in every CTA of `cta_mask`; each destination CTA's mbarrier (same offset)
-// receives the complete_tx for the bytes written into that CTA.  One L2 read feeds all the destination SMs.
-__device__ __forceinline__ void bulk_g2s_multicast(void* dst_smem, const void* src_gmem, uint32_t bytes, uint64_t* bar,
-                                                   uint16_t cta_mask) {
-    asm volatile(
-        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;\n" ::"r"(
-            smem_u32(dst_smem)),
-        "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar)), "h"(cta_mask)
-        : "memory");
 }
 
 // ---- ordered source lists of one resample (coefficient packs) ----

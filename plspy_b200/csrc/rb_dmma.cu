@@ -64,7 +64,6 @@ static bool rd_plan(int N, int K, const int32_t* cs, int ncell, int unit_cells, 
     r.warps = r.nks <= 32 ? 16 : 8;
     r.nstd = ncell - unit_cells;
     const size_t coef_bytes = (size_t)r.nks * r.nblk * 32 * sizeof(double);
-    static const char* const env = getenv("PLSB200_RB_MOMENTS");         // "fma" forces the scalar-moment kernel (A/B runs)
     // moments on DMMA: weight fragments of one batch of 8 bootstraps, block sizes, running moments, per-warp scale tables
     // of the batch ([8 bootstraps][standardised cell][8 voxels]), barriers
     const size_t fixed_md = ((size_t)r.nks * 32 + 16 + 3 * r.nblk * 2 * r.warps * 32 + (size_t)r.warps * 64 * (r.nstd > 0 ? r.nstd : 1)) * sizeof(double) + 256;
@@ -72,7 +71,7 @@ static bool rd_plan(int N, int K, const int32_t* cs, int ncell, int unit_cells, 
     if (ns > 4) ns = 4;
     // (only the 16-warp bucket: with 8 warps -- 2 per scheduler -- the serial moment phase of a batch is not covered by other
     // warps; cfg 4 pass 2, 92 k-steps of which 30 standardised: 7.79 ms with the scalar moments, 8.41 ms with the DMMA moments)
-    r.md = ns >= 2 && r.nstd > 0 && r.warps == 16 && !(env && env[0] == 'f');
+    r.md = ns >= 2 && r.nstd > 0 && r.warps == 16;
     if (r.md) {
         r.nstage = ns;
         r.smem_bytes = ns * coef_bytes + fixed_md;

@@ -535,7 +535,7 @@ class Engine:
             T = self._empty(R, Kt, K)
         G = self.G
         ws_bytes = lib.plsb200_nspace_dmma_f64_workspace(self.N, K, Kt, R) if R > 0 else 0
-        if ws_bytes and os.environ.get("PLSB200_NSPACE", "dmma") != "fma":
+        if ws_bytes:
             if packed is None or packed["R"] != R or packed["K"] != K:
                 packed = self.pack_coef(E, idx)
             if packed is not None:
@@ -829,8 +829,8 @@ class Engine:
         with torch.cuda.device(self.device):
             nbytes = lib.plsb200_boot_factor_coef_bytes(self.N, K, J)
             if nbytes == 0:
-                raise _lib.PlsB200Error(f"boot_factor_quad: unsupported shape N={self.N} K={K} J={J} (the row-split "
-                                        "kernel of PLSB200_TALL=rs has no factored layout)")
+                raise _lib.PlsB200Error(f"boot_factor_quad: unsupported shape N={self.N} K={K} J={J} (the factored "
+                                        "pack needs 1 <= K <= 24 and J >= 1)")
             coef = self._ws(nbytes)
             check(lib.plsb200_boot_factor_pack_f64(self._p(E), self.N, K, self._p(L), J, self._p(sid), self._p(coef),
                                                    self._stream()), "boot_factor_pack_f64")

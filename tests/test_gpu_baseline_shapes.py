@@ -7,8 +7,8 @@ real workloads:
 * cfg 3m  mct (the north-star target), same design, K = 12                      16 perm + 16 boot
 * cfg 4   mb, bscan = [1, 2], 2 x 30 x 4 (N = 240 + 120 bscan rows) x 200 000 voxels, 4 behaviours, K = 24
                                                                                  3 perm + 3 boot + 2 splits (lv = 1)
-* cfg 5 shape (rows): mct 4 x 50 x 6 (N = 1200, K = 24) x 200 000 voxels -- the row-split DMMA kernel `boot_rs`
-  that only tall designs reach                                                    3 perm + 4 boot
+* cfg 5 shape (rows): mct 4 x 50 x 6 (N = 1200, K = 24) x 200 000 voxels -- the output-stationary DMMA kernel
+  `boot_os` that only tall designs reach                                          3 perm + 4 boot
 
 Both sides draw their indices from numpy's global stream after the same seed (the product through its native
 generator), so index generation is part of the check.  Tolerances are those of tests/test_gpu_parity.py: p-values and
@@ -95,7 +95,8 @@ def test_cfg3m_mct_200k_matches_oracle():
 
 
 def test_cfg5_rows_mct_n1200_matches_oracle():
-    """N = 1200 rows (4 x 50 x 6, K = 24): the exact bootstrap GEMM takes the row-split kernel (csrc/boot_rs.cu)."""
+    """N = 1200 rows (4 x 50 x 6, K = 24): the exact bootstrap GEMM takes the output-stationary kernel
+    (csrc/boot_os.cu)."""
     import plspy_b200
     groups, C, p = (50, 50, 50, 50), 6, 200_000
     _, X, _ = _planted(20260005, groups, C, p)

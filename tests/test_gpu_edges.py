@@ -124,27 +124,10 @@ def test_cst_single_contrast_and_cmb():
 @pytest.mark.parametrize("groups,C,p", [((60, 60), 3, 300), ((40, 45, 35), 6, 300), ((40, 45, 35), 6, 301),
                                         ((150, 160, 150), 3, 140)])
 def test_tall_designs(groups, C, p):
-    """N > 320 rows (360, 720, 720 with an odd voxel count, 1380 > the 1280 limit of the row-split kernel): the
-    output-stationary bootstrap GEMM (boot_os.cu), both operands staged through shared memory."""
+    """N > 320 rows (360, 720, 720 with an odd voxel count, 1380): the output-stationary bootstrap GEMM
+    (boot_os.cu), both operands staged through shared memory."""
     o, res = _both("mct", groups, C, p, nperm=4, nboot=11, seed=8)
     _check(o, res)
-
-
-@pytest.mark.parametrize("groups,C", [((60, 60), 3), ((40, 45, 35), 6)])     # N = 360 (2-way row split), 720 (4-way)
-def test_tall_designs_row_split_kernel(groups, C, monkeypatch):
-    """the row-split kernel (boot_rs.cu: A fragments split over 2 or 4 warps per voxel group, cluster pairs with a
-    multicast coefficient stream) stays selectable with PLSB200_TALL=rs; the choice is read once per process, so it
-    is exercised in a child process"""
-    import subprocess, sys, os
-    code = (
-        "import numpy as np, sys; sys.path.insert(0, %r); sys.path.insert(0, %r)\n"
-        "import test_gpu_edges as t\n"
-        "o, res = t._both('mct', %r, %d, 300, nperm=4, nboot=11, seed=8); t._check(o, res); print('ok')\n"
-        % (os.path.dirname(os.path.dirname(os.path.abspath(__file__))), os.path.dirname(os.path.abspath(__file__)),
-           tuple(groups), C))
-    env = dict(os.environ, PLSB200_TALL="rs")
-    out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=600)
-    assert out.returncode == 0 and "ok" in out.stdout, out.stderr[-2000:]
 
 
 def test_wide_k_fails_loudly():
