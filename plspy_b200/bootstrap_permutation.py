@@ -18,13 +18,14 @@ x_v^T Cov_r(c_rk) x_v -- see `check_boot_algo`; `boot_algo` of the result is the
 ("resamples", default, or "voxels": the layout of X in a multi-process run -- see `check_shard`).
 """
 import abc
+import functools
 
 import numpy as np
 import torch
 from scipy.stats import norm
 
 from . import class_functions, dist, exceptions, resample
-from .engine import Engine
+from .engine import Engine, check_choice
 
 VERBOSE = False
 
@@ -241,8 +242,7 @@ def _perm_multiblock(eng, X, U, s, cond_order, mctype, niter, pls_alg, contrast,
     raw_sq = float(eng.nspace_coef(st["Gw"], eng.to_device(C0[None], torch.float64))[0].sum())   # sum_k C0_k^T Gw C0_k
     org_s = np.sqrt(s ** 2 / np.sum(s ** 2) * raw_sq)
     totcov_org = _stepdown_tail(org_s)
-    Ucoef = np.asarray(U, dtype=float) if contrast is None else class_functions._normalize(
-        np.asarray(contrast, dtype=float))
+    Ucoef = _ucoef(U, contrast)
     Kc = Ucoef.shape[1]
     lo, hi = dist.shard(niter)
     it = _index_shard(eng, idx_t, niter, lo, hi); ib = _index_shard(eng, idx_b, niter, lo, hi)
@@ -292,13 +292,11 @@ def _boot_multiblock(eng, U, s, V, cond_order, mctype, niter, pls_alg, contrast,
     Lop = (class_functions._cell_mean_operator(cond_order) if pls_alg == "cmb"
            else class_functions._centring_operator(cond_order, mctype))
     Abar = class_functions._cell_mean_operator(cond_order)
-    Ucoef = np.asarray(U, dtype=float) if contrast is None else class_functions._normalize(
-        np.asarray(contrast, dtype=float))
+    Ucoef = _ucoef(U, contrast)
     Kc = Ucoef.shape[1]
     N, Nb = eng.N, st["Nb"]
     dev = eng.device
-    Vd = eng.to_device(V, torch.float64)
-    numer = Vd * eng.to_device(np.asarray(s, dtype=float), torch.float64) if contrast is None else Vd
+    numer = _numerator(eng, V, s, contrast)
     lo, hi = dist.shard(niter)
     it = _index_shard(eng, idx_t, niter, lo, hi); ib = _index_shard(eng, idx_b, niter, lo, hi)
     R = hi - lo
@@ -344,20 +342,57 @@ def _boot_multiblock(eng, U, s, V, cond_order, mctype, niter, pls_alg, contrast,
     return conf_int, conf_int_T, std_errs_h, boot_ratios_h, LV_h, debug
 
 
+def _ucoef(U, contrast):
+    """The design-side weights the saliences are projected on: U, or the normalised contrasts (:385-389, :620)."""
+    if contrast is None:
+        return np.asarray(U, dtype=float)
+    return class_functions._normalize(np.asarray(contrast, dtype=float))
+
+
+def _numerator(eng, V, s, contrast):
+    """Numerator of the bootstrap ratios, the original salience (:700-703): V s, or V with contrasts; also the pivot
+    that keeps the running sums of squares well conditioned.  V may already be a device tensor."""
+    Vd = eng.to_device(V, torch.float64)
+    return Vd * eng.to_device(np.asarray(s, dtype=float), torch.float64) if contrast is None else Vd
+
+
 def _task_operators(pls_alg, cond_order, mctype, U, contrast):
     """Row-space pull-back of the design-side weights: E = Lop^T @ Ucoef (N x K).
     mct: Lop = centring operator, Ucoef = U (bootstrap_permutation.py:385-387, 404);
     cst: Lop = cell-mean operator, Ucoef = normalised contrasts (:389, :430-432, :620)."""
     if pls_alg == "mct":
         Lop = class_functions._centring_operator(cond_order, mctype)
-        Ucoef = np.asarray(U, dtype=float)
+        Ucoef = _ucoef(U, None)
     else:
         Lop = class_functions._cell_mean_operator(cond_order)
-        Ucoef = class_functions._normalize(np.asarray(contrast, dtype=float))
+        Ucoef = _ucoef(U, contrast)
     return Lop, Ucoef, Lop.T @ Ucoef
 
 
 BOOT_ALGOS = ("auto", "direct", "collapsed")
+
+
+def _factor_layout_missing(cond_order, nboot):
+    """What the design lacks for the factored collapsed bootstrap (None: nothing): a `cond_order` with every group the
+    same size in each condition, and more bootstraps than the ns - G columns of the factor (else M is singular)."""
+    if cond_order is None:
+        return "no cond_order"
+    co = np.asarray(cond_order)
+    if co.ndim != 2 or co.size == 0 or (co != co[:, :1]).any():
+        return "unequal subject counts across conditions"
+    ns_g = int(co[:, 0].sum()) - co.shape[0]
+    if nboot is None or not nboot > ns_g >= 1:
+        return f"num_boot={nboot}, ns - G = {ns_g}"
+    return None
+
+
+def _no_collapsed_route(N, missing):
+    return exceptions.NotImplementedError(
+        f'boot_algo="collapsed" for a design of {N} rows: the N x N covariance route is limited to '
+        f'{Engine.QUAD_MAX_ROWS} rows, and the factored route needs a cond_order in which every group has the same '
+        'number of subjects in each condition, more bootstraps than ns - G (subjects minus groups), design weights '
+        'constant within each cell and bootstrap draws with the subject structure of resample.bootstrap_indices (each '
+        f'row drawn from its own cell, one subject map for all conditions) ({missing}); use boot_algo="direct"')
 
 
 def check_boot_algo(boot_algo, pls_alg, precision, N, nboot=None, cond_order=None):
@@ -374,8 +409,7 @@ def check_boot_algo(boot_algo, pls_alg, precision, N, nboot=None, cond_order=Non
     whole run's) than ns - G; draws passed in must also have the subject structure (checked on the device).
     "auto" (default) is "collapsed" for mct / cst with precision="fp64", N <= 320 and more bootstraps than rows, else
     "direct"."""
-    if boot_algo not in BOOT_ALGOS:
-        raise ValueError(f'boot_algo must be one of {BOOT_ALGOS}, got {boot_algo!r}')
+    check_choice("boot_algo", boot_algo, BOOT_ALGOS)
     if boot_algo == "auto":
         fits = N is not None and N <= Engine.QUAD_MAX_ROWS and nboot is not None and nboot > N
         return "collapsed" if (pls_alg in ("mct", "cst") and precision == "fp64" and fits) else "direct"
@@ -388,21 +422,10 @@ def check_boot_algo(boot_algo, pls_alg, precision, N, nboot=None, cond_order=Non
             'boot_algo="collapsed" applies to the task methods (mct, cst): the block standardisation of the behaviour '
             'and multiblock methods makes their saliences non-linear in the bootstrap draw')
     if N is not None and N > Engine.QUAD_MAX_ROWS:
-        co = None if cond_order is None else np.asarray(cond_order)
-        balanced = co is not None and co.ndim == 2 and co.size > 0 and bool((co == co[:, :1]).all())
-        ns_g = int(co[:, 0].sum()) - co.shape[0] if balanced else None
-        if not (balanced and nboot is not None and nboot > ns_g >= 1):
-            have = ("no cond_order" if co is None else "unequal subject counts across conditions" if not balanced
-                    else f"num_boot={nboot}, ns - G = {ns_g}")
-            raise exceptions.NotImplementedError(
-                f'boot_algo="collapsed" for a design of {N} rows: the N x N covariance route is limited to '
-                f'{Engine.QUAD_MAX_ROWS} rows, and the factored route needs a cond_order in which every group has the '
-                f'same number of subjects in each condition and more bootstraps than ns - G (subjects minus groups) '
-                f'({have}); use boot_algo="direct"')
+        missing = _factor_layout_missing(cond_order, nboot)
+        if missing is not None:
+            raise _no_collapsed_route(N, missing)
     return boot_algo
-
-
-X_STORAGES = ("fp64", "fp32")
 
 
 def check_x_storage(x_storage, pls_alg):
@@ -412,15 +435,11 @@ def check_x_storage(x_storage, pls_alg):
     (half the memory and half the bytes of every pass over X) and every kernel widens an element where it loads it,
     so all results equal, bit for bit, those of the "fp64" run on the widened matrix.  Task methods (mct, cst) only:
     the block standardisation kernels of the behaviour and multiblock methods read float64."""
-    if x_storage not in X_STORAGES:
-        raise ValueError(f'x_storage must be one of {X_STORAGES}, got {x_storage!r}')
+    check_choice("x_storage", x_storage, Engine.X_STORAGES)
     if x_storage == "fp32" and pls_alg not in ("mct", "cst"):
         raise exceptions.NotImplementedError(
             'x_storage="fp32" applies to the task methods (mct, cst); the behaviour and multiblock methods keep X '
             'in float64')
-
-
-SHARDS = Engine.SHARDS
 
 
 def check_shard(shard, pls_alg):
@@ -432,45 +451,56 @@ def check_shard(shard, pls_alg):
     resample-sharded through the all-reduced Gram matrix, and the p x K results are gathered.  Task methods (mct,
     cst): the behaviour and multiblock bootstraps reduce over voxels per resample.  One process: the two are the
     same."""
-    if shard not in SHARDS:
-        raise ValueError(f'shard must be one of {SHARDS}, got {shard!r}')
+    check_choice("shard", shard, Engine.SHARDS)
     if shard == "voxels" and pls_alg not in ("mct", "cst"):
         raise exceptions.NotImplementedError(
             'shard="voxels" applies to the task methods (mct, cst); the behaviour and multiblock bootstraps need '
             'per-resample norms over all voxels')
 
 
+def resolve_options(pls_alg, engine=None, X=None, nboot=None, cond_order=None, precision="fp64", boot_algo="auto",
+                    x_storage=None, shard=None):
+    """The engine options of one analysis, validated before any GPU work: (precision, boot_algo, x_storage, shard).
+    A given `engine` sets the precision and row count (else X's rows), and its x_storage and shard, which a value
+    passed too must match (None: the engine's, else "fp64" / "resamples").  `boot_algo` None: not checked (a caller
+    that does not know `nboot` and `cond_order` yet)."""
+    check_choice("precision", precision, Engine.PRECISIONS)
+    if engine is not None:
+        for name, given in (("x_storage", x_storage), ("shard", shard)):
+            if given is not None and given != getattr(engine, name):
+                raise ValueError(f"{name}={given!r} but the engine holds X with {name}={getattr(engine, name)!r}")
+        precision, N, x_storage, shard = engine.precision, engine.N, engine.x_storage, engine.shard
+    else:
+        N = int(X.shape[0]) if getattr(X, "shape", None) else None
+        x_storage, shard = ("fp64" if x_storage is None else x_storage), ("resamples" if shard is None else shard)
+    check_x_storage(x_storage, pls_alg)
+    check_shard(shard, pls_alg)
+    if boot_algo is not None:
+        boot_algo = check_boot_algo(boot_algo, pls_alg, precision, N, nboot, cond_order)
+    return precision, boot_algo, x_storage, shard
+
+
 def _factor_plan(eng, pls_alg, U, contrast, cond_order, mctype, niter, indices):
     """The subject layout for the factored collapsed bootstrap (DESIGN.md section 3), or None when its preconditions
-    do not hold and the N x N covariance route runs instead: every group has the same number of subjects in each
-    condition, E = Lop^T Ucoef is bit-identical within each cell, there are more bootstraps than the factor's ns - G
-    columns (fewer make the count covariance singular), and every draw keeps each row in its cell with one subject map
-    for all conditions.  Indices drawn here (`indices` None) have that structure by construction; given ones are
-    checked on the device, each rank its shard, with the flag all-reduced.  Designs of more than 320 rows have no
-    N x N route: there exceptions.NotImplementedError replaces None (on every rank)."""
-    plan = _factor_plan_or_none(eng, pls_alg, U, contrast, cond_order, mctype, niter, indices)
-    if plan is None and eng.N > Engine.QUAD_MAX_ROWS:
-        raise exceptions.NotImplementedError(
-            f'boot_algo="collapsed" for a design of {eng.N} rows: the N x N covariance route is limited to '
-            f'{Engine.QUAD_MAX_ROWS} rows, and the factored route needs every group to have the same number of '
-            'subjects in each condition, more bootstraps than ns - G, design weights constant within each cell and '
-            'bootstrap draws with the subject structure of resample.bootstrap_indices (each row drawn from its own '
-            'cell, one subject map for all conditions); use boot_algo="direct"')
-    return plan
-
-
-def _factor_plan_or_none(eng, pls_alg, U, contrast, cond_order, mctype, niter, indices):
+    do not hold and the N x N covariance route runs instead: those of `_factor_layout_missing`, E = Lop^T Ucoef
+    bit-identical within each cell, and every draw keeping each row in its cell with one subject map for all
+    conditions.  Indices drawn by the library (pass None) have that structure by construction; given ones are checked
+    on the device, each rank its shard, with the flag all-reduced.  Designs of more than 320 rows have no N x N route:
+    there exceptions.NotImplementedError replaces None (on every rank)."""
+    def none_or_raise(missing):
+        if eng.N > Engine.QUAD_MAX_ROWS:
+            raise _no_collapsed_route(eng.N, missing)
+        return None
+    missing = _factor_layout_missing(cond_order, niter)
+    if missing is not None:
+        return none_or_raise(missing)
     co = np.asarray(cond_order)
-    if co.ndim != 2 or (co != co[:, :1]).any():
-        return None
     sizes = co[:, 0].astype(np.int64)
-    G, C, ns = co.shape[0], co.shape[1], int(sizes.sum())
-    if niter <= ns - G or ns <= G:
-        return None
+    G, C = co.shape
     _, _, E = _task_operators(pls_alg, cond_order, mctype, U, contrast)
     cells = _cell_offsets(co)
     if any((E[a:b] != E[a]).any() for a, b in zip(cells[:-1], cells[1:])):
-        return None
+        return none_or_raise("design weights that differ within a cell")
     gstart = np.concatenate(([0], np.cumsum(sizes))).astype(np.int32)
     base = np.repeat(cells[:-1], co.reshape(-1))                         # first row of each row's cell
     sid = np.concatenate([gstart[g] + np.arange(sizes[g]) for g in range(G) for _ in range(C)])
@@ -485,7 +515,7 @@ def _factor_plan_or_none(eng, pls_alg, U, contrast, cond_order, mctype, niter, i
                else torch.zeros(1, dtype=torch.int32, device=eng.device)).to(torch.int64)
         dist.allreduce_sum_(bad)
         if int(bad.item()) != 0:
-            return None
+            return none_or_raise("bootstrap draws without the subject structure")
     return plan
 
 
@@ -504,23 +534,68 @@ def _collapsed_sumsq(eng, E, idx_dev, niter, lo, hi, factor=None):
               else torch.zeros(ns + 1, ns + 1, dtype=torch.float64, device=eng.device))
         dist.allreduce_sum_(Mg)
         L = eng.boot_factor(Mg, niter, factor["gstart"])
-        if dist.world()[1] == 1 or eng.voxel_sharded:
-            return eng.boot_factor_quad(E, L, factor["sid"])
-        v0, v1 = dist.shard(eng.p)
-        return dist.gather_rows(eng.boot_factor_quad(E, L, factor["sid"], v0, v1), eng.p, v0)
-    if hi > lo:
-        S1, S2 = eng.boot_cov(E, idx_dev)
+        quad = lambda *vox: eng.boot_factor_quad(E, L, factor["sid"], *vox)        # noqa: E731
     else:
-        K = E.shape[1]
-        S1 = torch.zeros(eng.N, K, dtype=torch.float64, device=eng.device)
-        S2 = torch.zeros(K, eng.N, eng.N, dtype=torch.float64, device=eng.device)
-    dist.allreduce_packed_([S1, S2])
-    s1t = S1.T
-    Sig = S2 - s1t[:, :, None] * s1t[:, None, :] / niter
+        if hi > lo:
+            S1, S2 = eng.boot_cov(E, idx_dev)
+        else:
+            K = E.shape[1]
+            S1 = torch.zeros(eng.N, K, dtype=torch.float64, device=eng.device)
+            S2 = torch.zeros(K, eng.N, eng.N, dtype=torch.float64, device=eng.device)
+        dist.allreduce_packed_([S1, S2])
+        s1t = S1.T
+        Sig = S2 - s1t[:, :, None] * s1t[:, None, :] / niter
+        quad = lambda *vox: eng.boot_quad(Sig, *vox)                                # noqa: E731
     if dist.world()[1] == 1 or eng.voxel_sharded:
-        return eng.boot_quad(Sig)
+        return quad()
     v0, v1 = dist.shard(eng.p)
-    return dist.gather_rows(eng.boot_quad(Sig, v0, v1), eng.p, v0)
+    return dist.gather_rows(quad(v0, v1), eng.p, v0)
+
+
+class _TaskPlan:
+    """The inputs of one mct / cst bootstrap: operators, this rank's draws (rows [lo, hi); `idx_all`: every draw, for
+    the moment stage of a voxel-sharded engine), the resolved `boot_algo` with its `_factor_plan` (None: the N x N
+    route), and the `moments` once `_boot_moments` has run.  `drawn`: the library drew `indices` (no draw check).  V
+    reaches the device at its first use: uploaded ahead of the collapsed stage it would hold back a pipelined X."""
+
+    def __init__(self, eng, pls_alg, U, s, V, cond_order, mctype, contrast, niter, indices, boot_algo, drawn=False):
+        if isinstance(indices, tuple):
+            indices = indices[0]
+        self.boot_algo, self.moments = boot_algo, None
+        self.Lop, self.Ucoef, self.E = _task_operators(pls_alg, cond_order, mctype, U, contrast)
+        self.factor = (_factor_plan(eng, pls_alg, U, contrast, cond_order, mctype, niter, None if drawn else indices)
+                       if boot_algo == "collapsed" else None)
+        self.lo, self.hi = dist.shard(niter)
+        self.idx = _index_shard(eng, indices, niter, self.lo, self.hi)
+        self.idx_all = _index_shard(eng, indices, niter, 0, niter) if eng.voxel_sharded else self.idx
+        self._eng, self._V, self._s, self._contrast = eng, V, s, contrast
+
+    @functools.cached_property
+    def V(self):
+        return self._eng.to_device(self._V, torch.float64)
+
+    @functools.cached_property
+    def numer(self):
+        """`_numerator`, its rows of the voxels this engine holds."""
+        numer, (v0, v1) = _numerator(self._eng, self.V, self._s, self._contrast), self._eng.voxel_range
+        return numer[v0:v1].contiguous() if self._eng.voxel_sharded else numer
+
+
+def _boot_moments(eng, plan, niter, packed=None):
+    """The moment stage of the mct / cst bootstrap: sums of VS_r - pivot and of its squares over all `niter` draws,
+    complete on every rank (p x K, this engine's voxels); "collapsed": (0, sum of squares about the mean), with no
+    p x K all-reduce.  `packed`: a `pack_coef` result for the plan's (E, idx) to reuse."""
+    if plan.boot_algo == "collapsed":
+        s2 = _collapsed_sumsq(eng, plan.E, plan.idx, niter, plan.lo, plan.hi, factor=plan.factor)
+        return torch.zeros_like(s2), s2
+    if eng.voxel_sharded:                       # every bootstrap on this rank's voxels: no moment all-reduce
+        return eng.boot_moments(plan.E, plan.idx_all, pivot=plan.numer)
+    if plan.hi > plan.lo:
+        s1, s2 = eng.boot_moments(plan.E, plan.idx, pivot=plan.numer, packed=packed)   # K4
+    else:
+        s1 = torch.zeros_like(plan.numer); s2 = torch.zeros_like(plan.numer)
+    dist.allreduce_packed_([s1, s2])
+    return s1, s2
 
 
 @ResampleTest._register_subclass("mct")
@@ -535,19 +610,10 @@ class _ResampleTestPLS(ResampleTest):
     def __init__(self, X, Y, U, s, V, cond_order, mctype, contrast=None, preprocess=None, nperm=1000,
                  nboot=1000, bscan=None, Xbscan=None, Ybscan=None, lvcorrs_orig=None, Tvsc_orig=None,
                  CI=0.95, *, perm_indices=None, boot_indices=None, engine=None, precision="fp64", rotate_method=2,
-                 device=None, boot_algo="auto", x_storage="fp64", shard=None):
+                 device=None, boot_algo="auto", x_storage=None, shard=None):
         self.CI = CI
-        boot_algo = check_boot_algo(boot_algo, self.pls_alg, engine.precision if engine is not None else precision,
-                                    engine.N if engine is not None else (int(X.shape[0]) if X is not None else None),
-                                    nboot, cond_order)
-        check_x_storage(x_storage, self.pls_alg)
-        if engine is not None:
-            check_x_storage(engine.x_storage, self.pls_alg)
-        if shard is None:                   # the layout of a given engine, else the default
-            shard = engine.shard if engine is not None else "resamples"
-        check_shard(shard, self.pls_alg)
-        if engine is not None and engine.shard != shard:
-            raise ValueError(f"shard={shard!r} but the engine holds X laid out for shard={engine.shard!r}")
+        precision, boot_algo, x_storage, shard = resolve_options(self.pls_alg, engine, X, nboot, cond_order, precision,
+                                                                 boot_algo, x_storage, shard)
         self.boot_algo = boot_algo
         if rotate_method not in (0, 1, 2):
             raise ValueError("rotate_method must be 0 (SVD), 1 (Procrustes) or 2 (derived)")
@@ -564,26 +630,26 @@ class _ResampleTestPLS(ResampleTest):
         if eng is not None and self.pls_alg in ("mct", "cst") and dist.world()[1] > 1:
             eng.gram_collective()          # all ranks are here: Gram from per-rank voxel ranges + one all-reduce
         perm_pending = None
-        early = None
-        factor = None
-        if eng is not None and nboot > 0 and boot_algo == "collapsed":
-            # (given indices are checked here, before the permutation work is enqueued: one small kernel and one wait)
-            factor = _factor_plan(eng, self.pls_alg, U, contrast, cond_order, mctype, nboot, boot_indices)
-        if (eng is not None and eng.upload_in_flight and nboot > 0 and self.pls_alg in ("mct", "cst")
-                and dist.world()[1] == 1):
-            # X is still crossing PCIe in voxel ranges (Engine._upload_pipelined): the bootstrap moment GEMM is the
-            # one kernel that can start on the ranges already there, so it is enqueued before the permutation test,
-            # whose Gram matrix needs all of X.  Index matrices are drawn first, in the reference's order.
+        plan = None
+        if eng is not None and nboot > 0 and self.pls_alg in ("mct", "cst"):
+            # the plan checks given draws (one small kernel and one wait) before the permutation work is enqueued;
+            # the index matrices are drawn first, in the reference's order
             if nperm > 0:
                 s[np.abs(s) < 1e-12] = 0                       # as _permutation_test does before anything reads s
                 if perm_indices is None:
                     perm_indices = resample.permutation_indices(self.pls_alg, nperm, cond_order, Y=Y, bscan=bscan,
                                                                 Ybscan=Ybscan)
-            if boot_indices is None:
+            drawn = boot_indices is None
+            if drawn:
                 boot_indices = resample.bootstrap_indices(self.pls_alg, nboot, cond_order, Y=Y, bscan=bscan,
                                                           Ybscan=Ybscan)
-            early = self._bootstrap_moments_early(eng, U, s, V, cond_order, mctype, nboot, self.pls_alg, contrast,
-                                                  boot_indices, boot_algo=boot_algo, _factor=factor)
+            plan = _TaskPlan(eng, self.pls_alg, U, s, V, cond_order, mctype, contrast, nboot, boot_indices, boot_algo,
+                             drawn=drawn)
+            if eng.upload_in_flight and dist.world()[1] == 1:
+                # X is still crossing PCIe in voxel ranges (Engine._upload_pipelined): the moment stage is the one
+                # that can start on the ranges already there, so it is enqueued before the permutation test, whose
+                # Gram matrix needs all of X
+                plan.moments = _boot_moments(eng, plan, nboot)
         if nperm > 0:
             # the permutation kernels and their device->host copies are enqueued here; the host only waits for
             # them after the bootstrap work has been enqueued too, so the GPU never idles between the two tests
@@ -598,7 +664,7 @@ class _ResampleTestPLS(ResampleTest):
             out = self._bootstrap_test(
                 X, Y, U, s, V, cond_order, mctype, nboot, self.pls_alg, preprocess=preprocess, contrast=contrast,
                 bscan=bscan, Xbscan=Xbscan, Ybscan=Ybscan, lvcorrs_orig=lvcorrs_orig, Tvsc_orig=Tvsc_orig, CI=CI,
-                indices=boot_indices, engine=eng, _early=early, boot_algo=boot_algo, _factor=factor)
+                indices=boot_indices, engine=eng, boot_algo=boot_algo, _plan=plan)
             if self.pls_alg in ("rb", "csb"):
                 self.conf_ints, self.std_errs, self.boot_ratios, self.LVcorr, self.boot_debug_dict = out
             elif self.pls_alg in ("mb", "cmb"):
@@ -685,8 +751,7 @@ class _ResampleTestPLS(ResampleTest):
             # only Y is permuted (:337-340, 395-396): X keeps its block z-scores, so everything lives in
             # N-space through Gz = Z Z^T
             cells = _cell_offsets(cond_order)
-            Ucoef = np.asarray(U, dtype=float) if contrast is None else class_functions._normalize(
-                np.asarray(contrast, dtype=float))
+            Ucoef = _ucoef(U, contrast)
             K = Ucoef.shape[1]
             Gz = _behaviour_state(eng, cells)["Gz"]
             if rotate_method == 0:
@@ -743,18 +808,17 @@ class _ResampleTestPLS(ResampleTest):
     @staticmethod
     def _bootstrap_test(X, Y, U, s, V, cond_order, mctype, niter, pls_alg, preprocess=None, dist_=(0.05, 0.95),
                         contrast=None, bscan=None, Xbscan=None, Ybscan=None, lvcorrs_orig=None, Tvsc_orig=None,
-                        CI=0.95, indices=None, engine=None, _early=None, boot_algo="direct", _factor=None):
-        """bootstrap_permutation.py:466-766 for the task methods (mct, cst).  `_early`: moments already enqueued by
-        `_bootstrap_moments_early` (pipelined upload of X).  `boot_algo`: see `check_boot_algo` ("auto" resolves here;
-        `_factor`: a `_factor_plan` for "collapsed").  A voxel-sharded engine
+                        CI=0.95, indices=None, engine=None, boot_algo="direct", _plan=None):
+        """bootstrap_permutation.py:466-766 for the task methods (mct, cst).  `boot_algo`: see `check_boot_algo`
+        ("auto" resolves here).  `_plan`: the `_TaskPlan` of these draws (mct / cst), with its moments when its moment
+        stage already ran; built here when None.  A voxel-sharded engine
         runs the moment GEMM of ALL bootstraps on its voxels (no moment all-reduce) and gathers the p x K results; the
         lazy `right_sv_sampled` and the salience percentiles are then gathered too, so every rank must ask for them."""
         eng = engine if engine is not None else Engine(X)
-        boot_algo = check_boot_algo(boot_algo, pls_alg, eng.precision, eng.N, niter, cond_order)
+        if _plan is None:
+            boot_algo = check_boot_algo(boot_algo, pls_alg, eng.precision, eng.N, niter, cond_order)
         if indices is None:
             indices = resample.bootstrap_indices(pls_alg, niter, cond_order, Y=Y, bscan=bscan, Ybscan=Ybscan)
-        if boot_algo == "collapsed" and _factor is None and _early is None and eng.N > Engine.QUAD_MAX_ROWS:
-            _factor = _factor_plan(eng, pls_alg, U, contrast, cond_order, mctype, niter, indices)   # the only route
         if pls_alg in ("mb", "cmb"):
             return _boot_multiblock(eng, U, s, V, cond_order, mctype, niter, pls_alg, contrast, bscan, Ybscan,
                                     lvcorrs_orig, Tvsc_orig, CI, indices)
@@ -763,28 +827,18 @@ class _ResampleTestPLS(ResampleTest):
         if pls_alg in ("rb", "csb"):
             return _ResampleTestPLS._bootstrap_behaviour(eng, Y, U, s, V, cond_order, niter, pls_alg, contrast,
                                                          lvcorrs_orig, CI, indices)
-        Lop, Ucoef, E = _task_operators(pls_alg, cond_order, mctype, U, contrast)
+        plan = _plan if _plan is not None else _TaskPlan(eng, pls_alg, U, s, V, cond_order, mctype, contrast, niter,
+                                                         indices, boot_algo)
+        Lop, Ucoef, E, idx_dev, lo, hi = plan.Lop, plan.Ucoef, plan.E, plan.idx, plan.lo, plan.hi
         Abar = class_functions._cell_mean_operator(cond_order)
-        # numerator of the bootstrap ratios = the original salience (:700-703); also the pivot that keeps
-        # the running sum of squares well conditioned.  V may already be a device tensor.
-        Vd = eng.to_device(V, torch.float64)
-        numer = Vd * eng.to_device(np.asarray(s, dtype=float), torch.float64) if contrast is None else Vd
-
-        lo, hi = dist.shard(niter)
-        idx_dev = _index_shard(eng, indices, niter, lo, hi)
+        numer_v = plan.numer
         vox = eng.voxel_sharded
-        if vox:         # this rank's voxels: rows [v0, v1) of the p x K operands, every bootstrap
-            v0, v1 = eng.voxel_range
-            numer_v = numer[v0:v1].contiguous()
-            idx_all = _index_shard(eng, indices, niter, 0, niter)
-        else:
-            numer_v = numer
         # exact mode, single launch: the packed coefficients serve the N-space pass and the moment GEMM
-        packed = (eng.pack_coef(E, idx_dev) if (hi > lo and eng.precision == "fp64" and _early is None
+        packed = (eng.pack_coef(E, idx_dev) if (hi > lo and eng.precision == "fp64" and plan.moments is None
                                                 and E.shape[1] <= eng.KMAX and not vox) else None)
         d2, Tdist = eng.nspace(E, idx_dev, Lmat=Abar, packed=packed)        # Tdistrib (:633-634, :665-666)
         if pls_alg == "mct":
-            XL = eng.xv(Vd)                                                 # X @ V once
+            XL = eng.xv(plan.V)                                             # X @ V once
             left = eng.uhat(XL, Lop, idx_dev)                               # U_hat (:617, :631)
         else:
             left = None
@@ -798,21 +852,7 @@ class _ResampleTestPLS(ResampleTest):
         defer = dist.world()[1] > 1
         fetch_small = (eng.to_host_async(eng.colstd(Tdist), side=True) if defer
                        else eng.to_host_async(eng.colstd(Tdist), Tdist, left, side=True))
-        if boot_algo == "collapsed":
-            # sum of squares about the bootstrap mean, already complete on every rank: no p x K all-reduce
-            s2 = _early if _early is not None else _collapsed_sumsq(eng, E, idx_dev, niter, lo, hi, factor=_factor)
-            s1 = torch.zeros_like(s2)
-        else:
-            if _early is not None:
-                s1, s2 = _early
-            elif vox:
-                s1, s2 = eng.boot_moments(E, idx_all, pivot=numer_v)
-            elif hi > lo:
-                s1, s2 = eng.boot_moments(E, idx_dev, pivot=numer, packed=packed)   # K4
-            else:
-                s1 = torch.zeros_like(numer); s2 = torch.zeros_like(numer)
-            if not vox:
-                dist.allreduce_packed_([s1, s2])
+        s1, s2 = plan.moments if plan.moments is not None else _boot_moments(eng, plan, niter, packed)
         std_errs, boot_ratios = eng.boot_finalize(s1, s2, niter, numer=numer_v)   # (:695-703)
         if vox:                                                             # ONE gather of [std_errs | boot_ratios]
             K = int(std_errs.shape[1])
@@ -858,33 +898,13 @@ class _ResampleTestPLS(ResampleTest):
 
     # ------------------------------------------------------------------------------------------
     @staticmethod
-    def _bootstrap_moments_early(eng, U, s, V, cond_order, mctype, niter, pls_alg, contrast, indices,
-                                 boot_algo="direct", _factor=None):
-        """The moment GEMM of `_bootstrap_test` for the task methods, on its own (single process).  Collapsed: the
-        N-space covariance build needs no X, so it runs while X is still crossing PCIe; the quadratic form follows
-        range by range as X arrives."""
-        if isinstance(indices, tuple):
-            indices = indices[0]
-        _, _, E = _task_operators(pls_alg, cond_order, mctype, U, contrast)
-        if boot_algo == "collapsed":
-            return _collapsed_sumsq(eng, E, _index_shard(eng, indices, niter, 0, niter), niter, 0, niter,
-                                    factor=_factor)
-        Vd = eng.to_device(V, torch.float64)
-        numer = Vd * eng.to_device(np.asarray(s, dtype=float), torch.float64) if contrast is None else Vd
-        idx_dev = _index_shard(eng, indices, niter, 0, niter)
-        return eng.boot_moments(E, idx_dev, pivot=numer)
-
-    # ------------------------------------------------------------------------------------------
-    @staticmethod
     def _bootstrap_behaviour(eng, Y, U, s, V, cond_order, niter, pls_alg, contrast, lvcorrs_orig, CI, indices):
         """bootstrap_permutation.py:537-675, 695-766 for rb / csb: X and Y rows are resampled together, the
         block z-scores of X change with every draw, so X is streamed once per bootstrap batch (K5)."""
         cells = _cell_offsets(cond_order)
-        Ucoef = np.asarray(U, dtype=float) if contrast is None else class_functions._normalize(
-            np.asarray(contrast, dtype=float))
+        Ucoef = _ucoef(U, contrast)
         nb = Y.shape[1]
-        Vd = eng.to_device(V, torch.float64)
-        numer = Vd * eng.to_device(np.asarray(s, dtype=float), torch.float64) if contrast is None else Vd
+        numer = _numerator(eng, V, s, contrast)
         Xc = _behaviour_state(eng, cells)["Xc"]
         lo, hi = dist.shard(niter)
         idx_dev = _index_shard(eng, indices, niter, lo, hi)

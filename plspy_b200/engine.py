@@ -18,6 +18,12 @@ F32 = torch.float32
 I32 = torch.int32
 
 
+def check_choice(name, value, allowed):
+    """ValueError unless `value` is one of `allowed` (the values of one option)."""
+    if value not in allowed:
+        raise ValueError(f"{name} must be one of {allowed}, got {value!r}")
+
+
 def _require_cuda():
     if not torch.cuda.is_available():
         raise RuntimeError(
@@ -60,12 +66,9 @@ class Engine:
         rank must call them at the same point.  With one process (or inside dist.local_only) the two layouts are the
         same."""
         _require_cuda()
-        if precision not in self.PRECISIONS:
-            raise ValueError(f"precision must be one of {self.PRECISIONS}")
-        if x_storage not in self.X_STORAGES:
-            raise ValueError(f"x_storage must be one of {self.X_STORAGES}, got {x_storage!r}")
-        if shard not in self.SHARDS:
-            raise ValueError(f"shard must be one of {self.SHARDS}, got {shard!r}")
+        check_choice("precision", precision, self.PRECISIONS)
+        check_choice("x_storage", x_storage, self.X_STORAGES)
+        check_choice("shard", shard, self.SHARDS)
         from . import dist
         self.shard = shard
         self._world = dist.world()
@@ -95,9 +98,32 @@ class Engine:
         """Address of column v0 of the device copy of X (float32 or float64 elements)."""
         return self._X.data_ptr() + self._X.element_size() * v0
 
-    @staticmethod
-    def _x32(M):
-        return M.dtype == F32
+    def _xfn(self, name, M=None):
+        """(function, name) of the entry point `name` reading M (default X), or of its float32 twin when M is float32:
+        `_x32` goes before the `_f64` suffix, in place of a trailing `_x`, or at the end."""
+        if (self._X if M is None else M).dtype == F32:
+            base, f64 = (name[:-4], "_f64") if name.endswith("_f64") else (name.removesuffix("_x"), "")
+            name = f"{base}_x32{f64}"
+        return getattr(lib, "plsb200_" + name), name
+
+    def _x_stream(self, v0=0, v1=None):
+        """The voxel ranges (lo, hi) of X clipped to [v0, v1), each yielded once the current stream waits for its upload."""
+        v1 = self.p if v1 is None else v1
+        cur = torch.cuda.current_stream(self.device)
+        for a, b, ev in self._x_ranges():
+            lo, hi = max(a, v0), min(b, v1)
+            if lo >= hi:
+                continue
+            if ev is not None:
+                cur.wait_event(ev)
+            yield lo, hi
+
+    def _column_blocks(self, K, part):
+        """A result of K > KMAX independent columns from `part(k0, k1)`, the result(s) of columns [k0, k1) <= KMAX wide."""
+        parts = [part(k0, min(K, k0 + self.KMAX)) for k0 in range(0, K, self.KMAX)]
+        if isinstance(parts[0], tuple):
+            return tuple(torch.cat(blocks, dim=1) for blocks in zip(*parts))
+        return torch.cat(parts, dim=1)
 
     def _collective(self):
         """The world this voxel-sharded engine was cut for must be the current one: a voxel-sharded engine used inside
@@ -376,7 +402,7 @@ class Engine:
     def gram_of(self, M):
         """K1: M M^T for a device matrix M (rows x p)."""
         n, p, ld = int(M.shape[0]), int(M.shape[1]), int(M.stride(0))
-        fn, what = (lib.plsb200_gram_x32_f64, "gram_x32_f64") if self._x32(M) else (lib.plsb200_gram_f64, "gram_f64")
+        fn, what = self._xfn("gram_f64", M)
         with torch.cuda.device(self.device):
             ws = self._ws(lib.plsb200_gram_f64_workspace(n, p))
             G = self._empty(n, n)
@@ -407,10 +433,8 @@ class Engine:
             elif self._pending is None:
                 self._G = self.gram_of(self.X)
             else:       # partial Gram matrices of the voxel ranges as they arrive, summed in a fixed order
-                cur = torch.cuda.current_stream(self.device)
                 G = None
-                for v0, v1, ev in self._x_ranges():
-                    cur.wait_event(ev)
+                for v0, v1 in self._x_stream():
                     Gc = self.gram_of(self._X[:, v0:v1])
                     G = Gc if G is None else G.add_(Gc)
                 self._G = G
@@ -418,22 +442,20 @@ class Engine:
                 self._collective().allreduce_sum_(self._G)
         return self._G
 
-    def _gram_tf32(self, ranges=None):
-        """K1 fast mode: G on the tcgen05 tensor cores, voxel range by voxel range as X arrives (TF32 split of a range
-        into the Gram kernel's operand image, then its partial Gram, accumulated in a fixed order)."""
+    def _gram_tf32(self, v0=0, v1=None):
+        """K1 fast mode: G of the voxels [v0, v1) on the tcgen05 tensor cores, voxel range by voxel range as X arrives
+        (TF32 split of a range into the Gram kernel's operand image, then its partial Gram, accumulated in a fixed
+        order)."""
         G = self._empty(self.N, self.N)
-        cur = torch.cuda.current_stream(self.device)
-        split = lib.plsb200_gram_tf32_split_x32 if self._x32(self._X) else lib.plsb200_gram_tf32_split
+        split, what = self._xfn("gram_tf32_split")
         with torch.cuda.device(self.device):
-            for i, (v0, v1, ev) in enumerate(self._x_ranges() if ranges is None else ranges):
-                if ev is not None:
-                    cur.wait_event(ev)
+            for i, (v0, v1) in enumerate(self._x_stream(v0, v1)):
                 pc = v1 - v0
                 img = self._ws(lib.plsb200_gram_tf32_image_bytes(self.N, pc))
                 nb = lib.plsb200_gram_tf32_workspace(self.N, pc)
                 ws = self._ws(nb)
                 self._mark("gram_tf32")
-                check(split(self._xp(v0), self.N, pc, self.ldx, self._p(img), self._stream()), "gram_tf32_split")
+                check(split(self._xp(v0), self.N, pc, self.ldx, self._p(img), self._stream()), what)
                 check(lib.plsb200_gram_tf32(self._p(img), self.N, pc, self._p(G), 1 if i else 0, self._p(ws), nb,
                                             self._stream()), "gram_tf32")
                 self._mark("gram_tf32")
@@ -452,7 +474,7 @@ class Engine:
             cut = [(self.p * r // size) // 64 * 64 for r in range(size)] + [self.p]
             if self.gram_tf32 and self.N <= self.GRAM_TF32_MAX_ROWS:
                 self.X                                      # (the whole of X is on the device from here on)
-                G = self._gram_tf32([(cut[rank], cut[rank + 1], None)])
+                G = self._gram_tf32(cut[rank], cut[rank + 1])
             else:
                 G = self.gram_of(self.X[:, cut[rank]:cut[rank + 1]])
             dist.allreduce_sum_(G)
@@ -472,7 +494,7 @@ class Engine:
         if self.p == 0:
             out = torch.zeros(self.N, K, dtype=F64, device=self.device)
         else:
-            fn, what = (lib.plsb200_xv_x32_f64, "xv_x32_f64") if self._x32(X) else (lib.plsb200_xv_f64, "xv_f64")
+            fn, what = self._xfn("xv_f64", X)
             with torch.cuda.device(self.device):
                 ws = self._ws(lib.plsb200_xv_f64_workspace(self.N, self.p, K))
                 out = self._empty(self.N, K)
@@ -638,8 +660,8 @@ class Engine:
                 torch.cuda.current_stream(self.device).wait_event(ev)
             with torch.cuda.device(self.device):
                 img = self._ws(lib.plsb200_tf32_ximage_bytes(self.N, v1 - v0))
-                split = lib.plsb200_tf32_split_x32 if self._x32(self._X) else lib.plsb200_tf32_split_x
-                check(split(self._xp(v0), self.N, v1 - v0, self.ldx, self._p(img), self._stream()), "tf32_split_x")
+                split, what = self._xfn("tf32_split_x")
+                check(split(self._xp(v0), self.N, v1 - v0, self.ldx, self._p(img), self._stream()), what)
             self._ximage[i] = (v0, v1, img)
         return self._ximage[i][2]
 
@@ -676,13 +698,9 @@ class Engine:
         R, K = int(idx.shape[0]), int(E.shape[1])
         if pivot is not None:
             pivot = self.to_device(pivot, F64)
-        if K > self.KMAX:   # columns are independent: split wide problems
-            parts = []
-            for k0 in range(0, K, self.KMAX):
-                sl = slice(k0, min(K, k0 + self.KMAX))
-                parts.append(self.boot_moments(E[:, sl].contiguous(), idx,
-                                               None if pivot is None else pivot[:, sl].contiguous()))
-            return torch.cat([a for a, _ in parts], dim=1), torch.cat([b for _, b in parts], dim=1)
+        if K > self.KMAX:
+            return self._column_blocks(K, lambda k0, k1: self.boot_moments(
+                E[:, k0:k1].contiguous(), idx, None if pivot is None else pivot[:, k0:k1].contiguous()))
         self._x_ranges()          # (starts a deferred upload of X now: every small input is already on its way)
         if self.p == 0:           # the empty voxel slice of a voxel-sharded rank
             return self._empty(0, K), self._empty(0, K)
@@ -695,12 +713,8 @@ class Engine:
                 raise _lib.PlsB200Error(f"boot_moments: unsupported shape N={self.N} K={K} R={R}")
             coef = packed["coef"]
             s1 = self._empty(self.p, K); s2 = self._empty(self.p, K)
-            cur = torch.cuda.current_stream(self.device)
-            fn, what = ((lib.plsb200_boot_moments_x32_f64, "boot_moments_x32_f64") if self._x32(self._X)
-                        else (lib.plsb200_boot_moments_f64, "boot_moments_f64"))
-            for v0, v1, ev in self._x_ranges():          # one launch per voxel range still arriving, else one in all
-                if ev is not None:
-                    cur.wait_event(ev)
+            fn, what = self._xfn("boot_moments_f64")
+            for v0, v1 in self._x_stream():             # one launch per voxel range still arriving, else one in all
                 pc = v1 - v0
                 ws = self._ws(lib.plsb200_boot_moments_f64_workspace(self.N, pc, K, R))
                 self._mark("boot_moments")
@@ -746,8 +760,8 @@ class Engine:
         v1 = self.p if v1 is None else int(v1)
         if N != self.N or tuple(Sig.shape) != (K, N, N):
             raise ValueError(f"boot_quad: Sig must be K x {self.N} x {self.N}")
-        if K > self.KMAX:   # columns are independent: split wide problems
-            return torch.cat([self.boot_quad(Sig[k0:k0 + self.KMAX], v0, v1) for k0 in range(0, K, self.KMAX)], dim=1)
+        if K > self.KMAX:
+            return self._column_blocks(K, lambda k0, k1: self.boot_quad(Sig[k0:k1], v0, v1))
         q = self._empty(max(v1 - v0, 0), K)
         if v1 <= v0:
             return q
@@ -758,15 +772,8 @@ class Engine:
             coef = self._ws(nbytes)
             check(lib.plsb200_boot_quad_coef_pack_f64(self._p(Sig), N, K, self._p(coef), self._stream()),
                   "boot_quad_coef_pack_f64")
-            cur = torch.cuda.current_stream(self.device)
-            fn, what = ((lib.plsb200_boot_quad_x32_f64, "boot_quad_x32_f64") if self._x32(self._X)
-                        else (lib.plsb200_boot_quad_f64, "boot_quad_f64"))
-            for a, b, ev in self._x_ranges():
-                lo, hi = max(a, v0), min(b, v1)
-                if lo >= hi:
-                    continue
-                if ev is not None:
-                    cur.wait_event(ev)
+            fn, what = self._xfn("boot_quad_f64")
+            for lo, hi in self._x_stream(v0, v1):
                 ws = self._ws(lib.plsb200_boot_quad_f64_workspace(N, hi - lo, K))
                 self._mark("boot_quad")
                 check(fn(self._xp(lo), N, hi - lo, self.ldx, self._p(coef), K, q.data_ptr() + 8 * (lo - v0) * K,
@@ -819,9 +826,8 @@ class Engine:
         E = self.to_device(E, F64); sid = self.to_device(sid, I32)
         K, J = int(E.shape[1]), int(L.shape[1])
         v1 = self.p if v1 is None else int(v1)
-        if K > self.KMAX:   # columns are independent: split wide problems
-            return torch.cat([self.boot_factor_quad(E[:, k0:k0 + self.KMAX].contiguous(), L, sid, v0, v1)
-                              for k0 in range(0, K, self.KMAX)], dim=1)
+        if K > self.KMAX:
+            return self._column_blocks(K, lambda k0, k1: self.boot_factor_quad(E[:, k0:k1].contiguous(), L, sid, v0, v1))
         q = self._empty(max(v1 - v0, 0), K)
         if v1 <= v0:
             return q
@@ -834,15 +840,8 @@ class Engine:
             coef = self._ws(nbytes)
             check(lib.plsb200_boot_factor_pack_f64(self._p(E), self.N, K, self._p(L), J, self._p(sid), self._p(coef),
                                                    self._stream()), "boot_factor_pack_f64")
-            cur = torch.cuda.current_stream(self.device)
-            fn, what = ((lib.plsb200_boot_moments_x32_f64, "boot_moments_x32_f64") if self._x32(self._X)
-                        else (lib.plsb200_boot_moments_f64, "boot_moments_f64"))
-            for a, b, ev in self._x_ranges():
-                lo, hi = max(a, v0), min(b, v1)
-                if lo >= hi:
-                    continue
-                if ev is not None:
-                    cur.wait_event(ev)
+            fn, what = self._xfn("boot_moments_f64")
+            for lo, hi in self._x_stream(v0, v1):
                 ws = self._ws(lib.plsb200_boot_moments_f64_workspace(self.N, hi - lo, K, J))
                 off = 8 * (lo - v0) * K
                 self._mark("boot_moments")
@@ -895,7 +894,7 @@ class Engine:
         lo = self._empty(self.p, K); hi = self._empty(self.p, K)
         vc = max(128, min(self.p, int(max_bytes // (R * K * 8)) // 128 * 128))
         X = self.X
-        series = lib.plsb200_salience_series_x32_f64 if self._x32(X) else lib.plsb200_salience_series_f64
+        series, what = self._xfn("salience_series_f64", X)
         nb = lib.plsb200_percentile_f64_workspace(R)
         with torch.cuda.device(self.device):
             ws = self._ws(nb)
@@ -905,7 +904,7 @@ class Engine:
                 # resample-major cube read in place with a stride of the chunk size cost 23-41 ms per chunk against 17)
                 cube = self._empty(v1 - v0, K, R)
                 check(series(self._xp(v0), self.N, v1 - v0, self.ldx, self._p(E), K, self._p(idx), R, self._p(cube),
-                             self._stream()), "salience_series_f64")
+                             self._stream()), what)
                 check(lib.plsb200_percentile_f64(self._p(cube), R, (v1 - v0) * K, 1, R, float(conf[0]), float(conf[1]),
                                                  lo.data_ptr() + 8 * v0 * K, hi.data_ptr() + 8 * v0 * K, self._p(ws), nb,
                                                  self._stream()), "percentile_f64")
@@ -921,9 +920,9 @@ class Engine:
         out = self._empty(R, p, K)
         if p == 0:
             return out
-        fn = lib.plsb200_salience_x32_f64 if self._x32(M) else lib.plsb200_salience_f64
+        fn, what = self._xfn("salience_f64", M)
         with torch.cuda.device(self.device):
-            check(fn(self._p(M), n, p, ld, self._p(E), K, self._p(idx), R, self._p(out), self._stream()), "salience_f64")
+            check(fn(self._p(M), n, p, ld, self._p(E), K, self._p(idx), R, self._p(out), self._stream()), what)
         return out
 
     # ------------------------------------------------------------------ split-half (K3)

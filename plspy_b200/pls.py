@@ -76,16 +76,9 @@ def PLS(*args, **kwargs):
     if "num_perm" in kwargs:
         if kwargs["num_perm"] < 0 or not isinstance(kwargs["num_perm"], int):
             raise ValueError("Invalid number of permutations provided. Value must be a positive integer.")
-    if "boot_algo" in kwargs:        # before any GPU work (the engine's upload of X starts with the analysis)
-        X = args[0] if args else kwargs.get("X")
-        engine = kwargs.get("engine")
-        nboot, cond_order = _boot_layout(pls_method, args, kwargs)
-        bootstrap_permutation.check_boot_algo(
-            kwargs["boot_algo"], pls_method, engine.precision if engine is not None else kwargs.get("precision", "fp64"),
-            engine.N if engine is not None else (int(X.shape[0]) if X is not None and hasattr(X, "shape") else None),
-            nboot, cond_order)
-    if "x_storage" in kwargs:
-        bootstrap_permutation.check_x_storage(kwargs["x_storage"], pls_method)
-    if "shard" in kwargs:
-        bootstrap_permutation.check_shard(kwargs["shard"], pls_method)
+    # the engine options, before any GPU work (the engine's upload of X starts with the analysis)
+    nboot, cond_order = _boot_layout(pls_method, args, kwargs)
+    bootstrap_permutation.resolve_options(
+        pls_method, kwargs.get("engine"), args[0] if args else kwargs.get("X"), nboot, cond_order,
+        kwargs.get("precision", "fp64"), kwargs.get("boot_algo", "auto"), kwargs.get("x_storage"), kwargs.get("shard"))
     return pls_classes.PLSBase._create(pls_method, *args, **kwargs)

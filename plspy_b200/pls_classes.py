@@ -58,24 +58,24 @@ class PLSBase(abc.ABC):
                 continue
             setattr(self, k, v)
             self._user_defined_attrs.add(k)
-        # storage of X on the device: the option, else that of a given engine (before any GPU work)
-        eng = self._engine_kwargs.get("engine")
-        xs = self._engine_kwargs.get("x_storage", eng.x_storage if eng is not None else "fp64")
-        if eng is not None and eng.x_storage != xs:
-            raise ValueError(f"x_storage={xs!r} but the engine holds X as {eng.x_storage!r}")
-        bootstrap_permutation.check_x_storage(xs, self.pls_alg)
-        self._engine_kwargs["x_storage"] = xs
-        # multi-process layout of X: the option, else that of a given engine
-        sh = self._engine_kwargs.get("shard", eng.shard if eng is not None else "resamples")
-        if eng is not None and eng.shard != sh:
-            raise ValueError(f"shard={sh!r} but the engine holds X laid out for shard={eng.shard!r}")
-        bootstrap_permutation.check_shard(sh, self.pls_alg)
-        self._engine_kwargs["shard"] = sh
+        # storage and multi-process layout of X: the options, else those of a given engine (before any GPU work; the
+        # bootstrap formulation is resolved with the resampling test, which knows the bootstrap count)
+        ek = self._engine_kwargs
+        _, _, ek["x_storage"], ek["shard"] = bootstrap_permutation.resolve_options(
+            self.pls_alg, ek.get("engine"), precision=ek.get("precision", "fp64"), boot_algo=None,
+            x_storage=ek.get("x_storage"), shard=ek.get("shard"))
 
-    def _shard_kw(self):
-        """Engine keyword for the layout of X: none for the default (the same construction as without the option)."""
-        sh = self._engine_kwargs["shard"]
-        return {} if sh == "resamples" else {"shard": sh}
+    def _new_engine(self, device=None, exact=False):
+        """An Engine holding X (the copy prepared for the device, else self.X) as the options ask; `exact`: whatever the
+        precision option.  No `shard` keyword for the default layout: the same construction as without the option."""
+        from .engine import Engine
+        ek = self._engine_kwargs
+        kw = {} if ek["shard"] == "resamples" else {"shard": ek["shard"]}
+        if not exact:
+            kw["precision"] = ek.get("precision", "fp64")
+        src = getattr(self, "_x_tensor", None)
+        return Engine(self.X if src is None else src, device=ek.get("device") if device is None else device,
+                      x_storage=ek["x_storage"], **kw)
 
     @staticmethod
     def _get_groups_info(groups_tuple):
@@ -176,12 +176,9 @@ class PLSBase(abc.ABC):
             return
         import concurrent.futures
         import torch
-        from .engine import Engine
         device = ek.get("device")
         if device is None and torch.cuda.is_available():
             device = torch.device("cuda", torch.cuda.current_device())     # (the current device is per thread)
-        xsrc = getattr(self, "_x_tensor", None)
-        xsrc = self.X if xsrc is None else xsrc
         Y = getattr(self, "Y", None) if self.pls_alg in ("rb", "csb", "mb", "cmb") else None
         multi = self.pls_alg in ("mb", "cmb")
         bscan, Ybscan = (self.bscan, self.Ybscan) if multi else (None, None)
@@ -189,8 +186,7 @@ class PLSBase(abc.ABC):
         def work():
             out = {}
             if want_eng:
-                out["engine"] = Engine(xsrc, device=device, precision=ek.get("precision", "fp64"),
-                                       x_storage=ek["x_storage"], **self._shard_kw())
+                out["engine"] = self._new_engine(device)
             if want_idx:
                 if self.num_perm > 0:
                     out["perm_indices"] = resample.permutation_indices(self.pls_alg, self.num_perm, self.cond_order, Y=Y,
@@ -221,11 +217,7 @@ class PLSBase(abc.ABC):
         if mode == "host":
             return False
         if self._engine_kwargs.get("engine") is None:
-            from .engine import Engine
-            self._engine_kwargs["engine"] = Engine(getattr(self, "_x_tensor", None) if getattr(self, "_x_tensor", None)
-                                                   is not None else self.X, device=self._engine_kwargs.get("device"),
-                                                   precision=self._engine_kwargs.get("precision", "fp64"),
-                                                   x_storage=self._engine_kwargs["x_storage"], **self._shard_kw())
+            self._engine_kwargs["engine"] = self._new_engine()
         return True
 
     def _resample(self, Y, mctype, preprocess, **kw):
@@ -233,10 +225,7 @@ class PLSBase(abc.ABC):
         V = getattr(self, "_V_dev", None)
         xt = getattr(self, "_x_tensor", None)
         if xt is not None and self._engine_kwargs.get("engine") is None and (self.num_perm > 0 or self.num_boot > 0):
-            from .engine import Engine
-            self._engine_kwargs["engine"] = Engine(xt, device=self._engine_kwargs.get("device"),
-                                                   precision=self._engine_kwargs.get("precision", "fp64"),
-                                                   x_storage=self._engine_kwargs["x_storage"], **self._shard_kw())
+            self._engine_kwargs["engine"] = self._new_engine()
         self.resample_tests = bootstrap_permutation.ResampleTest._create(
             self.pls_alg, self.X, Y, self.U, self.s, self.V if V is None else V, self.cond_order, mctype, preprocess=preprocess,
             nperm=self.num_perm, nboot=self.num_boot, CI=self.CI,
@@ -262,10 +251,7 @@ class PLSBase(abc.ABC):
                                     or self._engine_kwargs["shard"] == "voxels"):
                     # no resampling engine: the split-half functions would each upload the (widened) host copy as
                     # float64 and whole; one engine holding X as asked (exact mode, as theirs) serves both instead
-                    from .engine import Engine
-                    src = getattr(self, "_x_tensor", None)
-                    eng = Engine(self.X if src is None else src, device=self._engine_kwargs.get("device"),
-                                 x_storage=self._engine_kwargs["x_storage"], **self._shard_kw())
+                    eng = self._new_engine(exact=True)
                 self.pls_repro_tt = split_half_resampling.split_half_test_train(
                     self.pls_alg, self.X, Y, self.cond_order, num_split=self.num_split, mctype=mctype,
                     contrasts=contrasts, engine=eng, **kw)

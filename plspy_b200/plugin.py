@@ -60,16 +60,10 @@ class _InstalledResampleTest(_bp._ResampleTestPLS):
     def __init__(self, X, Y, U, s, V, cond_order, mctype, *args, **kwargs):
         nperm = kwargs.get("nperm", 1000)
         nboot = kwargs.get("nboot", 1000)
-        kwargs.setdefault("x_storage", _options["x_storage"])
-        kwargs.setdefault("shard", _options["shard"])
-        kwargs.setdefault("precision", _options["precision"])
-        kwargs.setdefault("boot_algo", _options["boot_algo"])
-        _bp.check_x_storage(kwargs["x_storage"], self.pls_alg)        # before the engine uploads X
-        _bp.check_shard(kwargs["shard"], self.pls_alg)
-        eng = kwargs.get("engine")
-        _bp.check_boot_algo(kwargs["boot_algo"], self.pls_alg, eng.precision if eng is not None else kwargs["precision"],
-                            eng.N if eng is not None else (int(X.shape[0]) if hasattr(X, "shape") else None), nboot,
-                            cond_order)
+        for name, value in _options.items():
+            kwargs.setdefault(name, value)
+        _bp.resolve_options(self.pls_alg, kwargs.get("engine"), X, nboot, cond_order,       # before the engine uploads X
+                            **{name: kwargs[name] for name in _options})
         if "engine" not in kwargs and (nperm > 0 or nboot > 0):
             kwargs["engine"] = shared_engine(X)
         super().__init__(X, Y, U, s, V, cond_order, mctype, *args, **kwargs)
@@ -111,16 +105,10 @@ def install(plspy_module=None, precision="fp64", boot_algo="auto", x_storage="fp
     multi-process run: every rank holds only its columns of X, see `bootstrap_permutation.check_shard`); behaviour and
     multiblock analyses raise NotImplementedError with "voxels"."""
     global _state
-    if precision not in ("fp64", "tf32x3", "tf32x3+gram"):
-        raise ValueError('precision must be "fp64", "tf32x3" or "tf32x3+gram"')
-    if boot_algo not in _bp.BOOT_ALGOS:
-        raise ValueError(f"boot_algo must be one of {_bp.BOOT_ALGOS}")
-    if boot_algo == "collapsed" and precision != "fp64":
-        raise ValueError('boot_algo="collapsed" is an exact (precision="fp64") formulation')
-    if x_storage not in _bp.X_STORAGES:
-        raise ValueError(f"x_storage must be one of {_bp.X_STORAGES}")
-    if shard not in _bp.SHARDS:
-        raise ValueError(f"shard must be one of {_bp.SHARDS}")
+    # the values themselves; what a method or design does not support is refused by each resampling test ("mct"
+    # supports every value)
+    _, _, x_storage, shard = _bp.resolve_options("mct", precision=precision, boot_algo=boot_algo, x_storage=x_storage,
+                                                 shard=shard)
     if plspy_module is None:
         import plspy as plspy_module
     ref_bp = plspy_module.core.bootstrap_permutation
