@@ -21,15 +21,17 @@
 //     x 8 columns; it is folded into per-thread running sums and discarded.  Column -> k is fixed per
 //     thread for the whole kernel because the period is a multiple of K.
 // Shared memory: nstage x (N/4 * NBLK * 256 B) ring (57.6 KB per stage at N=300, K=12 -> 3 stages).
+// The ring, the A fragments and the DMMA stream are ring_pipeline (boot_plan.cuh), shared with nspace_dmma_kernel below
+// and boot_quad_kernel (boot_quad.cu); boot_moments_kernel adds MomentsEpilogue: the chains start from -pivot, the D
+// fragments are folded into running moments with the ragged last period masked, and fold_slots_store writes them.
 #include "common.cuh"
 #include "boot_plan.cuh"
 
 namespace plsb {
 
 // ------------------------------------------------------------------------------------------------
-// coefficient packing: C_r = scatter(E, idx_r) written in B-fragment order.
-// offset(per, s, jb, lane) = ((per*nks + s)*nblk + jb)*32 + lane,  lane = 4*n + q,
-// column-in-period c = (r % nb)*Kp + k -> jb = c/8, n = c%8 ; row i -> s = i/4, q = i%4.
+// coefficient packing: C_r = scatter(E, idx_r) written in B-fragment order (bfrag_offset, boot_plan.cuh): resample r
+// is slot r % nb of period r / nb, column c = (r % nb)*Kp + k ; row i -> s = i/4, q = i%4.
 // One CTA per PERIOD (nb resamples): thread i scans idx for sources of target row i in index order (deterministic),
 // the period's block is assembled in shared memory in fragment order and written out as one contiguous, coalesced
 // piece.  (Round 1 wrote every coefficient straight to its fragment position: 8-byte stores at a stride of
@@ -64,8 +66,7 @@ __global__ void __launch_bounds__(256) boot_coef_pack_kernel(const double* __res
 #pragma unroll
             for (int k = 0; k < 24; ++k) {
                 if (k < K) {
-                    const int c = cbase + k;
-                    blk[(s * nblk + (c >> 3)) * 32 + 4 * (c & 7) + q] = acc[k];
+                    blk[bfrag_offset(s, cbase + k, q, nblk)] = acc[k];
                 }
             }
         }
@@ -93,10 +94,7 @@ __global__ void __launch_bounds__(256) boot_factor_pack_kernel(const double* __r
         if (j >= J) continue;
         const double w = L[(size_t)sid[i] * J + j];
         const int s = i >> 2, q = i & 3;
-        for (int k = 0; k < K; ++k) {
-            const int c = slot * Kp + k;
-            smf[(s * nblk + (c >> 3)) * 32 + 4 * (c & 7) + q] = E[(size_t)i * K + k] * w;
-        }
+        for (int k = 0; k < K; ++k) smf[bfrag_offset(s, slot * Kp + k, q, nblk)] = E[(size_t)i * K + k] * w;
     }
     __syncthreads();
     double2* out = reinterpret_cast<double2*>(coef + (size_t)per * stage_doubles);
@@ -105,159 +103,67 @@ __global__ void __launch_bounds__(256) boot_factor_pack_kernel(const double* __r
 }
 
 // ------------------------------------------------------------------------------------------------
-// NKS (k-steps of 4 rows) is a compile-time constant so that the whole period is one straight-line
-// stream of NKS*NBLK {LDS.64, DMMA} pairs that ptxas can software-pipeline; kernels are instantiated
-// for every multiple of 4 up to 80 (N <= 320).  T: element type of X (float: X stored as float32, widened as the A
-// fragments are loaded -- the same DMMA operands as from the widened matrix).
+// The moments epilogue: the chains start from -pivot, so a D fragment holds VS - pivot for 8 voxels x 8 columns; it is
+// folded into per-thread running sums and sums of squares (s[0], s[1]) and discarded.  Column -> k is fixed per thread
+// for the whole kernel because the period is a multiple of K.  The padding slots of a ragged last period are masked.
+template <int NBLK>
+struct MomentsEpilogue : RingEpilogue {
+    struct Args { const double* pivot; long long v, p; int R, Kp, K; double* osum; double* osumsq; };
+    const Args a;
+    const RingThread th;
+    double piv[NBLK][2], s[2][NBLK][2];
+    int nb;
+    __device__ __forceinline__ MomentsEpilogue(const Args& args, const RingThread& t) : a(args), th(t) {
+#pragma unroll
+        for (int j = 0; j < NBLK; ++j)
+#pragma unroll
+            for (int e = 0; e < 2; ++e) {
+                const int c = 8 * j + 2 * th.q + e, k = c % a.Kp;
+                piv[j][e] = (a.pivot != nullptr && k < a.K && a.v < a.p) ? __ldg(a.pivot + a.v * a.K + k) : 0.0;
+                s[0][j][e] = 0.0; s[1][j][e] = 0.0;
+            }
+        nb = 8 * NBLK / a.Kp;
+    }
+    __device__ __forceinline__ double d0(int j, int e) const { return -piv[j][e]; }
+    __device__ __forceinline__ void fold(const double (&d)[NBLK][2], int it) {
+        if (it + 1 < th.nit || (th.per0 + it + 1) * nb <= a.R) {      // every slot of the period is a real resample
+#pragma unroll
+            for (int j = 0; j < NBLK; ++j)
+#pragma unroll
+                for (int e = 0; e < 2; ++e) {
+                    s[0][j][e] += d[j][e];
+                    s[1][j][e] = fma(d[j][e], d[j][e], s[1][j][e]);
+                }
+        } else {                                                      // ragged last period: mask the padding slots
+            const int rbase = (th.per0 + it) * nb;
+#pragma unroll
+            for (int j = 0; j < NBLK; ++j)
+#pragma unroll
+                for (int e = 0; e < 2; ++e) {
+                    if (rbase + (8 * j + 2 * th.q + e) / a.Kp < a.R) {
+                        s[0][j][e] += d[j][e];
+                        s[1][j][e] = fma(d[j][e], d[j][e], s[1][j][e]);
+                    }
+                }
+        }
+    }
+    __device__ __forceinline__ void finish(double* red) {
+        fold_slots_store<2, NBLK>(s, red, th, nb, a.Kp, a.K, a.p, {a.osum, a.osumsq});
+    }
+};
+
+// T: element type of X (float: X stored as float32, widened as the A fragments are loaded -- the same DMMA operands as
+// from the widened matrix).
 template <typename T, int NKS, int NBLK>
 __global__ void __launch_bounds__(BM_THREADS, 1)
 boot_moments_kernel(const T* __restrict__ X, long long ldx, int N, long long p,
                     const double* __restrict__ coef, int nper, int per_per_split, int nstage,
                     int R, int Kp, int K, const double* __restrict__ pivot,
                     double* __restrict__ osum, double* __restrict__ osumsq) {
-    extern __shared__ __align__(128) unsigned char smraw[];
-    constexpr int stage_doubles = NKS * NBLK * 32;
-    constexpr uint32_t stage_bytes = (uint32_t)stage_doubles * 8u;
-    double* ring = reinterpret_cast<double*>(smraw);
-    double* red = ring + (size_t)nstage * stage_doubles;              // [8 warps][2][8][Kp]
-    uint64_t* full = reinterpret_cast<uint64_t*>(red + BM_WARPS * 16 * Kp);
-    uint64_t* empty = full + nstage;
-
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int q = lane & 3, vr = lane >> 2;
-    const long long v = (long long)blockIdx.x * BM_VOX + warp * 8 + vr;
-    const int per0 = blockIdx.y * per_per_split;
-    const int per1 = min(nper, per0 + per_per_split);
-    const int nit = per1 - per0;
-
-    if (tid == 0) {
-        for (int s = 0; s < nstage; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, BM_WARPS); }
-        mbar_fence_init();
-    }
-    __syncthreads();
-
-    auto issue = [&](int it, int slot) {   // thread 0 only: stream period per0+it into `slot`
-        mbar_expect_tx(full + slot, stage_bytes);
-        const char* src = reinterpret_cast<const char*>(coef + (size_t)(per0 + it) * stage_doubles);
-        char* dst = reinterpret_cast<char*>(ring + (size_t)slot * stage_doubles);
-#pragma unroll 1
-        for (uint32_t off = 0; off < stage_bytes; off += 16384u) {
-            const uint32_t n = min(16384u, stage_bytes - off);
-            bulk_g2s(dst + off, src + off, n, full + slot);
-        }
-    };
-    if (tid == 0)
-        for (int it = 0; it < min(nstage, nit); ++it) issue(it, it);
-
-    // ---- A fragments: this warp's 8 voxels x all rows, resident in registers
-    double a[NKS];
-#pragma unroll
-    for (int s = 0; s < NKS; ++s) {
-        const int row = 4 * s + q;
-        a[s] = (row < N && v < p) ? (double)__ldg(X + (long long)row * ldx + v) : 0.0;
-    }
-
-    // ---- per-thread column bookkeeping (fixed for the whole kernel)
-    double piv[NBLK][2], s1[NBLK][2], s2[NBLK][2];
-#pragma unroll
-    for (int j = 0; j < NBLK; ++j)
-#pragma unroll
-        for (int e = 0; e < 2; ++e) {
-            const int c = 8 * j + 2 * q + e, k = c % Kp;
-            piv[j][e] = (pivot != nullptr && k < K && v < p) ? __ldg(pivot + v * K + k) : 0.0;
-            s1[j][e] = 0.0; s2[j][e] = 0.0;
-        }
-    const int nb = 8 * NBLK / Kp;
-
-    // The two warps that share an SM sub-partition (w and w+4) run half a period apart, so that one of
-    // them always has a full MMA stream in flight while the other folds its accumulators and waits on
-    // the next stage (otherwise all eight warps drain the DMMA pipe at the same instant).
-    if (warp >= 4) __nanosleep((unsigned)(NKS * NBLK * 8));
-
-    int slot = 0, prev_slot = 0;
-    uint32_t phase = 0, prev_phase = 0;
-    for (int it = 0; it < nit; ++it) {
-        if (tid == 0 && it > 0) {
-            // refill the slot drained in the previous iteration with period it-1+nstage
-            const int nx = it - 1 + nstage;
-            if (nx < nit) {
-                mbar_wait(empty + prev_slot, prev_phase);
-                issue(nx, prev_slot);
-            }
-        }
-        __syncwarp();
-        mbar_wait(full + slot, phase);
-
-        double d[NBLK][2];
-#pragma unroll
-        for (int j = 0; j < NBLK; ++j) { d[j][0] = -piv[j][0]; d[j][1] = -piv[j][1]; }
-        // volatile: ptxas must keep these loads in program order (s-major, chains round-robin), which
-        // keeps the NBLK accumulator chains interleaved; without it the straight-line stream is
-        // re-ordered chain by chain (fewest live registers) and every DMMA waits on its predecessor.
-        const volatile double* bs = ring + (size_t)slot * stage_doubles + lane;
-#pragma unroll
-        for (int s = 0; s < NKS; ++s) {
-#pragma unroll
-            for (int j = 0; j < NBLK; ++j) {
-                const double b = bs[(s * NBLK + j) * 32];
-                dmma884(d[j][0], d[j][1], a[s], b);
-            }
-        }
-        __syncwarp();
-        if (lane == 0) mbar_arrive(empty + slot);
-
-        if (it + 1 < nit || (per0 + it + 1) * nb <= R) {      // every slot of the period is a real resample
-#pragma unroll
-            for (int j = 0; j < NBLK; ++j)
-#pragma unroll
-                for (int e = 0; e < 2; ++e) {
-                    s1[j][e] += d[j][e];
-                    s2[j][e] = fma(d[j][e], d[j][e], s2[j][e]);
-                }
-        } else {                                              // ragged last period: mask the padding slots
-            const int rbase = (per0 + it) * nb;
-#pragma unroll
-            for (int j = 0; j < NBLK; ++j)
-#pragma unroll
-                for (int e = 0; e < 2; ++e) {
-                    if (rbase + (8 * j + 2 * q + e) / Kp < R) {
-                        s1[j][e] += d[j][e];
-                        s2[j][e] = fma(d[j][e], d[j][e], s2[j][e]);
-                    }
-                }
-        }
-        prev_slot = slot; prev_phase = phase;
-        if (++slot == nstage) { slot = 0; phase ^= 1u; }
-    }
-
-    // ---- fold the nb resample slots of a period onto k, in slot order (deterministic)
-    double* r1 = red + warp * (16 * Kp);
-    double* r2 = r1 + 8 * Kp;
-    for (int i = lane; i < 16 * Kp; i += 32) r1[i] = 0.0;
-    __syncwarp();
-    for (int round = 0; round < nb; ++round) {
-#pragma unroll
-        for (int j = 0; j < NBLK; ++j)
-#pragma unroll
-            for (int e = 0; e < 2; ++e) {
-                const int c = 8 * j + 2 * q + e;
-                if (c / Kp == round) {
-                    r1[vr * Kp + c % Kp] += s1[j][e];
-                    r2[vr * Kp + c % Kp] += s2[j][e];
-                }
-            }
-        __syncwarp();
-    }
-    const long long vbase = (long long)blockIdx.x * BM_VOX + warp * 8;
-    double* o1 = osum + (size_t)blockIdx.y * p * K;
-    double* o2 = osumsq + (size_t)blockIdx.y * p * K;
-    for (int i = lane; i < 8 * K; i += 32) {
-        const int rr = i / K, k = i % K;
-        if (vbase + rr < p) {
-            o1[(vbase + rr) * K + k] = r1[rr * Kp + k];
-            o2[(vbase + rr) * K + k] = r2[rr * Kp + k];
-        }
-    }
+    const RingThread th(threadIdx.x, nper, per_per_split);
+    const long long v = (long long)blockIdx.x * BM_VOX + th.warp * 8 + th.vr;
+    ring_pipeline<NKS, NBLK, MomentsEpilogue<NBLK>>(th, X, ldx, N, v, v < p, coef, nstage, BM_WARPS * 16 * Kp,
+                                                    {pivot, v, p, R, Kp, K, osum, osumsq});
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -268,7 +174,9 @@ boot_moments_kernel(const T* __restrict__ X, long long ldx, int N, long long p,
 // up to 8), so a warp's 8 "voxels" are either rows of H -- its D fragment is multiplied element-wise with the
 // coefficients of those rows (read from the stage in shared memory), reduced over the 8 rows with shuffles and written
 // as one partial per (voxel group, resample, k) -- or rows of T, which are stored as they are.  Partials are summed in
-// a fixed order by nspace_finish_kernel (deterministic), which also applies 1/sqrt(d2) to T.
+// a fixed order by nspace_finish_kernel (deterministic), which also applies 1/sqrt(d2) to T.  The pipeline is
+// ring_pipeline with W as the data matrix; NspaceEpilogue adds the read of the row's own coefficients from the stage
+// before it is released, and the shuffle reduction or the store of T.
 // Replaces nspace_kernel (FMA, bound by the shared-memory pipe: profiles/ncu_nspace_r02.md) for N <= 320.
 struct NsArgs {
     const double* W; long long ldw; int N, Nv, Npad;
@@ -277,86 +185,31 @@ struct NsArgs {
     double* Traw;       // [R][Kt][K] or NULL
 };
 
-template <int NKS, int NBLK>
-__global__ void __launch_bounds__(BM_THREADS, 1) nspace_dmma_kernel(const NsArgs a) {
-    extern __shared__ __align__(128) unsigned char smraw[];
-    constexpr int stage_doubles = NKS * NBLK * 32;
-    constexpr uint32_t stage_bytes = (uint32_t)stage_doubles * 8u;
-    double* ring = reinterpret_cast<double*>(smraw);
-    uint64_t* full = reinterpret_cast<uint64_t*>(ring + (size_t)a.nstage * stage_doubles);
-    uint64_t* empty = full + a.nstage;
-
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int q = lane & 3, vr = lane >> 2;
-    const int group = blockIdx.x * BM_WARPS + warp;          // 8 consecutive columns of W
-    const int v = group * 8 + vr;
-    const int per0 = blockIdx.y * a.per_per_split;
-    const int per1 = min(a.nper, per0 + a.per_per_split);
-    const int nit = per1 - per0;
-
-    if (tid == 0) {
-        for (int s = 0; s < a.nstage; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, BM_WARPS); }
-        mbar_fence_init();
-    }
-    __syncthreads();
-    auto issue = [&](int it, int slot) {
-        mbar_expect_tx(full + slot, stage_bytes);
-        const char* src = reinterpret_cast<const char*>(a.coef + (size_t)(per0 + it) * stage_doubles);
-        char* dst = reinterpret_cast<char*>(ring + (size_t)slot * stage_doubles);
-#pragma unroll 1
-        for (uint32_t off = 0; off < stage_bytes; off += 16384u)
-            bulk_g2s(dst + off, src + off, min(16384u, stage_bytes - off), full + slot);
-    };
-    if (tid == 0)
-        for (int it = 0; it < min(a.nstage, nit); ++it) issue(it, it);
-
-    double x[NKS];
-#pragma unroll
-    for (int s = 0; s < NKS; ++s) {
-        const int row = 4 * s + q;
-        x[s] = (row < a.N && v < a.Nv) ? __ldg(a.W + (long long)row * a.ldw + v) : 0.0;
-    }
-    const bool is_h = group * 8 < a.Npad;                    // warp-uniform: rows of H, else rows of T
-    const int nb = 8 * NBLK / a.Kp;
-    if (warp >= 4) __nanosleep((unsigned)(NKS * NBLK * 8));
-
-    int slot = 0, prev_slot = 0;
-    uint32_t phase = 0, prev_phase = 0;
-    for (int it = 0; it < nit; ++it) {
-        if (tid == 0 && it > 0) {
-            const int nx = it - 1 + a.nstage;
-            if (nx < nit) {
-                mbar_wait(empty + prev_slot, prev_phase);
-                issue(nx, prev_slot);
-            }
-        }
-        __syncwarp();
-        mbar_wait(full + slot, phase);
-        double d[NBLK][2];
-#pragma unroll
-        for (int j = 0; j < NBLK; ++j) d[j][0] = d[j][1] = 0.0;
-        const volatile double* bs = ring + (size_t)slot * stage_doubles + lane;
-#pragma unroll
-        for (int s = 0; s < NKS; ++s) {
-#pragma unroll
-            for (int j = 0; j < NBLK; ++j) {
-                const double b = bs[(s * NBLK + j) * 32];
-                dmma884(d[j][0], d[j][1], x[s], b);
-            }
-        }
-        // the coefficients of this thread's own row (v) for its columns: C[v, c] sits at k-step v/4, element v%4
-        double cv[NBLK][2];
+// The N-space epilogue.  A warp over rows of H reads, before the stage is released, the coefficients of its thread's
+// own row v for the thread's columns; the product with the D element is reduced over the warp's 8 rows and stored as a
+// partial of d2.  A warp over rows of T stores its D elements.
+template <int NBLK>
+struct NspaceEpilogue : RingEpilogue {
+    struct Args { const NsArgs& a; int group, v; };
+    const Args x;
+    const RingThread th;
+    const bool is_h;                                         // warp-uniform: rows of H, else rows of T
+    const int nb;
+    double cv[NBLK][2];
+    __device__ __forceinline__ NspaceEpilogue(const Args& args, const RingThread& t)
+        : x(args), th(t), is_h(args.group * 8 < args.a.Npad), nb(8 * NBLK / args.a.Kp) {}
+    __device__ __forceinline__ void read_stage(const double* stage) {
         if (is_h) {
-            const double* cs = ring + (size_t)slot * stage_doubles + (size_t)(v >> 2) * NBLK * 32 + (v & 3);
 #pragma unroll
             for (int j = 0; j < NBLK; ++j)
 #pragma unroll
-                for (int e = 0; e < 2; ++e) cv[j][e] = v < a.N ? cs[j * 32 + 4 * (2 * q + e)] : 0.0;
+                for (int e = 0; e < 2; ++e)
+                    cv[j][e] = x.v < x.a.N ? stage[bfrag_offset(x.v >> 2, 8 * j + 2 * th.q + e, x.v & 3, NBLK)] : 0.0;
         }
-        __syncwarp();
-        if (lane == 0) mbar_arrive(empty + slot);
-
-        const int rbase = (per0 + it) * nb;
+    }
+    __device__ __forceinline__ void fold(const double (&d)[NBLK][2], int it) {
+        const NsArgs& a = x.a;
+        const int rbase = (th.per0 + it) * nb;
         if (is_h) {
 #pragma unroll
             for (int j = 0; j < NBLK; ++j)
@@ -366,22 +219,29 @@ __global__ void __launch_bounds__(BM_THREADS, 1) nspace_dmma_kernel(const NsArgs
                     pr += __shfl_xor_sync(0xffffffffu, pr, 4);
                     pr += __shfl_xor_sync(0xffffffffu, pr, 8);
                     pr += __shfl_xor_sync(0xffffffffu, pr, 16);
-                    const int c = 8 * j + 2 * q + e, r = rbase + c / a.Kp, k = c % a.Kp;
-                    if (vr == 0 && k < a.K && r < a.R) a.dpart[((size_t)group * a.R + r) * a.K + k] = pr;
+                    const int c = 8 * j + 2 * th.q + e, r = rbase + c / a.Kp, k = c % a.Kp;
+                    if (th.vr == 0 && k < a.K && r < a.R) a.dpart[((size_t)x.group * a.R + r) * a.K + k] = pr;
                 }
         } else if (a.Traw != nullptr) {
-            const int ci = v - a.Npad;
+            const int ci = x.v - a.Npad;
 #pragma unroll
             for (int j = 0; j < NBLK; ++j)
 #pragma unroll
                 for (int e = 0; e < 2; ++e) {
-                    const int c = 8 * j + 2 * q + e, r = rbase + c / a.Kp, k = c % a.Kp;
+                    const int c = 8 * j + 2 * th.q + e, r = rbase + c / a.Kp, k = c % a.Kp;
                     if (ci < a.Kt && k < a.K && r < a.R) a.Traw[((size_t)r * a.Kt + ci) * a.K + k] = d[j][e];
                 }
         }
-        prev_slot = slot; prev_phase = phase;
-        if (++slot == a.nstage) { slot = 0; phase ^= 1u; }
     }
+};
+
+template <int NKS, int NBLK>
+__global__ void __launch_bounds__(BM_THREADS, 1) nspace_dmma_kernel(const NsArgs a) {
+    const RingThread th(threadIdx.x, a.nper, a.per_per_split);
+    const int group = blockIdx.x * BM_WARPS + th.warp;      // 8 consecutive columns of W
+    const int v = group * 8 + th.vr;
+    ring_pipeline<NKS, NBLK, NspaceEpilogue<NBLK>>(th, a.W, a.ldw, a.N, v, v < a.Nv, a.coef, a.nstage, 0,
+                                                   {a, group, v});
 }
 
 // W = [G | 0 | (Lmat G)^T]: N rows, ldw columns
@@ -414,13 +274,17 @@ __global__ void nspace_finish_kernel(const double* __restrict__ dpart, int ngrou
     }
 }
 
-__global__ void moments_reduce_kernel(const double* __restrict__ part1, const double* __restrict__ part2, int nsplit,
-                                      long long n, double* __restrict__ sum, double* __restrict__ sumsq) {
+__global__ void split_sum_kernel(const double* __restrict__ part1, const double* __restrict__ part2, int nsplit,
+                                 long long n, double* __restrict__ out1, double* __restrict__ out2) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    double a = 0.0, b = 0.0;
-    for (int s = 0; s < nsplit; ++s) { a += part1[(size_t)s * n + i]; b += part2[(size_t)s * n + i]; }
-    sum[i] = a; sumsq[i] = b;
+    double a = 0.0;
+    for (int s = 0; s < nsplit; ++s) a += part1[(size_t)s * n + i];
+    out1[i] = a;
+    if (out2 == nullptr) return;
+    double b = 0.0;
+    for (int s = 0; s < nsplit; ++s) b += part2[(size_t)s * n + i];
+    out2[i] = b;
 }
 
 __global__ void boot_finalize_kernel(const double* __restrict__ sum, const double* __restrict__ sumsq, long long n,
@@ -536,33 +400,6 @@ __global__ void xv_reduce_kernel(const double* __restrict__ part, int nchunk, in
     out[i] = s;
 }
 
-template <typename T, int NKS, int NBLK>
-static int launch_moments(const BootPlan& b, const T* X, int N, int64_t p, int64_t ldx, const double* coef, int K,
-                          int R, const double* pivot, double* o1, double* o2, cudaStream_t st) {
-    PLSB_CUDA(cudaFuncSetAttribute(boot_moments_kernel<T, NKS, NBLK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                   (int)b.smem_bytes));
-    dim3 grid((unsigned)cdiv(p, BM_VOX), (unsigned)b.nsplit);
-    boot_moments_kernel<T, NKS, NBLK><<<grid, BM_THREADS, b.smem_bytes, st>>>(
-        X, ldx, N, p, coef, b.nper, b.per_per_split, b.nstage, R, b.Kp, K, pivot, o1, o2);
-    PLSB_LAUNCH_CHECK("boot_moments_kernel");
-    return PLSB200_OK;
-}
-
-template <typename T, int NBLK>
-static int dispatch_nks(const BootPlan& b, const T* X, int N, int64_t p, int64_t ldx, const double* coef, int K,
-                        int R, const double* pivot, double* o1, double* o2, cudaStream_t st) {
-    switch (b.nks) {
-#define PLSB_CASE(n) case n: return launch_moments<T, n, NBLK>(b, X, N, p, ldx, coef, K, R, pivot, o1, o2, st);
-        PLSB_CASE(4) PLSB_CASE(8) PLSB_CASE(12) PLSB_CASE(16) PLSB_CASE(20) PLSB_CASE(24) PLSB_CASE(28)
-        PLSB_CASE(32) PLSB_CASE(36) PLSB_CASE(40) PLSB_CASE(44) PLSB_CASE(48) PLSB_CASE(52) PLSB_CASE(56)
-        PLSB_CASE(60) PLSB_CASE(64) PLSB_CASE(68) PLSB_CASE(72) PLSB_CASE(76) PLSB_CASE(80)
-#undef PLSB_CASE
-        default:
-            set_err("boot_moments_f64: no kernel for nks=%d", b.nks);
-            return PLSB200_EUNSUPPORTED;
-    }
-}
-
 }  // namespace plsb
 
 using namespace plsb;
@@ -659,17 +496,20 @@ static int boot_moments(const T* X, int N, int64_t p, int64_t ldx, const double*
         o1 = (double*)workspace;
         o2 = o1 + (size_t)b.nsplit * p * K;
     }
-    int rc;
-    switch (b.nblk) {
-        case 1: rc = dispatch_nks<T, 1>(b, X, N, p, ldx, coef, K, R, pivot, o1, o2, st); break;
-        case 2: rc = dispatch_nks<T, 2>(b, X, N, p, ldx, coef, K, R, pivot, o1, o2, st); break;
-        default: rc = dispatch_nks<T, 3>(b, X, N, p, ldx, coef, K, R, pivot, o1, o2, st); break;
-    }
+    const dim3 grid((unsigned)cdiv(p, BM_VOX), (unsigned)b.nsplit);
+    const int rc = ring_dispatch(b, "boot_moments_f64", [&](auto nks, auto nblk) {
+        const auto kernel = boot_moments_kernel<T, decltype(nks)::value, decltype(nblk)::value>;
+        PLSB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b.smem_bytes));
+        kernel<<<grid, BM_THREADS, b.smem_bytes, st>>>(X, ldx, N, p, coef, b.nper, b.per_per_split, b.nstage, R, b.Kp,
+                                                       K, pivot, o1, o2);
+        PLSB_LAUNCH_CHECK("boot_moments_kernel");
+        return PLSB200_OK;
+    });
     if (rc != PLSB200_OK) return rc;
     if (b.nsplit > 1) {
         const long long n = (long long)p * K;
-        moments_reduce_kernel<<<(unsigned)cdiv(n, 256), 256, 0, st>>>(o1, o2, b.nsplit, n, sum, sumsq);
-        PLSB_LAUNCH_CHECK("moments_reduce_kernel");
+        split_sum_kernel<<<(unsigned)cdiv(n, 256), 256, 0, st>>>(o1, o2, b.nsplit, n, sum, sumsq);
+        PLSB_LAUNCH_CHECK("split_sum_kernel");
     }
     return PLSB200_OK;
 }
@@ -798,26 +638,6 @@ static NsLayout ns_layout(int N, int K, int Kt, int R) {
     return L;
 }
 
-template <int NKS, int NBLK>
-static int ns_launch(const BootPlan& b, const NsArgs& a, int tiles, cudaStream_t st) {
-    PLSB_CUDA(cudaFuncSetAttribute(nspace_dmma_kernel<NKS, NBLK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                   (int)b.smem_bytes));
-    dim3 grid((unsigned)tiles, (unsigned)b.nsplit);
-    nspace_dmma_kernel<NKS, NBLK><<<grid, BM_THREADS, b.smem_bytes, st>>>(a);
-    PLSB_LAUNCH_CHECK("nspace_dmma_kernel");
-    return PLSB200_OK;
-}
-template <int NBLK>
-static int ns_dispatch(const BootPlan& b, const NsArgs& a, int tiles, cudaStream_t st) {
-    switch (b.nks) {
-#define PLSB_CASE(n) case n: return ns_launch<n, NBLK>(b, a, tiles, st);
-        PLSB_CASE(4) PLSB_CASE(8) PLSB_CASE(12) PLSB_CASE(16) PLSB_CASE(20) PLSB_CASE(24) PLSB_CASE(28)
-        PLSB_CASE(32) PLSB_CASE(36) PLSB_CASE(40) PLSB_CASE(44) PLSB_CASE(48) PLSB_CASE(52) PLSB_CASE(56)
-        PLSB_CASE(60) PLSB_CASE(64) PLSB_CASE(68) PLSB_CASE(72) PLSB_CASE(76) PLSB_CASE(80)
-#undef PLSB_CASE
-        default: set_err("nspace_dmma_f64: no kernel for nks=%d", b.nks); return PLSB200_EUNSUPPORTED;
-    }
-}
 }  // namespace plsb
 
 extern "C" size_t plsb200_nspace_dmma_f64_workspace(int N, int K, int Kt, int R) {
@@ -869,12 +689,14 @@ extern "C" int plsb200_nspace_dmma_f64(const double* G, int N, const double* Lma
     a.W = W; a.ldw = L.ldw; a.N = N; a.Nv = L.Nv; a.Npad = L.Npad; a.coef = coef; a.nper = b.nper;
     a.per_per_split = b.per_per_split; a.nstage = b.nstage; a.R = R; a.Kp = b.Kp; a.K = K; a.Kt = Kt;
     a.dpart = dpart; a.Traw = T;
-    int rc;
-    switch (b.nblk) {
-        case 1: rc = ns_dispatch<1>(b, a, tiles, st); break;
-        case 2: rc = ns_dispatch<2>(b, a, tiles, st); break;
-        default: rc = ns_dispatch<3>(b, a, tiles, st); break;
-    }
+    const dim3 grid((unsigned)tiles, (unsigned)b.nsplit);
+    const int rc = ring_dispatch(b, "nspace_dmma_f64", [&](auto nks, auto nblk) {
+        const auto kernel = nspace_dmma_kernel<decltype(nks)::value, decltype(nblk)::value>;
+        PLSB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b.smem_bytes));
+        kernel<<<grid, BM_THREADS, b.smem_bytes, st>>>(a);
+        PLSB_LAUNCH_CHECK("nspace_dmma_kernel");
+        return PLSB200_OK;
+    });
     if (rc != PLSB200_OK) return rc;
     const long long n = (long long)R * K;
     nspace_finish_kernel<<<(unsigned)cdiv(n, 256), 256, 0, st>>>(dpart, L.ngH, R, K, Kt, d2, T);

@@ -22,6 +22,7 @@
 // moments of (VS - pivot) -- the column -> k map is tile-invariant because 96 is a multiple of every padded K -- and
 // the CTA moves to the next column tile.  There is no limit on N.
 #include "common.cuh"
+#include "boot_plan.cuh"
 
 namespace plsb {
 
@@ -43,14 +44,8 @@ struct OsPlan {
 
 static bool os_plan(int N, int K, int R, int64_t p, OsPlan& b) {
     if (K < 1 || K > 24 || N < 1 || R < 1) return false;
-    int best_kp = 0, best_blk = 0;
-    for (int blk = 3; blk >= 1; --blk) {
-        const int cols = 8 * blk;
-        for (int kp = K; kp <= cols; ++kp)
-            if (cols % kp == 0) { if (best_kp == 0 || kp < best_kp) { best_kp = kp; best_blk = blk; } break; }
-    }
-    if (!best_kp) return false;
-    b.Kp = best_kp; b.nacc = best_blk; b.nb = 8 * best_blk / best_kp;
+    if (!pad_period(K, b.Kp, b.nacc)) return false;
+    b.nb = 8 * b.nacc / b.Kp;
     {
         const int need = (int)cdiv(N, 4);
         // padded k-steps are wasted DMMAs; shallower stages cost about 1.5 % per k-step below 8 (more barrier rounds
@@ -316,15 +311,6 @@ boot_moments_os_kernel(const double* __restrict__ Ximg, int N, long long p,
     }
 }
 
-__global__ void os_moments_reduce_kernel(const double* __restrict__ p1, const double* __restrict__ p2, int nsplit,
-                                         long long n, double* __restrict__ sum, double* __restrict__ sumsq) {
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    double a = 0.0, b = 0.0;
-    for (int s = 0; s < nsplit; ++s) { a += p1[(size_t)s * n + i]; b += p2[(size_t)s * n + i]; }
-    sum[i] = a; sumsq[i] = b;
-}
-
 template <int NACC, int KS>
 static int os_launch_ks(const OsPlan& b, const double* Ximg, int N, int64_t p, const double* coef, int K, int R,
                         const double* pivot, double* o1, double* o2, cudaStream_t st) {
@@ -430,8 +416,8 @@ static int os_moments(const T* X, int N, int64_t p, int64_t ldx, const double* c
     if (rc != PLSB200_OK) return rc;
     if (b.nsplit > 1) {
         const long long n = (long long)p * K;
-        os_moments_reduce_kernel<<<(unsigned)cdiv(n, 256), 256, 0, st>>>(o1, o2, b.nsplit, n, sum, sumsq);
-        PLSB_LAUNCH_CHECK("os_moments_reduce_kernel");
+        split_sum_kernel<<<(unsigned)cdiv(n, 256), 256, 0, st>>>(o1, o2, b.nsplit, n, sum, sumsq);
+        PLSB_LAUNCH_CHECK("split_sum_kernel");
     }
     return PLSB200_OK;
 }

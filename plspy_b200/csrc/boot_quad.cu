@@ -7,11 +7,11 @@
 // file evaluates the p x K quadratic forms, 2 p N^2 K flops instead of the 2 p N K B of the direct moment GEMM.
 //
 // The kernel is boot_moments_kernel (boot.cu) with N "pseudo-resamples" in place of the B resamples: pseudo-resample m
-// has the N x K coefficient matrix P_m[n,k] = S_k[n,m], packed in exactly the B-fragment / period order of
-// boot_coef_pack_kernel, so the plan, the ring of bulk copies and the mbarriers are the same.  A D element is then
-// (S_k x_v)[m]; the epilogue folds it as acc[v,k] += X[m,v] . d.  X[m,v] comes from an __ldg issued before the
-// period's MMA stream (the A registers cannot serve it: m is a runtime index).  Pseudo-resamples m >= N and columns
-// k >= K are zero in the pack; the loads of rows m >= N are masked.
+// has the N x K coefficient matrix P_m[n,k] = S_k[n,m], packed in the layout of boot_coef_pack_kernel (bfrag_offset),
+// and the plan, the ring of bulk copies, the mbarriers and the DMMA stream are the same code, ring_pipeline
+// (boot_plan.cuh).  What boot_quad_kernel adds is QuadEpilogue: a D element is (S_k x_v)[m], folded as
+// acc[v,k] += X[m,v] . d with X[m,v] loaded before the period's wait, and fold_slots_store writes the one output.
+// Pseudo-resamples m >= N and columns k >= K are zero in the pack.
 #include <float.h>
 
 #include "common.cuh"
@@ -19,182 +19,74 @@
 
 namespace plsb {
 
-// S ([K][N][N], row-major) -> B-fragment order: offset ((per*nks + s)*nblk + jb)*32 + lane, lane = 4*n + qq,
-// column c = 8*jb + n = slot*Kp + k of pseudo-resample m = per*nb + slot, row i = 4*s + qq.
+// S ([K][N][N], row-major) -> the packed layout (bfrag_offset): element i of the pack, enumerated as period per, k-step
+// s, column c and row 4*s + q in the order of the layout, is S_k[row, m] for column c = slot*Kp + k of pseudo-resample
+// m = per*nb + slot.
 __global__ void quad_coef_pack_kernel(const double* __restrict__ S, int N, int K, int Kp, int nblk, int nb, int nks,
                                       long long total, double* __restrict__ coef) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= total) return;
-    const int lane = (int)(i & 31);
-    long long t = i >> 5;
-    const int jb = (int)(t % nblk); t /= nblk;
+    const int q = (int)(i & 3);
+    long long t = i >> 2;
+    const int c = (int)(t % (8 * nblk)); t /= 8 * nblk;
     const int s = (int)(t % nks);
     const int per = (int)(t / nks);
-    const int c = 8 * jb + (lane >> 2), row = 4 * s + (lane & 3);
-    const int k = c % Kp, m = per * nb + c / Kp;
-    coef[i] = (row < N && m < N && k < K) ? S[((size_t)k * N + row) * N + m] : 0.0;
+    const int row = 4 * s + q, k = c % Kp, m = per * nb + c / Kp;
+    coef[(size_t)per * nks * nblk * 32 + bfrag_offset(s, c, q, nblk)] =
+        (row < N && m < N && k < K) ? S[((size_t)k * N + row) * N + m] : 0.0;
 }
 
-// T: element type of X (float: X stored as float32, widened at every load -- the same FP64 operations as on the
-// widened matrix).
-template <typename T, int NKS, int NBLK>
-__global__ void __launch_bounds__(BM_THREADS, 1)
-boot_quad_kernel(const T* __restrict__ X, long long ldx, int N, long long p, const double* __restrict__ coef,
-                 int nper, int per_per_split, int nstage, int Kp, int K, double* __restrict__ out) {
-    extern __shared__ __align__(128) unsigned char smraw[];
-    constexpr int stage_doubles = NKS * NBLK * 32;
-    constexpr uint32_t stage_bytes = (uint32_t)stage_doubles * 8u;
-    double* ring = reinterpret_cast<double*>(smraw);
-    double* red = ring + (size_t)nstage * stage_doubles;              // [8 warps][8][Kp] (the plan reserves twice that)
-    uint64_t* full = reinterpret_cast<uint64_t*>(red + BM_WARPS * 16 * Kp);
-    uint64_t* empty = full + nstage;
-
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int q = lane & 3, vr = lane >> 2;
-    const long long v = (long long)blockIdx.x * BM_VOX + warp * 8 + vr;
-    const int per0 = blockIdx.y * per_per_split;
-    const int per1 = min(nper, per0 + per_per_split);
-    const int nit = per1 - per0;
-
-    if (tid == 0) {
-        for (int s = 0; s < nstage; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, BM_WARPS); }
-        mbar_fence_init();
+// The quadratic-form epilogue: the chains start from 0, so a D element is (S_k x_v)[m] for the pseudo-resample m of
+// its column; it is folded as acc += X[m,v] . d.  X[m,v] comes from an __ldg issued before the period's wait (the A
+// registers cannot serve it: m is a runtime index); the loads of rows m >= N are masked.
+template <typename T, int NBLK>
+struct QuadEpilogue : RingEpilogue {
+    struct Args { const T* X; long long ldx, v, p; int N, Kp, K; double* out; };
+    const Args a;
+    const RingThread th;
+    const long long vc;                                   // (address of the masked lanes' X loads)
+    int slot_of[NBLK][2];                                 // pseudo-resample slot of each column
+    double acc[1][NBLK][2], xm[NBLK][2];
+    int nb;
+    __device__ __forceinline__ QuadEpilogue(const Args& args, const RingThread& t)
+        : a(args), th(t), vc(args.v < args.p ? args.v : 0) {
+#pragma unroll
+        for (int j = 0; j < NBLK; ++j)
+#pragma unroll
+            for (int e = 0; e < 2; ++e) { slot_of[j][e] = (8 * j + 2 * th.q + e) / a.Kp; acc[0][j][e] = 0.0; }
+        nb = 8 * NBLK / a.Kp;
     }
-    __syncthreads();
-
-    auto issue = [&](int it, int slot) {   // thread 0 only: stream period per0+it into `slot`
-        mbar_expect_tx(full + slot, stage_bytes);
-        const char* src = reinterpret_cast<const char*>(coef + (size_t)(per0 + it) * stage_doubles);
-        char* dst = reinterpret_cast<char*>(ring + (size_t)slot * stage_doubles);
-#pragma unroll 1
-        for (uint32_t off = 0; off < stage_bytes; off += 16384u)
-            bulk_g2s(dst + off, src + off, min(16384u, stage_bytes - off), full + slot);
-    };
-    if (tid == 0)
-        for (int it = 0; it < min(nstage, nit); ++it) issue(it, it);
-
-    // ---- A fragments: this warp's 8 voxels x all rows, resident in registers
-    double a[NKS];
-#pragma unroll
-    for (int s = 0; s < NKS; ++s) {
-        const int row = 4 * s + q;
-        a[s] = (row < N && v < p) ? (double)__ldg(X + (long long)row * ldx + v) : 0.0;
-    }
-    const long long vc = v < p ? v : 0;                                // (address of the masked lanes' X loads)
-
-    // ---- per-thread column bookkeeping (fixed for the whole kernel): pseudo-resample slot of each column
-    int slot_of[NBLK][2];
-    double acc[NBLK][2];
-#pragma unroll
-    for (int j = 0; j < NBLK; ++j)
-#pragma unroll
-        for (int e = 0; e < 2; ++e) { slot_of[j][e] = (8 * j + 2 * q + e) / Kp; acc[j][e] = 0.0; }
-    const int nb = 8 * NBLK / Kp;
-
-    if (warp >= 4) __nanosleep((unsigned)(NKS * NBLK * 8));
-
-    int slot = 0, prev_slot = 0;
-    uint32_t phase = 0, prev_phase = 0;
-    for (int it = 0; it < nit; ++it) {
-        if (tid == 0 && it > 0) {
-            const int nx = it - 1 + nstage;
-            if (nx < nit) {
-                mbar_wait(empty + prev_slot, prev_phase);
-                issue(nx, prev_slot);
-            }
-        }
-        // X[m, v] of this thread's columns, loaded before the MMA stream so that its latency is hidden
-        const int mbase = (per0 + it) * nb;
-        double xm[NBLK][2];
+    __device__ __forceinline__ void before_wait(int it) {
+        const int mbase = (th.per0 + it) * nb;
 #pragma unroll
         for (int j = 0; j < NBLK; ++j)
 #pragma unroll
             for (int e = 0; e < 2; ++e) {
                 const int m = mbase + slot_of[j][e];
-                xm[j][e] = m < N ? (double)__ldg(X + (long long)m * ldx + vc) : 0.0;
+                xm[j][e] = m < a.N ? (double)__ldg(a.X + (long long)m * a.ldx + vc) : 0.0;
             }
-        __syncwarp();
-        mbar_wait(full + slot, phase);
-
-        double d[NBLK][2];
-#pragma unroll
-        for (int j = 0; j < NBLK; ++j) { d[j][0] = 0.0; d[j][1] = 0.0; }
-        // volatile: keeps the loads in program order, so the NBLK accumulator chains stay interleaved (see boot.cu)
-        const volatile double* bs = ring + (size_t)slot * stage_doubles + lane;
-#pragma unroll
-        for (int s = 0; s < NKS; ++s) {
-#pragma unroll
-            for (int j = 0; j < NBLK; ++j) {
-                const double b = bs[(s * NBLK + j) * 32];
-                dmma884(d[j][0], d[j][1], a[s], b);
-            }
-        }
-        __syncwarp();
-        if (lane == 0) mbar_arrive(empty + slot);
+    }
+    __device__ __forceinline__ void fold(const double (&d)[NBLK][2], int) {
 #pragma unroll
         for (int j = 0; j < NBLK; ++j)
 #pragma unroll
-            for (int e = 0; e < 2; ++e) acc[j][e] = fma(xm[j][e], d[j][e], acc[j][e]);
-        prev_slot = slot; prev_phase = phase;
-        if (++slot == nstage) { slot = 0; phase ^= 1u; }
+            for (int e = 0; e < 2; ++e) acc[0][j][e] = fma(xm[j][e], d[j][e], acc[0][j][e]);
     }
-
-    // ---- fold the nb pseudo-resample slots of a period onto k, in slot order (deterministic)
-    double* r1 = red + warp * (8 * Kp);
-    for (int i = lane; i < 8 * Kp; i += 32) r1[i] = 0.0;
-    __syncwarp();
-    for (int round = 0; round < nb; ++round) {
-#pragma unroll
-        for (int j = 0; j < NBLK; ++j)
-#pragma unroll
-            for (int e = 0; e < 2; ++e) {
-                const int c = 8 * j + 2 * q + e;
-                if (slot_of[j][e] == round) r1[vr * Kp + c % Kp] += acc[j][e];
-            }
-        __syncwarp();
+    __device__ __forceinline__ void finish(double* red) {
+        fold_slots_store<1, NBLK>(acc, red, th, nb, a.Kp, a.K, a.p, {a.out});
     }
-    const long long vbase = (long long)blockIdx.x * BM_VOX + warp * 8;
-    double* o = out + (size_t)blockIdx.y * p * K;
-    for (int i = lane; i < 8 * K; i += 32) {
-        const int rr = i / K, k = i % K;
-        if (vbase + rr < p) o[(vbase + rr) * K + k] = r1[rr * Kp + k];
-    }
-}
+};
 
-// q = sum of the split partials, in split order (deterministic)
-__global__ void quad_reduce_kernel(const double* __restrict__ part, int nsplit, long long n, double* __restrict__ q) {
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    double a = 0.0;
-    for (int s = 0; s < nsplit; ++s) a += part[(size_t)s * n + i];
-    q[i] = a;
-}
-
+// T: element type of X (float: X stored as float32, widened at every load -- the same FP64 operations as on the
+// widened matrix).  The plan reserves shared memory for two outputs per warp; this kernel uses one.
 template <typename T, int NKS, int NBLK>
-static int launch_quad(const BootPlan& b, const T* X, int N, int64_t p, int64_t ldx, const double* coef, int K,
-                       double* o, cudaStream_t st) {
-    PLSB_CUDA(cudaFuncSetAttribute(boot_quad_kernel<T, NKS, NBLK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                   (int)b.smem_bytes));
-    dim3 grid((unsigned)cdiv(p, BM_VOX), (unsigned)b.nsplit);
-    boot_quad_kernel<T, NKS, NBLK><<<grid, BM_THREADS, b.smem_bytes, st>>>(X, ldx, N, p, coef, b.nper, b.per_per_split,
-                                                                       b.nstage, b.Kp, K, o);
-    PLSB_LAUNCH_CHECK("boot_quad_kernel");
-    return PLSB200_OK;
-}
-
-template <typename T, int NBLK>
-static int quad_dispatch_nks(const BootPlan& b, const T* X, int N, int64_t p, int64_t ldx, const double* coef,
-                             int K, double* o, cudaStream_t st) {
-    switch (b.nks) {
-#define PLSB_CASE(n) case n: return launch_quad<T, n, NBLK>(b, X, N, p, ldx, coef, K, o, st);
-        PLSB_CASE(4) PLSB_CASE(8) PLSB_CASE(12) PLSB_CASE(16) PLSB_CASE(20) PLSB_CASE(24) PLSB_CASE(28)
-        PLSB_CASE(32) PLSB_CASE(36) PLSB_CASE(40) PLSB_CASE(44) PLSB_CASE(48) PLSB_CASE(52) PLSB_CASE(56)
-        PLSB_CASE(60) PLSB_CASE(64) PLSB_CASE(68) PLSB_CASE(72) PLSB_CASE(76) PLSB_CASE(80)
-#undef PLSB_CASE
-        default:
-            set_err("boot_quad_f64: no kernel for nks=%d", b.nks);
-            return PLSB200_EUNSUPPORTED;
-    }
+__global__ void __launch_bounds__(BM_THREADS, 1)
+boot_quad_kernel(const T* __restrict__ X, long long ldx, int N, long long p, const double* __restrict__ coef,
+                 int nper, int per_per_split, int nstage, int Kp, int K, double* __restrict__ out) {
+    const RingThread th(threadIdx.x, nper, per_per_split);
+    const long long v = (long long)blockIdx.x * BM_VOX + th.warp * 8 + th.vr;
+    ring_pipeline<NKS, NBLK, QuadEpilogue<T, NBLK>>(th, X, ldx, N, v, v < p, coef, nstage, BM_WARPS * 16 * Kp,
+                                                    {X, ldx, v, p, N, Kp, K, out});
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -379,17 +271,20 @@ static int boot_quad(const T* X, int N, int64_t p, int64_t ldx, const double* co
         }
         o = (double*)workspace;
     }
-    int rc;
-    switch (b.nblk) {
-        case 1: rc = quad_dispatch_nks<T, 1>(b, X, N, p, ldx, coef, K, o, st); break;
-        case 2: rc = quad_dispatch_nks<T, 2>(b, X, N, p, ldx, coef, K, o, st); break;
-        default: rc = quad_dispatch_nks<T, 3>(b, X, N, p, ldx, coef, K, o, st); break;
-    }
+    const dim3 grid((unsigned)cdiv(p, BM_VOX), (unsigned)b.nsplit);
+    const int rc = ring_dispatch(b, "boot_quad_f64", [&](auto nks, auto nblk) {
+        const auto kernel = boot_quad_kernel<T, decltype(nks)::value, decltype(nblk)::value>;
+        PLSB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b.smem_bytes));
+        kernel<<<grid, BM_THREADS, b.smem_bytes, st>>>(X, ldx, N, p, coef, b.nper, b.per_per_split, b.nstage, b.Kp, K,
+                                                       o);
+        PLSB_LAUNCH_CHECK("boot_quad_kernel");
+        return PLSB200_OK;
+    });
     if (rc != PLSB200_OK) return rc;
     if (b.nsplit > 1) {
         const long long n = (long long)p * K;
-        quad_reduce_kernel<<<(unsigned)cdiv(n, 256), 256, 0, st>>>(o, b.nsplit, n, q);
-        PLSB_LAUNCH_CHECK("quad_reduce_kernel");
+        split_sum_kernel<<<(unsigned)cdiv(n, 256), 256, 0, st>>>(o, nullptr, b.nsplit, n, q, nullptr);
+        PLSB_LAUNCH_CHECK("split_sum_kernel");
     }
     return PLSB200_OK;
 }

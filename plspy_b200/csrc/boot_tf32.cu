@@ -528,15 +528,6 @@ __global__ void __launch_bounds__(TF_THREADS, 1) boot_moments_tf32_kernel(const 
     }
 }
 
-__global__ void moments_reduce_tf32_kernel(const double* __restrict__ part1, const double* __restrict__ part2, int nsplit,
-                                           long long n, double* __restrict__ sum, double* __restrict__ sumsq) {
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    double x = 0.0, y = 0.0;
-    for (int s = 0; s < nsplit; ++s) { x += part1[(size_t)s * n + i]; y += part2[(size_t)s * n + i]; }
-    sum[i] = x; sumsq[i] = y;
-}
-
 template <int KP, int CG>
 static int launch_tf32_cg(const TfPlan& t, const TfArgs& a, cudaStream_t st) {
     PLSB_CUDA(cudaFuncSetAttribute(boot_moments_tf32_kernel<KP, CG>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -666,8 +657,8 @@ extern "C" int plsb200_boot_moments_tf32(const void* ximage, int N, int64_t p, c
     if (rc != PLSB200_OK) return rc;
     if (t.nsplit > 1) {
         const long long n = (long long)p * K;
-        moments_reduce_tf32_kernel<<<(unsigned)cdiv(n, 256), 256, 0, st>>>(o1, o2, t.nsplit, n, sum, sumsq);
-        PLSB_LAUNCH_CHECK("moments_reduce_tf32_kernel");
+        split_sum_kernel<<<(unsigned)cdiv(n, 256), 256, 0, st>>>(o1, o2, t.nsplit, n, sum, sumsq);
+        PLSB_LAUNCH_CHECK("split_sum_kernel");
     }
     return PLSB200_OK;
 }

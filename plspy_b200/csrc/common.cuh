@@ -74,6 +74,12 @@ int boot_os_moments(const float* X, int N, int64_t p, int64_t ldx, const double*
 // ---------------------------------------------------------------- device side
 #ifdef __CUDACC__
 
+// The split partials of the bootstrap GEMMs, whose period or column range is divided over the grid: out1[i] = sum of
+// part1[s*n + i] over s = 0 .. nsplit-1 in that order (deterministic), and out2 likewise from part2 unless out2 is
+// null.  Defined in boot.cu.
+__global__ void split_sum_kernel(const double* __restrict__ part1, const double* __restrict__ part2, int nsplit,
+                                 long long n, double* __restrict__ out1, double* __restrict__ out2);
+
 // D(8x8) += A(8x4, row) * B(4x8, col), FP64 tensor core (SASS: DMMA.8x8x4 -- the only native f64
 // MMA shape on sm_100a; the m16n8k{4,8,16} PTX shapes lower to sequences of it).
 //   a : A[row = lane/4][k = lane%4]      b : B[k = lane%4][col = lane/4]
