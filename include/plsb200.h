@@ -267,6 +267,9 @@ int plsb200_salience_series_x32_f64(const float* X, int N, int64_t p, int64_t ld
  *   block std of the RESAMPLED rows (class_functions.py:219-245 as called at bootstrap_permutation.py:613);
  *   accumulates sum/sumsq of (VS - pivot) INTO sum/sumsq (p x K, caller zeroes before the first chunk) and
  *   writes T[b] = Xc . VS_b (N x K) and nrm2[b] = ||VS_b[:,k]||^2 for the LV correlations.
+ *   The `_vs` variants also store VS_b itself (the reference's right_sv_sampled[b], before the pivot is subtracted)
+ *   into VS, resample-major like T: VS[b * p * K + v * K + k] for b in [b0, b0+nbt), p x K per bootstrap.  The
+ *   plain entry points are the `_vs` ones with VS = NULL (nothing stored).
  * rb_lvcorr: LVcorr[b] = _compute_corr(X_new @ V_hat, Y_new) (ncell*nb x K)  (bootstrap_permutation.py:636-642). */
 int plsb200_cell_standardize_f64(const double* X, int N, int64_t p, int64_t ldx, const int32_t* cell_start,
                                  int ncell, double* Xc, double* Z, void* stream);
@@ -296,6 +299,11 @@ int plsb200_rb_boot_f64(const double* Xc, int N, int64_t p, const double* Xc2, i
                         int nbt, const int32_t* cell_start, int ncell, int unit_cells, const double* pivot,
                         double* sum, double* sumsq, double* T, double* nrm2, void* workspace,
                         size_t workspace_bytes, void* stream);
+int plsb200_rb_boot_vs_f64(const double* Xc, int N, int64_t p, const double* Xc2, int n1, int64_t ld2, const double* Q,
+                           const double* W, int K, int b0,
+                           int nbt, const int32_t* cell_start, int ncell, int unit_cells, const double* pivot,
+                           double* sum, double* sumsq, double* T, double* nrm2, double* VS, void* workspace,
+                           size_t workspace_bytes, void* stream);
 /* rb_boot on the FP64 tensor path (DMMA): same contract as plsb200_rb_boot_f64 except that the block offsets are
  * read on the HOST (`cell_start_host`), T may be NULL (squared norms only: first pass of the multiblock bootstrap)
  * and designs whose blocks, each padded to a multiple of 4 rows, exceed 384 rows are not supported: the workspace
@@ -308,6 +316,11 @@ int plsb200_rb_boot_dmma_f64(const double* Xc, int N, int64_t p, const double* X
                              int nbt, const int32_t* cell_start_host, int ncell, int unit_cells, const double* pivot,
                              double* sum, double* sumsq, double* T, double* nrm2, void* workspace,
                              size_t workspace_bytes, void* stream);
+int plsb200_rb_boot_dmma_vs_f64(const double* Xc, int N, int64_t p, const double* Xc2, int n1, int64_t ld2,
+                                const double* Q, const double* W, int K, int b0,
+                                int nbt, const int32_t* cell_start_host, int ncell, int unit_cells, const double* pivot,
+                                double* sum, double* sumsq, double* T, double* nrm2, double* VS, void* workspace,
+                                size_t workspace_bytes, void* stream);
 /* multiblock glue (class_functions.py:454-516): the last `unit_cells` blocks of rb_boot are plain linear rows
  * (task part of the multiblock matrix, no standardisation).
  * scatter_coef: C[r] (N x K) = scatter(E, idx_r) written out explicitly.

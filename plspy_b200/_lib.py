@@ -118,11 +118,19 @@ SIGNATURES = {
                                     c_int, c_int,
                                     c_int32_p, c_int, c_int, c_double_p, c_double_p, c_double_p, c_double_p,
                                     c_double_p, c_void_p, c_size_t, c_void_p]),
+    "plsb200_rb_boot_vs_f64": (c_int, [c_double_p, c_int, c_int64, c_double_p, c_int, c_int64, c_double_p, c_double_p,
+                                       c_int, c_int, c_int,
+                                       c_int32_p, c_int, c_int, c_double_p, c_double_p, c_double_p, c_double_p,
+                                       c_double_p, c_double_p, c_void_p, c_size_t, c_void_p]),
     "plsb200_rb_boot_dmma_f64_workspace": (c_size_t, [c_int, c_int64, c_int, c_int, c_void_p, c_int, c_int, c_int]),
     "plsb200_rb_boot_dmma_f64": (c_int, [c_double_p, c_int, c_int64, c_double_p, c_int, c_int64, c_double_p, c_double_p,
                                          c_int, c_int, c_int,
                                          c_void_p, c_int, c_int, c_double_p, c_double_p, c_double_p, c_double_p,
                                          c_double_p, c_void_p, c_size_t, c_void_p]),
+    "plsb200_rb_boot_dmma_vs_f64": (c_int, [c_double_p, c_int, c_int64, c_double_p, c_int, c_int64, c_double_p,
+                                            c_double_p, c_int, c_int, c_int,
+                                            c_void_p, c_int, c_int, c_double_p, c_double_p, c_double_p, c_double_p,
+                                            c_double_p, c_double_p, c_void_p, c_size_t, c_void_p]),
     "plsb200_rb_lvcorr_f64": (c_int, [c_double_p, c_double_p, c_double_p, c_int32_p, c_int, c_int, c_int, c_int,
                                       c_int32_p, c_int, c_double_p, c_void_p]),
     "plsb200_half_gram_f64_workspace": (c_size_t, [c_int64, c_int, c_int]),

@@ -142,6 +142,19 @@ def _p_sized_to_host(eng, *tensors):
     return out if isinstance(out, (list, tuple)) else [out]
 
 
+# Largest `right_sv_sampled` cube (B x p x K float64) a read builds.  The bootstrap itself never stores the cube: it
+# accumulates the moments on the fly, and the lazy entry rebuilds the saliences only when asked for.
+RIGHT_SV_MAX_BYTES = 2 << 30
+
+
+def _check_right_sv_bytes(niter, p, K):
+    """Raises MemoryError, before anything is allocated, when the niter x p x K cube exceeds RIGHT_SV_MAX_BYTES."""
+    nbytes = niter * p * K * 8
+    if nbytes > RIGHT_SV_MAX_BYTES:
+        raise MemoryError(f"right_sv_sampled would need {nbytes / 2**30:.1f} GiB; the B200 path "
+                          "accumulates its moments on the fly instead of storing it")
+
+
 def _stepdown_tail(s):
     return np.cumsum((np.asarray(s, dtype=float) ** 2)[::-1])[::-1].copy()
 
@@ -278,34 +291,22 @@ def _perm_multiblock(eng, X, U, s, cond_order, mctype, niter, pls_alg, contrast,
     return counts[:Kc] / (niter + 1), counts[Kc:] / (niter + 1), debug
 
 
-def _boot_multiblock(eng, U, s, V, cond_order, mctype, niter, pls_alg, contrast, bscan, Ybscan, lvcorrs_orig,
-                     Tvsc_orig, CI, indices):
-    """bootstrap_permutation.py:545-554, 609-675, 695-766 for mb / cmb: independent bootstrap draws for the
-    task block (rows of X) and the behaviour block (bscan rows).  Two p-space passes per bootstrap batch:
-    (1) squared norms of the behaviour rows (their per-voxel std depends on the draw), (2) the projected
-    cross-block matrix VS = permuted^T U of the row-normalised multiblock, with fused moments and the
-    latent products [Xcb; X] @ VS needed for LVcorr and Tdistrib."""
-    st = _multiblock_state(eng, cond_order, bscan)
+def _multiblock_boot_coef(eng, st, Lop, Ucoef, Ybscan, bscan, cond_order, it, ib, want_yz=False):
+    """Row coefficients of pass 2 of the mb / cmb bootstrap for the draws (it, ib), rows ordered like W2 = [Xcb; X]:
+    task rows (scatter of Lop^T, squared norms through G), behaviour rows (raw correlation rows, squared norms from
+    pass 1), each row normalised and projected on Ucoef.  Returns (C2, Wfull, cells2, Yz); Yz only with want_yz.  The
+    bootstrap and the lazy `right_sv_sampled` both build their coefficients here, so the cube comes from exactly the
+    coefficients the moments used."""
     nb = Ybscan.shape[1]
     tcol, bcol, K = _multiblock_columns(cond_order, bscan, nb)
-    idx_t, idx_b = _multiblock_indices(pls_alg, indices, niter, cond_order, bscan, Ybscan, boot=True)
-    Lop = (class_functions._cell_mean_operator(cond_order) if pls_alg == "cmb"
-           else class_functions._centring_operator(cond_order, mctype))
-    Abar = class_functions._cell_mean_operator(cond_order)
-    Ucoef = _ucoef(U, contrast)
-    Kc = Ucoef.shape[1]
-    N, Nb = eng.N, st["Nb"]
-    dev = eng.device
-    numer = _numerator(eng, V, s, contrast)
-    lo, hi = dist.shard(niter)
-    it = _index_shard(eng, idx_t, niter, lo, hi); ib = _index_shard(eng, idx_b, niter, lo, hi)
-    R = hi - lo
+    N, Nb, dev = eng.N, st["Nb"], eng.device
+    R = int(it.shape[0])
     tcol_d = torch.as_tensor(tcol, device=dev); bcol_d = torch.as_tensor(bcol, device=dev)
     # task rows: coefficients over the rows of X and their squared norms through G
     Ct = eng.scatter_coef(np.ascontiguousarray(Lop.T), it)                          # R x N x GC
     d2t, _ = eng.nspace_coef(eng.G, Ct)
     # behaviour rows: raw (un-normalised) correlation rows and pass 1 for their squared norms
-    Qraw, Wb, Yz = eng.rb_coef(Ybscan, ib, st["cells_b"], np.eye(len(bcol)), scatter=True, want_yz=True)
+    Qraw, Wb, Yz = eng.rb_coef(Ybscan, ib, st["cells_b"], np.eye(len(bcol)), scatter=True, want_yz=want_yz)
     _, _, _, nrm_b = eng.rb_boot(st["Xcb"], Qraw, Wb, st["cells_b"], want_t=False)
     d2row = torch.zeros(R, K, dtype=torch.float64, device=dev)
     d2row[:, tcol_d] = d2t
@@ -316,6 +317,28 @@ def _boot_multiblock(eng, U, s, V, cond_order, mctype, niter, pls_alg, contrast,
     C2 = eng.coef_project(C1, d2row, Ucoef)                                         # R x (Nb+N) x Kc
     Wfull = torch.cat([Wb, torch.zeros(R, N, dtype=torch.float64, device=dev)], dim=1)
     cells2 = np.concatenate([st["cells_b"], [Nb + N]]).astype(np.int32)
+    return C2, Wfull, cells2, Yz
+
+
+def _boot_multiblock(eng, U, s, V, cond_order, mctype, niter, pls_alg, contrast, bscan, Ybscan, lvcorrs_orig,
+                     Tvsc_orig, CI, indices):
+    """bootstrap_permutation.py:545-554, 609-675, 695-766 for mb / cmb: independent bootstrap draws for the
+    task block (rows of X) and the behaviour block (bscan rows).  Two p-space passes per bootstrap batch:
+    (1) squared norms of the behaviour rows (their per-voxel std depends on the draw), (2) the projected
+    cross-block matrix VS = permuted^T U of the row-normalised multiblock, with fused moments and the
+    latent products [Xcb; X] @ VS needed for LVcorr and Tdistrib."""
+    st = _multiblock_state(eng, cond_order, bscan)
+    nb = Ybscan.shape[1]
+    idx_t, idx_b = _multiblock_indices(pls_alg, indices, niter, cond_order, bscan, Ybscan, boot=True)
+    Lop = (class_functions._cell_mean_operator(cond_order) if pls_alg == "cmb"
+           else class_functions._centring_operator(cond_order, mctype))
+    Abar = class_functions._cell_mean_operator(cond_order)
+    Ucoef = _ucoef(U, contrast)
+    Nb = st["Nb"]
+    numer = _numerator(eng, V, s, contrast)
+    lo, hi = dist.shard(niter)
+    it = _index_shard(eng, idx_t, niter, lo, hi); ib = _index_shard(eng, idx_b, niter, lo, hi)
+    C2, Wfull, cells2, Yz = _multiblock_boot_coef(eng, st, Lop, Ucoef, Ybscan, bscan, cond_order, it, ib, want_yz=True)
     s1, s2, T, nrm2 = eng.rb_boot(st["Xcb"], C2, Wfull, cells2, pivot=numer, unit_cells=1, X2=eng.X)   # pass 2
     dist.allreduce_packed_([s1, s2])
     std_errs, boot_ratios = eng.boot_finalize(s1, s2, niter, numer=numer)
@@ -339,6 +362,16 @@ def _boot_multiblock(eng, U, s, V, cond_order, mctype, niter, pls_alg, contrast,
     debug["Tdistrib"] = Td_h
     debug.set_lazy("indices", lambda: _indices_to_host(idx_t, niter))
     debug.set_lazy("indices_behaviour", lambda: _indices_to_host(idx_b, niter))
+
+    def _right():   # the reference's B x p x K cube, only on request: every draw on this rank, no collective
+        _check_right_sv_bytes(niter, eng.p, Ucoef.shape[1])
+        st_ = _multiblock_state(eng, cond_order, bscan)
+        it_all = _index_shard(eng, idx_t, niter, 0, niter); ib_all = _index_shard(eng, idx_b, niter, 0, niter)
+        C2_, W_, cells_, _ = _multiblock_boot_coef(eng, st_, Lop, Ucoef, Ybscan, bscan, cond_order, it_all, ib_all)
+        VS = torch.empty(niter, eng.p, Ucoef.shape[1], dtype=torch.float64, device=eng.device)
+        eng.rb_boot(st_["Xcb"], C2_, W_, cells_, unit_cells=1, X2=eng.X, want_t=False, vs_out=VS)
+        return VS.cpu().numpy()
+    debug.set_lazy("right_sv_sampled", _right)
     return conf_int, conf_int_T, std_errs_h, boot_ratios_h, LV_h, debug
 
 
@@ -876,10 +909,7 @@ class _ResampleTestPLS(ResampleTest):
         debug.set_lazy("indices", lambda: _indices_to_host(indices, niter))
 
         def _right():   # the reference's B x p x K cube, only on request
-            nbytes = niter * eng.p_total * E.shape[1] * 8
-            if nbytes > (2 << 30):
-                raise MemoryError(f"right_sv_sampled would need {nbytes / 2**30:.1f} GiB; the B200 path "
-                                  "accumulates its moments on the fly instead of storing it")
+            _check_right_sv_bytes(niter, eng.p_total, E.shape[1])
             VS = eng.salience(E, _index_shard(eng, indices, niter, 0, niter))
             if vox:     # voxel-major for the gather
                 VS = eng.gather_voxels(VS.transpose(0, 1).contiguous()).transpose(0, 1).contiguous()
@@ -926,6 +956,15 @@ class _ResampleTestPLS(ResampleTest):
         debug = _LazyDebugDict()
         debug["left_sv_sampled"] = LV_h
         debug.set_lazy("indices", lambda: _indices_to_host(indices, niter))
+
+        def _right():   # the reference's B x p x K cube, only on request: every draw on this rank, no collective
+            _check_right_sv_bytes(niter, eng.p, Ucoef.shape[1])
+            Xc_ = _behaviour_state(eng, cells)["Xc"]
+            Q_, W_, _ = eng.rb_coef(Y, _index_shard(eng, indices, niter, 0, niter), cells, Ucoef, scatter=True)
+            VS = torch.empty(niter, eng.p, Ucoef.shape[1], dtype=torch.float64, device=eng.device)
+            eng.rb_boot(Xc_, Q_, W_, cells, want_t=False, vs_out=VS)
+            return VS.cpu().numpy()
+        debug.set_lazy("right_sv_sampled", _right)
         return conf_int, std_errs_h, boot_ratios_h, LV_h, debug
 
     # ------------------------------------------------------------------------------------------

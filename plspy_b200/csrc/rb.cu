@@ -113,13 +113,13 @@ __global__ void __launch_bounds__(256) rb_coef_kernel(const double* __restrict__
 // ------------------------------------------------------------------------------------------------
 // Bootstrap p-space pass.  CTA = 256 voxels; loops over the bootstraps of the chunk.
 //  phase 1 (thread per voxel): block moments with multiplicity weights, VS[v, k0..k0+kc), fused
-//          running sum / sum of squares of (VS - pivot);
+//          running sum / sum of squares of (VS - pivot), VS itself into the resample-major cube when VS != NULL;
 //  phase 2 (thread per (row, 4 columns)): partial T[b] = Xc[:, tile] . VS_tile  and  ||VS||^2 partials,
 //          written per (tile, bootstrap) and summed over tiles in a fixed order by rb_reduce_kernel.
 constexpr int RB_VT = 256;
 constexpr int RB_VCH = 32;
 
-template <int KC>
+template <int KC, bool EXPORT>     // EXPORT: also store VS into the cube (instantiations without it keep their registers)
 __global__ void __launch_bounds__(RB_VT) rb_boot_kernel(const double* __restrict__ Xc, int N, long long p,
                                                        const double* __restrict__ Xc2, int n1, long long ld2,
                                                        const double* __restrict__ Q, const double* __restrict__ W,
@@ -128,7 +128,8 @@ __global__ void __launch_bounds__(RB_VT) rb_boot_kernel(const double* __restrict
                                                        int unit_cells,
                                                        const double* __restrict__ pivot, int Kfull,
                                                        double* __restrict__ sum, double* __restrict__ sumsq,
-                                                       double* __restrict__ Tpart, double* __restrict__ Npart) {
+                                                       double* __restrict__ Tpart, double* __restrict__ Npart,
+                                                       double* __restrict__ VS) {
     extern __shared__ __align__(16) double smb[];
     double* Qs = smb;                               // [N][KC]
     double* Ws = Qs + (size_t)N * KC;               // [N]
@@ -188,6 +189,8 @@ __global__ void __launch_bounds__(RB_VT) rb_boot_kernel(const double* __restrict
                 const double d = vs[k] - ((ok && pivot) ? __ldg(pivot + v * Kfull + k0 + k) : 0.0);
                 s1[k] += d;
                 s2[k] = fma(d, d, s2[k]);
+                if constexpr (EXPORT)
+                    if (ok) VS[((size_t)bb * p + v) * Kfull + k0 + k] = vs[k];
             }
             VSs[k * RB_VT + tid] = ok ? vs[k] : 0.0;
         }
@@ -525,12 +528,11 @@ extern "C" size_t plsb200_rb_boot_f64_workspace(int N, int64_t p, int K, int nbt
     return ntile * nbt * ((size_t)N * K + K) * sizeof(double);
 }
 
-extern "C" int plsb200_rb_boot_f64(const double* Xc, int N, int64_t p, const double* Xc2, int n1, int64_t ld2,
-                                   const double* Q, const double* W, int K, int b0,
-                                   int nbt, const int32_t* cell_start, int ncell, int unit_cells, const double* pivot,
-                                   double* sum,
-                                   double* sumsq, double* T, double* nrm2, void* workspace, size_t workspace_bytes,
-                                   void* stream) {
+extern "C" int plsb200_rb_boot_vs_f64(const double* Xc, int N, int64_t p, const double* Xc2, int n1, int64_t ld2,
+                                      const double* Q, const double* W, int K, int b0,
+                                      int nbt, const int32_t* cell_start, int ncell, int unit_cells, const double* pivot,
+                                      double* sum, double* sumsq, double* T, double* nrm2, double* VS, void* workspace,
+                                      size_t workspace_bytes, void* stream) {
     PLSB_CHECK_ARG(Xc && Q && W && cell_start && sum && sumsq && T && nrm2 && workspace, "rb_boot_f64: null pointer");
     PLSB_CHECK_ARG(N > 0 && p > 0 && K > 0 && nbt > 0 && ncell > 0, "rb_boot_f64: bad shape");
     if (Xc2 == nullptr) { n1 = N; ld2 = p; }
@@ -546,6 +548,7 @@ extern "C" int plsb200_rb_boot_f64(const double* Xc, int N, int64_t p, const dou
     double* Npart = Tpart + (size_t)ntile * nbt * N * K;
     const int nch = (int)cdiv(K, 16);
     const int kc_max = (int)cdiv(K, nch);
+    double* VSb = VS ? VS + (size_t)b0 * p * K : nullptr;
     for (int k0 = 0; k0 < K; k0 += kc_max) {
         const int kc = K - k0 < kc_max ? K - k0 : kc_max;
         if ((long long)N * ((kc + 3) / 4) > 8 * RB_VT) {
@@ -556,10 +559,10 @@ extern "C" int plsb200_rb_boot_f64(const double* Xc, int N, int64_t p, const dou
     do {                                                                                                            \
         size_t smem = ((size_t)N * KCV + N + (size_t)KCV * RB_VT + (size_t)N * (RB_VCH + 1)) * sizeof(double);      \
         if (smem > 220 * 1024) { set_err("rb_boot_f64: N=%d too large for shared memory", N); return PLSB200_EUNSUPPORTED; } \
-        PLSB_CUDA(cudaFuncSetAttribute(rb_boot_kernel<KCV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        rb_boot_kernel<KCV><<<ntile, RB_VT, smem, st>>>(Xc, N, p, Xc2, n1, ld2, Q, W, K, k0, kc, b0, nbt, cell_start, ncell,          \
-                                                        unit_cells, pivot, K,                                       \
-                                                        sum, sumsq, Tpart, Npart);                                  \
+        auto kern = VSb ? rb_boot_kernel<KCV, true> : rb_boot_kernel<KCV, false>;                                   \
+        PLSB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));              \
+        kern<<<ntile, RB_VT, smem, st>>>(Xc, N, p, Xc2, n1, ld2, Q, W, K, k0, kc, b0, nbt, cell_start, ncell,       \
+                                         unit_cells, pivot, K, sum, sumsq, Tpart, Npart, VSb);                      \
     } while (0)
         if (kc <= 8) PLSB_RB_LAUNCH(8);
         else if (kc <= 12) PLSB_RB_LAUNCH(12);
@@ -573,6 +576,16 @@ extern "C" int plsb200_rb_boot_f64(const double* Xc, int N, int64_t p, const dou
     rb_reduce_kernel<<<(unsigned)cdiv(nN, 256), 256, 0, st>>>(Npart, ntile, nN, nrm2 + (size_t)b0 * K);
     PLSB_LAUNCH_CHECK("rb_reduce_kernel");
     return PLSB200_OK;
+}
+
+extern "C" int plsb200_rb_boot_f64(const double* Xc, int N, int64_t p, const double* Xc2, int n1, int64_t ld2,
+                                   const double* Q, const double* W, int K, int b0,
+                                   int nbt, const int32_t* cell_start, int ncell, int unit_cells, const double* pivot,
+                                   double* sum,
+                                   double* sumsq, double* T, double* nrm2, void* workspace, size_t workspace_bytes,
+                                   void* stream) {
+    return plsb200_rb_boot_vs_f64(Xc, N, p, Xc2, n1, ld2, Q, W, K, b0, nbt, cell_start, ncell, unit_cells, pivot, sum, sumsq,
+                                  T, nrm2, nullptr, workspace, workspace_bytes, stream);
 }
 
 extern "C" int plsb200_rb_lvcorr_f64(const double* T, const double* nrm2, const double* Yz, const int32_t* idx, int N,

@@ -136,6 +136,7 @@ struct RdArgs {
     double* sum;
     double* sumsq;
     double* VSt;       // [nbt][kcp][p]  (may be NULL when T is not wanted)
+    double* VS;        // [nbt][p][Kfull] from the launch's first bootstrap: the saliences themselves (NULL: not exported)
     double* Npart;     // [nbt][kcp][tiles*8]
     long long p;
     int Kfull, k0, kc, nbt, npass, pass, nstage, ncell, nwarps;
@@ -171,7 +172,10 @@ __device__ __noinline__ void rd_store_scales(double* dst0, double* dst1, double 
 // weight-fragment (the multiplicity weights of the 8 bootstraps packed as a B fragment, rd_wpack_kernel), once per batch of 8
 // bootstraps -- 2 DMMAs + 1 DMUL per k-step and batch instead of 24 scalar operations and 8 quad reductions -- and the lane
 // that ends up with (voxel, bootstraps 2q, 2q+1) stores their two scales into the batch's scale table.
-template <int NKS, int NBLK, int W, bool MD>
+// EXPORT = also store VS_b into a.VS.  A template flag, not only a run-time test of a.VS: the 8-warp bucket holds up to
+// 96 k-steps of X fragments in 254 of its 255 registers, and the instantiations without the store keep exactly the
+// registers (and the code) of the kernel without the feature.
+template <int NKS, int NBLK, int W, bool MD, bool EXPORT>
 __global__ void __launch_bounds__(W * 32, 1) rb_vs_kernel(const RdArgs a) {
     constexpr int RD_WARPS = W, RD_THREADS = W * 32;
     extern __shared__ __align__(128) unsigned char smraw[];
@@ -407,7 +411,8 @@ __global__ void __launch_bounds__(W * 32, 1) rb_vs_kernel(const RdArgs a) {
         __syncwarp();
         if (lane == 0) mbar_arrive(empty + slot);
 
-        // ---- fold: moments, squared column norms (this warp's 8 voxels), transposed VS for the latent GEMM
+        // ---- fold: moments, squared column norms (this warp's 8 voxels), transposed VS for the latent GEMM, and the
+        //      exported salience (before the pivot is subtracted: the reference's permuted^T U)
 #pragma unroll
         for (int j = 0; j < NBLK; ++j)
 #pragma unroll
@@ -424,6 +429,8 @@ __global__ void __launch_bounds__(W * 32, 1) rb_vs_kernel(const RdArgs a) {
                 if (vr == 0)
                     a.Npart[((size_t)bb * (8 * NBLK) + c) * ((size_t)gridDim.x * nwarps) + blockIdx.x * nwarps + warp] = n2;
                 if (a.VSt && ok) a.VSt[((size_t)bb * (8 * NBLK) + c) * a.p + v] = val;
+                if constexpr (EXPORT)
+                    if (ok && c < a.kc) a.VS[((size_t)bb * a.p + v) * a.Kfull + a.k0 + c] = val;
             }
         if constexpr (!MD)
             if (has_next) scales();                               // scales of bootstrap bb+1 from its moments
@@ -602,12 +609,16 @@ static RdLayout rd_layout(const RdPlan& r, int N, int64_t p, int nbt, bool want_
     return L;
 }
 
-template <int NKS, int NBLK, int W, bool MD>
-static int launch_vs_md(const RdPlan& r, const RdArgs& a, int ntile, cudaStream_t st) {
-    PLSB_CUDA(cudaFuncSetAttribute(rb_vs_kernel<NKS, NBLK, W, MD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)r.smem_bytes));
-    rb_vs_kernel<NKS, NBLK, W, MD><<<ntile, a.nwarps * 32, r.smem_bytes, st>>>(a);
+template <int NKS, int NBLK, int W, bool MD, bool EXPORT>
+static int launch_vs_kernel(const RdPlan& r, const RdArgs& a, int ntile, cudaStream_t st) {
+    PLSB_CUDA(cudaFuncSetAttribute(rb_vs_kernel<NKS, NBLK, W, MD, EXPORT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)r.smem_bytes));
+    rb_vs_kernel<NKS, NBLK, W, MD, EXPORT><<<ntile, a.nwarps * 32, r.smem_bytes, st>>>(a);
     PLSB_LAUNCH_CHECK("rb_vs_kernel");
     return PLSB200_OK;
+}
+template <int NKS, int NBLK, int W, bool MD>
+static int launch_vs_md(const RdPlan& r, const RdArgs& a, int ntile, cudaStream_t st) {
+    return a.VS ? launch_vs_kernel<NKS, NBLK, W, MD, true>(r, a, ntile, st) : launch_vs_kernel<NKS, NBLK, W, MD, false>(r, a, ntile, st);
 }
 template <int NKS, int NBLK, int W>
 static int launch_vs(const RdPlan& r, const RdArgs& a, int ntile, cudaStream_t st) {
@@ -652,10 +663,10 @@ extern "C" size_t plsb200_rb_boot_dmma_f64_workspace(int N, int64_t p, int K, in
     return rd_layout(r, N, p, nbt, want_t != 0).total;
 }
 
-extern "C" int plsb200_rb_boot_dmma_f64(const double* Xc, int N, int64_t p, const double* Xc2, int n1, int64_t ld2,
-                                        const double* Q, const double* W, int K, int b0, int nbt, const int32_t* cell_start_host, int ncell, int unit_cells,
-                                        const double* pivot, double* sum, double* sumsq, double* T, double* nrm2,
-                                        void* workspace, size_t workspace_bytes, void* stream) {
+extern "C" int plsb200_rb_boot_dmma_vs_f64(const double* Xc, int N, int64_t p, const double* Xc2, int n1, int64_t ld2,
+                                           const double* Q, const double* W, int K, int b0, int nbt, const int32_t* cell_start_host, int ncell, int unit_cells,
+                                           const double* pivot, double* sum, double* sumsq, double* T, double* nrm2, double* VS,
+                                           void* workspace, size_t workspace_bytes, void* stream) {
     PLSB_CHECK_ARG(Xc && Q && cell_start_host && sum && sumsq && nrm2 && workspace, "rb_boot_dmma_f64: null pointer");
     PLSB_CHECK_ARG(N > 0 && p > 0 && K > 0 && nbt > 0 && ncell > 0, "rb_boot_dmma_f64: bad shape");
     if (Xc2 == nullptr) { n1 = N; ld2 = p; }
@@ -691,7 +702,7 @@ extern "C" int plsb200_rb_boot_dmma_f64(const double* Xc, int N, int64_t p, cons
     for (int pass = 0; pass < r.npass; ++pass) {
         RdArgs a;
         a.Xc = Xc; a.Xc2 = Xc2; a.n1 = n1; a.ld2 = ld2; a.pack = d_pack; a.wpack = d_wpack; a.nstd = r.nstd; a.pivot = pivot; a.krow = d_krow; a.celln = d_celln; a.sum = sum; a.sumsq = sumsq;
-        a.VSt = d_vst; a.Npart = d_npart; a.p = p; a.Kfull = K; a.k0 = pass * r.kcp;
+        a.VSt = d_vst; a.VS = VS ? VS + (size_t)b0 * p * K : nullptr; a.Npart = d_npart; a.p = p; a.Kfull = K; a.k0 = pass * r.kcp;
         a.kc = K - a.k0 < r.kcp ? K - a.k0 : r.kcp;
         a.nbt = nbt; a.npass = r.npass; a.pass = pass; a.nstage = r.nstage; a.ncell = r.ncell; a.nwarps = L.nwarps; a.ks_unit = r.ks_unit;
         a.cend[0] = r.cend[0]; a.cend[1] = r.cend[1]; a.cend[2] = r.cend[2];
@@ -726,4 +737,12 @@ extern "C" int plsb200_rb_boot_dmma_f64(const double* Xc, int N, int64_t p, cons
         }
     }
     return PLSB200_OK;
+}
+
+extern "C" int plsb200_rb_boot_dmma_f64(const double* Xc, int N, int64_t p, const double* Xc2, int n1, int64_t ld2,
+                                        const double* Q, const double* W, int K, int b0, int nbt, const int32_t* cell_start_host, int ncell, int unit_cells,
+                                        const double* pivot, double* sum, double* sumsq, double* T, double* nrm2,
+                                        void* workspace, size_t workspace_bytes, void* stream) {
+    return plsb200_rb_boot_dmma_vs_f64(Xc, N, p, Xc2, n1, ld2, Q, W, K, b0, nbt, cell_start_host, ncell, unit_cells, pivot,
+                                       sum, sumsq, T, nrm2, nullptr, workspace, workspace_bytes, stream);
 }

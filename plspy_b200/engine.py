@@ -1011,9 +1011,12 @@ class Engine:
                                           self._stream()), "rb_coef_f64")
         return Q, W, Yz
 
-    def rb_boot(self, Xc, Q, W, cell_start, pivot=None, unit_cells=0, max_ws_bytes=2 << 30, want_t=True, X2=None):
+    def rb_boot(self, Xc, Q, W, cell_start, pivot=None, unit_cells=0, max_ws_bytes=2 << 30, want_t=True, X2=None,
+                vs_out=None):
         """p-space pass over all bootstraps in Q: returns (sum, sumsq) of VS - pivot (p x K),
-        T (R x N x K) = Xc @ VS_b (None when want_t is False) and nrm2 (R x K).
+        T (R x N x K) = Xc @ VS_b (None when want_t is False) and nrm2 (R x K).  `vs_out`: an R x p x K float64 device
+        tensor that receives the saliences VS_b themselves (the reference's right_sv_sampled); with want_t=False the
+        call is the p-space pass alone.
         Runs on the FP64 tensor path (plsb200_rb_boot_dmma_f64) when the design fits its register-resident
         fragments, else on the general FMA kernel.  `X2`: the data matrix is the row stack [Xc; X2] (not built: the
         kernels take the two row segments; multiblock bootstraps pass [Xcb; X])."""
@@ -1025,6 +1028,9 @@ class Engine:
         ld2 = int(X2.stride(0)) if X2 is not None else p
         if n1 + (int(X2.shape[0]) if X2 is not None else 0) != N:
             raise ValueError("rb_boot: coefficient rows do not match the data matrix")
+        if vs_out is not None and (vs_out.dtype != F64 or tuple(vs_out.shape) != (R, p, K) or not vs_out.is_contiguous()
+                                   or vs_out.device != torch.device(self.device)):
+            raise ValueError(f"rb_boot: vs_out must be a contiguous float64 tensor of shape {(R, p, K)} on {self.device}")
         ncell = int(cs_host.size) - 1
         s1 = torch.zeros(p, K, dtype=F64, device=self.device); s2 = torch.zeros_like(s1)
         T = self._empty(R, N, K) if want_t else None
@@ -1044,10 +1050,11 @@ class Engine:
                 self._mark("rb_boot")
                 for b0 in range(0, R, nbt):
                     n = min(nbt, R - b0)
-                    check(lib.plsb200_rb_boot_dmma_f64(self._p(Xc), N, p, self._p(X2), n1, ld2, self._p(Q), self._p(W), K, b0, n,
-                                                       cs_host.ctypes.data, ncell, int(unit_cells), self._p(pivot),
-                                                       self._p(s1), self._p(s2), self._p(T), self._p(nrm2),
-                                                       self._p(ws), ws.numel(), self._stream()), "rb_boot_dmma_f64")
+                    check(lib.plsb200_rb_boot_dmma_vs_f64(self._p(Xc), N, p, self._p(X2), n1, ld2, self._p(Q), self._p(W), K,
+                                                          b0, n, cs_host.ctypes.data, ncell, int(unit_cells),
+                                                          self._p(pivot), self._p(s1), self._p(s2), self._p(T),
+                                                          self._p(nrm2), self._p(vs_out), self._p(ws), ws.numel(),
+                                                          self._stream()), "rb_boot_dmma_f64")
                 self._mark("rb_boot")
             return s1, s2, T, nrm2
         # design outside the tensor-core kernel's buckets (more than 16 blocks or 384 rows after padding every block to a
@@ -1069,11 +1076,10 @@ class Engine:
             self._mark("rb_boot")
             for b0 in range(0, R, nbt):
                 n = min(nbt, R - b0)
-                check(lib.plsb200_rb_boot_f64(self._p(Xc), N, p, self._p(X2), n1, ld2, self._p(Q), self._p(W), K, b0, n, self._p(cs),
-                                              ncell, int(unit_cells), self._p(pivot), self._p(s1),
-                                              self._p(s2),
-                                              self._p(T), self._p(nrm2), self._p(ws), ws.numel(), self._stream()),
-                      "rb_boot_f64")
+                check(lib.plsb200_rb_boot_vs_f64(self._p(Xc), N, p, self._p(X2), n1, ld2, self._p(Q), self._p(W), K, b0, n,
+                                                 self._p(cs), ncell, int(unit_cells), self._p(pivot), self._p(s1),
+                                                 self._p(s2), self._p(T), self._p(nrm2), self._p(vs_out), self._p(ws),
+                                                 ws.numel(), self._stream()), "rb_boot_f64")
             self._mark("rb_boot")
         return s1, s2, (T if want_t else None), nrm2
 
