@@ -237,6 +237,13 @@ size_t plsb200_percentile_f64_workspace(int B);
 int plsb200_percentile_f64(const double* samples, int B, int64_t nseries, int64_t stride_sample,
                            int64_t stride_series, double q_lo, double q_hi, double* lower, double* upper,
                            void* workspace, size_t workspace_bytes, void* stream);
+/* the bias-corrected percentile interval (Efron) of the same series: orig[s] is the original value theta of series s,
+ * prop[s] = #{r : sample_r <= theta} / B, z0 = Phi^-1(prop), and the bounds are taken as above at the levels
+ * Phi(2 z0 + Phi^-1(q_lo)) and Phi(2 z0 + Phi^-1(q_hi)) (q = 0 / 1: the minimum / maximum).  prop 0 or 1 gives NaN
+ * bounds; a NaN theta gives NaN bounds and prop.  Workspace: plsb200_percentile_f64_workspace(B).                    */
+int plsb200_percentile_bc_f64(const double* samples, int B, int64_t nseries, int64_t stride_sample,
+                              int64_t stride_series, const double* orig, double q_lo, double q_hi, double* lower,
+                              double* upper, double* prop, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- explicit saliences for a small batch: VS[r] = X^T . C_r  (R x p x K), for callers that ask for
  * boot_debug_dict["right_sv_sampled"] on problems small enough to hold it.                          */

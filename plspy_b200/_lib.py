@@ -149,6 +149,8 @@ SIGNATURES = {
     "plsb200_percentile_f64_workspace": (c_size_t, [c_int]),
     "plsb200_percentile_f64": (c_int, [c_double_p, c_int, c_int64, c_int64, c_int64, c_double, c_double, c_double_p,
                                        c_double_p, c_void_p, c_size_t, c_void_p]),
+    "plsb200_percentile_bc_f64": (c_int, [c_double_p, c_int, c_int64, c_int64, c_int64, c_double_p, c_double, c_double,
+                                          c_double_p, c_double_p, c_double_p, c_void_p, c_size_t, c_void_p]),
     "plsb200_salience_f64": (c_int, [c_double_p, c_int, c_int64, c_int64, c_double_p, c_int, c_int32_p, c_int,
                                      c_double_p, c_void_p]),
     "plsb200_salience_series_f64": (c_int, [c_double_p, c_int, c_int64, c_int64, c_double_p, c_int, c_int32_p, c_int,

@@ -389,6 +389,12 @@ def _numerator(eng, V, s, contrast):
     return Vd * eng.to_device(np.asarray(s, dtype=float), torch.float64) if contrast is None else Vd
 
 
+def _local_numerator(eng, V, s, contrast):
+    """`_numerator`, its rows of the voxels this engine holds."""
+    numer, (v0, v1) = _numerator(eng, V, s, contrast), eng.voxel_range
+    return numer[v0:v1].contiguous() if eng.voxel_sharded else numer
+
+
 def _task_operators(pls_alg, cond_order, mctype, U, contrast):
     """Row-space pull-back of the design-side weights: E = Lop^T @ Ucoef (N x K).
     mct: Lop = centring operator, Ucoef = U (bootstrap_permutation.py:385-387, 404);
@@ -609,9 +615,7 @@ class _TaskPlan:
 
     @functools.cached_property
     def numer(self):
-        """`_numerator`, its rows of the voxels this engine holds."""
-        numer, (v0, v1) = _numerator(self._eng, self.V, self._s, self._contrast), self._eng.voxel_range
-        return numer[v0:v1].contiguous() if self._eng.voxel_sharded else numer
+        return _local_numerator(self._eng, self.V, self._s, self._contrast)
 
 
 def _boot_moments(eng, plan, niter, packed=None):
@@ -645,6 +649,7 @@ class _ResampleTestPLS(ResampleTest):
                  CI=0.95, *, perm_indices=None, boot_indices=None, engine=None, precision="fp64", rotate_method=2,
                  device=None, boot_algo="auto", x_storage=None, shard=None):
         self.CI = CI
+        self._Tvsc_orig, self._lvcorrs_orig = Tvsc_orig, lvcorrs_orig     # centres of bias_corrected_conf_ints
         precision, boot_algo, x_storage, shard = resolve_options(self.pls_alg, engine, X, nboot, cond_order, precision,
                                                                  boot_algo, x_storage, shard)
         self.boot_algo = boot_algo
@@ -743,6 +748,51 @@ class _ResampleTestPLS(ResampleTest):
             raise exceptions.NotImplementedError(
                 "salience percentile intervals are available for the task methods (mct, cst) after a bootstrap test")
         return fn(self._default_conf(conf), max_bytes)
+
+    def _bc_conf(self, conf):
+        if self._engine is None or not hasattr(self, "boot_debug_dict"):
+            raise exceptions.MissingParameterError("bias-corrected intervals need a bootstrap test (num_boot > 0)")
+        conf = self._default_conf(conf)
+        if not all(0.0 <= q <= 1.0 for q in conf):
+            raise ValueError(f"conf must hold two fractions in [0, 1], got {conf}")
+        return conf
+
+    def bias_corrected_conf_ints(self, conf=None):
+        """Bias-corrected percentile intervals (Efron) of the design-side bootstrap distributions, with the share of
+        bootstrap samples at or below the original value (the `*_adj` bounds and `prop` of the MATLAB PLS toolbox).
+        The original value theta is the centre of the normal-theory interval: `Tvsc_orig` for "Tdistrib" (mct, cst,
+        mb, cmb: `conf_ints`, or `conf_ints_T` for mb / cmb), `lvcorrs_orig` for "left_sv_sampled" (rb, csb, mb, cmb:
+        `conf_ints`), broadcast against the distribution's elements as there.  prop = #{samples <= theta} / B, and the
+        bounds are the samples at the levels Phi(2 Phi^-1(prop) + Phi^-1(q)) (NaN where prop is 0 or 1), interpolated
+        like `percentile_conf_ints` (DESIGN.md section 5.8).  conf: (lower, upper) fractions, default from CI.
+        Returns {name: (lower, upper, prop)}."""
+        conf = self._bc_conf(conf)
+        centres = {"Tdistrib": self._Tvsc_orig if self.pls_alg in ("mct", "cst", "mb", "cmb") else None,
+                   "left_sv_sampled": self._lvcorrs_orig if self.pls_alg in ("rb", "csb", "mb", "cmb") else None}
+        out = {}
+        for key, theta in centres.items():
+            if theta is None or key not in self.boot_debug_dict:
+                continue
+            a = np.asarray(self.boot_debug_dict[key])
+            if a.ndim >= 2 and a.size:
+                theta = np.asarray(theta, dtype=float)
+                shape = np.broadcast_shapes(theta.shape, a.shape[1:])
+                a, theta = np.broadcast_to(a, a.shape[:1] + shape), np.broadcast_to(theta, shape)
+                out[key] = tuple(self._engine.to_host(*self._engine.percentile_interval_bc(a, theta, conf)))
+        return out
+
+    def salience_bias_corrected_intervals(self, conf=None, max_bytes=4 << 30):
+        """Bias-corrected percentile interval of every brain salience over the bootstrap samples, with prop, as
+        `bias_corrected_conf_ints` defines them; theta is the numerator of `boot_ratios` (V s for mct, V for cst).
+        Streamed in voxel chunks like `salience_percentile_intervals`.  Task methods (mct, cst).  Returns (lower,
+        upper, prop), p x K.  With shard="voxels" every rank works on its voxels and the results are gathered: every
+        rank must call it."""
+        conf = self._bc_conf(conf)
+        fn = getattr(self.boot_debug_dict, "salience_percentiles_bc", None)
+        if fn is None:
+            raise exceptions.NotImplementedError(
+                "bias-corrected salience intervals are available for the task methods (mct, cst)")
+        return fn(conf, max_bytes)
 
     # ------------------------------------------------------------------------------------------
     @staticmethod
@@ -916,14 +966,22 @@ class _ResampleTestPLS(ResampleTest):
             return VS.cpu().numpy()
         debug.set_lazy("right_sv_sampled", _right)
 
-        def _salience_percentiles(conf, max_bytes=4 << 30):
-            lo_, hi_ = eng.salience_percentiles(E, _index_shard(eng, indices, niter, 0, niter), conf, max_bytes)
+        def _to_host_gathered(*parts):       # p x K parts of this engine's voxels; voxel-sharded: one gather
             if vox:
-                K = int(lo_.shape[1])
-                both = eng.gather_voxels(torch.cat([lo_, hi_], dim=1))
-                lo_, hi_ = both[:, :K], both[:, K:]
-            return tuple(eng.to_host(lo_, hi_))
+                K = int(parts[0].shape[1])
+                both = eng.gather_voxels(torch.cat(parts, dim=1))
+                parts = [both[:, i * K:(i + 1) * K] for i in range(len(parts))]
+            return tuple(eng.to_host(*parts))
+
+        def _salience_percentiles(conf, max_bytes=4 << 30):
+            return _to_host_gathered(*eng.salience_percentiles(E, _index_shard(eng, indices, niter, 0, niter), conf,
+                                                               max_bytes))
         debug.salience_percentiles = _salience_percentiles
+
+        def _salience_percentiles_bc(conf, max_bytes=4 << 30):
+            return _to_host_gathered(*eng.salience_percentiles_bc(
+                E, _index_shard(eng, indices, niter, 0, niter), _local_numerator(eng, V, s, contrast), conf, max_bytes))
+        debug.salience_percentiles_bc = _salience_percentiles_bc
         return conf_int, std_errs_h, boot_ratios_h, debug
 
     # ------------------------------------------------------------------------------------------

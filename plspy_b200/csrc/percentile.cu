@@ -56,18 +56,23 @@ __device__ __forceinline__ void pc_pass(double* a_, int L, int a, int k, int war
     }
 }
 
-template <bool GLOBAL>
+// Bias-corrected bounds (BC): with prop = #{s <= theta} / B (theta = orig[s], the original value) and z0 = Phi^-1(prop),
+// the levels are Phi(2 z0 + Phi^-1(q)) instead of q.  prop is counted by binary search over the first B sorted slots
+// (the +inf padding never counts); prop 0 or 1 (z0 infinite) and a NaN theta give NaN bounds.
+template <bool GLOBAL, bool BC>
 __global__ void __launch_bounds__(PC_THREADS) percentile_kernel(const double* __restrict__ S, int B, long long nseries,
                                                                long long stride_sample, long long stride_series,
                                                                double q_lo, double q_hi, int L,
                                                                double* __restrict__ lower, double* __restrict__ upper,
-                                                               double* __restrict__ scratch) {
+                                                               double* __restrict__ scratch,
+                                                               const double* __restrict__ orig, double* __restrict__ prop) {
     extern __shared__ __align__(16) double pc_sm[];
     double* a = GLOBAL ? scratch + (size_t)blockIdx.x * pc_slots(L) : pc_sm;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int span = L / (PC_THREADS / 32);                 // elements owned by a warp (L >= 512: span >= 64)
     int logL = 0;
     while ((1 << logL) < L) ++logL;
+    const double zq = BC && tid < 2 ? normcdfinv(tid == 0 ? q_lo : q_hi) : 0.0;   // -inf / +inf at q = 0 / 1
     for (long long s = blockIdx.x; s < nseries; s += gridDim.x) {
         const double* src = S + s * stride_series;
         for (int r = tid; r < L; r += PC_THREADS) a[pc_phys(r)] = r < B ? src[(long long)r * stride_sample] : CUDART_INF;
@@ -89,12 +94,26 @@ __global__ void __launch_bounds__(PC_THREADS) percentile_kernel(const double* __
         }
         __syncthreads();
         if (tid < 2) {
-            double t = (tid == 0 ? q_lo : q_hi) * B - 0.5;        // fractional index into the sorted samples
+            double q = tid == 0 ? q_lo : q_hi;
+            bool defined = true;
+            if (BC) {                                       // both threads count (same addresses: broadcast reads)
+                const double theta = orig[s];
+                int lo = 0, hi = B;                         // first sorted slot > theta
+                while (lo < hi) {
+                    const int mid = (lo + hi) >> 1;
+                    if (a[pc_phys(mid)] <= theta) lo = mid + 1; else hi = mid;
+                }
+                const double pr = isnan(theta) ? CUDART_NAN : (double)lo / B;
+                if (tid == 0) prop[s] = pr;
+                defined = pr > 0.0 && pr < 1.0;             // false for NaN too
+                if (defined) q = normcdf(2.0 * normcdfinv(pr) + zq);
+            }
+            double t = q * B - 0.5;                         // fractional index into the sorted samples
             t = fmin(fmax(t, 0.0), (double)(B - 1));
             const int lo = (int)floor(t), hi = min(lo + 1, B - 1);
             const double w = t - lo;
             const double v = a[pc_phys(lo)] * (1.0 - w) + a[pc_phys(hi)] * w;
-            (tid == 0 ? lower : upper)[s] = v;
+            (tid == 0 ? lower : upper)[s] = defined ? v : CUDART_NAN;
         }
         __syncthreads();
     }
@@ -116,34 +135,51 @@ extern "C" size_t plsb200_percentile_f64_workspace(int B) {
     return L > PC_MAX_SMEM_L ? (size_t)2 * num_sms() * pc_slots(L) * sizeof(double) : 16;
 }
 
-extern "C" int plsb200_percentile_f64(const double* samples, int B, int64_t nseries, int64_t stride_sample,
-                                      int64_t stride_series, double q_lo, double q_hi, double* lower, double* upper,
-                                      void* workspace, size_t workspace_bytes, void* stream) {
-    PLSB_CHECK_ARG(samples && lower && upper, "percentile_f64: null pointer");
-    PLSB_CHECK_ARG(B >= 1 && B <= (1 << 24) && nseries >= 1, "percentile_f64: bad shape B=%d nseries=%lld", B,
+// one launcher for both entry points: the plain interval (BC = false, orig / prop unused) and the bias-corrected one
+template <bool BC>
+static int pc_launch(const char* what, const double* samples, int B, int64_t nseries, int64_t stride_sample,
+                     int64_t stride_series, const double* orig, double q_lo, double q_hi, double* lower, double* upper,
+                     double* prop, void* workspace, size_t workspace_bytes, void* stream) {
+    PLSB_CHECK_ARG(samples && lower && upper && (!BC || (orig && prop)), "%s: null pointer", what);
+    PLSB_CHECK_ARG(B >= 1 && B <= (1 << 24) && nseries >= 1, "%s: bad shape B=%d nseries=%lld", what, B,
                    (long long)nseries);
-    PLSB_CHECK_ARG(q_lo >= 0.0 && q_lo <= 1.0 && q_hi >= 0.0 && q_hi <= 1.0, "percentile_f64: quantiles must lie in [0, 1]");
+    PLSB_CHECK_ARG(q_lo >= 0.0 && q_lo <= 1.0 && q_hi >= 0.0 && q_hi <= 1.0, "%s: quantiles must lie in [0, 1]", what);
     const int L = pc_padded(B);
     cudaStream_t st = (cudaStream_t)stream;
     if (L <= PC_MAX_SMEM_L) {
         const size_t smem = pc_slots(L) * sizeof(double);
-        PLSB_CUDA(cudaFuncSetAttribute(percentile_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        PLSB_CUDA(cudaFuncSetAttribute(percentile_kernel<false, BC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         const int per_sm = (int)((220 * 1024) / smem) < 8 ? (int)((220 * 1024) / smem) : 8;
         const long long cap = (long long)num_sms() * per_sm * 4;
         const unsigned grid = (unsigned)(nseries < cap ? nseries : cap);
-        percentile_kernel<false><<<grid, PC_THREADS, smem, st>>>(samples, B, nseries, stride_sample, stride_series, q_lo,
-                                                                q_hi, L, lower, upper, nullptr);
+        percentile_kernel<false, BC><<<grid, PC_THREADS, smem, st>>>(samples, B, nseries, stride_sample, stride_series,
+                                                                    q_lo, q_hi, L, lower, upper, nullptr, orig, prop);
     } else {
         const size_t need = (size_t)2 * num_sms() * pc_slots(L) * sizeof(double);
         if (!workspace || workspace_bytes < need) {
-            set_err("percentile_f64: workspace %zu < %zu bytes", workspace_bytes, need);
+            set_err("%s: workspace %zu < %zu bytes", what, workspace_bytes, need);
             return PLSB200_EWORKSPACE;
         }
         const long long cap = 2LL * num_sms();
         const unsigned grid = (unsigned)(nseries < cap ? nseries : cap);
-        percentile_kernel<true><<<grid, PC_THREADS, 0, st>>>(samples, B, nseries, stride_sample, stride_series, q_lo, q_hi,
-                                                            L, lower, upper, (double*)workspace);
+        percentile_kernel<true, BC><<<grid, PC_THREADS, 0, st>>>(samples, B, nseries, stride_sample, stride_series, q_lo,
+                                                                q_hi, L, lower, upper, (double*)workspace, orig, prop);
     }
     PLSB_LAUNCH_CHECK("percentile_kernel");
     return PLSB200_OK;
+}
+
+extern "C" int plsb200_percentile_f64(const double* samples, int B, int64_t nseries, int64_t stride_sample,
+                                      int64_t stride_series, double q_lo, double q_hi, double* lower, double* upper,
+                                      void* workspace, size_t workspace_bytes, void* stream) {
+    return pc_launch<false>("percentile_f64", samples, B, nseries, stride_sample, stride_series, nullptr, q_lo, q_hi,
+                            lower, upper, nullptr, workspace, workspace_bytes, stream);
+}
+
+extern "C" int plsb200_percentile_bc_f64(const double* samples, int B, int64_t nseries, int64_t stride_sample,
+                                         int64_t stride_series, const double* orig, double q_lo, double q_hi,
+                                         double* lower, double* upper, double* prop, void* workspace,
+                                         size_t workspace_bytes, void* stream) {
+    return pc_launch<true>("percentile_bc_f64", samples, B, nseries, stride_sample, stride_series, orig, q_lo, q_hi,
+                           lower, upper, prop, workspace, workspace_bytes, stream);
 }

@@ -884,14 +884,31 @@ class Engine:
                                              self._p(hi), self._p(ws), nb, self._stream()), "percentile_f64")
         return lo, hi
 
-    def salience_percentiles(self, E, idx, conf=(0.05, 0.95), max_bytes=4 << 30):
-        """Percentile interval of every element of the bootstrap salience distribution VS[r] = X^T scatter(E, idx_r)
-        (what `confidence_interval(right_sv_sampled)` would give) without holding the R x p x K cube: voxel chunks
-        of at most `max_bytes` are made explicit (`salience`), reduced to their two bounds and dropped.
-        Returns (lower, upper), p x K device tensors."""
+    def percentile_interval_bc(self, A, orig, conf=(0.05, 0.95)):
+        """Bias-corrected percentile interval (Efron) over the first axis of a (B x ...) stack: `orig`, shaped like
+        A[0], holds the original value theta of every element; prop = #{samples <= theta} / B and the bounds are taken
+        at the levels Phi(2 Phi^-1(prop) + Phi^-1(q)) (DESIGN.md section 5.8).  Returns (lower, upper, prop) device
+        tensors shaped like A[0]; lower / upper are NaN where prop is 0 or 1."""
+        A = self.to_device(A, F64)
+        orig = self.to_device(orig, F64)
+        if tuple(orig.shape) != tuple(A.shape[1:]):
+            raise ValueError(f"orig has shape {tuple(orig.shape)}, the elements of the stack {tuple(A.shape[1:])}")
+        B = int(A.shape[0]); M = int(A.numel() // B)
+        lo, hi, prop = (self._empty(*A.shape[1:]) for _ in range(3))
+        with torch.cuda.device(self.device):
+            nb = lib.plsb200_percentile_f64_workspace(B)
+            ws = self._ws(nb)
+            check(lib.plsb200_percentile_bc_f64(self._p(A), B, M, M, 1, self._p(orig), float(conf[0]), float(conf[1]),
+                                                self._p(lo), self._p(hi), self._p(prop), self._p(ws), nb,
+                                                self._stream()), "percentile_bc_f64")
+        return lo, hi, prop
+
+    def _salience_chunks(self, E, idx, max_bytes, reduce):
+        """Streams the bootstrap salience distribution VS[r] = X^T scatter(E, idx_r) without holding the R x p x K
+        cube: voxel chunks of at most `max_bytes` are made explicit series-major and handed to
+        `reduce(cube, R, v0, v1, ws, nb)` (ws: nb bytes of percentile workspace), then dropped."""
         E = self.to_device(E, F64); idx = self.to_device(idx, I32)
         R, K = int(idx.shape[0]), int(E.shape[1])
-        lo = self._empty(self.p, K); hi = self._empty(self.p, K)
         vc = max(128, min(self.p, int(max_bytes // (R * K * 8)) // 128 * 128))
         X = self.X
         series, what = self._xfn("salience_series_f64", X)
@@ -905,11 +922,42 @@ class Engine:
                 cube = self._empty(v1 - v0, K, R)
                 check(series(self._xp(v0), self.N, v1 - v0, self.ldx, self._p(E), K, self._p(idx), R, self._p(cube),
                              self._stream()), what)
-                check(lib.plsb200_percentile_f64(self._p(cube), R, (v1 - v0) * K, 1, R, float(conf[0]), float(conf[1]),
-                                                 lo.data_ptr() + 8 * v0 * K, hi.data_ptr() + 8 * v0 * K, self._p(ws), nb,
-                                                 self._stream()), "percentile_f64")
+                reduce(cube, R, v0, v1, ws, nb)
                 del cube
+
+    def salience_percentiles(self, E, idx, conf=(0.05, 0.95), max_bytes=4 << 30):
+        """Percentile interval of every element of the bootstrap salience distribution VS[r] = X^T scatter(E, idx_r)
+        (what `confidence_interval(right_sv_sampled)` would give) without holding the R x p x K cube: voxel chunks
+        of at most `max_bytes` are made explicit (`salience`), reduced to their two bounds and dropped.
+        Returns (lower, upper), p x K device tensors."""
+        K = int(E.shape[1])
+        lo = self._empty(self.p, K); hi = self._empty(self.p, K)
+
+        def reduce(cube, R, v0, v1, ws, nb):
+            check(lib.plsb200_percentile_f64(self._p(cube), R, (v1 - v0) * K, 1, R, float(conf[0]), float(conf[1]),
+                                             lo.data_ptr() + 8 * v0 * K, hi.data_ptr() + 8 * v0 * K, self._p(ws), nb,
+                                             self._stream()), "percentile_f64")
+        self._salience_chunks(E, idx, max_bytes, reduce)
         return lo, hi
+
+    def salience_percentiles_bc(self, E, idx, orig, conf=(0.05, 0.95), max_bytes=4 << 30):
+        """Bias-corrected percentile interval (`percentile_interval_bc`) of every element of the same streamed
+        distribution; `orig` (p x K, this engine's voxels) is the original salience of every element.
+        Returns (lower, upper, prop), p x K device tensors."""
+        K = int(E.shape[1])
+        orig = self.to_device(orig, F64)
+        if tuple(orig.shape) != (self.p, K):
+            raise ValueError(f"orig has shape {tuple(orig.shape)}, the saliences {(self.p, K)}")
+        lo, hi, prop = (self._empty(self.p, K) for _ in range(3))
+
+        def reduce(cube, R, v0, v1, ws, nb):
+            off = 8 * v0 * K
+            check(lib.plsb200_percentile_bc_f64(self._p(cube), R, (v1 - v0) * K, 1, R, orig.data_ptr() + off,
+                                                float(conf[0]), float(conf[1]), lo.data_ptr() + off,
+                                                hi.data_ptr() + off, prop.data_ptr() + off, self._p(ws), nb,
+                                                self._stream()), "percentile_bc_f64")
+        self._salience_chunks(E, idx, max_bytes, reduce)
+        return lo, hi, prop
 
     def salience(self, E, idx, M=None):
         """Explicit VS[r] = M^T scatter(E, idx_r) (R x p x K), M = X by default -- small R only."""
