@@ -142,6 +142,16 @@ def _p_sized_to_host(eng, *tensors):
     return out if isinstance(out, (list, tuple)) else [out]
 
 
+def _p_sized_to_host_async(eng, *tensors):
+    """`_p_sized_to_host` with the copies on the side stream, so that they overlap the kernels enqueued next: returns a
+    function that waits for them and hands back what `_p_sized_to_host` would."""
+    if dist.world()[1] > 1 and dist.world()[0] != 0:
+        out = [_DeviceResult(eng, t) for t in tensors]
+        return lambda: out
+    fetch = eng.to_host_async(*tensors, side=True)
+    return lambda: list(fetch()) if len(tensors) > 1 else [fetch()]
+
+
 # Largest `right_sv_sampled` cube (B x p x K float64) a read builds.  The bootstrap itself never stores the cube: it
 # accumulates the moments on the fly, and the lazy entry rebuilds the saliences only when asked for.
 RIGHT_SV_MAX_BYTES = 2 << 30
@@ -594,13 +604,13 @@ def _collapsed_sumsq(eng, E, idx_dev, niter, lo, hi, factor=None):
 class _TaskPlan:
     """The inputs of one mct / cst bootstrap: operators, this rank's draws (rows [lo, hi); `idx_all`: every draw, for
     the moment stage of a voxel-sharded engine), the resolved `boot_algo` with its `_factor_plan` (None: the N x N
-    route), and the `moments` once `_boot_moments` has run.  `drawn`: the library drew `indices` (no draw check).  V
+    route), and the `results` once `_boot_results` has run.  `drawn`: the library drew `indices` (no draw check).  V
     reaches the device at its first use: uploaded ahead of the collapsed stage it would hold back a pipelined X."""
 
     def __init__(self, eng, pls_alg, U, s, V, cond_order, mctype, contrast, niter, indices, boot_algo, drawn=False):
         if isinstance(indices, tuple):
             indices = indices[0]
-        self.boot_algo, self.moments = boot_algo, None
+        self.boot_algo, self.results = boot_algo, None
         self.Lop, self.Ucoef, self.E = _task_operators(pls_alg, cond_order, mctype, U, contrast)
         self.factor = (_factor_plan(eng, pls_alg, U, contrast, cond_order, mctype, niter, None if drawn else indices)
                        if boot_algo == "collapsed" else None)
@@ -633,6 +643,18 @@ def _boot_moments(eng, plan, niter, packed=None):
         s1 = torch.zeros_like(plan.numer); s2 = torch.zeros_like(plan.numer)
     dist.allreduce_packed_([s1, s2])
     return s1, s2
+
+
+def _boot_results(eng, plan, niter, packed=None):
+    """The moment stage of the mct / cst bootstrap, the standard errors and bootstrap ratios from it, and their copy to
+    the host started on the side stream; returns the function that waits for [std_errs, boot_ratios]."""
+    s1, s2 = _boot_moments(eng, plan, niter, packed)
+    std_errs, boot_ratios = eng.boot_finalize(s1, s2, niter, numer=plan.numer)   # (:695-703)
+    if eng.voxel_sharded:                                                       # ONE gather of [std_errs | boot_ratios]
+        K = int(std_errs.shape[1])
+        both = eng.gather_voxels(torch.cat([std_errs, boot_ratios], dim=1))
+        std_errs, boot_ratios = both[:, :K], both[:, K:]
+    return _p_sized_to_host_async(eng, std_errs, boot_ratios)
 
 
 @ResampleTest._register_subclass("mct")
@@ -683,11 +705,24 @@ class _ResampleTestPLS(ResampleTest):
                                                           Ybscan=Ybscan)
             plan = _TaskPlan(eng, self.pls_alg, U, s, V, cond_order, mctype, contrast, nboot, boot_indices, boot_algo,
                              drawn=drawn)
-            if eng.upload_in_flight and dist.world()[1] == 1:
-                # X is still crossing PCIe in voxel ranges (Engine._upload_pipelined): the moment stage is the one
-                # that can start on the ranges already there, so it is enqueued before the permutation test, whose
-                # Gram matrix needs all of X
-                plan.moments = _boot_moments(eng, plan, nboot)
+            if self.pls_alg == "mct" and not eng.upload_in_flight:
+                eng.prepare_xv(plan.V)          # X V for U_hat out of the Gram launch, where that is free
+            if plan.boot_algo == "collapsed" or (eng.upload_in_flight and dist.world()[1] == 1):
+                # The moment stage runs first, and the copy of its p x K results to the host (38 MB at the bench
+                # shape) overlaps the N-space work of both tests.  When X is still crossing PCIe in voxel ranges
+                # (Engine._upload_pipelined), the moment stage is also the one that can start on the ranges already
+                # there.  The direct route on a resident X keeps it last, where it shares the packed coefficients of
+                # the bootstrap's N-space pass.  The bootstrap's N-space outputs come next, so that their copy
+                # (Tdistrib, U_hat) overlaps the permutation kernels and the step ends on the small copy of the
+                # permutation results.  (The same order on every rank: boot_algo is the whole run's.)
+                plan.results = _boot_results(eng, plan, nboot)
+        boot_first = nboot > 0 and plan is not None and plan.results is not None
+        boot_pending = None
+        if boot_first:
+            boot_pending = self._bootstrap_test(
+                X, Y, U, s, V, cond_order, mctype, nboot, self.pls_alg, preprocess=preprocess, contrast=contrast,
+                Tvsc_orig=Tvsc_orig, CI=CI, indices=boot_indices, engine=eng, boot_algo=boot_algo, _plan=plan,
+                _defer=True)
         if nperm > 0:
             # the permutation kernels and their device->host copies are enqueued here; the host only waits for
             # them after the bootstrap work has been enqueued too, so the GPU never idles between the two tests
@@ -699,7 +734,7 @@ class _ResampleTestPLS(ResampleTest):
             self.permute_ratio = "NA"
             self.stepdown_ratio = "NA"
         if nboot > 0:
-            out = self._bootstrap_test(
+            out = boot_pending() if boot_first else self._bootstrap_test(
                 X, Y, U, s, V, cond_order, mctype, nboot, self.pls_alg, preprocess=preprocess, contrast=contrast,
                 bscan=bscan, Xbscan=Xbscan, Ybscan=Ybscan, lvcorrs_orig=lvcorrs_orig, Tvsc_orig=Tvsc_orig, CI=CI,
                 indices=boot_indices, engine=eng, boot_algo=boot_algo, _plan=plan)
@@ -891,10 +926,11 @@ class _ResampleTestPLS(ResampleTest):
     @staticmethod
     def _bootstrap_test(X, Y, U, s, V, cond_order, mctype, niter, pls_alg, preprocess=None, dist_=(0.05, 0.95),
                         contrast=None, bscan=None, Xbscan=None, Ybscan=None, lvcorrs_orig=None, Tvsc_orig=None,
-                        CI=0.95, indices=None, engine=None, boot_algo="direct", _plan=None):
+                        CI=0.95, indices=None, engine=None, boot_algo="direct", _plan=None, _defer=False):
         """bootstrap_permutation.py:466-766 for the task methods (mct, cst).  `boot_algo`: see `check_boot_algo`
-        ("auto" resolves here).  `_plan`: the `_TaskPlan` of these draws (mct / cst), with its moments when its moment
-        stage already ran; built here when None.  A voxel-sharded engine
+        ("auto" resolves here).  `_plan`: the `_TaskPlan` of these draws (mct / cst), with its results when its moment
+        stage already ran; built here when None.  `_defer=True` (mct / cst) returns a function that waits for the
+        device results and builds the outputs.  A voxel-sharded engine
         runs the moment GEMM of ALL bootstraps on its voxels (no moment all-reduce) and gathers the p x K results; the
         lazy `right_sv_sampled` and the salience percentiles are then gathered too, so every rank must ask for them."""
         eng = engine if engine is not None else Engine(X)
@@ -914,10 +950,9 @@ class _ResampleTestPLS(ResampleTest):
                                                          indices, boot_algo)
         Lop, Ucoef, E, idx_dev, lo, hi = plan.Lop, plan.Ucoef, plan.E, plan.idx, plan.lo, plan.hi
         Abar = class_functions._cell_mean_operator(cond_order)
-        numer_v = plan.numer
         vox = eng.voxel_sharded
         # exact mode, single launch: the packed coefficients serve the N-space pass and the moment GEMM
-        packed = (eng.pack_coef(E, idx_dev) if (hi > lo and eng.precision == "fp64" and plan.moments is None
+        packed = (eng.pack_coef(E, idx_dev) if (hi > lo and eng.precision == "fp64" and plan.results is None
                                                 and E.shape[1] <= eng.KMAX and not vox) else None)
         d2, Tdist = eng.nspace(E, idx_dev, Lmat=Abar, packed=packed)        # Tdistrib (:633-634, :665-666)
         if pls_alg == "mct":
@@ -926,7 +961,8 @@ class _ResampleTestPLS(ResampleTest):
         else:
             left = None
         # the per-bootstrap N-space outputs are complete here: assemble them across ranks and start their
-        # device -> host copies on a second stream, so that they overlap the moment GEMM enqueued next
+        # device -> host copies on a second stream, so that they overlap the kernels enqueued next (the moment GEMM, or
+        # the permutation test when the moment stage ran first)
         Tdist = dist.gather_rows(Tdist, niter, lo)
         if left is not None:
             left = dist.gather_rows(left, niter, lo)
@@ -935,54 +971,53 @@ class _ResampleTestPLS(ResampleTest):
         defer = dist.world()[1] > 1
         fetch_small = (eng.to_host_async(eng.colstd(Tdist), side=True) if defer
                        else eng.to_host_async(eng.colstd(Tdist), Tdist, left, side=True))
-        s1, s2 = plan.moments if plan.moments is not None else _boot_moments(eng, plan, niter, packed)
-        std_errs, boot_ratios = eng.boot_finalize(s1, s2, niter, numer=numer_v)   # (:695-703)
-        if vox:                                                             # ONE gather of [std_errs | boot_ratios]
-            K = int(std_errs.shape[1])
-            both = eng.gather_voxels(torch.cat([std_errs, boot_ratios], dim=1))
-            std_errs, boot_ratios = both[:, :K], both[:, K:]
-        z = norm.ppf(1 - (1 - CI) / 2)                                      # (:709)
-        std_errs_h, boot_ratios_h = _p_sized_to_host(eng, std_errs, boot_ratios)
-        std_T, Tdist_h, left_h = (fetch_small(), None, None) if defer else fetch_small()
-        half = std_T * z                                                    # (:715-716)
-        conf_int = (Tvsc_orig - half, Tvsc_orig + half)
+        fetch_p = plan.results if plan.results is not None else _boot_results(eng, plan, niter, packed)
 
-        debug = _LazyDebugDict()
-        if defer:
-            debug.set_lazy("Tdistrib", lambda: eng.to_host(Tdist))
-            debug.set_lazy("left_sv_sampled", (lambda: eng.to_host(left)) if left is not None
-                           else (lambda: np.zeros((niter, Ucoef.shape[0], Ucoef.shape[1]))))
-        else:
-            debug["left_sv_sampled"] = (left_h if left_h is not None
-                                        else np.zeros((niter, Ucoef.shape[0], Ucoef.shape[1])))
-            debug["Tdistrib"] = Tdist_h
-        debug.set_lazy("indices", lambda: _indices_to_host(indices, niter))
+        def finish():
+            z = norm.ppf(1 - (1 - CI) / 2)                                      # (:709)
+            std_errs_h, boot_ratios_h = fetch_p()
+            std_T, Tdist_h, left_h = (fetch_small(), None, None) if defer else fetch_small()
+            half = std_T * z                                                    # (:715-716)
+            conf_int = (Tvsc_orig - half, Tvsc_orig + half)
 
-        def _right():   # the reference's B x p x K cube, only on request
-            _check_right_sv_bytes(niter, eng.p_total, E.shape[1])
-            VS = eng.salience(E, _index_shard(eng, indices, niter, 0, niter))
-            if vox:     # voxel-major for the gather
-                VS = eng.gather_voxels(VS.transpose(0, 1).contiguous()).transpose(0, 1).contiguous()
-            return VS.cpu().numpy()
-        debug.set_lazy("right_sv_sampled", _right)
+            debug = _LazyDebugDict()
+            if defer:
+                debug.set_lazy("Tdistrib", lambda: eng.to_host(Tdist))
+                debug.set_lazy("left_sv_sampled", (lambda: eng.to_host(left)) if left is not None
+                               else (lambda: np.zeros((niter, Ucoef.shape[0], Ucoef.shape[1]))))
+            else:
+                debug["left_sv_sampled"] = (left_h if left_h is not None
+                                            else np.zeros((niter, Ucoef.shape[0], Ucoef.shape[1])))
+                debug["Tdistrib"] = Tdist_h
+            debug.set_lazy("indices", lambda: _indices_to_host(indices, niter))
 
-        def _to_host_gathered(*parts):       # p x K parts of this engine's voxels; voxel-sharded: one gather
-            if vox:
-                K = int(parts[0].shape[1])
-                both = eng.gather_voxels(torch.cat(parts, dim=1))
-                parts = [both[:, i * K:(i + 1) * K] for i in range(len(parts))]
-            return tuple(eng.to_host(*parts))
+            def _right():   # the reference's B x p x K cube, only on request
+                _check_right_sv_bytes(niter, eng.p_total, E.shape[1])
+                VS = eng.salience(E, _index_shard(eng, indices, niter, 0, niter))
+                if vox:     # voxel-major for the gather
+                    VS = eng.gather_voxels(VS.transpose(0, 1).contiguous()).transpose(0, 1).contiguous()
+                return VS.cpu().numpy()
+            debug.set_lazy("right_sv_sampled", _right)
 
-        def _salience_percentiles(conf, max_bytes=4 << 30):
-            return _to_host_gathered(*eng.salience_percentiles(E, _index_shard(eng, indices, niter, 0, niter), conf,
-                                                               max_bytes))
-        debug.salience_percentiles = _salience_percentiles
+            def _to_host_gathered(*parts):       # p x K parts of this engine's voxels; voxel-sharded: one gather
+                if vox:
+                    K = int(parts[0].shape[1])
+                    both = eng.gather_voxels(torch.cat(parts, dim=1))
+                    parts = [both[:, i * K:(i + 1) * K] for i in range(len(parts))]
+                return tuple(eng.to_host(*parts))
 
-        def _salience_percentiles_bc(conf, max_bytes=4 << 30):
-            return _to_host_gathered(*eng.salience_percentiles_bc(
-                E, _index_shard(eng, indices, niter, 0, niter), _local_numerator(eng, V, s, contrast), conf, max_bytes))
-        debug.salience_percentiles_bc = _salience_percentiles_bc
-        return conf_int, std_errs_h, boot_ratios_h, debug
+            def _salience_percentiles(conf, max_bytes=4 << 30):
+                return _to_host_gathered(*eng.salience_percentiles(E, _index_shard(eng, indices, niter, 0, niter),
+                                                                   conf, max_bytes))
+            debug.salience_percentiles = _salience_percentiles
+
+            def _salience_percentiles_bc(conf, max_bytes=4 << 30):
+                return _to_host_gathered(*eng.salience_percentiles_bc(
+                    E, _index_shard(eng, indices, niter, 0, niter), _local_numerator(eng, V, s, contrast), conf,
+                    max_bytes))
+            debug.salience_percentiles_bc = _salience_percentiles_bc
+            return conf_int, std_errs_h, boot_ratios_h, debug
+        return finish if _defer else finish()
 
     # ------------------------------------------------------------------------------------------
     @staticmethod

@@ -153,21 +153,24 @@ __global__ void __launch_bounds__(GTHREADS) gram_partial_kernel(const T* __restr
         }
 }
 
-__global__ void gram_reduce_kernel(const double* __restrict__ part, int npair, int nsplit, int ntile, int N,
-                                   double* __restrict__ G) {
+// One thread per element of a tile pair (grid: pairs x GT*GT/GRED_THREADS): the split partials of an element are summed
+// in split order.  One CTA per pair (15 CTAs at N = 300) left most SMs idle while it read the partials.
+constexpr int GRED_THREADS = 256;
+__global__ void __launch_bounds__(GRED_THREADS) gram_reduce_kernel(const double* __restrict__ part, int npair,
+                                                                   int nsplit, int ntile, int N, double* __restrict__ G) {
     const int pair = blockIdx.x;
     int ti = 0, rem = pair, row = ntile;
     while (rem >= row) { rem -= row; --row; ++ti; }
     const int tj = ti + rem;
-    for (int e = threadIdx.x; e < GT * GT; e += blockDim.x) {
-        double s = 0.0;
-        for (int c = 0; c < nsplit; ++c) s += part[((long long)c * npair + pair) * (GT * GT) + e];
-        const int r = ti * GT + e / GT, cc = tj * GT + e % GT;
-        if (r < N && cc < N) {
-            G[(long long)r * N + cc] = s;
-            if (ti != tj) G[(long long)cc * N + r] = s;
-        }
-    }
+    const int e = blockIdx.y * GRED_THREADS + threadIdx.x;
+    const int r = ti * GT + e / GT, cc = tj * GT + e % GT;
+    if (r >= N || cc >= N) return;
+    const double* src = part + (long long)pair * (GT * GT) + e;
+    const long long stride = (long long)npair * (GT * GT);
+    double s = 0.0;
+    for (int c = 0; c < nsplit; ++c) s += __ldg(src + c * stride);
+    G[(long long)r * N + cc] = s;
+    if (ti != tj) G[(long long)cc * N + r] = s;
 }
 
 }  // namespace plsb
@@ -204,7 +207,8 @@ static int gram_launch(const T* X, int n1, int64_t ldx, const T* X2, int n2, int
         gram_partial_kernel<T, 1><<<grid, GTHREADS, smem, st>>>(X, N, p, ldx, X2, n1, ld2, g.chunk, g.ntile, (double*)workspace);
     }
     PLSB_LAUNCH_CHECK("gram_partial_kernel");
-    gram_reduce_kernel<<<g.npair, 256, 0, st>>>((const double*)workspace, g.npair, g.nsplit, g.ntile, N, G);
+    gram_reduce_kernel<<<dim3(g.npair, GT * GT / GRED_THREADS), GRED_THREADS, 0, st>>>((const double*)workspace, g.npair,
+                                                                                       g.nsplit, g.ntile, N, G);
     PLSB_LAUNCH_CHECK("gram_reduce_kernel");
     return PLSB200_OK;
 }

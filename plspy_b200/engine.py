@@ -90,6 +90,8 @@ class Engine:
         self.N, self.p = int(self._X.shape[0]), int(self._X.shape[1])     # p: the width held here
         self.ldx = int(self._X.stride(0))
         self._G = None
+        self._xv_next = None          # the V of a later xv(V) whose product comes out of the Gram launch (prepare_xv)
+        self._xv_done = None          # (V, X V) of that launch
         self.kernel_events = None     # set to {} to record CUDA events around named kernels (bench.py)
         self.on_mark = None           # optional callable(name) invoked at every _mark (bench.py: clock sampling)
         self.h2d_bytes = 0 if (torch.is_tensor(X) and X.is_cuda) else self._X.numel() * self._X.element_size()
@@ -430,6 +432,8 @@ class Engine:
                 self._G = torch.zeros(self.N, self.N, dtype=F64, device=self.device)
             elif self.gram_tf32 and self.N <= self.GRAM_TF32_MAX_ROWS:
                 self._G = self._gram_tf32()
+            elif self._xv_next is not None:
+                self._G = self._gram_xv()
             elif self._pending is None:
                 self._G = self.gram_of(self.X)
             else:       # partial Gram matrices of the voxel ranges as they arrive, summed in a fixed order
@@ -481,10 +485,36 @@ class Engine:
             self._G = G
         return self.G
 
+    GRAM_TILE_ROWS = 64     # row tile of the exact Gram kernel (gram.cu GT)
+
+    def prepare_xv(self, V):
+        """Announces the V (p x K) of a later `xv(V)`.  If G is not formed yet, X is float64, whole and resident, G is
+        exact, and the stack [X; V^T] has no more 64-row tiles than X, G is then formed as the Gram matrix of that stack
+        in one launch: its X block is bit-identical to `gram_of(X)` (same tiles, same voxel splits; a row of G only
+        reads its own two rows of the stack) and its X-V^T block is X V, which `xv(V)` returns without a pass of its
+        own over X.  Otherwise nothing changes.  Returns whether the product will come from the Gram launch."""
+        V = self.to_device(V, F64)
+        K, t = int(V.shape[1]), self.GRAM_TILE_ROWS
+        fused = (self._G is None and self._pending is None and not self.voxel_sharded and self._X.dtype == F64
+                 and not (self.gram_tf32 and self.N <= self.GRAM_TF32_MAX_ROWS) and self.p > 0
+                 and V.dim() == 2 and int(V.shape[0]) == self.p and -(-(self.N + K) // t) == -(-self.N // t))
+        self._xv_next = V if fused else None
+        return fused
+
+    def _gram_xv(self):
+        V, self._xv_next = self._xv_next, None
+        Gs = self.gram_stacked(self.X, V.T.contiguous())
+        self._xv_done = (V, Gs[:self.N, self.N:].contiguous())
+        return Gs[:self.N, :self.N].contiguous()
+
     def xv(self, V):
         """XL = X @ V (N x K) for V of p_total x K.  Voxel-sharded: the product of this rank's columns with its rows of V
-        plus one all-reduce of N x K doubles (COLLECTIVE)."""
+        plus one all-reduce of N x K doubles (COLLECTIVE).  The V of `prepare_xv`: the product of the Gram launch."""
         V = self.to_device(V, F64)
+        if self._xv_next is V:
+            self.G
+        if self._xv_done is not None and self._xv_done[0] is V:
+            return self._xv_done[1]
         K = int(V.shape[1])
         if self.voxel_sharded:
             if int(V.shape[0]) != self.p_total:

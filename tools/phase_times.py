@@ -1,5 +1,7 @@
 """Where does one pass of the bench workload spend its time?  Wraps every Engine method with host timestamps and
-CUDA events (development aid; run on the GPU box: PYTHONPATH=. python tools/phase_times.py [--precision tf32x3])."""
+CUDA events (development aid; run on the GPU box: PYTHONPATH=. python tools/phase_times.py [--precision tf32x3]).
+--profile DIR: instead, one pass under torch.profiler (CUDA activities), its kernel and copy list written to
+DIR/kernels.txt and the trace to DIR/trace.json (no wrappers: the profiler run is kept apart from the timeline)."""
 import os as _os, sys as _sys
 _sys.path.insert(0, _os.path.dirname(_os.path.dirname(_os.path.abspath(__file__))))
 import argparse, json, time
@@ -12,6 +14,7 @@ ap = argparse.ArgumentParser()
 ap.add_argument("--precision", default="fp64")
 ap.add_argument("--voxels", type=int, default=bench.P_VOX)
 ap.add_argument("--n", type=int, default=5000)
+ap.add_argument("--profile", metavar="DIR", default=None)
 a = ap.parse_args()
 
 X = bench.make_data(p=a.voxels)
@@ -34,14 +37,38 @@ def wrap(name, fn):
         log.append((name, t0, time.perf_counter(), e0, e1))
         return out
     return w
-for name in ("gram_of", "xv", "nspace", "perm_count", "uhat", "boot_moments", "boot_finalize", "colstd", "to_host",
-             "to_device"):
-    setattr(Engine, name, wrap(name, getattr(Engine, name)))
 
 def one():
     eng = Engine(Xd, device=dev, precision=a.precision)
     return bp.ResampleTest._create("mct", Xd, None, U, s.copy(), Vd, co, 0, preprocess=cf._mean_centre, nperm=a.n,
                                    nboot=a.n, Tvsc_orig=Tvsc, CI=0.95, perm_indices=ipd, boot_indices=ibd, engine=eng)
+
+
+if a.profile:
+    from torch.profiler import ProfilerActivity, profile
+    for _ in range(3):
+        one()
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CPU, ProfilerActivity.CUDA]) as prof:
+        one(); torch.cuda.synchronize()
+    _os.makedirs(a.profile, exist_ok=True)
+    prof.export_chrome_trace(_os.path.join(a.profile, "trace.json"))
+    with open(_os.path.join(a.profile, "kernels.txt"), "w") as f:
+        f.write(prof.key_averages().table(sort_by="cuda_time_total", row_limit=60, max_name_column_width=70) + "\n")
+        # device activity in start order, ms from the first one
+        ev = sorted((e for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA),
+                    key=lambda e: e.time_range.start)
+        t0 = ev[0].time_range.start if ev else 0
+        for e in ev:
+            f.write(f"{(e.time_range.start - t0) / 1e3:9.3f} {(e.time_range.end - e.time_range.start) / 1e3:8.3f}  "
+                    f"{e.name[:110]}\n")
+    print(open(_os.path.join(a.profile, "kernels.txt")).read())
+    raise SystemExit(0)
+
+for name in ("gram_of", "gram_stacked", "xv", "nspace", "pack_coef", "perm_count", "uhat", "boot_moments",
+             "boot_count_gram", "boot_factor", "boot_factor_quad", "boot_finalize", "colstd", "to_host",
+             "to_host_async", "to_device"):
+    setattr(Engine, name, wrap(name, getattr(Engine, name)))
 for _ in range(3):
     one()
 torch.cuda.synchronize(); log.clear()
