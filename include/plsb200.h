@@ -328,6 +328,25 @@ int plsb200_rb_boot_dmma_vs_f64(const double* Xc, int N, int64_t p, const double
                                 int nbt, const int32_t* cell_start_host, int ncell, int unit_cells, const double* pivot,
                                 double* sum, double* sumsq, double* T, double* nrm2, double* VS, void* workspace,
                                 size_t workspace_bytes, void* stream);
+/* rb_salience: the export-only pass of rb_boot over the voxel window [v0, v1): VS[b][v - v0][k] (nbt x (v1 - v0) x K,
+ * resample-major, the reference's right_sv_sampled[b, v0:v1]) for the bootstraps [0, nbt) of Q / W, bit-identical to
+ * the VS of the `_vs` entry points; no moments, norms or latent products.  The first row segment Xc has the row stride
+ * ld1 (the second, if any, ld2 >= v1), so a window is read in place.
+ * The DMMA path packs the coefficients of all nbt bootstraps once (plsb200_rb_salience_dmma_pack_f64 into the
+ * workspace) and every window's launch reads them; its workspace query returns 0 for a design the DMMA kernels do not
+ * hold, as plsb200_rb_boot_dmma_f64_workspace does, and the caller uses plsb200_rb_salience_f64 (cell_start in device
+ * memory, no workspace).                                                                                          */
+size_t plsb200_rb_salience_dmma_f64_workspace(int N, int K, int nbt, const int32_t* cell_start_host, int ncell,
+                                             int unit_cells);
+int plsb200_rb_salience_dmma_pack_f64(const double* Q, const double* W, int N, int K, int nbt,
+                                      const int32_t* cell_start_host, int ncell, int unit_cells, void* workspace,
+                                      size_t workspace_bytes, void* stream);
+int plsb200_rb_salience_dmma_f64(const double* Xc, int N, int64_t ld1, const double* Xc2, int n1, int64_t ld2,
+                                 int64_t v0, int64_t v1, int K, int nbt, const int32_t* cell_start_host, int ncell,
+                                 int unit_cells, double* VS, const void* workspace, size_t workspace_bytes, void* stream);
+int plsb200_rb_salience_f64(const double* Xc, int N, int64_t ld1, const double* Xc2, int n1, int64_t ld2, int64_t v0,
+                            int64_t v1, const double* Q, const double* W, int K, int nbt, const int32_t* cell_start,
+                            int ncell, int unit_cells, double* VS, void* stream);
 /* multiblock glue (class_functions.py:454-516): the last `unit_cells` blocks of rb_boot are plain linear rows
  * (task part of the multiblock matrix, no standardisation).
  * scatter_coef: C[r] (N x K) = scatter(E, idx_r) written out explicitly.

@@ -131,6 +131,15 @@ SIGNATURES = {
                                             c_double_p, c_int, c_int, c_int,
                                             c_void_p, c_int, c_int, c_double_p, c_double_p, c_double_p, c_double_p,
                                             c_double_p, c_double_p, c_void_p, c_size_t, c_void_p]),
+    "plsb200_rb_salience_dmma_f64_workspace": (c_size_t, [c_int, c_int, c_int, c_void_p, c_int, c_int]),
+    "plsb200_rb_salience_dmma_pack_f64": (c_int, [c_double_p, c_double_p, c_int, c_int, c_int, c_void_p, c_int, c_int,
+                                                  c_void_p, c_size_t, c_void_p]),
+    "plsb200_rb_salience_dmma_f64": (c_int, [c_double_p, c_int, c_int64, c_double_p, c_int, c_int64, c_int64, c_int64,
+                                             c_int, c_int, c_void_p, c_int, c_int, c_double_p, c_void_p, c_size_t,
+                                             c_void_p]),
+    "plsb200_rb_salience_f64": (c_int, [c_double_p, c_int, c_int64, c_double_p, c_int, c_int64, c_int64, c_int64,
+                                        c_double_p, c_double_p, c_int, c_int, c_int32_p, c_int, c_int, c_double_p,
+                                        c_void_p]),
     "plsb200_rb_lvcorr_f64": (c_int, [c_double_p, c_double_p, c_double_p, c_int32_p, c_int, c_int, c_int, c_int,
                                       c_int32_p, c_int, c_double_p, c_void_p]),
     "plsb200_half_gram_f64_workspace": (c_size_t, [c_int64, c_int, c_int]),

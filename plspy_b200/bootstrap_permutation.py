@@ -382,6 +382,14 @@ def _boot_multiblock(eng, U, s, V, cond_order, mctype, niter, pls_alg, contrast,
         eng.rb_boot(st_["Xcb"], C2_, W_, cells_, unit_cells=1, X2=eng.X, want_t=False, vs_out=VS)
         return VS.cpu().numpy()
     debug.set_lazy("right_sv_sampled", _right)
+
+    def _right_chunks(max_bytes):   # the same cube in voxel chunks: pass 1 over all of X, then windows of pass 2
+        st_ = _multiblock_state(eng, cond_order, bscan)
+        it_all = _index_shard(eng, idx_t, niter, 0, niter); ib_all = _index_shard(eng, idx_b, niter, 0, niter)
+        C2_, W_, cells_, _ = _multiblock_boot_coef(eng, st_, Lop, Ucoef, Ybscan, bscan, cond_order, it_all, ib_all)
+        fill = eng.rb_salience(st_["Xcb"], C2_, W_, cells_, unit_cells=1, X2=eng.X)
+        yield from eng.stream_chunks(fill, niter, Ucoef.shape[1], max_bytes)
+    debug.right_sv_chunks = _right_chunks
     return conf_int, conf_int_T, std_errs_h, boot_ratios_h, LV_h, debug
 
 
@@ -784,6 +792,30 @@ class _ResampleTestPLS(ResampleTest):
                 "salience percentile intervals are available for the task methods (mct, cst) after a bootstrap test")
         return fn(self._default_conf(conf), max_bytes)
 
+    def right_sv_sampled_chunks(self, max_bytes=1 << 30):
+        """The per-bootstrap brain saliences `boot_debug_dict["right_sv_sampled"]` (B x p x K) at any size, in voxel
+        chunks: a generator of (v0, v1, chunk), chunk a float64 array B x (v1 - v0) x K equal, bit for bit, to
+        right_sv_sampled[:, v0:v1, :].  The chunks cover the voxels in increasing order, each holds at most `max_bytes`
+        (but at least one voxel), and they are computed on the GPU while the previous chunk is copied to the host.
+
+        A yielded array is valid until the next step of the generator (two pinned buffers are reused); copy what you
+        keep, e.g. the whole cube to disk:
+
+            out = np.lib.format.open_memmap("right_sv.npy", mode="w+", dtype=np.float64, shape=(B, p, K))
+            for v0, v1, chunk in rt.right_sv_sampled_chunks():
+                out[:, v0:v1] = chunk
+
+        Nothing runs on the GPU until the first step; closing the generator early waits for the work in flight and
+        frees its buffers.  In a multi-process run every rank streams every bootstrap on its own (no collective); with
+        shard="voxels" a rank yields only its own voxels (global v0, v1 of its `voxel_range`).  The lazy
+        `right_sv_sampled` entry stays bounded by RIGHT_SV_MAX_BYTES; this one is not."""
+        fn = getattr(getattr(self, "boot_debug_dict", None), "right_sv_chunks", None)
+        if self._engine is None or fn is None:
+            raise exceptions.MissingParameterError("right_sv_sampled_chunks needs a bootstrap test (num_boot > 0)")
+        if not max_bytes > 0:
+            raise ValueError(f"max_bytes must be positive, got {max_bytes}")
+        return fn(int(max_bytes))
+
     def _bc_conf(self, conf):
         if self._engine is None or not hasattr(self, "boot_debug_dict"):
             raise exceptions.MissingParameterError("bias-corrected intervals need a bootstrap test (num_boot > 0)")
@@ -999,6 +1031,11 @@ class _ResampleTestPLS(ResampleTest):
                 return VS.cpu().numpy()
             debug.set_lazy("right_sv_sampled", _right)
 
+            def _right_chunks(max_bytes):   # this engine's voxels in chunks (voxel-sharded: no gather)
+                fill = eng.salience_window(E, _index_shard(eng, indices, niter, 0, niter))
+                yield from eng.stream_chunks(fill, niter, E.shape[1], max_bytes, v_offset=eng.voxel_range[0])
+            debug.right_sv_chunks = _right_chunks
+
             def _to_host_gathered(*parts):       # p x K parts of this engine's voxels; voxel-sharded: one gather
                 if vox:
                     K = int(parts[0].shape[1])
@@ -1058,6 +1095,13 @@ class _ResampleTestPLS(ResampleTest):
             eng.rb_boot(Xc_, Q_, W_, cells, want_t=False, vs_out=VS)
             return VS.cpu().numpy()
         debug.set_lazy("right_sv_sampled", _right)
+
+        def _right_chunks(max_bytes):   # the same cube in voxel chunks, from the same coefficients
+            Xc_ = _behaviour_state(eng, cells)["Xc"]
+            Q_, W_, _ = eng.rb_coef(Y, _index_shard(eng, indices, niter, 0, niter), cells, Ucoef, scatter=True)
+            fill = eng.rb_salience(Xc_, Q_, W_, cells)
+            yield from eng.stream_chunks(fill, niter, Ucoef.shape[1], max_bytes)
+        debug.right_sv_chunks = _right_chunks
         return conf_int, std_errs_h, boot_ratios_h, LV_h, debug
 
     # ------------------------------------------------------------------------------------------

@@ -119,7 +119,9 @@ __global__ void __launch_bounds__(256) rb_coef_kernel(const double* __restrict__
 constexpr int RB_VT = 256;
 constexpr int RB_VCH = 32;
 
-template <int KC, bool EXPORT>     // EXPORT: also store VS into the cube (instantiations without it keep their registers)
+// ONLY (with EXPORT): phase 1 alone over the voxel window [vw0, p) of a matrix whose first segment has the row stride
+// ld1, storing VS[b][v - vw0][k]; no moments, norms or phase 2.  blockIdx.y takes the bootstraps [y bslice, (y+1) bslice).
+template <int KC, bool EXPORT, bool ONLY = false>     // EXPORT: also store VS into the cube (instantiations without it keep their registers)
 __global__ void __launch_bounds__(RB_VT) rb_boot_kernel(const double* __restrict__ Xc, int N, long long p,
                                                        const double* __restrict__ Xc2, int n1, long long ld2,
                                                        const double* __restrict__ Q, const double* __restrict__ W,
@@ -129,23 +131,27 @@ __global__ void __launch_bounds__(RB_VT) rb_boot_kernel(const double* __restrict
                                                        const double* __restrict__ pivot, int Kfull,
                                                        double* __restrict__ sum, double* __restrict__ sumsq,
                                                        double* __restrict__ Tpart, double* __restrict__ Npart,
-                                                       double* __restrict__ VS) {
+                                                       double* __restrict__ VS, long long vw0, long long ld1,
+                                                       int bslice) {
+    static_assert(EXPORT || !ONLY, "ONLY is an export mode");
     extern __shared__ __align__(16) double smb[];
     double* Qs = smb;                               // [N][KC]
     double* Ws = Qs + (size_t)N * KC;               // [N]
     double* VSs = Ws + N;                           // [KC][RB_VT]
     double* Xs = VSs + (size_t)KC * RB_VT;          // [N][RB_VCH + 1]
     const int tid = threadIdx.x;
-    const long long v0 = (long long)blockIdx.x * RB_VT;
+    const long long v0 = (ONLY ? vw0 : 0) + (long long)blockIdx.x * RB_VT;
     const long long v = v0 + tid;
     const bool ok = v < p;
     double s1[KC], s2[KC];
 #pragma unroll
     for (int k = 0; k < KC; ++k) {
-        s1[k] = (ok && k < kc) ? sum[v * Kfull + k0 + k] : 0.0;
-        s2[k] = (ok && k < kc) ? sumsq[v * Kfull + k0 + k] : 0.0;
+        s1[k] = (!ONLY && ok && k < kc) ? sum[v * Kfull + k0 + k] : 0.0;
+        s2[k] = (!ONLY && ok && k < kc) ? sumsq[v * Kfull + k0 + k] : 0.0;
     }
-    for (int bb = 0; bb < nbt; ++bb) {
+    const int bb_lo = ONLY ? (int)blockIdx.y * bslice : 0;
+    const int bb_hi = ONLY ? min(nbt, bb_lo + bslice) : nbt;
+    for (int bb = bb_lo; bb < bb_hi; ++bb) {
         const int b = b0 + bb;
         __syncthreads();
         for (int i = tid; i < N * KC; i += RB_VT) {
@@ -165,7 +171,7 @@ __global__ void __launch_bounds__(RB_VT) rb_boot_kernel(const double* __restrict
             for (int k = 0; k < KC; ++k) P[k] = 0.0;
             for (int i = s; i < e; ++i) {
                 // rows [0, n1) of the data matrix live in Xc, rows [n1, N) in Xc2 (n1 == N: a single matrix)
-                const double x = ok ? __ldg((i < n1 ? Xc + (long long)i * p : Xc2 + (long long)(i - n1) * ld2) + v) : 0.0;
+                const double x = ok ? __ldg((i < n1 ? Xc + (long long)i * (ONLY ? ld1 : p) : Xc2 + (long long)(i - n1) * ld2) + v) : 0.0;
                 const double wx = Ws[i] * x;
                 m1 += wx;
                 m2 = fma(wx, x, m2);
@@ -182,6 +188,12 @@ __global__ void __launch_bounds__(RB_VT) rb_boot_kernel(const double* __restrict
                                   : ((var > 1e-13 * m2 && var > 0.0) ? 1.0 / sqrt(var * (double)(e - s)) : 0.0);
 #pragma unroll
             for (int k = 0; k < KC; ++k) vs[k] = fma(sc, P[k], vs[k]);
+        }
+        if constexpr (ONLY) {
+#pragma unroll
+            for (int k = 0; k < KC; ++k)
+                if (ok && k < kc) VS[((size_t)bb * (p - vw0) + (v - vw0)) * Kfull + k0 + k] = vs[k];
+            continue;
         }
 #pragma unroll
         for (int k = 0; k < KC; ++k) {
@@ -251,7 +263,7 @@ __global__ void __launch_bounds__(RB_VT) rb_boot_kernel(const double* __restrict
             }
         }
     }
-    if (ok) {
+    if (!ONLY && ok) {
 #pragma unroll
         for (int k = 0; k < KC; ++k)
             if (k < kc) { sum[v * Kfull + k0 + k] = s1[k]; sumsq[v * Kfull + k0 + k] = s2[k]; }
@@ -562,7 +574,7 @@ extern "C" int plsb200_rb_boot_vs_f64(const double* Xc, int N, int64_t p, const 
         auto kern = VSb ? rb_boot_kernel<KCV, true> : rb_boot_kernel<KCV, false>;                                   \
         PLSB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));              \
         kern<<<ntile, RB_VT, smem, st>>>(Xc, N, p, Xc2, n1, ld2, Q, W, K, k0, kc, b0, nbt, cell_start, ncell,       \
-                                         unit_cells, pivot, K, sum, sumsq, Tpart, Npart, VSb);                      \
+                                         unit_cells, pivot, K, sum, sumsq, Tpart, Npart, VSb, 0, 0, 0);             \
     } while (0)
         if (kc <= 8) PLSB_RB_LAUNCH(8);
         else if (kc <= 12) PLSB_RB_LAUNCH(12);
@@ -586,6 +598,44 @@ extern "C" int plsb200_rb_boot_f64(const double* Xc, int N, int64_t p, const dou
                                    void* stream) {
     return plsb200_rb_boot_vs_f64(Xc, N, p, Xc2, n1, ld2, Q, W, K, b0, nbt, cell_start, ncell, unit_cells, pivot, sum, sumsq,
                                   T, nrm2, nullptr, workspace, workspace_bytes, stream);
+}
+
+// The export-only pass of rb_boot over the voxel window [v0, v1) (right_sv_sampled in voxel chunks): VS[b][v - v0][k]
+// for the bootstraps [0, nbt) of Q / W, the same per-voxel arithmetic as plsb200_rb_boot_vs_f64.
+extern "C" int plsb200_rb_salience_f64(const double* Xc, int N, int64_t ld1, const double* Xc2, int n1, int64_t ld2,
+                                       int64_t v0, int64_t v1, const double* Q, const double* W, int K, int nbt,
+                                       const int32_t* cell_start, int ncell, int unit_cells, double* VS, void* stream) {
+    PLSB_CHECK_ARG(Xc && Q && W && cell_start && VS, "rb_salience_f64: null pointer");
+    PLSB_CHECK_ARG(N > 0 && K > 0 && nbt > 0 && ncell > 0 && v0 >= 0 && v1 > v0 && ld1 >= v1, "rb_salience_f64: bad shape");
+    if (Xc2 == nullptr) { n1 = N; ld2 = ld1; }
+    PLSB_CHECK_ARG(n1 > 0 && n1 <= N && ld2 >= v1, "rb_salience_f64: bad row split");
+    cudaStream_t st = (cudaStream_t)stream;
+    const int ntile = (int)cdiv(v1 - v0, RB_VT);
+    int nsl = (int)cdiv(4LL * num_sms(), ntile);          // bootstrap slices: fill the SMs when the window is narrow
+    if (nsl > nbt) nsl = nbt;
+    if (nsl > 65535) nsl = 65535;
+    const int bslice = (int)cdiv(nbt, nsl);
+    nsl = (int)cdiv(nbt, bslice);
+    const int nch = (int)cdiv(K, 16);                     // the column passes of plsb200_rb_boot_vs_f64
+    const int kc_max = (int)cdiv(K, nch);
+    for (int k0 = 0; k0 < K; k0 += kc_max) {
+        const int kc = K - k0 < kc_max ? K - k0 : kc_max;
+#define PLSB_RS_LAUNCH(KCV)                                                                                         \
+    do {                                                                                                            \
+        size_t smem = ((size_t)N * KCV + N) * sizeof(double);                                                       \
+        if (smem > 220 * 1024) { set_err("rb_salience_f64: N=%d too large for shared memory", N); return PLSB200_EUNSUPPORTED; } \
+        PLSB_CUDA(cudaFuncSetAttribute(rb_boot_kernel<KCV, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+        rb_boot_kernel<KCV, true, true><<<dim3(ntile, nsl), RB_VT, smem, st>>>(                                     \
+            Xc, N, v1, Xc2, n1, ld2, Q, W, K, k0, kc, 0, nbt, cell_start, ncell, unit_cells, nullptr, K, nullptr,   \
+            nullptr, nullptr, nullptr, VS, v0, ld1, bslice);                                                        \
+    } while (0)
+        if (kc <= 8) PLSB_RS_LAUNCH(8);
+        else if (kc <= 12) PLSB_RS_LAUNCH(12);
+        else PLSB_RS_LAUNCH(16);
+#undef PLSB_RS_LAUNCH
+        PLSB_LAUNCH_CHECK("rb_boot_kernel");
+    }
+    return PLSB200_OK;
 }
 
 extern "C" int plsb200_rb_lvcorr_f64(const double* T, const double* nrm2, const double* Yz, const int32_t* idx, int N,

@@ -138,11 +138,14 @@ struct RdArgs {
     double* VSt;       // [nbt][kcp][p]  (may be NULL when T is not wanted)
     double* VS;        // [nbt][p][Kfull] from the launch's first bootstrap: the saliences themselves (NULL: not exported)
     double* Npart;     // [nbt][kcp][tiles*8]
-    long long p;
+    long long p;       // ONLY: the end of the voxel window
     int Kfull, k0, kc, nbt, npass, pass, nstage, ncell, nwarps;
     int ks_unit;       // first k-step of the trailing unit cells (plain linear rows: no block moments needed); nks if none
     int nstd;          // standardised cells
     uint32_t cend[3];
+    long long v0;      // ONLY: first voxel of the window; VS is [nbt][p - v0][Kfull]
+    long long ld1;     // ONLY: row stride of Xc (the other instantiations: p)
+    int bslice;        // ONLY: bootstraps per blockIdx.y (a multiple of 8)
 };
 
 constexpr int RD_MAXCELL = 16;
@@ -175,8 +178,13 @@ __device__ __noinline__ void rd_store_scales(double* dst0, double* dst1, double 
 // EXPORT = also store VS_b into a.VS.  A template flag, not only a run-time test of a.VS: the 8-warp bucket holds up to
 // 96 k-steps of X fragments in 254 of its 255 registers, and the instantiations without the store keep exactly the
 // registers (and the code) of the kernel without the feature.
-template <int NKS, int NBLK, int W, bool MD, bool EXPORT>
+// ONLY (with EXPORT) = the export alone, over the voxel window [a.v0, a.p) of a matrix whose first segment has the row
+// stride a.ld1, into VS[b][v - v0][k]: no pivot moments, norms or transposed VS.  blockIdx.y takes the bootstraps
+// [y * bslice, (y + 1) * bslice); bslice is a multiple of 8, so the MD path forms the batches of the whole-p pass.  The
+// saliences of a voxel depend on its own column of X only, so a window's values are those of the whole-p pass.
+template <int NKS, int NBLK, int W, bool MD, bool EXPORT, bool ONLY = false>
 __global__ void __launch_bounds__(W * 32, 1) rb_vs_kernel(const RdArgs a) {
+    static_assert(EXPORT || !ONLY, "ONLY is an export mode");
     constexpr int RD_WARPS = W, RD_THREADS = W * 32;
     extern __shared__ __align__(128) unsigned char smraw[];
     constexpr int coef_doubles = NKS * NBLK * 32;                 // B fragments of one bootstrap and pass
@@ -200,8 +208,14 @@ __global__ void __launch_bounds__(W * 32, 1) rb_vs_kernel(const RdArgs a) {
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int q = lane & 3, vr = lane >> 2;
     const int nwarps = a.nwarps;                                  // warps launched (<= W, see rd_balanced_warps)
-    const long long v = (long long)blockIdx.x * (nwarps * 8) + warp * 8 + vr;
+    long long v = (long long)blockIdx.x * (nwarps * 8) + warp * 8 + vr;
+    if constexpr (ONLY) v += a.v0;
     const bool ok = v < a.p;
+    // ONLY: this CTA's bootstraps are [bofs, bofs + nbt_s) of the launch; everything below counts from bofs (the other
+    // instantiations read a.nbt as before: bofs and nbt_s are not used there)
+    const int bofs = ONLY ? (int)blockIdx.y * a.bslice : 0;
+    const int nbt_s = ONLY ? min(a.bslice, a.nbt - bofs) : 0;
+#define RD_NBT (ONLY ? nbt_s : a.nbt)
 
     if (tid == 0) {
         for (int s = 0; s < a.nstage; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, nwarps); }
@@ -214,7 +228,7 @@ __global__ void __launch_bounds__(W * 32, 1) rb_vs_kernel(const RdArgs a) {
     const size_t bstride = (size_t)a.npass * pack_doubles;        // doubles between consecutive bootstraps
     auto issue = [&](int bb, int slot) {                          // coefficients of bootstrap bb -> ring slot
         mbar_expect_tx(full + slot, coef_bytes);
-        const char* src = reinterpret_cast<const char*>(a.pack + (size_t)bb * bstride + (size_t)a.pass * pack_doubles);
+        const char* src = reinterpret_cast<const char*>(a.pack + (size_t)(ONLY ? bb + bofs : bb) * bstride + (size_t)a.pass * pack_doubles);
         char* dst = reinterpret_cast<char*>(ring + (size_t)slot * coef_doubles);
 #pragma unroll 1
         for (uint32_t off = 0; off < coef_bytes; off += 16384u)
@@ -224,11 +238,11 @@ __global__ void __launch_bounds__(W * 32, 1) rb_vs_kernel(const RdArgs a) {
         const int ws_ = bb % WSLOTS;
         mbar_expect_tx(wfull + ws_, w_bytes);
         bulk_g2s(wring + ws_ * w_doubles,
-                 a.pack + (size_t)bb * bstride + (size_t)a.pass * pack_doubles + coef_doubles, w_bytes, wfull + ws_);
+                 a.pack + (size_t)(ONLY ? bb + bofs : bb) * bstride + (size_t)a.pass * pack_doubles + coef_doubles, w_bytes, wfull + ws_);
     };
     auto issue_w8 = [&](int batch) {                              // MD: weight fragments of bootstraps 8 batch ... 8 batch + 7
         mbar_expect_tx(wfull, w8_bytes);
-        const char* src = reinterpret_cast<const char*>(a.wpack + (size_t)batch * w8_doubles);
+        const char* src = reinterpret_cast<const char*>(a.wpack + (size_t)(ONLY ? batch + bofs / 8 : batch) * w8_doubles);
         char* dst = reinterpret_cast<char*>(wring);
 #pragma unroll 1
         for (uint32_t off = 0; off < w8_bytes; off += 16384u)
@@ -237,15 +251,15 @@ __global__ void __launch_bounds__(W * 32, 1) rb_vs_kernel(const RdArgs a) {
     if (tid == 0) {
         if constexpr (MD) issue_w8(0);
         else
-            for (int bb = 0; bb < min(WSLOTS, a.nbt); ++bb) issue_w(bb);
-        for (int bb = 0; bb < min(a.nstage, a.nbt); ++bb) issue(bb, bb);
+            for (int bb = 0; bb < min(WSLOTS, RD_NBT); ++bb) issue_w(bb);
+        for (int bb = 0; bb < min(a.nstage, RD_NBT); ++bb) issue(bb, bb);
     }
 
     double x[NKS];
 #pragma unroll
     for (int s = 0; s < NKS; ++s) {
         const int row = __ldg(a.krow + 4 * s + q);
-        x[s] = (row >= 0 && ok) ? __ldg((row < a.n1 ? a.Xc + (long long)row * a.p
+        x[s] = (row >= 0 && ok) ? __ldg((row < a.n1 ? a.Xc + (long long)row * (ONLY ? a.ld1 : a.p)
                                                      : a.Xc2 + (long long)(row - a.n1) * a.ld2) + v) : 0.0;
     }
     // running moments live in shared memory (one slot per thread and fragment element): registers are for X
@@ -257,7 +271,7 @@ __global__ void __launch_bounds__(W * 32, 1) rb_vs_kernel(const RdArgs a) {
 #pragma unroll
         for (int e = 0; e < 2; ++e) {
             const int c = 8 * j + 2 * q + e;
-            const bool live = ok && c < a.kc;
+            const bool live = !ONLY && ok && c < a.kc;                // (ONLY: no moments)
             my1[(2 * j + e) * RD_THREADS] = live ? a.sum[v * a.Kfull + a.k0 + c] : 0.0;
             my2[(2 * j + e) * RD_THREADS] = live ? a.sumsq[v * a.Kfull + a.k0 + c] : 0.0;
             // (the pivot is the same for every bootstrap: read once -- as a per-bootstrap __ldg its L2 latency sat on
@@ -329,23 +343,23 @@ __global__ void __launch_bounds__(W * 32, 1) rb_vs_kernel(const RdArgs a) {
 
     int slot = 0, prev_slot = 0;
     uint32_t phase = 0, prev_phase = 0;
-    for (int bb = 0; bb < a.nbt; ++bb) {
+    for (int bb = 0; bb < RD_NBT; ++bb) {
         if (tid == 0 && bb > 0) {
             // every warp has finished iteration bb-1: its coefficient slot is free, and so are the weight slots of
             // bootstraps <= bb (the weights of bootstrap j are read during iteration j-1); weights 0..3 were issued
             // in the prologue, bootstrap bb+3 goes into the slot bootstrap bb-1 occupied
             mbar_wait(empty + prev_slot, prev_phase);
             const int nx = bb - 1 + a.nstage;
-            if (nx < a.nbt) issue(nx, prev_slot);
+            if (nx < RD_NBT) issue(nx, prev_slot);
             if constexpr (MD) {
                 // every warp has finished iteration 8g, so it has also read the weights of batch g (before that iteration)
-                if ((bb & 7) == 1 && 8 * (bb / 8 + 1) < a.nbt) issue_w8(bb / 8 + 1);
+                if ((bb & 7) == 1 && 8 * (bb / 8 + 1) < RD_NBT) issue_w8(bb / 8 + 1);
             } else {
-                if (bb + WSLOTS - 1 < a.nbt) issue_w(bb + WSLOTS - 1);
+                if (bb + WSLOTS - 1 < RD_NBT) issue_w(bb + WSLOTS - 1);
             }
         }
         __syncwarp();
-        const bool has_next = bb + 1 < a.nbt;
+        const bool has_next = bb + 1 < RD_NBT;
         if constexpr (MD) {
             if ((bb & 7) == 0 && bb > 0) batch_scales((uint32_t)((bb >> 3) & 1));
         } else {
@@ -419,6 +433,10 @@ __global__ void __launch_bounds__(W * 32, 1) rb_vs_kernel(const RdArgs a) {
             for (int e = 0; e < 2; ++e) {
                 const int c = 8 * j + 2 * q + e;
                 const double val = ok ? vs[j][e] : 0.0;
+                if constexpr (ONLY) {
+                    if (ok && c < a.kc) a.VS[((size_t)(bb + bofs) * (a.p - a.v0) + (v - a.v0)) * a.Kfull + a.k0 + c] = val;
+                    continue;
+                }
                 const double dd = val - myp[(2 * j + e) * RD_THREADS];
                 my1[(2 * j + e) * RD_THREADS] += dd;
                 my2[(2 * j + e) * RD_THREADS] = fma(dd, dd, my2[(2 * j + e) * RD_THREADS]);
@@ -437,7 +455,7 @@ __global__ void __launch_bounds__(W * 32, 1) rb_vs_kernel(const RdArgs a) {
         prev_slot = slot; prev_phase = phase;
         if (++slot == a.nstage) { slot = 0; phase ^= 1u; }
     }
-    if (ok) {
+    if (!ONLY && ok) {
 #pragma unroll
         for (int j = 0; j < NBLK; ++j)
 #pragma unroll
@@ -449,6 +467,7 @@ __global__ void __launch_bounds__(W * 32, 1) rb_vs_kernel(const RdArgs a) {
                 }
             }
     }
+#undef RD_NBT
 }
 
 // nrm2[b0 + bb][k0 + c] = sum over the (tile, warp) partials: one warp per output, lanes stride over the contiguous
@@ -609,37 +628,39 @@ static RdLayout rd_layout(const RdPlan& r, int N, int64_t p, int nbt, bool want_
     return L;
 }
 
-template <int NKS, int NBLK, int W, bool MD, bool EXPORT>
-static int launch_vs_kernel(const RdPlan& r, const RdArgs& a, int ntile, cudaStream_t st) {
-    PLSB_CUDA(cudaFuncSetAttribute(rb_vs_kernel<NKS, NBLK, W, MD, EXPORT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)r.smem_bytes));
-    rb_vs_kernel<NKS, NBLK, W, MD, EXPORT><<<ntile, a.nwarps * 32, r.smem_bytes, st>>>(a);
+template <int NKS, int NBLK, int W, bool MD, bool EXPORT, bool ONLY>
+static int launch_vs_kernel(const RdPlan& r, const RdArgs& a, dim3 grid, cudaStream_t st) {
+    PLSB_CUDA(cudaFuncSetAttribute(rb_vs_kernel<NKS, NBLK, W, MD, EXPORT, ONLY>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)r.smem_bytes));
+    rb_vs_kernel<NKS, NBLK, W, MD, EXPORT, ONLY><<<grid, a.nwarps * 32, r.smem_bytes, st>>>(a);
     PLSB_LAUNCH_CHECK("rb_vs_kernel");
     return PLSB200_OK;
 }
+// only: the export-only instantiation (plsb200_rb_salience_dmma_f64), grid = (voxel tiles, bootstrap slices)
 template <int NKS, int NBLK, int W, bool MD>
-static int launch_vs_md(const RdPlan& r, const RdArgs& a, int ntile, cudaStream_t st) {
-    return a.VS ? launch_vs_kernel<NKS, NBLK, W, MD, true>(r, a, ntile, st) : launch_vs_kernel<NKS, NBLK, W, MD, false>(r, a, ntile, st);
+static int launch_vs_md(const RdPlan& r, const RdArgs& a, dim3 grid, bool only, cudaStream_t st) {
+    if (only) return launch_vs_kernel<NKS, NBLK, W, MD, true, true>(r, a, grid, st);
+    return a.VS ? launch_vs_kernel<NKS, NBLK, W, MD, true, false>(r, a, grid, st) : launch_vs_kernel<NKS, NBLK, W, MD, false, false>(r, a, grid, st);
 }
 template <int NKS, int NBLK, int W>
-static int launch_vs(const RdPlan& r, const RdArgs& a, int ntile, cudaStream_t st) {
+static int launch_vs(const RdPlan& r, const RdArgs& a, dim3 grid, bool only, cudaStream_t st) {
     if constexpr (W == 16) {
-        if (r.md) return launch_vs_md<NKS, NBLK, W, true>(r, a, ntile, st);
+        if (r.md) return launch_vs_md<NKS, NBLK, W, true>(r, a, grid, only, st);
     }
-    return launch_vs_md<NKS, NBLK, W, false>(r, a, ntile, st);
+    return launch_vs_md<NKS, NBLK, W, false>(r, a, grid, only, st);
 }
 
 template <int NBLK>
-static int dispatch_vs(const RdPlan& r, const RdArgs& a, int ntile, cudaStream_t st) {
+static int dispatch_vs(const RdPlan& r, const RdArgs& a, dim3 grid, bool only, cudaStream_t st) {
     if (r.warps == 16) {
         switch (r.nks) {
-#define PLSB_CASE(n) case n: return launch_vs<n, NBLK, 16>(r, a, ntile, st);
+#define PLSB_CASE(n) case n: return launch_vs<n, NBLK, 16>(r, a, grid, only, st);
             PLSB_CASE(4) PLSB_CASE(8) PLSB_CASE(12) PLSB_CASE(16) PLSB_CASE(20) PLSB_CASE(24) PLSB_CASE(28) PLSB_CASE(32)
 #undef PLSB_CASE
             default: break;
         }
     } else {
         switch (r.nks) {
-#define PLSB_CASE(n) case n: return launch_vs<n, NBLK, 8>(r, a, ntile, st);
+#define PLSB_CASE(n) case n: return launch_vs<n, NBLK, 8>(r, a, grid, only, st);
             PLSB_CASE(36) PLSB_CASE(40) PLSB_CASE(44) PLSB_CASE(48) PLSB_CASE(52) PLSB_CASE(56) PLSB_CASE(60) PLSB_CASE(64) PLSB_CASE(68) PLSB_CASE(72)
             PLSB_CASE(76) PLSB_CASE(80) PLSB_CASE(84) PLSB_CASE(88) PLSB_CASE(92) PLSB_CASE(96)
 #undef PLSB_CASE
@@ -706,11 +727,12 @@ extern "C" int plsb200_rb_boot_dmma_vs_f64(const double* Xc, int N, int64_t p, c
         a.kc = K - a.k0 < r.kcp ? K - a.k0 : r.kcp;
         a.nbt = nbt; a.npass = r.npass; a.pass = pass; a.nstage = r.nstage; a.ncell = r.ncell; a.nwarps = L.nwarps; a.ks_unit = r.ks_unit;
         a.cend[0] = r.cend[0]; a.cend[1] = r.cend[1]; a.cend[2] = r.cend[2];
+        a.v0 = 0; a.ld1 = p; a.bslice = nbt;
         int rc;
         switch (r.nblk) {
-            case 1: rc = dispatch_vs<1>(r, a, L.ntile, st); break;
-            case 2: rc = dispatch_vs<2>(r, a, L.ntile, st); break;
-            default: rc = dispatch_vs<3>(r, a, L.ntile, st); break;
+            case 1: rc = dispatch_vs<1>(r, a, L.ntile, false, st); break;
+            case 2: rc = dispatch_vs<2>(r, a, L.ntile, false, st); break;
+            default: rc = dispatch_vs<3>(r, a, L.ntile, false, st); break;
         }
         if (rc != PLSB200_OK) return rc;
         rd_norm_reduce_kernel<<<(unsigned)cdiv((int64_t)nbt * a.kc * 32, 256), 256, 0, st>>>(
@@ -745,4 +767,112 @@ extern "C" int plsb200_rb_boot_dmma_f64(const double* Xc, int N, int64_t p, cons
                                         void* workspace, size_t workspace_bytes, void* stream) {
     return plsb200_rb_boot_dmma_vs_f64(Xc, N, p, Xc2, n1, ld2, Q, W, K, b0, nbt, cell_start_host, ncell, unit_cells, pivot,
                                        sum, sumsq, T, nrm2, nullptr, workspace, workspace_bytes, stream);
+}
+
+// ---- export-only pass over a voxel window (right_sv_sampled in voxel chunks) -------------------------------------------
+// Workspace: block rows, block sizes and the packed coefficients of all nbt bootstraps (rd_pack_kernel, and the MD weight
+// fragments), filled once by plsb200_rb_salience_dmma_pack_f64 and read by every window.
+struct RsLayout {
+    size_t off_krow, off_celln, off_pack, off_wpack, total;
+};
+
+static RsLayout rs_layout(const RdPlan& r, int nbt) {
+    RsLayout L;
+    auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
+    size_t o = 0;
+    L.off_krow = o; o = al(o + (size_t)r.nks * 4 * sizeof(int));
+    L.off_celln = o; o = al(o + 16 * sizeof(double));
+    L.off_pack = o; o = al(o + (size_t)nbt * r.npass * r.stage_doubles * sizeof(double));
+    L.off_wpack = o; o = al(o + (size_t)cdiv(nbt, 8) * r.nks * 32 * sizeof(double));
+    L.total = o;
+    return L;
+}
+
+extern "C" size_t plsb200_rb_salience_dmma_f64_workspace(int N, int K, int nbt, const int32_t* cell_start_host, int ncell,
+                                                        int unit_cells) {
+    RdPlan r;
+    if (!cell_start_host || nbt < 1 || !rd_plan(N, K, cell_start_host, ncell, unit_cells, r)) return 0;
+    return rs_layout(r, nbt).total;
+}
+
+extern "C" int plsb200_rb_salience_dmma_pack_f64(const double* Q, const double* W, int N, int K, int nbt,
+                                                 const int32_t* cell_start_host, int ncell, int unit_cells, void* workspace,
+                                                 size_t workspace_bytes, void* stream) {
+    PLSB_CHECK_ARG(Q && W && cell_start_host && workspace, "rb_salience_dmma_pack_f64: null pointer");
+    PLSB_CHECK_ARG(N > 0 && K > 0 && nbt > 0 && ncell > 0, "rb_salience_dmma_pack_f64: bad shape");
+    RdPlan r;
+    if (!rd_plan(N, K, cell_start_host, ncell, unit_cells, r)) {
+        set_err("rb_salience_dmma_pack_f64: design not supported (N=%d, %d cells): use rb_salience_f64", N, ncell);
+        return PLSB200_EUNSUPPORTED;
+    }
+    const RsLayout L = rs_layout(r, nbt);
+    if (workspace_bytes < L.total) {
+        set_err("rb_salience_dmma_pack_f64: workspace %zu < %zu bytes", workspace_bytes, L.total);
+        return PLSB200_EWORKSPACE;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    char* ws = (char*)workspace;
+    int* d_krow = (int*)(ws + L.off_krow);
+    PLSB_CUDA(cudaMemcpyAsync(d_krow, r.krow, (size_t)r.nks * 4 * sizeof(int), cudaMemcpyHostToDevice, st));
+    PLSB_CUDA(cudaMemcpyAsync(ws + L.off_celln, r.celln, 16 * sizeof(double), cudaMemcpyHostToDevice, st));
+    rd_pack_kernel<<<dim3(nbt, r.npass), 256, 0, st>>>(Q, W, N, K, 0, d_krow, r.nks, r.nblk, r.npass, (double*)(ws + L.off_pack));
+    PLSB_LAUNCH_CHECK("rd_pack_kernel");
+    if (r.md) {
+        rd_wpack_kernel<<<(unsigned)cdiv(nbt, 8), 256, 0, st>>>(W, N, 0, nbt, d_krow, r.nks, (double*)(ws + L.off_wpack));
+        PLSB_LAUNCH_CHECK("rd_wpack_kernel");
+    }
+    return PLSB200_OK;
+}
+
+extern "C" int plsb200_rb_salience_dmma_f64(const double* Xc, int N, int64_t ld1, const double* Xc2, int n1, int64_t ld2,
+                                            int64_t v0, int64_t v1, int K, int nbt, const int32_t* cell_start_host,
+                                            int ncell, int unit_cells, double* VS, const void* workspace,
+                                            size_t workspace_bytes, void* stream) {
+    PLSB_CHECK_ARG(Xc && cell_start_host && VS && workspace, "rb_salience_dmma_f64: null pointer");
+    PLSB_CHECK_ARG(N > 0 && K > 0 && nbt > 0 && ncell > 0 && v0 >= 0 && v1 > v0 && ld1 >= v1,
+                   "rb_salience_dmma_f64: bad shape");
+    if (Xc2 == nullptr) { n1 = N; ld2 = ld1; }
+    PLSB_CHECK_ARG(n1 > 0 && n1 <= N && ld2 >= v1, "rb_salience_dmma_f64: bad row split");
+    RdPlan r;
+    if (!rd_plan(N, K, cell_start_host, ncell, unit_cells, r)) {
+        set_err("rb_salience_dmma_f64: design not supported (N=%d, %d cells): use rb_salience_f64", N, ncell);
+        return PLSB200_EUNSUPPORTED;
+    }
+    const RsLayout L = rs_layout(r, nbt);
+    if (workspace_bytes < L.total) {
+        set_err("rb_salience_dmma_f64: workspace %zu < %zu bytes", workspace_bytes, L.total);
+        return PLSB200_EWORKSPACE;
+    }
+    const char* ws = (const char*)workspace;
+    const int nwarps = rd_balanced_warps(r.warps, v1 - v0);
+    const int ntile = (int)cdiv(v1 - v0, nwarps * 8);
+    // bootstrap slices: a window of a few thousand voxels is a few dozen tiles, too few CTAs for the SMs on their own
+    // (one CTA per SM); aim for about four CTAs per SM, in slices of whole batches of 8 bootstraps
+    const int nbatch = (int)cdiv(nbt, 8);
+    int nsl = (int)cdiv(4LL * num_sms(), ntile);
+    if (nsl > nbatch) nsl = nbatch;
+    if (nsl > 65535) nsl = 65535;
+    const int bslice = (int)cdiv(nbatch, nsl) * 8;
+    nsl = (int)cdiv(nbt, bslice);
+    for (int pass = 0; pass < r.npass; ++pass) {
+        RdArgs a{};
+        a.Xc = Xc; a.Xc2 = Xc2; a.n1 = n1; a.ld2 = ld2; a.pack = (const double*)(ws + L.off_pack);
+        a.wpack = r.md ? (const double*)(ws + L.off_wpack) : nullptr; a.nstd = r.nstd; a.pivot = nullptr;
+        a.krow = (const int*)(ws + L.off_krow); a.celln = (const double*)(ws + L.off_celln); a.sum = a.sumsq = nullptr;
+        a.VSt = nullptr; a.VS = VS; a.Npart = nullptr; a.p = v1; a.Kfull = K; a.k0 = pass * r.kcp;
+        a.kc = K - a.k0 < r.kcp ? K - a.k0 : r.kcp;
+        a.nbt = nbt; a.npass = r.npass; a.pass = pass; a.nstage = r.nstage; a.ncell = r.ncell; a.nwarps = nwarps; a.ks_unit = r.ks_unit;
+        a.cend[0] = r.cend[0]; a.cend[1] = r.cend[1]; a.cend[2] = r.cend[2];
+        a.v0 = v0; a.ld1 = ld1; a.bslice = bslice;
+        const dim3 grid((unsigned)ntile, (unsigned)nsl);
+        cudaStream_t st = (cudaStream_t)stream;
+        int rc;
+        switch (r.nblk) {
+            case 1: rc = dispatch_vs<1>(r, a, grid, true, st); break;
+            case 2: rc = dispatch_vs<2>(r, a, grid, true, st); break;
+            default: rc = dispatch_vs<3>(r, a, grid, true, st); break;
+        }
+        if (rc != PLSB200_OK) return rc;
+    }
+    return PLSB200_OK;
 }

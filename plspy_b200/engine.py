@@ -1003,6 +1003,70 @@ class Engine:
             check(fn(self._p(M), n, p, ld, self._p(E), K, self._p(idx), R, self._p(out), self._stream()), what)
         return out
 
+    def salience_window(self, E, idx):
+        """The task-method saliences VS[r] = X^T scatter(E, idx_r) over a voxel window: returns `fill(v0, v1, out)`,
+        which writes voxels [v0, v1) of this engine's columns into `out` (R x (v1 - v0) x K, contiguous float64) with
+        `salience_f64` (or its float32 twin) read in place through the row stride of X.  E and the index matrix are
+        uploaded once, here; the values are those of `salience` bit for bit."""
+        E = self.to_device(E, F64); idx = self.to_device(idx, I32)
+        R, K = int(idx.shape[0]), int(E.shape[1])
+        X = self.X
+        fn, what = self._xfn("salience_f64", X)
+
+        def fill(v0, v1, out):
+            with torch.cuda.device(self.device):
+                check(fn(self._xp(v0), self.N, v1 - v0, self.ldx, self._p(E), K, self._p(idx), R, self._p(out),
+                         self._stream()), what)
+        return fill
+
+    def stream_chunks(self, fill, B, K, max_bytes, v_offset=0):
+        """Generator over the B x p x K cube that `fill(v0, v1, out)` computes window by window (out: B x (v1 - v0) x K,
+        contiguous float64 on the device), in voxel chunks of at most `max_bytes` (at least one voxel): yields
+        (v_offset + v0, v_offset + v1, chunk), chunk a float64 numpy array B x (v1 - v0) x K that stays valid until the
+        next step.  Two device buffers and two pinned host buffers: chunk c is copied on the side stream (the one of
+        `to_host_async(side=True)`) while chunk c+1 is computed, and is yielded once its copy has finished; chunk c+1
+        is then copied while the caller reads chunk c.  Closing the generator early waits for the work in flight and
+        frees the buffers."""
+        p = self.p
+        vc = max(1, min(p, int(max_bytes) // (B * K * 8)))
+        spans = [(v0, min(p, v0 + vc)) for v0 in range(0, p, vc)]
+        if not spans:
+            return
+        cur = torch.cuda.current_stream(self.device)
+        if getattr(self, "_copy_stream", None) is None:
+            self._copy_stream = torch.cuda.Stream(device=self.device)
+        side = self._copy_stream
+        n = B * vc * K
+        dev = [self._empty(n) for _ in range(min(2, len(spans)))]
+        host = [torch.empty(n, dtype=F64, pin_memory=True) for _ in dev]
+        computed = [torch.cuda.Event() for _ in dev]
+        copied = [torch.cuda.Event() for _ in dev]
+
+        def launch(c):          # compute chunk c on the current stream, then copy it on the side stream
+            v0, v1 = spans[c]
+            i, m = c % 2, B * (v1 - v0) * K
+            with torch.cuda.stream(cur):
+                fill(v0, v1, dev[i][:m].view(B, v1 - v0, K))
+                computed[i].record(cur)
+            side.wait_event(computed[i])
+            with torch.cuda.stream(side):
+                host[i][:m].copy_(dev[i][:m], non_blocking=True)
+                copied[i].record(side)
+        try:
+            launch(0)
+            for c, (v0, v1) in enumerate(spans):
+                if c + 1 < len(spans):
+                    # chunk c+1 is computed while chunk c is copied, and copied while the caller reads chunk c: its
+                    # buffers held chunk c-1, whose copy finished before chunk c-1 was yielded and which the caller
+                    # has let go of by asking for the next step
+                    launch(c + 1)
+                copied[c % 2].synchronize()
+                yield v_offset + v0, v_offset + v1, host[c % 2][:B * (v1 - v0) * K].numpy().reshape(B, v1 - v0, K)
+        finally:
+            side.synchronize()
+            cur.synchronize()
+            del dev, host
+
     # ------------------------------------------------------------------ split-half (K3)
     def sym_eig(self, A):
         """Batched symmetric eigendecomposition (B x K x K, K <= 112): evals descending, evecs in columns.
@@ -1160,6 +1224,46 @@ class Engine:
                                                  ws.numel(), self._stream()), "rb_boot_f64")
             self._mark("rb_boot")
         return s1, s2, (T if want_t else None), nrm2
+
+    def rb_salience(self, Xc, Q, W, cell_start, unit_cells=0, X2=None):
+        """The export-only p-space pass of `rb_boot` over a voxel window: returns `fill(v0, v1, out)`, which writes the
+        saliences VS_b of voxels [v0, v1) of every bootstrap in Q into `out` (R x (v1 - v0) x K, contiguous float64),
+        bit-identical to the `vs_out` of `rb_boot`.  Runs on the DMMA kernel when the design fits it (its coefficients
+        are packed once, here, for every window) and on the FMA kernel otherwise or with `force_rb_fma`, like
+        `rb_boot`.  `X2`: the data matrix is the row stack [Xc; X2]."""
+        self._need_f64(Xc, "rb_salience"); self._need_f64(X2, "rb_salience"); self._need_whole_x("rb_salience")
+        cs_host = np.ascontiguousarray(np.asarray(cell_start, dtype=np.int32))
+        R, N, K = int(Q.shape[0]), int(Q.shape[1]), int(Q.shape[2])
+        n1, ld1 = int(Xc.shape[0]), int(Xc.stride(0))
+        ld2 = int(X2.stride(0)) if X2 is not None else ld1
+        if n1 + (int(X2.shape[0]) if X2 is not None else 0) != N:
+            raise ValueError("rb_salience: coefficient rows do not match the data matrix")
+        ncell = int(cs_host.size) - 1
+        nbytes = lib.plsb200_rb_salience_dmma_f64_workspace(N, K, R, cs_host.ctypes.data, ncell, int(unit_cells))
+        if nbytes and not getattr(self, "force_rb_fma", False):
+            self.last_rb_path = "dmma"
+            with torch.cuda.device(self.device):
+                ws = self._ws(nbytes)
+                check(lib.plsb200_rb_salience_dmma_pack_f64(self._p(Q), self._p(W), N, K, R, cs_host.ctypes.data, ncell,
+                                                            int(unit_cells), self._p(ws), ws.numel(), self._stream()),
+                      "rb_salience_dmma_pack_f64")
+
+            def fill(v0, v1, out):
+                with torch.cuda.device(self.device):
+                    check(lib.plsb200_rb_salience_dmma_f64(self._p(Xc), N, ld1, self._p(X2), n1, ld2, v0, v1, K, R,
+                                                           cs_host.ctypes.data, ncell, int(unit_cells), self._p(out),
+                                                           self._p(ws), ws.numel(), self._stream()),
+                          "rb_salience_dmma_f64")
+            return fill
+        self.last_rb_path = "fma"
+        cs = self.to_device(cs_host, I32)
+
+        def fill(v0, v1, out):
+            with torch.cuda.device(self.device):
+                check(lib.plsb200_rb_salience_f64(self._p(Xc), N, ld1, self._p(X2), n1, ld2, v0, v1, self._p(Q),
+                                                  self._p(W), K, R, self._p(cs), ncell, int(unit_cells), self._p(out),
+                                                  self._stream()), "rb_salience_f64")
+        return fill
 
     def rb_lvcorr(self, T, nrm2, Yz, idx, cell_start, nb):
         cs = self.to_device(np.asarray(cell_start, dtype=np.int32), I32)
