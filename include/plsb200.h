@@ -244,6 +244,22 @@ int plsb200_percentile_f64(const double* samples, int B, int64_t nseries, int64_
 int plsb200_percentile_bc_f64(const double* samples, int B, int64_t nseries, int64_t stride_sample,
                               int64_t stride_series, const double* orig, double q_lo, double q_hi, double* lower,
                               double* upper, double* prop, void* workspace, size_t workspace_bytes, void* stream);
+/* the bias-corrected and accelerated interval (BCa, Efron 1987) of the same series: prop and z0 as in the BC interval,
+ * accel[s] the acceleration a of series s, w = z0 + Phi^-1(q), and the bounds taken at the levels
+ * Phi(z0 + w / (1 - a w)).  q = 0 / 1 give the minimum / maximum; the bound is NaN where 1 - a w <= 0 (or a is NaN),
+ * where prop is 0 or 1, and for a NaN theta (whose prop is NaN).  a = 0 gives the BC bounds.
+ * Workspace: plsb200_percentile_f64_workspace(B).                                                                   */
+int plsb200_percentile_bca_f64(const double* samples, int B, int64_t nseries, int64_t stride_sample,
+                               int64_t stride_series, const double* orig, const double* accel, double q_lo,
+                               double q_hi, double* lower, double* upper, double* prop, void* workspace,
+                               size_t workspace_bytes, void* stream);
+/* the stratified jackknife acceleration of nseries series S[s][j] (J contiguous samples each, s-major), the samples
+ * in G groups [goff[g], goff[g+1]) (goff: G + 1 int32 in device memory, goff[0] = 0, goff[G] = J, every group
+ * non-empty).  With d_j = S[s][j] - theta[s], m_g the mean of d over group g (n_g samples) and
+ * l_j = (n_g - 1)(m_g - d_j):  accel[s] = (1/6) sum_g n_g^-3 sum l^3 / (sum_g n_g^-2 sum l^2)^(3/2), 0 where the
+ * denominator is 0 (NaN where it is NaN).  theta is only a pivot: a does not depend on it.                       */
+int plsb200_jack_accel_f64(const double* S, int64_t nseries, int J, const int32_t* goff, int G, const double* theta,
+                           double* accel, void* stream);
 
 /* ---- explicit saliences for a small batch: VS[r] = X^T . C_r  (R x p x K), for callers that ask for
  * boot_debug_dict["right_sv_sampled"] on problems small enough to hold it.                          */
@@ -257,6 +273,13 @@ int plsb200_salience_series_f64(const double* X, int N, int64_t p, int64_t ldx, 
                                 const int32_t* idx, int R, double* VS, void* stream);
 int plsb200_salience_series_x32_f64(const float* X, int N, int64_t p, int64_t ldx, const double* E, int K,
                                     const int32_t* idx, int R, double* VS, void* stream);
+/* saliences over explicit per-sample coefficients, series-major: VS[v][k][j] = sum_i X[i, v] . C[j][i][k] (C: J x N x K,
+ * VS: p x K x J), the leave-one-subject-out jackknife of the saliences (C zero on the removed rows).  X is read in
+ * place through ldx, so a voxel window is X + v0; p <= 65535 * 128 per call, N K <= 25600.                      */
+int plsb200_salience_coef_series_f64(const double* X, int N, int64_t p, int64_t ldx, const double* C, int K, int J,
+                                     double* VS, void* stream);
+int plsb200_salience_coef_series_x32_f64(const float* X, int N, int64_t p, int64_t ldx, const double* C, int K, int J,
+                                         double* VS, void* stream);
 
 /* ---- K5: behaviour PLS (rb / csb) -----------------------------------------------------------------
  * Cells = (group, condition) blocks of consecutive rows, given as ncell+1 int32 offsets `cell_start`.

@@ -160,6 +160,11 @@ SIGNATURES = {
                                        c_double_p, c_void_p, c_size_t, c_void_p]),
     "plsb200_percentile_bc_f64": (c_int, [c_double_p, c_int, c_int64, c_int64, c_int64, c_double_p, c_double, c_double,
                                           c_double_p, c_double_p, c_double_p, c_void_p, c_size_t, c_void_p]),
+    "plsb200_percentile_bca_f64": (c_int, [c_double_p, c_int, c_int64, c_int64, c_int64, c_double_p, c_double_p,
+                                           c_double, c_double, c_double_p, c_double_p, c_double_p, c_void_p, c_size_t,
+                                           c_void_p]),
+    "plsb200_jack_accel_f64": (c_int, [c_double_p, c_int64, c_int, c_int32_p, c_int, c_double_p, c_double_p,
+                                       c_void_p]),
     "plsb200_salience_f64": (c_int, [c_double_p, c_int, c_int64, c_int64, c_double_p, c_int, c_int32_p, c_int,
                                      c_double_p, c_void_p]),
     "plsb200_salience_series_f64": (c_int, [c_double_p, c_int, c_int64, c_int64, c_double_p, c_int, c_int32_p, c_int,
@@ -168,6 +173,10 @@ SIGNATURES = {
                                          c_double_p, c_void_p]),
     "plsb200_salience_series_x32_f64": (c_int, [c_void_p, c_int, c_int64, c_int64, c_double_p, c_int, c_int32_p,
                                                 c_int, c_double_p, c_void_p]),
+    "plsb200_salience_coef_series_f64": (c_int, [c_double_p, c_int, c_int64, c_int64, c_double_p, c_int, c_int,
+                                                 c_double_p, c_void_p]),
+    "plsb200_salience_coef_series_x32_f64": (c_int, [c_void_p, c_int, c_int64, c_int64, c_double_p, c_int, c_int,
+                                                     c_double_p, c_void_p]),
 }
 
 for _name, (_res, _args) in SIGNATURES.items():

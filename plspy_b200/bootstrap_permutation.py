@@ -426,17 +426,65 @@ def _task_operators(pls_alg, cond_order, mctype, U, contrast):
     return Lop, Ucoef, Lop.T @ Ucoef
 
 
+def _jackknife_coefficients(pls_alg, cond_order, mctype, Ucoef):
+    """The leave-one-subject-out jackknife of the task-method saliences, in row space (DESIGN.md section 5.8).  The
+    jackknife unit is the subject that resample.bootstrap_indices draws: group g, subject s, in every condition.
+    Without it the design has n_g - 1 subjects in group g, and its saliences are X_(-gs)^T Lop'^T Ucoef with Lop' the
+    method's operator for that design (centring for mct, cell means for cst) and Ucoef the original design weights
+    (U, or the normalised contrasts): no re-SVD, as for the bootstrap samples.  In row space that is X^T C_gs, C_gs
+    (N x K) zero on the C removed rows.  Lop' depends on the group only, so one product per group is scattered.
+
+    Returns (C, goff): C (J x N x K), J the number of subjects, group-major in the order of the rows; goff (G + 1,
+    int32) the offsets of the groups in C.  Raises exceptions.NotImplementedError (host only, before any GPU work)
+    unless every group has the same number of subjects in each condition and at least two subjects."""
+    missing = _balance_missing(cond_order)
+    co = np.asarray(cond_order) if missing is None else None
+    if missing is None and (co[:, 0] < 2).any():
+        g = int(np.flatnonzero(co[:, 0] < 2)[0])
+        missing = f"group {g} has {int(co[g, 0])} subject(s)"
+    if missing is not None:
+        raise exceptions.NotImplementedError(
+            "BCa salience intervals need a leave-one-subject-out jackknife: a cond_order in which every group has the "
+            f"same number of subjects in each condition, and at least two subjects in every group ({missing})")
+    G, C = co.shape
+    n = co[:, 0].astype(np.int64)
+    N, K = int(co.sum()), int(Ucoef.shape[1])
+    goff = np.concatenate(([0], np.cumsum(n))).astype(np.int32)
+    gstart = np.concatenate(([0], np.cumsum(n * C)))
+    jack = np.zeros((int(n.sum()), N, K))
+    for g in range(G):
+        co_r = co.copy()
+        co_r[g] -= 1
+        Lop = (class_functions._centring_operator(co_r, mctype) if pls_alg == "mct"
+               else class_functions._cell_mean_operator(co_r))
+        E_r = Lop.T @ Ucoef                                   # (N - C) x K, the rows of the reduced design
+        for sub in range(n[g]):
+            keep = np.ones(N, dtype=bool)
+            keep[gstart[g] + np.arange(C) * n[g] + sub] = False   # subject `sub` of group g in every condition
+            jack[goff[g] + sub, keep] = E_r
+    return jack, goff
+
+
 BOOT_ALGOS = ("auto", "direct", "collapsed")
 
 
-def _factor_layout_missing(cond_order, nboot):
-    """What the design lacks for the factored collapsed bootstrap (None: nothing): a `cond_order` with every group the
-    same size in each condition, and more bootstraps than the ns - G columns of the factor (else M is singular)."""
+def _balance_missing(cond_order):
+    """None when `cond_order` gives every group the same number of subjects in each condition, else what is missing."""
     if cond_order is None:
         return "no cond_order"
     co = np.asarray(cond_order)
     if co.ndim != 2 or co.size == 0 or (co != co[:, :1]).any():
         return "unequal subject counts across conditions"
+    return None
+
+
+def _factor_layout_missing(cond_order, nboot):
+    """What the design lacks for the factored collapsed bootstrap (None: nothing): a `cond_order` with every group the
+    same size in each condition, and more bootstraps than the ns - G columns of the factor (else M is singular)."""
+    missing = _balance_missing(cond_order)
+    if missing is not None:
+        return missing
+    co = np.asarray(cond_order)
     ns_g = int(co[:, 0].sum()) - co.shape[0]
     if nboot is None or not nboot > ns_g >= 1:
         return f"num_boot={nboot}, ns - G = {ns_g}"
@@ -861,6 +909,29 @@ class _ResampleTestPLS(ResampleTest):
                 "bias-corrected salience intervals are available for the task methods (mct, cst)")
         return fn(conf, max_bytes)
 
+    def salience_bca_intervals(self, conf=None, max_bytes=4 << 30):
+        """Bias-corrected and accelerated percentile interval (BCa, Efron 1987) of every brain salience over the
+        bootstrap samples, with prop and the acceleration.  theta, prop and z0 = Phi^-1(prop) are those of
+        `salience_bias_corrected_intervals`.  The acceleration a of every salience comes from its leave-one-subject-out
+        jackknife (the subject is the unit resample.bootstrap_indices draws; the saliences without subject (g, s) are
+        projected on the original design weights, with no re-SVD), stratified by group: with theta_(-gs) the jackknife
+        values and l_gs = (n_g - 1)(mean_s theta_(-gs) - theta_(-gs)),
+        a = (1/6) sum_g n_g^-3 sum_s l_gs^3 / (sum_g n_g^-2 sum_s l_gs^2)^(3/2), 0 where the denominator is 0.
+        With w = z0 + Phi^-1(q) the bounds are the samples at the levels Phi(z0 + w / (1 - a w)), interpolated like
+        `percentile_conf_ints`; they are NaN where 1 - a w <= 0, where prop is 0 or 1 and for a NaN theta, and q = 0 / 1
+        give the minimum / maximum.  With a = 0 they are the bias-corrected bounds (DESIGN.md section 5.8).
+
+        Streamed in voxel chunks like `salience_percentile_intervals`; `max_bytes` bounds the bootstrap and the
+        jackknife chunks together.  Task methods (mct, cst) on a design in which every group has the same number of
+        subjects in each condition and at least two subjects (else exceptions.NotImplementedError, before any GPU work).
+        Returns (lower, upper, prop, accel), p x K.  With shard="voxels" every rank works on its voxels and the results
+        are gathered: every rank must call it."""
+        conf = self._bc_conf(conf)
+        fn = getattr(self.boot_debug_dict, "salience_percentiles_bca", None)
+        if fn is None:
+            raise exceptions.NotImplementedError("BCa salience intervals are available for the task methods (mct, cst)")
+        return fn(conf, max_bytes)
+
     # ------------------------------------------------------------------------------------------
     @staticmethod
     def _permutation_test(X, Y, U, s, V, cond_order, mctype, niter, pls_alg, preprocess=None, contrast=None,
@@ -1053,6 +1124,13 @@ class _ResampleTestPLS(ResampleTest):
                     E, _index_shard(eng, indices, niter, 0, niter), _local_numerator(eng, V, s, contrast), conf,
                     max_bytes))
             debug.salience_percentiles_bc = _salience_percentiles_bc
+
+            def _salience_percentiles_bca(conf, max_bytes=4 << 30):
+                jack = _jackknife_coefficients(pls_alg, cond_order, mctype, Ucoef)      # raises before any GPU work
+                return _to_host_gathered(*eng.salience_percentiles_bca(
+                    E, _index_shard(eng, indices, niter, 0, niter), _local_numerator(eng, V, s, contrast), jack, conf,
+                    max_bytes))
+            debug.salience_percentiles_bca = _salience_percentiles_bca
             return conf_int, std_errs_h, boot_ratios_h, debug
         return finish if _defer else finish()
 

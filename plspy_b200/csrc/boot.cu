@@ -305,7 +305,9 @@ __global__ void boot_finalize_kernel(const double* __restrict__ sum, const doubl
 // SERIES: output [v][k][r] (the R samples of an element contiguous: the layout percentile_kernel sorts fastest) with the
 // resample as the FAST grid index, so that the CTAs running at one time share their rows of X in L2 and write
 // neighbouring 8-byte slots of the same sectors.
-template <typename T, int KT, bool SERIES>
+// COEF: explicit per-sample coefficients instead of a gather, VS[r][v][k] = sum_i X[i, v] . E[r][i][k] (E: R x N x K,
+// idx unused) -- the leave-one-subject-out jackknife of the saliences, whose coefficients are zero on the removed rows.
+template <typename T, int KT, bool SERIES, bool COEF = false>
 __global__ void __launch_bounds__(128) salience_kernel(const T* __restrict__ X, int N, long long p, long long ldx,
                                                       const double* __restrict__ E, int K,
                                                       const int32_t* __restrict__ idx, int R, double* __restrict__ VS) {
@@ -313,8 +315,10 @@ __global__ void __launch_bounds__(128) salience_kernel(const T* __restrict__ X, 
     double* Es = sms;
     int* ids = reinterpret_cast<int*>(Es + (size_t)N * K);
     const int r = SERIES ? blockIdx.x : blockIdx.y;
-    for (int i = threadIdx.x; i < N * K; i += blockDim.x) Es[i] = E[i];
-    for (int i = threadIdx.x; i < N; i += blockDim.x) ids[i] = idx[(size_t)r * N + i];
+    const double* Er = COEF ? E + (size_t)r * N * K : E;
+    for (int i = threadIdx.x; i < N * K; i += blockDim.x) Es[i] = Er[i];
+    if (!COEF)
+        for (int i = threadIdx.x; i < N; i += blockDim.x) ids[i] = idx[(size_t)r * N + i];
     __syncthreads();
     const long long v = (long long)(SERIES ? blockIdx.y : blockIdx.x) * blockDim.x + threadIdx.x;
     if (v >= p) return;
@@ -322,11 +326,21 @@ __global__ void __launch_bounds__(128) salience_kernel(const T* __restrict__ X, 
         double acc[KT];
 #pragma unroll
         for (int t = 0; t < KT; ++t) acc[t] = 0.0;
-        for (int i = 0; i < N; ++i) {
-            const double x = (double)__ldg(X + (long long)ids[i] * ldx + v);
+        if (COEF) {
+#pragma unroll 2
+            for (int i = 0; i < N; ++i) {              // unrolled twice: the compiler's default unroll spills here
+                const double x = (double)__ldg(X + (long long)i * ldx + v);
 #pragma unroll
-            for (int t = 0; t < KT; ++t)
-                if (k0 + t < K) acc[t] = fma(x, Es[i * K + k0 + t], acc[t]);
+                for (int t = 0; t < KT; ++t)
+                    if (k0 + t < K) acc[t] = fma(x, Es[i * K + k0 + t], acc[t]);
+            }
+        } else {
+            for (int i = 0; i < N; ++i) {
+                const double x = (double)__ldg(X + (long long)ids[i] * ldx + v);
+#pragma unroll
+                for (int t = 0; t < KT; ++t)
+                    if (k0 + t < K) acc[t] = fma(x, Es[i * K + k0 + t], acc[t]);
+            }
         }
 #pragma unroll
         for (int t = 0; t < KT; ++t)
@@ -398,6 +412,36 @@ __global__ void xv_reduce_kernel(const double* __restrict__ part, int nchunk, in
     double s = 0.0;
     for (int c = 0; c < nchunk; ++c) s += part[(size_t)c * n + i];
     out[i] = s;
+}
+
+// The stratified jackknife acceleration of every series: S[s][j] (J samples per series, groups [goff[g], goff[g+1])),
+// one thread per series, summed with a pivot at theta[s] (translation leaves a unchanged; the pivot keeps large
+// per-voxel baselines from cancelling).  With d_j = S_j - theta, m_g the mean of d over group g and
+// l_j = (n_g - 1)(m_g - d_j):  a = (1/6) sum_g n_g^-3 sum l^3 / (sum_g n_g^-2 sum l^2)^(3/2), 0 where the denominator
+// is 0.  The J samples of a series are read twice (mean, then moments); the second pass hits L1 / L2.
+__global__ void jack_accel_kernel(const double* __restrict__ S, long long nseries, int J, const int32_t* __restrict__ goff,
+                                  int G, const double* __restrict__ theta, double* __restrict__ accel) {
+    const long long s = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= nseries) return;
+    const double* row = S + s * J;
+    const double th = theta[s];
+    double num = 0.0, den = 0.0;
+    for (int g = 0; g < G; ++g) {
+        const int j0 = goff[g], j1 = goff[g + 1], n = j1 - j0;
+        double m = 0.0;
+        for (int j = j0; j < j1; ++j) m += row[j] - th;
+        m /= n;
+        double s2 = 0.0, s3 = 0.0;
+        for (int j = j0; j < j1; ++j) {
+            const double l = (n - 1) * (m - (row[j] - th));
+            s2 = fma(l, l, s2);
+            s3 = fma(l * l, l, s3);
+        }
+        const double inv = 1.0 / n;
+        num += s3 * inv * inv * inv;
+        den += s2 * inv * inv;
+    }
+    accel[s] = den > 0.0 ? num / (6.0 * den * sqrt(den)) : (isnan(den) ? den : 0.0);
 }
 
 }  // namespace plsb
@@ -566,6 +610,27 @@ static int salience_launch(const T* X, int N, int64_t p, int64_t ldx, const doub
     return PLSB200_OK;
 }
 
+// the jackknife pass: explicit coefficients C (J x N x K), series-major output VS[v][k][j] of the voxel window [0, p)
+template <typename T>
+static int salience_coef_series(const T* X, int N, int64_t p, int64_t ldx, const double* C, int K, int J, double* VS,
+                                void* stream, const char* what) {
+    PLSB_CHECK_ARG(X && C && VS, "%s: null pointer", what);
+    PLSB_CHECK_ARG(N > 0 && p > 0 && K > 0 && J >= 0 && ldx >= p, "%s: bad shape", what);
+    PLSB_CHECK_ARG(cdiv(p, 128) <= 65535, "%s: more than 65535 voxel blocks per call", what);
+    if (J == 0) return PLSB200_OK;
+    const size_t smem = (size_t)N * K * sizeof(double);
+    if (smem > 200 * 1024) {
+        set_err("%s: N*K too large", what);
+        return PLSB200_EUNSUPPORTED;
+    }
+    PLSB_CUDA(cudaFuncSetAttribute(salience_kernel<T, 12, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   (int)smem));
+    const dim3 grid((unsigned)J, (unsigned)cdiv(p, 128));
+    salience_kernel<T, 12, true, true><<<grid, 128, smem, (cudaStream_t)stream>>>(X, N, p, ldx, C, K, nullptr, J, VS);
+    PLSB_LAUNCH_CHECK("salience_kernel");
+    return PLSB200_OK;
+}
+
 extern "C" int plsb200_salience_f64(const double* X, int N, int64_t p, int64_t ldx, const double* E, int K,
                                     const int32_t* idx, int R, double* VS, void* stream) {
     return salience_launch(X, N, p, ldx, E, K, idx, R, VS, false, stream, "salience_f64");
@@ -584,6 +649,27 @@ extern "C" int plsb200_salience_x32_f64(const float* X, int N, int64_t p, int64_
 extern "C" int plsb200_salience_series_x32_f64(const float* X, int N, int64_t p, int64_t ldx, const double* E, int K,
                                                const int32_t* idx, int R, double* VS, void* stream) {
     return salience_launch(X, N, p, ldx, E, K, idx, R, VS, true, stream, "salience_series_x32_f64");
+}
+
+extern "C" int plsb200_salience_coef_series_f64(const double* X, int N, int64_t p, int64_t ldx, const double* C, int K,
+                                                int J, double* VS, void* stream) {
+    return salience_coef_series(X, N, p, ldx, C, K, J, VS, stream, "salience_coef_series_f64");
+}
+
+extern "C" int plsb200_salience_coef_series_x32_f64(const float* X, int N, int64_t p, int64_t ldx, const double* C,
+                                                    int K, int J, double* VS, void* stream) {
+    return salience_coef_series(X, N, p, ldx, C, K, J, VS, stream, "salience_coef_series_x32_f64");
+}
+
+extern "C" int plsb200_jack_accel_f64(const double* S, int64_t nseries, int J, const int32_t* goff, int G,
+                                      const double* theta, double* accel, void* stream) {
+    PLSB_CHECK_ARG(S && goff && theta && accel, "jack_accel_f64: null pointer");
+    PLSB_CHECK_ARG(nseries >= 1 && J >= 1 && G >= 1 && G <= J, "jack_accel_f64: bad shape nseries=%lld J=%d G=%d",
+                   (long long)nseries, J, G);
+    jack_accel_kernel<<<(unsigned)cdiv(nseries, 256), 256, 0, (cudaStream_t)stream>>>(S, nseries, J, goff, G, theta,
+                                                                                      accel);
+    PLSB_LAUNCH_CHECK("jack_accel_kernel");
+    return PLSB200_OK;
 }
 
 extern "C" size_t plsb200_xv_f64_workspace(int N, int64_t p, int K) {

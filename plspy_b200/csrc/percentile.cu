@@ -56,16 +56,25 @@ __device__ __forceinline__ void pc_pass(double* a_, int L, int a, int k, int war
     }
 }
 
+// The three intervals one kernel takes: the plain percentile interval, the bias-corrected one and the bias-corrected and
+// accelerated one.
+enum PcMode { PC_PLAIN, PC_BC, PC_BCA };
+
 // Bias-corrected bounds (BC): with prop = #{s <= theta} / B (theta = orig[s], the original value) and z0 = Phi^-1(prop),
 // the levels are Phi(2 z0 + Phi^-1(q)) instead of q.  prop is counted by binary search over the first B sorted slots
 // (the +inf padding never counts); prop 0 or 1 (z0 infinite) and a NaN theta give NaN bounds.
-template <bool GLOBAL, bool BC>
+// Bias-corrected and accelerated bounds (BCa, Efron 1987): with the acceleration a = accel[s] and w = z0 + Phi^-1(q),
+// the levels are Phi(z0 + w / (1 - a w)); the bound is NaN where 1 - a w <= 0 (or a is NaN).  q = 0 / 1 keep the
+// minimum / maximum, as in BC.  a = 0 gives the BC levels.
+template <bool GLOBAL, PcMode MODE>
 __global__ void __launch_bounds__(PC_THREADS) percentile_kernel(const double* __restrict__ S, int B, long long nseries,
                                                                long long stride_sample, long long stride_series,
                                                                double q_lo, double q_hi, int L,
                                                                double* __restrict__ lower, double* __restrict__ upper,
                                                                double* __restrict__ scratch,
-                                                               const double* __restrict__ orig, double* __restrict__ prop) {
+                                                               const double* __restrict__ orig, double* __restrict__ prop,
+                                                               const double* __restrict__ accel) {
+    constexpr bool BC = MODE != PC_PLAIN;
     extern __shared__ __align__(16) double pc_sm[];
     double* a = GLOBAL ? scratch + (size_t)blockIdx.x * pc_slots(L) : pc_sm;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -106,7 +115,15 @@ __global__ void __launch_bounds__(PC_THREADS) percentile_kernel(const double* __
                 const double pr = isnan(theta) ? CUDART_NAN : (double)lo / B;
                 if (tid == 0) prop[s] = pr;
                 defined = pr > 0.0 && pr < 1.0;             // false for NaN too
-                if (defined) q = normcdf(2.0 * normcdfinv(pr) + zq);
+                if (MODE == PC_BCA) {
+                    if (defined && q > 0.0 && q < 1.0) {
+                        const double z0 = normcdfinv(pr), ac = accel[s], w = z0 + zq, den = 1.0 - ac * w;
+                        defined = den > 0.0;                // false for a NaN acceleration too
+                        q = normcdf(ac == 0.0 ? 2.0 * z0 + zq : z0 + w / den);   // a = 0: the BC level, bit for bit
+                    }
+                } else if (defined) {
+                    q = normcdf(2.0 * normcdfinv(pr) + zq);
+                }
             }
             double t = q * B - 0.5;                         // fractional index into the sorted samples
             t = fmin(fmax(t, 0.0), (double)(B - 1));
@@ -135,12 +152,14 @@ extern "C" size_t plsb200_percentile_f64_workspace(int B) {
     return L > PC_MAX_SMEM_L ? (size_t)2 * num_sms() * pc_slots(L) * sizeof(double) : 16;
 }
 
-// one launcher for both entry points: the plain interval (BC = false, orig / prop unused) and the bias-corrected one
-template <bool BC>
+// one launcher for the three entry points: the plain interval (orig / prop / accel unused), the bias-corrected one
+// (accel unused) and the bias-corrected and accelerated one
+template <PcMode MODE>
 static int pc_launch(const char* what, const double* samples, int B, int64_t nseries, int64_t stride_sample,
-                     int64_t stride_series, const double* orig, double q_lo, double q_hi, double* lower, double* upper,
-                     double* prop, void* workspace, size_t workspace_bytes, void* stream) {
-    PLSB_CHECK_ARG(samples && lower && upper && (!BC || (orig && prop)), "%s: null pointer", what);
+                     int64_t stride_series, const double* orig, const double* accel, double q_lo, double q_hi,
+                     double* lower, double* upper, double* prop, void* workspace, size_t workspace_bytes, void* stream) {
+    PLSB_CHECK_ARG(samples && lower && upper && (MODE == PC_PLAIN || (orig && prop)) && (MODE != PC_BCA || accel),
+                   "%s: null pointer", what);
     PLSB_CHECK_ARG(B >= 1 && B <= (1 << 24) && nseries >= 1, "%s: bad shape B=%d nseries=%lld", what, B,
                    (long long)nseries);
     PLSB_CHECK_ARG(q_lo >= 0.0 && q_lo <= 1.0 && q_hi >= 0.0 && q_hi <= 1.0, "%s: quantiles must lie in [0, 1]", what);
@@ -148,12 +167,14 @@ static int pc_launch(const char* what, const double* samples, int B, int64_t nse
     cudaStream_t st = (cudaStream_t)stream;
     if (L <= PC_MAX_SMEM_L) {
         const size_t smem = pc_slots(L) * sizeof(double);
-        PLSB_CUDA(cudaFuncSetAttribute(percentile_kernel<false, BC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        PLSB_CUDA(cudaFuncSetAttribute(percentile_kernel<false, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)smem));
         const int per_sm = (int)((220 * 1024) / smem) < 8 ? (int)((220 * 1024) / smem) : 8;
         const long long cap = (long long)num_sms() * per_sm * 4;
         const unsigned grid = (unsigned)(nseries < cap ? nseries : cap);
-        percentile_kernel<false, BC><<<grid, PC_THREADS, smem, st>>>(samples, B, nseries, stride_sample, stride_series,
-                                                                    q_lo, q_hi, L, lower, upper, nullptr, orig, prop);
+        percentile_kernel<false, MODE><<<grid, PC_THREADS, smem, st>>>(samples, B, nseries, stride_sample,
+                                                                      stride_series, q_lo, q_hi, L, lower, upper,
+                                                                      nullptr, orig, prop, accel);
     } else {
         const size_t need = (size_t)2 * num_sms() * pc_slots(L) * sizeof(double);
         if (!workspace || workspace_bytes < need) {
@@ -162,8 +183,9 @@ static int pc_launch(const char* what, const double* samples, int B, int64_t nse
         }
         const long long cap = 2LL * num_sms();
         const unsigned grid = (unsigned)(nseries < cap ? nseries : cap);
-        percentile_kernel<true, BC><<<grid, PC_THREADS, 0, st>>>(samples, B, nseries, stride_sample, stride_series, q_lo,
-                                                                q_hi, L, lower, upper, (double*)workspace, orig, prop);
+        percentile_kernel<true, MODE><<<grid, PC_THREADS, 0, st>>>(samples, B, nseries, stride_sample, stride_series,
+                                                                  q_lo, q_hi, L, lower, upper, (double*)workspace, orig,
+                                                                  prop, accel);
     }
     PLSB_LAUNCH_CHECK("percentile_kernel");
     return PLSB200_OK;
@@ -172,14 +194,22 @@ static int pc_launch(const char* what, const double* samples, int B, int64_t nse
 extern "C" int plsb200_percentile_f64(const double* samples, int B, int64_t nseries, int64_t stride_sample,
                                       int64_t stride_series, double q_lo, double q_hi, double* lower, double* upper,
                                       void* workspace, size_t workspace_bytes, void* stream) {
-    return pc_launch<false>("percentile_f64", samples, B, nseries, stride_sample, stride_series, nullptr, q_lo, q_hi,
-                            lower, upper, nullptr, workspace, workspace_bytes, stream);
+    return pc_launch<PC_PLAIN>("percentile_f64", samples, B, nseries, stride_sample, stride_series, nullptr, nullptr,
+                               q_lo, q_hi, lower, upper, nullptr, workspace, workspace_bytes, stream);
 }
 
 extern "C" int plsb200_percentile_bc_f64(const double* samples, int B, int64_t nseries, int64_t stride_sample,
                                          int64_t stride_series, const double* orig, double q_lo, double q_hi,
                                          double* lower, double* upper, double* prop, void* workspace,
                                          size_t workspace_bytes, void* stream) {
-    return pc_launch<true>("percentile_bc_f64", samples, B, nseries, stride_sample, stride_series, orig, q_lo, q_hi,
-                           lower, upper, prop, workspace, workspace_bytes, stream);
+    return pc_launch<PC_BC>("percentile_bc_f64", samples, B, nseries, stride_sample, stride_series, orig, nullptr, q_lo,
+                            q_hi, lower, upper, prop, workspace, workspace_bytes, stream);
+}
+
+extern "C" int plsb200_percentile_bca_f64(const double* samples, int B, int64_t nseries, int64_t stride_sample,
+                                          int64_t stride_series, const double* orig, const double* accel, double q_lo,
+                                          double q_hi, double* lower, double* upper, double* prop, void* workspace,
+                                          size_t workspace_bytes, void* stream) {
+    return pc_launch<PC_BCA>("percentile_bca_f64", samples, B, nseries, stride_sample, stride_series, orig, accel, q_lo,
+                             q_hi, lower, upper, prop, workspace, workspace_bytes, stream);
 }

@@ -933,13 +933,37 @@ class Engine:
                                                 self._stream()), "percentile_bc_f64")
         return lo, hi, prop
 
-    def _salience_chunks(self, E, idx, max_bytes, reduce):
+    def percentile_interval_bca(self, A, orig, accel, conf=(0.05, 0.95)):
+        """Bias-corrected and accelerated percentile interval (BCa, Efron 1987) over the first axis of a (B x ...)
+        stack: `orig` and `accel`, shaped like A[0], hold the original value theta and the acceleration a of every
+        element.  prop and z0 = Phi^-1(prop) are those of `percentile_interval_bc`; with w = z0 + Phi^-1(q) the bounds
+        are taken at the levels Phi(z0 + w / (1 - a w)) (DESIGN.md section 5.8).  Returns (lower, upper, prop) device
+        tensors shaped like A[0]; lower / upper are NaN where prop is 0 or 1 and where 1 - a w <= 0, and q = 0 / 1
+        give the minimum / maximum.  With a = 0 the bounds are those of `percentile_interval_bc`."""
+        A = self.to_device(A, F64)
+        orig = self.to_device(orig, F64)
+        accel = self.to_device(accel, F64)
+        for name, t in (("orig", orig), ("accel", accel)):
+            if tuple(t.shape) != tuple(A.shape[1:]):
+                raise ValueError(f"{name} has shape {tuple(t.shape)}, the elements of the stack {tuple(A.shape[1:])}")
+        B = int(A.shape[0]); M = int(A.numel() // B)
+        lo, hi, prop = (self._empty(*A.shape[1:]) for _ in range(3))
+        with torch.cuda.device(self.device):
+            nb = lib.plsb200_percentile_f64_workspace(B)
+            ws = self._ws(nb)
+            check(lib.plsb200_percentile_bca_f64(self._p(A), B, M, M, 1, self._p(orig), self._p(accel), float(conf[0]),
+                                                 float(conf[1]), self._p(lo), self._p(hi), self._p(prop), self._p(ws),
+                                                 nb, self._stream()), "percentile_bca_f64")
+        return lo, hi, prop
+
+    def _salience_chunks(self, E, idx, max_bytes, reduce, extra_series=0):
         """Streams the bootstrap salience distribution VS[r] = X^T scatter(E, idx_r) without holding the R x p x K
         cube: voxel chunks of at most `max_bytes` are made explicit series-major and handed to
-        `reduce(cube, R, v0, v1, ws, nb)` (ws: nb bytes of percentile workspace), then dropped."""
+        `reduce(cube, R, v0, v1, ws, nb)` (ws: nb bytes of percentile workspace), then dropped.  `extra_series`
+        samples per element that `reduce` holds next to the chunk count against `max_bytes` too."""
         E = self.to_device(E, F64); idx = self.to_device(idx, I32)
         R, K = int(idx.shape[0]), int(E.shape[1])
-        vc = max(128, min(self.p, int(max_bytes // (R * K * 8)) // 128 * 128))
+        vc = max(128, min(self.p, int(max_bytes // ((R + extra_series) * K * 8)) // 128 * 128))
         X = self.X
         series, what = self._xfn("salience_series_f64", X)
         nb = lib.plsb200_percentile_f64_workspace(R)
@@ -988,6 +1012,39 @@ class Engine:
                                                 self._stream()), "percentile_bc_f64")
         self._salience_chunks(E, idx, max_bytes, reduce)
         return lo, hi, prop
+
+    def salience_percentiles_bca(self, E, idx, orig, jack, conf=(0.05, 0.95), max_bytes=4 << 30):
+        """Bias-corrected and accelerated percentile interval (`percentile_interval_bca`) of every element of the same
+        streamed distribution.  `orig` (p x K, this engine's voxels) is the original salience of every element;
+        `jack` = (C, goff): C (J x N x K) the coefficients of the J leave-one-subject-out saliences X^T C_j, and goff
+        (G + 1 offsets) the groups of the J subjects.  Per voxel chunk the bootstrap cube and the jackknife cube
+        (voxel x K x J, `salience_coef_series_f64`) are made explicit -- `max_bytes` bounds the two together -- the
+        stratified jackknife acceleration of every element is formed (`jack_accel_f64`, pivot at `orig`) and the
+        chunk is sorted.  Returns (lower, upper, prop, accel), p x K device tensors."""
+        K = int(E.shape[1])
+        orig = self.to_device(orig, F64)
+        if tuple(orig.shape) != (self.p, K):
+            raise ValueError(f"orig has shape {tuple(orig.shape)}, the saliences {(self.p, K)}")
+        Cj = self.to_device(jack[0], F64); goff = self.to_device(jack[1], I32)
+        J, G = int(Cj.shape[0]), int(goff.shape[0]) - 1
+        if tuple(Cj.shape) != (J, self.N, K):
+            raise ValueError(f"jackknife coefficients of shape {tuple(Cj.shape)}, need (J, {self.N}, {K})")
+        lo, hi, prop, accel = (self._empty(self.p, K) for _ in range(4))
+        jfn, jwhat = self._xfn("salience_coef_series_f64", self.X)
+
+        def reduce(cube, R, v0, v1, ws, nb):
+            off, n = 8 * v0 * K, (v1 - v0) * K
+            jc = self._empty(v1 - v0, K, J)
+            check(jfn(self._xp(v0), self.N, v1 - v0, self.ldx, self._p(Cj), K, J, self._p(jc), self._stream()), jwhat)
+            check(lib.plsb200_jack_accel_f64(self._p(jc), n, J, self._p(goff), G, orig.data_ptr() + off,
+                                             accel.data_ptr() + off, self._stream()), "jack_accel_f64")
+            del jc
+            check(lib.plsb200_percentile_bca_f64(self._p(cube), R, n, 1, R, orig.data_ptr() + off,
+                                                 accel.data_ptr() + off, float(conf[0]), float(conf[1]),
+                                                 lo.data_ptr() + off, hi.data_ptr() + off, prop.data_ptr() + off,
+                                                 self._p(ws), nb, self._stream()), "percentile_bca_f64")
+        self._salience_chunks(E, idx, max_bytes, reduce, extra_series=J)
+        return lo, hi, prop, accel
 
     def salience(self, E, idx, M=None):
         """Explicit VS[r] = M^T scatter(E, idx_r) (R x p x K), M = X by default -- small R only."""
