@@ -79,6 +79,9 @@ int plsb200_gram_x32_f64(const float* X, int N, int64_t p, int64_t ldx, double* 
  * plsb200_gram_f64_workspace(N1 + N2, p).                                                                      */
 int plsb200_gram_stacked_f64(const double* X1, int N1, int64_t ld1, const double* X2, int N2, int64_t ld2, int64_t p,
                              double* G, void* workspace, size_t workspace_bytes, void* stream);
+/* 1 when the stack of N rows and K more has the same row tiles as the N rows alone: then the N x N block of its Gram
+ * matrix is bit-identical to plsb200_gram_f64 of the N rows (same tiles, same voxel splits).                    */
+int plsb200_gram_stack_fuses(int N, int K);
 
 /* ---- latent projection XL = X . V (N x K); replaces class_functions._compute_X_latents
  * (class_functions.py:165-182) as used for U_hat (bootstrap_permutation.py:617).

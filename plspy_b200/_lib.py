@@ -43,6 +43,7 @@ SIGNATURES = {
     "plsb200_gram_x32_f64": (c_int, [c_void_p, c_int, c_int64, c_int64, c_double_p, c_void_p, c_size_t, c_void_p]),
     "plsb200_gram_stacked_f64": (c_int, [c_double_p, c_int, c_int64, c_double_p, c_int, c_int64, c_int64, c_double_p,
                                          c_void_p, c_size_t, c_void_p]),
+    "plsb200_gram_stack_fuses": (c_int, [c_int, c_int]),
     "plsb200_gram_tf32_image_bytes": (c_size_t, [c_int, c_int64]),
     "plsb200_gram_tf32_split": (c_int, [c_double_p, c_int, c_int64, c_int64, c_void_p, c_void_p]),
     "plsb200_gram_tf32_split_x32": (c_int, [c_void_p, c_int, c_int64, c_int64, c_void_p, c_void_p]),

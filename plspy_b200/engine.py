@@ -485,19 +485,17 @@ class Engine:
             self._G = G
         return self.G
 
-    GRAM_TILE_ROWS = 64     # row tile of the exact Gram kernel (gram.cu GT)
-
     def prepare_xv(self, V):
         """Announces the V (p x K) of a later `xv(V)`.  If G is not formed yet, X is float64, whole and resident, G is
-        exact, and the stack [X; V^T] has no more 64-row tiles than X, G is then formed as the Gram matrix of that stack
-        in one launch: its X block is bit-identical to `gram_of(X)` (same tiles, same voxel splits; a row of G only
+        exact, and the stack [X; V^T] has the same row tiles as X (plsb200_gram_stack_fuses), G is then formed as the
+        Gram matrix of that stack in one launch: its X block is bit-identical to `gram_of(X)` (same tiles, same voxel splits; a row of G only
         reads its own two rows of the stack) and its X-V^T block is X V, which `xv(V)` returns without a pass of its
         own over X.  Otherwise nothing changes.  Returns whether the product will come from the Gram launch."""
         V = self.to_device(V, F64)
-        K, t = int(V.shape[1]), self.GRAM_TILE_ROWS
+        K = int(V.shape[1])
         fused = (self._G is None and self._pending is None and not self.voxel_sharded and self._X.dtype == F64
                  and not (self.gram_tf32 and self.N <= self.GRAM_TF32_MAX_ROWS) and self.p > 0
-                 and V.dim() == 2 and int(V.shape[0]) == self.p and -(-(self.N + K) // t) == -(-self.N // t))
+                 and V.dim() == 2 and int(V.shape[0]) == self.p and lib.plsb200_gram_stack_fuses(self.N, K) == 1)
         self._xv_next = V if fused else None
         return fused
 
